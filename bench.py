@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- fwd+bwd warp+photometric loss throughput of the view-synthesis loss path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--config cfg2] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--config cfg2] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one pass of the hot path (pyramid / tables / smoothness prologue + fused loss forward+backward + epilogue,
@@ -243,7 +243,7 @@ def replay_timed_steps(runner, steps, first, per_step, one_step_per_graph):
         g0 = (first + G - 1) // G
         for j in range(steps // G):
             runner.group_graphs[(g0 + j) % len(runner.group_graphs)].replay()
-        runner.last = first + steps - 1
+        runner.last = G * g0 + steps - 1                     # the groups start at the first group boundary >= first
         return G
     for k in range(steps):
         runner.step(first + k)
@@ -341,6 +341,16 @@ class Workload(object):
             self.graphs[k % self.nsets].replay()
         else:
             self.launch(k, self.torch.cuda.current_stream().cuda_stream)
+
+    def outputs(self, k):
+        """What a caller of step k receives, copied to the host: the five losses and every gradient."""
+        t = self.sets[k % self.nsets]
+        out = dict(losses=t['losses'][:5], gposes=t['gposes'])
+        for s in range(4):
+            out['gdisp%d' % s] = t['gdisps'][s]
+            if self.exp:
+                out['glogits%d' % s] = t['glogits'][s]
+        return {name: v.cpu().numpy() for name, v in out.items()}
 
     def time_steps(self, steps, warmup, per_step=None, one_step_per_graph=False):
         torch = self.torch
@@ -737,6 +747,28 @@ def strong_scaling_block(args, device, world, rank, comm, peer, peak):
     return out
 
 
+DUMP_LIMIT_BYTES = 64 * 1000 * 1000
+NPY_HEADER_BYTES = 128
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes {name: array} as out_dir/<name>.npy in float32, at most DUMP_LIMIT_BYTES in all.  Smaller arrays are kept
+    whole; an array larger than its share of the remaining budget is cut to that many elements, taken at positions drawn
+    with a seed derived from its name and kept in flat order, so the same configuration always yields the same sample."""
+    import zlib
+    os.makedirs(out_dir, exist_ok=True)
+    budget = DUMP_LIMIT_BYTES - NPY_HEADER_BYTES * len(arrays)
+    items = sorted(arrays.items(), key=lambda kv: (kv[1].size, kv[0]))
+    for i, (name, a) in enumerate(items):
+        a = np.asarray(a, np.float32)
+        share = budget // (len(items) - i) // a.itemsize                  # elements
+        if a.size > share:
+            idx = np.random.RandomState(zlib.crc32(name.encode())).choice(a.size, share, replace=False)
+            a = a.reshape(-1)[np.sort(idx)]
+        budget -= a.nbytes
+        np.save(os.path.join(out_dir, name + '.npy'), a)
+
+
 def run_b200(args):
     import torch
     import torch.distributed as dist
@@ -801,6 +833,8 @@ def run_b200(args):
     ms, t0, t1 = runner.time(args.steps, args.warmup)
     torch.cuda.synchronize()
     trace('timed %.4f ms' % ms)
+    # the steps below reuse the buffer sets: take the last timed step's results now, write them at the end
+    dumped = wl.outputs(runner.last) if args.dump_outputs and rank == 0 else None
     steps_per_graph = runner.timed_steps_per_graph
     ms_single = ms
     if steps_per_graph > 1:                                   # the same K steps replayed one step per graph, for comparison
@@ -939,6 +973,8 @@ def run_b200(args):
             ss = strong_scaling_block(args, device, world, rank, comm, peer, peak)
             if rank == 0:
                 line['strong_scaling'] = ss
+    if dumped is not None:
+        dump_outputs(args.dump_outputs, dumped)
     if rank == 0:
         print(json.dumps(line))
     if world > 1:
@@ -963,7 +999,15 @@ def main():
     ap.add_argument('--no-other', action='store_true', help='skip the other_configs sweep (N = 1) / the strong_scaling block (N > 1)')
     ap.add_argument('--no-cpu', action='store_true', help='skip the cpu_baseline leg')
     ap.add_argument('--no-allreduce', action='store_true', help='(diagnostic) skip the loss-partial allreduce at N > 1')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write what the last timed step computed (rank 0: losses.npy, gposes.npy, gdisp<s>.npy, glogits<s>.npy '
+                         'with explainability) as float32 .npy files into DIR, at most 64 MB in all; the inputs are seeded, so '
+                         'runs with the same arguments compare output for output')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs is for the b200 arm')
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == 'reference':

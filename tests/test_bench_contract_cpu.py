@@ -5,6 +5,7 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -88,13 +89,46 @@ def test_timed_steps_are_exactly_K_with_grouped_graphs():
     r = Runner(28, 4)
     assert bench.replay_timed_steps(r, 20, 3, None, False) == 4
     assert len(r.log) == 20 and r.log == [(4 + k) % 28 for k in range(20)]      # starts at the first group boundary after the warm-up
+    assert r.last % 28 == r.log[-1]                                             # --dump-outputs reads the last step's buffer set
     r = Runner(28, 4)
     assert bench.replay_timed_steps(r, 2000, 50, None, False) == 4
     assert len(r.log) == 2000 and set(r.log) == set(range(28))
     assert all(b == (a + 1) % 28 for a, b in zip(r.log, r.log[1:]))              # consecutive steps never share a buffer set
+    assert r.last % 28 == r.log[-1]
     for args in ((21, 3, None, False), (20, 3, None, True), (20, 3, lambda k: None, False)):
         r = Runner(28, 4)
         assert bench.replay_timed_steps(r, *args) == 1
         assert r.log == [(3 + k) % 28 for k in range(args[0])]
     r = Runner(3, 1)
     assert bench.replay_timed_steps(r, 20, 3, None, False) == 1 and len(r.log) == 20
+
+
+def test_dump_outputs_keeps_small_arrays_whole_and_samples_within_the_limit(tmp_path, monkeypatch):
+    sys.path.insert(0, ROOT)
+    import bench
+    monkeypatch.setattr(bench, 'DUMP_LIMIT_BYTES', 64 * 1024)
+    rs = np.random.RandomState(0)
+    arrays = dict(losses=rs.standard_normal(5).astype(np.float32), gposes=rs.standard_normal((4, 2, 6)).astype(np.float32),
+                  gdisp0=rs.standard_normal((4, 1, 64, 208)).astype(np.float32),
+                  gdisp1=rs.standard_normal((4, 1, 32, 104)).astype(np.float32))
+    for d in ('a', 'b'):
+        bench.dump_outputs(str(tmp_path / d), arrays)
+    files = sorted(os.listdir(tmp_path / 'a'))
+    assert files == ['gdisp0.npy', 'gdisp1.npy', 'gposes.npy', 'losses.npy']
+    assert sum(os.path.getsize(tmp_path / 'a' / f) for f in files) <= 64 * 1024
+    for f in files:
+        a, b = np.load(tmp_path / 'a' / f), np.load(tmp_path / 'b' / f)
+        assert a.dtype == np.float32
+        np.testing.assert_array_equal(a, b)                                      # the same sample every time
+    for name in ('losses', 'gposes'):
+        np.testing.assert_array_equal(np.load(tmp_path / 'a' / (name + '.npy')), arrays[name])
+    big = np.load(tmp_path / 'a' / 'gdisp0.npy')
+    assert big.ndim == 1 and 0 < big.size < arrays['gdisp0'].size
+    assert np.isin(big, arrays['gdisp0']).all()
+
+
+def test_bench_rejects_a_step_count_below_one_and_dumps_of_the_reference_arm():
+    for extra in (['--steps', '0'], ['--impl', 'reference', '--dump-outputs', 'x']):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, 'bench.py')] + extra, stdout=subprocess.PIPE,
+                             stderr=subprocess.PIPE, text=True, timeout=120, cwd=ROOT)
+        assert out.returncode == 2 and out.stdout == '', out.stderr[-2000:]

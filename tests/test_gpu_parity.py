@@ -769,3 +769,33 @@ def test_fewer_scales_match_oracle(ns):
         assert_grad_close(host(grads['gdisps'][s]), G['gdisp'][s], what='gdisp[%d]' % s)
     tp, sp = op.pyramid(to_dev(d['tgt']), to_dev(d['src']))
     assert len(tp) == ns and len(sp) == ns
+
+
+@pytest.mark.parametrize('cfg', ['cfg2', 'cfg4'])
+def test_bench_dump_outputs_are_the_last_timed_step(cfg, tmp_path):
+    """bench.py --dump-outputs writes the losses and gradients of its last timed step: on the bench's seeded snippets (four,
+    tiled to the batch) they match the oracle."""
+    import subprocess
+    import sys
+    from sfm_learner_chainer_b200.synthetic import CONFIGS
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    env = {k: v for k, v in os.environ.items() if k not in ('WORLD_SIZE', 'RANK', 'LOCAL_RANK')}
+    out = subprocess.run([sys.executable, os.path.join(root, 'bench.py'), '--config', cfg, '--steps', '10', '--warmup', '3',
+                          '--no-other', '--no-cpu', '--dump-outputs', str(tmp_path)],
+                         stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, timeout=600, cwd=root, env=env)
+    assert out.returncode == 0, out.stderr[-2000:]
+    c = dict(CONFIGS[cfg])
+    B, S, H, W = c.pop('B'), c.pop('S'), c.pop('H'), c.pop('W')
+    d = make_snippets(4, S, H, W, seed=0)
+    tile = lambda a: np.concatenate([a] * (B // 4), 0)
+    L, G, _ = O.sfm_loss(tile(d['tgt']), tile(d['src']), tile(d['intrinsics']), [tile(x) for x in d['disps']],
+                         tile(d['poses']), [tile(x) for x in d['logits']], O.LossConfig(**c))
+    load = lambda name: np.load(os.path.join(str(tmp_path), name + '.npy'))
+    names = ['losses', 'gposes'] + ['gdisp%d' % s for s in range(4)] + (['glogits%d' % s for s in range(4)] if c['exp_reg'] else [])
+    assert sorted(os.listdir(str(tmp_path))) == sorted(n + '.npy' for n in names)
+    np.testing.assert_allclose(load('losses'), O.losses_vec(L), rtol=1e-5, atol=1e-9)
+    assert_grad_close(load('gposes'), G['gpose'], what='gpose')
+    for s in range(4):
+        assert_grad_close(load('gdisp%d' % s), G['gdisp'][s], what='gdisp[%d]' % s)
+        if c['exp_reg']:
+            assert_grad_close(load('glogits%d' % s), G['glogits'][s], what='glogits[%d]' % s)
