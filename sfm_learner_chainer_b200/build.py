@@ -8,7 +8,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
 CSRC = os.path.join(HERE, 'csrc')
 LIB = os.path.join(HERE, 'libsfmloss.so')
-SOURCES = ['api.cu', 'prep.cu', 'smooth.cu', 'fused_loss.cu', 'stage.cu', 'ingest.cu', 'eval.cu', 'comm.cu']
+SOURCES = ['api.cu', 'plan.cu', 'prep.cu', 'smooth.cu', 'fused_loss.cu', 'stage.cu', 'ingest.cu', 'eval.cu', 'comm.cu']
 HEADERS = ['common.cuh', 'kernels.h', 'ssim_march.cuh', 'smooth_task.cuh', os.path.join(ROOT, 'include', 'sfmloss.h')]
 
 
@@ -33,7 +33,6 @@ def build(force=False, verbose=False):
     cmd = [_nvcc(), '--threads', '0', '-gencode', 'arch=compute_100a,code=sm_100a', '-O3', '-lineinfo', '-std=c++17',
            '-Xcompiler', '-fPIC', '-shared', '-I', os.path.join(ROOT, 'include'), '-I', CSRC,
            '-o', LIB] + [os.path.join(CSRC, s) for s in SOURCES] + ['-ldl']
-    cmd[1:1] = os.environ.get('SFM_NVCC_FLAGS', '').split()      # development knob, e.g. -DSFM_MINB=16
     if verbose:
         cmd.insert(1, '-Xptxas=-v')
     res = subprocess.run(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)

@@ -1,7 +1,6 @@
 // api.cu -- extern "C" entry points of libsfmloss.so (see include/sfmloss.h for the contract and the
 // reference interfaces each one replaces).
 #include <stdarg.h>
-#include <stdlib.h>
 #include <string.h>
 
 #include <new>
@@ -31,15 +30,6 @@ extern "C" int sfm_set_kernel_events(void* start_event, void* stop_event) {
   return 0;
 }
 extern "C" int sfm_version(void) { return SFM_VERSION; }
-
-bool sfm_pdl_enabled() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("SFM_NO_PDL");
-    v = (e && e[0] == '1') ? 0 : 1;
-  }
-  return v != 0;
-}
 
 int sfm_validate_desc(const SfmDesc* d) {
   if (!d) { sfm_set_error("SfmDesc is NULL"); return SFM_E_NULL_POINTER; }
@@ -134,27 +124,44 @@ int check_grads(const SfmDesc* d, const SfmGrads* g) {
   return 0;
 }
 
-int run_prep(const SfmDesc* d, const SfmInputs* in, void* workspace, bool do_pyramid, const SfmSmoothParams* sm, int sm_mode,
-             cudaStream_t st) {
+// Parameters of the prologue kernel.  It builds the pyramid of (tgt, src) into the workspace when tgt is given, the
+// projection tables of (poses, intrinsics) when proj_out is given, and with `step` (a loss call) also resets the
+// workspace's fp64 cells and stores the reduced pose vectors there.
+SfmPrepParams prep_params(const SfmDesc* d, int band, char* ws, const float* tgt, const float* src, const float* intrinsics,
+                          const float* poses, float* proj_out, float* kinv_out, bool step) {
   SfmWsLayout L;
   sfm_ws_layout(d, &L);
-  char* ws = (char*)workspace;
   SfmPrepParams p{};
   p.B = d->B; p.S = d->S; p.H = d->H; p.W = d->W; p.ns = d->n_scales;
-  p.do_pyramid = do_pyramid ? 1 : 0;
-  p.build_tables = (d->flags & SFM_FLAG_TABLES_PROVIDED) ? 0 : 1;
-  p.tgt = in->tgt; p.src = in->src; p.intrinsics = in->intrinsics; p.poses = in->poses;
-  for (int s = 0; s < d->n_scales; ++s) {
-    p.tgt_pyr[s] = (float*)(ws + L.off_tgt[s]);
-    p.src_pyr[s] = (float*)(ws + L.off_src[s]);
-  }
-  p.proj_out = (float*)(ws + L.off_proj);
-  p.kinv_out = (float*)(ws + L.off_kinv);
-  p.acc = (double*)(ws + L.off_acc);
-  p.n_acc = (int)L.acc_doubles;
+  p.band = band;
+  p.do_pyramid = tgt ? 1 : 0;
+  p.build_tables = proj_out ? 1 : 0;
+  p.tgt = tgt; p.src = src; p.intrinsics = intrinsics; p.poses = poses;
+  if (tgt)
+    for (int s = 0; s < d->n_scales; ++s) {
+      p.tgt_pyr[s] = (float*)(ws + L.off_tgt[s]);
+      p.src_pyr[s] = (float*)(ws + L.off_src[s]);
+    }
+  p.proj_out = proj_out;
+  p.kinv_out = kinv_out;
   p.raw_pose_hw = d->raw_pose_hw;
-  p.posevec_out = (float*)(ws + L.off_posevec);
-  return sfm_launch_prep(p, sm, sm_mode, st);
+  if (step) {
+    p.acc = (double*)(ws + L.off_acc);
+    p.n_acc = (int)L.acc_doubles;
+    p.posevec_out = (float*)(ws + L.off_posevec);
+  }
+  return p;
+}
+
+// SM count of the device, queried once
+int num_sms() {
+  static int n = 0;
+  if (n == 0) {
+    int dev = 0;
+    cudaGetDevice(&dev);
+    if (cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || n <= 0) n = SFM_REF_SMS;
+  }
+  return n;
 }
 
 int run_loss(const SfmDesc* d, const SfmInputs* in, float* losses_out, const SfmGrads* grads, const float* gy,
@@ -173,10 +180,18 @@ int run_loss(const SfmDesc* d, const SfmInputs* in, float* losses_out, const Sfm
     return SFM_E_NO_DEVICE;
   }
   const Modes m = modes_of(d);
+  int mode = 0;
+  if (m.use_exp) mode |= SFM_MODE_EXP;
+  if (m.use_ssim) mode |= SFM_MODE_SSIM;
+  if (m.use_smooth) mode |= SFM_MODE_SMOOTH;
+  if (grads) mode |= SFM_MODE_GRAD;
+  if (dbg) mode |= SFM_MODE_DEBUG;
+  const SfmStepPlan plan = sfm_plan_step(d, mode, num_sms());
   SfmWsLayout L;
   sfm_ws_layout(d, &L);
   char* ws = (char*)workspace;
   SfmFusedParams p{};
+  SfmSmoothParams sm = plan.smooth;
   p.B = d->B; p.S = d->S; p.ns = d->n_scales;
   const double Bg = (double)(d->B_global > 0 ? d->B_global : d->B);
   for (int s = 0; s < d->n_scales; ++s) {
@@ -196,6 +211,11 @@ int run_loss(const SfmDesc* d, const SfmInputs* in, float* losses_out, const Sfm
     p.sm_dy2[s] = (float)(wgt / (Bg * (h - 2) * w));
     p.sm_ex[s] = (float)(wgt / (Bg * h * (w - 1)));
     p.sm_ey[s] = (float)(wgt / (Bg * (h - 1) * w));
+    p.hwf[s] = (float)((w - 1) / 2.0);
+    p.hhf[s] = (float)((h - 1) / 2.0);
+    sm.disp[s] = p.disp[s];
+    sm.gdisp[s] = p.gdisp[s];
+    sm.k_dx2[s] = p.sm_dx2[s]; sm.k_mix[s] = p.sm_mix[s]; sm.k_dy2[s] = p.sm_dy2[s];
     if (dbg) {
       p.dbg_P[s] = dbg->P[s]; p.dbg_u0[s] = dbg->u0[s]; p.dbg_v0[s] = dbg->v0[s]; p.dbg_inb[s] = dbg->inb[s];
     }
@@ -218,27 +238,19 @@ int run_loss(const SfmDesc* d, const SfmInputs* in, float* losses_out, const Sfm
   p.ssim_rate = d->ssim_rate;     // enters `total` even when the SSIM term itself is skipped (base_model.py:117)
   p.use_smooth = m.use_smooth ? 1 : 0;
   p.edge_smooth = (d->flags & SFM_FLAG_EDGE_AWARE_SMOOTH) ? 1 : 0;
-  int mode = 0;
-  if (m.use_exp) mode |= SFM_MODE_EXP;
-  if (m.use_ssim) mode |= SFM_MODE_SSIM;
-  if (grads) mode |= SFM_MODE_GRAD;
-  if (dbg) mode |= SFM_MODE_DEBUG;
   // prologue kernel: pyramid + tables + cell reset and, in the same grid, the second-order smoothness tasks (the
   // edge-aware variant reads the pyramid and is launched by sfm_launch_fused after it)
-  SfmSmoothParams sm{};
-  int sm_mode = 0;
-  p.sm_part = nullptr;
-  p.n_sm_part = 0;
-  if (m.use_smooth && !p.edge_smooth) {
-    sfm_plan_smooth(p, sm);
-    sm.part = (float*)(ws + L.off_smpart);
-    sm_mode = grads ? 2 : 1;
-    p.sm_part = sm.part;
-    p.n_sm_part = sm.n_ctas;
-  }
-  rc = run_prep(d, in, workspace, !reuse, &sm, sm_mode, st);
+  sm.gy = gy;
+  sm.raw_disp_mask = p.raw_disp_mask;
+  sm.part = (float*)(ws + L.off_smpart);
+  p.sm_part = sm.part;
+  p.n_sm_part = sm.n_ctas;
+  SfmPrepParams pp = prep_params(d, plan.band, ws, reuse ? nullptr : in->tgt, in->src, in->intrinsics, in->poses,
+                                 tables ? nullptr : (float*)(ws + L.off_proj), (float*)(ws + L.off_kinv), true);
+  pp.n_mix_region = plan.n_mix_region;
+  rc = sfm_launch_prep(pp, &sm, grads ? 2 : 1, st);
   if (rc) return rc;
-  return sfm_launch_fused(p, mode, st);
+  return sfm_launch_fused(p, plan, st);
 }
 
 }  // namespace
@@ -294,19 +306,7 @@ extern "C" int sfm_pyramid(const SfmDesc* desc, const float* tgt, const float* s
   int rc = sfm_validate_desc(desc);
   if (rc) return rc;
   if (!tgt || !src || !workspace) { sfm_set_error("sfm_pyramid: null pointer"); return SFM_E_NULL_POINTER; }
-  SfmWsLayout L;
-  sfm_ws_layout(desc, &L);
-  char* ws = (char*)workspace;
-  SfmPrepParams p{};
-  p.B = desc->B; p.S = desc->S; p.H = desc->H; p.W = desc->W; p.ns = desc->n_scales;
-  p.do_pyramid = 1; p.build_tables = 0;
-  p.tgt = tgt; p.src = src;
-  for (int s = 0; s < desc->n_scales; ++s) {
-    p.tgt_pyr[s] = (float*)(ws + L.off_tgt[s]);
-    p.src_pyr[s] = (float*)(ws + L.off_src[s]);
-  }
-  p.acc = (double*)(ws + L.off_acc);
-  p.n_acc = 0;
+  const SfmPrepParams p = prep_params(desc, sfm_plan_band(desc), (char*)workspace, tgt, src, nullptr, nullptr, nullptr, nullptr, false);
   return sfm_launch_prep(p, nullptr, 0, (cudaStream_t)stream);
 }
 
@@ -335,13 +335,7 @@ extern "C" int sfm_build_tables(const SfmDesc* desc, const float* poses, const f
   int rc = sfm_validate_desc(desc);
   if (rc) return rc;
   if (!poses || !intrinsics || !proj_out || !kinv_out) { sfm_set_error("sfm_build_tables: null pointer"); return SFM_E_NULL_POINTER; }
-  SfmPrepParams p{};
-  p.B = desc->B; p.S = desc->S; p.H = desc->H; p.W = desc->W; p.ns = desc->n_scales;
-  p.do_pyramid = 0; p.build_tables = 1;
-  p.intrinsics = intrinsics; p.poses = poses;
-  p.proj_out = proj_out; p.kinv_out = kinv_out;
-  p.acc = nullptr; p.n_acc = 0;
-  p.raw_pose_hw = desc->raw_pose_hw; p.posevec_out = nullptr;
+  const SfmPrepParams p = prep_params(desc, sfm_plan_band(desc), nullptr, nullptr, nullptr, intrinsics, poses, proj_out, kinv_out, false);
   return sfm_launch_prep(p, nullptr, 0, (cudaStream_t)stream);
 }
 

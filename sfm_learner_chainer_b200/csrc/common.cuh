@@ -52,8 +52,12 @@ struct SfmWsLayout {
 
 static inline size_t sfm_align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 
+// SM count of a B200.  The fixed reference of the decisions that must not depend on the device the code runs on (the
+// workspace layout) and of the ones tuned for it without a query (the prologue's band rule, grid caps).
+constexpr int SFM_REF_SMS = 148;
+
 // Decomposition of the second-order smoothness term into warp tasks (strips of SFM_SMOOTH_IW interior columns x hseg
-// rows of every (snippet, scale)); shared by the launcher (smooth.cu) and the workspace layout (one loss-partial slot
+// rows of every (snippet, scale)); shared by the planner (plan.cu) and the workspace layout (one loss-partial slot
 // per 8 tasks).  Segment height: enough warps to cover the chip a few times, few enough that the 4 halo rows stay cheap.
 #define SFM_SMOOTH_IW 28
 static inline int sfm_smooth_plan(int B, int ns, int H, int W, int* hseg_out) {
@@ -62,7 +66,7 @@ static inline int sfm_smooth_plan(int B, int ns, int H, int W, int* hseg_out) {
   for (;;) {
     n = 0;
     for (int s = 0; s < ns; ++s) n += (long long)B * (((W >> s) + SFM_SMOOTH_IW - 1) / SFM_SMOOTH_IW) * (((H >> s) + hseg - 1) / hseg);
-    if (n >= 148 * 4 * 8 || hseg <= 8) break;
+    if (n >= SFM_REF_SMS * 4 * 8 || hseg <= 8) break;
     hseg >>= 1;
   }
   if (hseg_out) *hseg_out = hseg;
@@ -263,9 +267,11 @@ __device__ __forceinline__ float sfm_blend(float w1, float w2, float w3, float w
   return __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(w1, a), __fmul_rn(w2, b)), __fmul_rn(w3, c)), __fmul_rn(w4, d));
 }
 
-__device__ __forceinline__ float sfm_sigmoid(float x) { return 1.f / (1.f + __expf(-x)); }
-// softplus(-x) = log1p(exp(-|x|)) + max(-x, 0)   (sigmoid_cross_entropy against label 1, base_model.py:157-167)
-__device__ __forceinline__ float sfm_softplus_neg(float x) { return log1pf(__expf(-fabsf(x))) + fmaxf(-x, 0.f); }
+// sign(v) * c for either sign of c, 0 when v == 0
+__device__ __forceinline__ float sfm_sign_times(float v, float c) {
+  const float t = __int_as_float((__float_as_int(v) & 0x80000000) ^ __float_as_int(c));
+  return (v == 0.f) ? 0.f : t;
+}
 
 __device__ __forceinline__ float sfm_warp_sum(float v) {
 #pragma unroll

@@ -199,7 +199,7 @@ int sfm_launch_eval_depth(int B, int h, int w, int Hg, int Wg, const float* pred
   EvalState* st = (EvalState*)(ws + L.off_state);
   SFM_CUDA_CHECK(cudaMemsetAsync(ws + L.off_hi, 0, L.total - L.off_hi, stream));
   const long long total = (long long)B * Hg * Wg;
-  const int blocks = (int)((total + 255) / 256 > 148 * 8 ? 148 * 8 : (total + 255) / 256);
+  const int blocks = (int)((total + 255) / 256 > SFM_REF_SMS * 8 ? SFM_REF_SMS * 8 : (total + 255) / 256);
   eval_resize_hist_kernel<<<blocks, 256, 0, stream>>>(pred, gt, mask, pred_full, hist_hi, st, B, h, w, Hg, Wg, lo, hi);
   eval_select_hi_kernel<<<1, 1024, 0, stream>>>(hist_hi, st);
   eval_hist_lo_kernel<<<blocks, 256, 0, stream>>>(gt, pred_full, mask, hist_lo, st, total);

@@ -21,14 +21,14 @@ struct SfmPrepParams {
   int n_acc;
   int raw_pose_hw;   // > 0: `poses` is the raw poseout map (B, 6S, raw_pose_hw); the reduced vectors go to posevec_out
   float* posevec_out;
-  // filled by the launcher
-  int n_pyr_blocks, n_tail_blocks;
+  int n_pyr_blocks, n_tail_blocks;   // filled by the launcher
   int n_mix_region;  // the smoothness CTAs are spread evenly over the first n_mix_region blocks after the tail blocks
   int band;          // full-resolution rows per pyramid CTA
 };
 
 // Second-order smoothness tasks that ride in the prologue kernel (smooth_task.cuh): strips x row segments of every
-// (snippet, scale), one per warp of n_ctas 8-warp CTAs; CTA k writes its loss partial to part[k].
+// (snippet, scale), one per warp of n_ctas 8-warp CTAs; CTA k writes its loss partial to part[k].  The planner fills
+// the task geometry (ns .. tile_begin), the caller the rest.
 struct SfmSmoothParams {
   int ns, hseg, n_tasks, n_ctas;
   int h[SFM_MAX_SCALES], w[SFM_MAX_SCALES];
@@ -67,15 +67,21 @@ struct SfmPeerDev {
   SfmPeerSlot* slots[SFM_MAX_PEERS];
 };
 
+// Warp tasks of a marching kernel: scale s holds tasks [task_begin[s], task_begin[s+1]), nseg[s] row segments of hseg
+// rows each (L1 kernel: rows = 32-pixel runs, nstrip[s] of them; SSIM kernel: image rows, nstrip[s] column strips of
+// SFM_SSIM_IW interior columns) per snippet.
+constexpr int SFM_SSIM_IW = 28;
+struct SfmTaskTable {
+  int hseg;
+  int nstrip[SFM_MAX_SCALES], nseg[SFM_MAX_SCALES];
+  int task_begin[SFM_MAX_SCALES + 1];
+};
+
 // Fused loss kernel parameters (one launch covers every scale, source and snippet).
 struct SfmFusedParams {
   int B, S, ns;
   int h[SFM_MAX_SCALES], w[SFM_MAX_SCALES];
-  // warp-task decomposition (marching kernels): a warp owns a 32-column strip x hseg rows of one (snippet, scale)
-  int hseg;
-  int nstrip[SFM_MAX_SCALES], nseg[SFM_MAX_SCALES];
-  int task_begin[SFM_MAX_SCALES + 1];
-  float wm1f[SFM_MAX_SCALES], hm1f[SFM_MAX_SCALES];   // (float)(w-1), (float)(h-1)
+  SfmTaskTable tasks;
   float hwf[SFM_MAX_SCALES], hhf[SFM_MAX_SCALES];     // (w-1)/2, (h-1)/2
   // images of every scale, planar fp32 [img][3][h][w]: scale 0 = the caller's tgt / src tensors themselves, scales >= 1 =
   // the pyramid in the workspace
@@ -116,34 +122,50 @@ struct SfmFusedParams {
   uint8_t* dbg_inb[SFM_MAX_SCALES];
 };
 
-// Launch helper: with pdl != 0 the kernel is a programmatic dependent launch on the previous kernel of the
-// stream (its CTAs may be scheduled while the predecessor drains; the kernel itself orders its dependent
-// accesses with cudaGridDependencySynchronize()).  SFM_NO_PDL=1 in the environment disables it.
-bool sfm_pdl_enabled();
+// Launch helper: with pdl the kernel is a programmatic dependent launch on the previous kernel of the stream (its
+// CTAs may be scheduled while the predecessor drains; the kernel itself orders its dependent accesses with
+// cudaGridDependencySynchronize()).
 template <typename K, typename... Args>
-static inline cudaError_t sfm_launch_kernel(K kernel, unsigned grid, unsigned block, cudaStream_t stream, bool pdl, Args... args) {
+static inline cudaError_t sfm_launch_kernel(K kernel, dim3 grid, unsigned block, cudaStream_t stream, bool pdl, Args... args) {
   cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(grid, 1, 1);
+  cfg.gridDim = grid;
   cfg.blockDim = dim3(block, 1, 1);
   cfg.dynamicSmemBytes = 0;
   cfg.stream = stream;
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
-  const bool use = pdl && sfm_pdl_enabled();
-  cfg.attrs = use ? attr : nullptr;
-  cfg.numAttrs = use ? 1 : 0;
+  cfg.attrs = pdl ? attr : nullptr;
+  cfg.numAttrs = pdl ? 1 : 0;
   return cudaLaunchKernelEx(&cfg, kernel, args...);
 }
 
 struct SfmPeer;
 const SfmPeerDev* sfm_peer_dev(const SfmPeer* q);      // comm.cu; nullptr until connected
 
-// mode bits for the launcher
-enum { SFM_MODE_EXP = 1, SFM_MODE_SSIM = 2, SFM_MODE_GRAD = 4, SFM_MODE_DEBUG = 8 };
-int sfm_launch_fused(SfmFusedParams& p, int mode, cudaStream_t stream);
-void sfm_plan_smooth(const SfmFusedParams& p, SfmSmoothParams& q);                 // smooth.cu
-int sfm_launch_edge_smooth(SfmFusedParams& p, int grad, cudaStream_t stream);      // smooth.cu
+// Resident warps per SM the SSIM marching kernel is compiled for (__launch_bounds__), which the planner's cost model
+// counts with: forward records in shared memory (168 registers) / in registers (250 registers).
+constexpr int SFM_SSIM_MIN_WARPS = 12;
+constexpr int SFM_SSIM_REG_MIN_WARPS = 8;
+
+// Launch plan of one fused step (plan.cu, the whole launch policy).  The marching kernel instance is
+// sfm_l1_march_kernel<exp, grad, accum, debug, raw> or sfm_ssim_march_kernel<grad, accum, debug, raw, nw, srec>.
+struct SfmStepPlan {
+  bool ssim;                           // kernel family
+  bool exp, grad, accum, debug, raw;   // accum: a smoothness kernel has initialised gdisp
+  int nw;                              // SSIM: warps per CTA (2: the two sources split over the warps of a CTA)
+  bool srec;                           // SSIM: forward records in shared memory (false: in registers)
+  bool edge_smooth;                    // the edge-aware smoothness kernel runs between the prologue and the march
+  SfmTaskTable tasks;
+  SfmSmoothParams smooth;              // second-order smoothness tasks of the prologue (n_ctas == 0: none)
+  int band, n_mix_region;              // SfmPrepParams
+};
+// mode bits of the planner
+enum { SFM_MODE_EXP = 1, SFM_MODE_SSIM = 2, SFM_MODE_GRAD = 4, SFM_MODE_DEBUG = 8, SFM_MODE_SMOOTH = 16 };
+SfmStepPlan sfm_plan_step(const SfmDesc* d, int mode, int num_sms);
+int sfm_plan_band(const SfmDesc* d);
+int sfm_launch_fused(SfmFusedParams& p, const SfmStepPlan& plan, cudaStream_t stream);
+int sfm_launch_edge_smooth(const SfmFusedParams& p, bool grad, cudaStream_t stream);   // smooth.cu
 extern thread_local cudaEvent_t sfm_ev_start, sfm_ev_stop;   // profiling hook (sfm_set_kernel_events)
 
 int sfm_launch_scale(float* const* ptrs, const long long* counts, int n, const float* gy, cudaStream_t stream);

@@ -6,8 +6,6 @@
 // alone and are issue-bound while the pyramid CTAs are memory-bound, so CTAs of both kinds are interleaved in one
 // launch and share the SMs (as separate dependent launches they ran almost back to back: a dependent grid is only
 // released when the last wave of its predecessor has started).
-#include <stdlib.h>
-
 #include "common.cuh"
 #include "kernels.h"
 #include "smooth_task.cuh"
@@ -204,42 +202,22 @@ __global__ void sfm_pose_reduce_kernel(const float* __restrict__ x, float* __res
 
 int sfm_launch_prep(const SfmPrepParams& p_in, const SfmSmoothParams* sm_in, int sm_mode, cudaStream_t stream) {
   SfmPrepParams p = p_in;
-  SfmSmoothParams sm = sm_in ? *sm_in : SfmSmoothParams{};
-  if (!sm_in || sm.n_ctas <= 0) sm_mode = 0;
-  // full-resolution rows per pyramid CTA: 8, or 4 / 2 while the grid would not fill the chip twice (small batches are
-  // latency-bound here: a thread walks band/2 rows of scale 1, so shorter bands mean shorter walks)
-  p.band = 8;
-  {
-    const char* e = getenv("SFM_PREP_BAND");      // development knob
-    if (e && (atoi(e) == 2 || atoi(e) == 4 || atoi(e) == 8)) p.band = atoi(e);
-    else
-      while (p.band > 2 && (long long)p.B * (1 + p.S) * ((p.H + p.band - 1) / p.band) < 148 * 2) p.band >>= 1;
-  }
+  const SfmSmoothParams sm = sm_in ? *sm_in : SfmSmoothParams{};
+  if (sm.n_ctas <= 0) sm_mode = 0;
   p.n_pyr_blocks = (p.do_pyramid && p.ns > 1) ? p.B * (1 + p.S) * ((p.H + p.band - 1) / p.band) : 0;
   const long long n_tail = (p.build_tables ? (long long)p.B * p.S * p.ns + (long long)p.B * p.ns : 0) + p.n_acc;
   p.n_tail_blocks = (int)((n_tail + kPrepThreads - 1) / kPrepThreads);
   const unsigned grid = (unsigned)(p.n_tail_blocks + p.n_pyr_blocks + (sm_mode ? sm.n_ctas : 0));
   if (grid == 0) return 0;                        // e.g. sfm_pyramid with a single scale: nothing to build
-  {
-    int pct = 75;
-    const char* e = getenv("SFM_SM_FRAC");        // development knob: share of the grid over which the smoothness CTAs are spread
-    if (e && atoi(e) > 0 && atoi(e) <= 100) pct = atoi(e);
-    const long long n_mix = (long long)p.n_pyr_blocks + sm.n_ctas;
-    long long R = n_mix * pct / 100;
-    if (R < sm.n_ctas) R = sm.n_ctas;
-    p.n_mix_region = (int)R;
-  }
-  if (sm_mode == 2) sfm_prep_kernel<2><<<grid, kPrepThreads, 0, stream>>>(p, sm);
-  else if (sm_mode == 1) sfm_prep_kernel<1><<<grid, kPrepThreads, 0, stream>>>(p, sm);
-  else sfm_prep_kernel<0><<<grid, kPrepThreads, 0, stream>>>(p, sm);
-  SFM_CUDA_CHECK(cudaGetLastError());
+  const auto kernel = sm_mode == 2 ? sfm_prep_kernel<2> : sm_mode == 1 ? sfm_prep_kernel<1> : sfm_prep_kernel<0>;
+  SFM_CUDA_CHECK(sfm_launch_kernel(kernel, grid, kPrepThreads, stream, false, p, sm));
   return 0;
 }
 
 int sfm_launch_disp_activation(long long n, const float* x, float* disp, float* dact, cudaStream_t stream) {
   if (n <= 0) return 0;
   const long long blocks = (n + 255) / 256;
-  sfm_disp_activation_kernel<<<(unsigned)(blocks > 148 * 16 ? 148 * 16 : blocks), 256, 0, stream>>>(x, disp, dact, n);
+  sfm_disp_activation_kernel<<<(unsigned)(blocks > SFM_REF_SMS * 16 ? SFM_REF_SMS * 16 : blocks), 256, 0, stream>>>(x, disp, dact, n);
   SFM_CUDA_CHECK(cudaGetLastError());
   return 0;
 }

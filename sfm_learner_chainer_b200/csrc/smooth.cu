@@ -60,16 +60,16 @@ __global__ void __launch_bounds__(256) sfm_edge_smooth_kernel(const __grid_const
     if (x + 1 < w) {
       const float dd = __fsub_rn(disp_at(i + 1, fd), d0), e = edge(t0, tex(i + 1));
       loss += fabsf(dd) * e * kx;
-      g -= sgnc(dd, kx) * e;
+      g -= sfm_sign_times(dd, kx) * e;
     }
     if (y + 1 < h) {
       const float dd = __fsub_rn(disp_at(i + w, fd), d0), e = edge(t0, tex(i + w));
       loss += fabsf(dd) * e * ky;
-      g -= sgnc(dd, ky) * e;
+      g -= sfm_sign_times(dd, ky) * e;
     }
     if (GRAD) {
-      if (x > 0) g += sgnc(__fsub_rn(d0, disp_at(i - 1, fd)), kx) * edge(tex(i - 1), t0);
-      if (y > 0) g += sgnc(__fsub_rn(d0, disp_at(i - w, fd)), ky) * edge(tex(i - w), t0);
+      if (x > 0) g += sfm_sign_times(__fsub_rn(d0, disp_at(i - 1, fd)), kx) * edge(tex(i - 1), t0);
+      if (y > 0) g += sfm_sign_times(__fsub_rn(d0, disp_at(i - w, fd)), ky) * edge(tex(i - w), t0);
       G[i] = raw ? (gyv * g) * f0 : gyv * g;
     }
   }
@@ -86,51 +86,9 @@ __global__ void __launch_bounds__(256) sfm_edge_smooth_kernel(const __grid_const
 
 }  // namespace
 
-int sfm_launch_edge_smooth(SfmFusedParams& p, int grad, cudaStream_t stream) {
+int sfm_launch_edge_smooth(const SfmFusedParams& p, bool grad, cudaStream_t stream) {
   const int per = (p.h[0] * p.w[0] + 255) / 256;
-  dim3 grid((unsigned)(per > 32 ? 32 : per), (unsigned)(p.B * p.ns));
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = grid;
-  cfg.blockDim = dim3(256, 1, 1);
-  cfg.stream = stream;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = sfm_pdl_enabled() ? attr : nullptr;
-  cfg.numAttrs = sfm_pdl_enabled() ? 1 : 0;
-  if (grad) SFM_CUDA_CHECK(cudaLaunchKernelEx(&cfg, sfm_edge_smooth_kernel<true>, p));
-  else SFM_CUDA_CHECK(cudaLaunchKernelEx(&cfg, sfm_edge_smooth_kernel<false>, p));
+  const dim3 grid((unsigned)(per > 32 ? 32 : per), (unsigned)(p.B * p.ns));
+  SFM_CUDA_CHECK(sfm_launch_kernel(grad ? sfm_edge_smooth_kernel<true> : sfm_edge_smooth_kernel<false>, grid, 256, stream, true, p));
   return 0;
-}
-
-// Strip decomposition of the smoothness tasks (tiles_x = strips, tiles_y = row segments, tile_begin) and the
-// number of 8-warp CTAs that walk them inside the prologue kernel (one task per warp).  With grad != 0 every
-// gdisp[s] is fully written.
-void sfm_plan_smooth(const SfmFusedParams& p, SfmSmoothParams& q) {
-  q = SfmSmoothParams{};
-  q.ns = p.ns;
-  int hseg = 64;
-  const int total_plan = sfm_smooth_plan(p.B, p.ns, p.h[0], p.w[0], &hseg);
-  q.hseg = hseg;
-  int total = 0;
-  for (int s = 0; s < SFM_MAX_SCALES; ++s) {
-    q.tile_begin[s] = total;
-    if (s < p.ns) {
-      q.h[s] = p.h[s]; q.w[s] = p.w[s];
-      q.tiles_x[s] = (p.w[s] + SM_IW - 1) / SM_IW;
-      q.tiles_y[s] = (p.h[s] + hseg - 1) / hseg;
-      total += p.B * q.tiles_x[s] * q.tiles_y[s];
-      q.disp[s] = p.disp[s];
-      q.gdisp[s] = p.gdisp[s];
-      q.k_dx2[s] = p.sm_dx2[s]; q.k_mix[s] = p.sm_mix[s]; q.k_dy2[s] = p.sm_dy2[s];
-    } else {
-      q.tiles_x[s] = q.tiles_y[s] = 1;
-    }
-  }
-  (void)total_plan;
-  q.tile_begin[SFM_MAX_SCALES] = total;
-  q.n_tasks = total;
-  q.n_ctas = (total + 7) / 8;
-  q.gy = p.gy;
-  q.raw_disp_mask = p.raw_disp_mask;
 }

@@ -10,11 +10,6 @@ namespace {
 
 constexpr int SM_IW = SFM_SMOOTH_IW;         // interior columns per strip
 
-__device__ __forceinline__ float sgnc(float v, float c) {   // sign(v) * c (c > 0), 0 when v == 0
-  const float t = __int_as_float((__float_as_int(v) & 0x80000000) | __float_as_int(c));
-  return (v == 0.f) ? 0.f : t;
-}
-
 // -> this lane's part of the task's loss (to be summed over the warp by the caller)
 template <bool GRAD>
 __device__ __forceinline__ float sfm_smooth_task(const SfmSmoothParams& p, int t, const int lane) {
@@ -67,7 +62,7 @@ __device__ __forceinline__ float sfm_smooth_task(const SfmSmoothParams& p, int t
     const float ex0 = __fsub_rn(__shfl_down_sync(0xffffffffu, d0, 1), d0);                 // D[r][x+1] - D[r][x]
     const float dx2 = __fsub_rn(__shfl_down_sync(0xffffffffu, ex0, 1), ex0);
     const bool vx = r_in && x_dx2;
-    const float sx = vx ? sgnc(dx2, k_dx2) : 0.f;
+    const float sx = vx ? sfm_sign_times(dx2, k_dx2) : 0.f;
     if (vx && col_own && r >= y0 && r < y1) loss += fabsf(dx2) * k_dx2;
     const float sxm1 = __shfl_up_sync(0xffffffffu, sx, 1), sxm2 = __shfl_up_sync(0xffffffffu, sx, 2);
     const float gx0 = (sxm2 - 2.f * sxm1) + sx;
@@ -76,14 +71,14 @@ __device__ __forceinline__ float sfm_smooth_task(const SfmSmoothParams& p, int t
     const float dy2 = __fsub_rn(ey1, ey2);
     const int ry = r - 2;
     const bool vy = col_in && (ry >= 0) && (ry <= h - 3);
-    const float sy2 = vy ? sgnc(dy2, k_dy2) : 0.f;
+    const float sy2 = vy ? sfm_sign_times(dy2, k_dy2) : 0.f;
     if (vy && col_own && ry >= y0 && ry < y1) loss += fabsf(dy2) * k_dy2;
     // ---- mixed terms of cell (r-1, x): dxdy = ex[r] - ex[r-1] ; dydx = ey[r-1][x+1] - ey[r-1][x]
     const float a = __fsub_rn(ex0, ex1);
     const float bq = __fsub_rn(__shfl_down_sync(0xffffffffu, ey1, 1), ey1);
     const int rm = r - 1;
     const bool vm = x_mix && (rm >= 0) && (rm <= h - 2);
-    const float m1 = vm ? (sgnc(a, k_mix) + sgnc(bq, k_mix)) : 0.f;
+    const float m1 = vm ? (sfm_sign_times(a, k_mix) + sfm_sign_times(bq, k_mix)) : 0.f;
     if (vm && col_own && rm >= y0 && rm < y1) loss += (fabsf(a) + fabsf(bq)) * k_mix;
     const float n1 = m1 - __shfl_up_sync(0xffffffffu, m1, 1);
     // ---- gradient of pixel (r-2, x)

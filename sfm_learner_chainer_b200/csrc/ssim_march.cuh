@@ -18,8 +18,6 @@
 
 namespace {
 
-constexpr int SSIM_IW = 28;     // interior columns per strip
-
 // Three channels as one packed pair (channels 0, 1: FFMA2 / FADD2 / FMUL2 of sm_100, one issue slot for two
 // lanes) plus a scalar (channel 2).  Used for the SSIM statistics and gradient fields (tolerance-checked region; the
 // individually rounded coordinate chain and the blend stay scalar).  The packed forms have the same FP32 throughput
@@ -50,16 +48,16 @@ __device__ __forceinline__ StripTask decode_strip(const SfmFusedParams& p, int t
   int s = 0;
 #pragma unroll
   for (int q = 1; q < SFM_MAX_SCALES; ++q)
-    if (q < p.ns && t >= p.task_begin[q]) s = q;
-  t -= p.task_begin[s];
+    if (q < p.ns && t >= p.tasks.task_begin[q]) s = q;
+  t -= p.tasks.task_begin[s];
   k.s = s;
-  const int seg = t % p.nseg[s];
-  t /= p.nseg[s];
-  const int strip = t % p.nstrip[s];
-  k.b = t / p.nstrip[s];
-  k.x0 = strip * SSIM_IW;
-  k.y0 = seg * p.hseg;
-  k.y1 = min(k.y0 + p.hseg, p.h[s]);
+  const int seg = t % p.tasks.nseg[s];
+  t /= p.tasks.nseg[s];
+  const int strip = t % p.tasks.nstrip[s];
+  k.b = t / p.tasks.nstrip[s];
+  k.x0 = strip * SFM_SSIM_IW;
+  k.y0 = seg * p.tasks.hseg;
+  k.y1 = min(k.y0 + p.tasks.hseg, p.h[s]);
   return k;
 }
 
@@ -75,15 +73,6 @@ struct Rec {
 template <int N>
 struct IC { static constexpr int value = N; };
 
-#ifndef SFM_SSIM_FENCE
-#define SFM_SSIM_FENCE 1      // basic-block fence after the refill (see step)
-#endif
-#ifndef SFM_MINB_SSIM
-#define SFM_MINB_SSIM 12      // resident warps per SM of the instances that keep the forward records in shared memory (168 registers)
-#endif
-#ifndef SFM_MINB_SSIM_REG
-#define SFM_MINB_SSIM_REG 8   // ... of the instances that keep them in registers (250 registers)
-#endif
 // NW = warps per CTA.  NW == 1: one warp walks the strip segment once per source.  NW == 2 (two sources, small
 // batches): the two warps of a CTA walk the same segment at the same time, one source each, so a task is half as
 // long and -- for the same number of resident warps -- twice as tall (half the halo rows).  gdisp stays
@@ -94,9 +83,8 @@ struct IC { static constexpr int value = N; };
 // registers, 2 warps per scheduler, 6 % fewer instructions and a third fewer L1 data-pipe wavefronts) -- faster whenever
 // the whole grid is resident at once anyway (cfg2: 29.3 -> 26.6 us), slower when occupancy counts (cfg5: 933 -> 952 us).
 template <bool GRAD, bool ACCUM, bool DEBUG, bool RAW, int NW, bool SREC = true>
-__global__ void __launch_bounds__(32 * NW, (SREC ? SFM_MINB_SSIM : SFM_MINB_SSIM_REG) / NW)
+__global__ void __launch_bounds__(32 * NW, (SREC ? SFM_SSIM_MIN_WARPS : SFM_SSIM_REG_MIN_WARPS) / NW)
 sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
-  constexpr bool SFM_SSIM_SREC = SREC;
   __shared__ float4 sP_all[NW][3];
   __shared__ float sG[(NW > 1) ? 3 * 2 * 32 : 1];       // [ring slot][gdd | dsc][lane] of warp 1's row term
   const int wi = (NW > 1) ? (int)(threadIdx.x >> 5) : 0;
@@ -114,7 +102,7 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
   // two-row delay line of forward records: [slot][field][lane], written in stage A of row r and read back by
   // the same lane in stages E/F two steps later (no synchronisation needed).  In registers these 51 values
   // pushed the kernel over its 168-register budget (17-27 local-memory spills per three rows).
-  __shared__ float sRec[(GRAD && SFM_SSIM_SREC) ? NW * 3 * 18 * 32 : 1];
+  __shared__ float sRec[(GRAD && SREC) ? NW * 3 * 18 * 32 : 1];
   const int lane = threadIdx.x & 31;
   float* const myrec = sRec + wi * (3 * 18 * 32) + lane;
   const StripTask t = decode_strip(p, blockIdx.x);
@@ -122,7 +110,7 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
   const Geo geo = make_geo(p, s);
   const int xx = t.x0 - 2 + lane;                       // this lane's image column (may be outside)
   const bool col_in = (xx >= 0) && (xx < w);
-  const bool col_own = (lane >= 2) && (lane < 2 + SSIM_IW) && (xx < w);
+  const bool col_own = (lane >= 2) && (lane < 2 + SFM_SSIM_IW) && (xx < w);
   const float gyv = p.gy ? __ldg(p.gy) : 1.f;
   const float inv_n3 = p.inv_n3[s];
   const float wpix = gyv * (1.f - p.ssim_rate) * inv_n3;
@@ -148,7 +136,7 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
   const size_t src_img = (size_t)3 * plane;
   float pix_part = 0.f, ssim_part = 0.f;
   const int r_begin = t.y0 - 2, r_end = t.y1 + 2;      // rows [r_begin, r_end) are warped
-  const bool opaque_true = p.hseg != 0x7fffffff;       // always true, unknown to ptxas: basic-block fence (see step)
+  const bool opaque_true = p.tasks.hseg != 0x7fffffff;       // always true, unknown to ptxas: basic-block fence (see step)
 
   for (int i = (NW > 1) ? wi : 0; i < ((NW > 1) ? wi + 1 : S); ++i) {
     __syncwarp();
@@ -181,7 +169,7 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
 #pragma unroll
       for (int c = 0; c < 3; ++c) rec[k].Ix[c] = rec[k].Iy[c] = rec[k].P[c] = rec[k].T[c] = 0.f;
       rec[k].q0 = rec[k].q1 = rec[k].q2 = rec[k].r = rec[k].depth = rec[k].dsc = 0.f;
-      if (GRAD && SFM_SSIM_SREC) {
+      if (GRAD && SREC) {
 #pragma unroll
         for (int q = 0; q < 18; ++q) myrec[(k * 18 + q) * 32] = 0.f;
       }
@@ -275,7 +263,7 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
           rc_.q0 = pq0; rc_.q1 = pq1; rc_.q2 = pq2; rc_.r = pr;
           rc_.depth = pdepth;
           rc_.dsc = RAW ? pdsc : pdepth;
-          if (SFM_SSIM_SREC) {
+          if (SREC) {
             float* o = myrec + cur * 18 * 32;
 #pragma unroll
             for (int c = 0; c < 3; ++c) {
@@ -301,9 +289,7 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
       // otherwise sinks the projection and the four gathers to the end of the step (seen in the SASS; ncu:
       // half of all stall samples were long-scoreboard waits on the taps ~60 instructions after their issue).
       // A branch it cannot fold keeps them ahead of stages B..F, which then cover the latency.
-#if SFM_SSIM_FENCE
       if (opaque_true) {
-#endif
       // ---------------- stage B: row sums of P, P^2, P.T, T, T^2 over lanes-1..+1 (zero outside the image)
       {
         const V3 pv = v3(rc_.P[0], rc_.P[1], rc_.P[2]), tv = v3(rc_.T[0], rc_.T[1], rc_.T[2]);
@@ -368,7 +354,7 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
         const V3* g1 = gs[pv1];
         const V3* g2 = gs[pv2];
         Rec rb = rec[pv2];
-        if (SFM_SSIM_SREC) {
+        if (SREC) {
           const float* o = myrec + pv2 * 18 * 32;
 #pragma unroll
           for (int c = 0; c < 3; ++c) {
@@ -393,7 +379,7 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
           const float gs3[3] = {gsv.a.x, gsv.a.y, gsv.b};
 #pragma unroll
           for (int c = 0; c < 3; ++c) {
-            const float gl1 = mf ? 0.f : sign_times(rb.P[c] - rb.T[c], wpix);
+            const float gl1 = mf ? 0.f : sfm_sign_times(rb.P[c] - rb.T[c], wpix);
             gP[c] = do_f ? gs3[c] + gl1 : 0.f;
           }
         }
@@ -419,9 +405,7 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
         }
         if (do_f && writer) st_global(gp, gval);
       }
-#if SFM_SSIM_FENCE
       }
-#endif
     };
 
     // prologue: rows r_begin (slot 0) and its lookahead
@@ -455,135 +439,3 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
 }
 
 }  // namespace
-
-template <typename K>
-static int launch_ssim_kernel(K kernel, const SfmFusedParams& p, cudaStream_t stream, int nw = 1) {
-  const int n_tasks = p.task_begin[SFM_MAX_SCALES];
-  if (sfm_ev_start) SFM_CUDA_CHECK(cudaEventRecord(sfm_ev_start, stream));
-  SFM_CUDA_CHECK(sfm_launch_kernel(kernel, n_tasks, 32 * nw, stream, !sfm_ev_start, p));
-  if (sfm_ev_stop) SFM_CUDA_CHECK(cudaEventRecord(sfm_ev_stop, stream));
-  return 0;
-}
-
-int launch_epilogue(const SfmFusedParams& p, cudaStream_t stream);
-
-static int sfm_launch_ssim(SfmFusedParams& p, bool grad, bool accum, bool debug, long long want_warps, cudaStream_t stream) {
-  // Task height (rows per strip segment).  Cost model, calibrated on B200 (tools/time_graph.py sweeps, DESIGN.md):
-  // a task marches 3*ceil((hseg+4)/3) rows per source (4 halo rows, row loop unrolled by three); up to
-  // SFM_MINB_SSIM single-warp CTAs are resident per SM, i.e. 3 per scheduler.  Above one wave the time is
-  // waves x rows; below one wave the busiest scheduler holds w = ceil(tasks / schedulers) warps and runs them at
-  // a relative issue efficiency of 0.66 / 0.9 / 1.0 for w = 1 / 2 / 3 (a lone warp cannot hide its own latencies).
-  // Example cfg2 (B=4, 128x416): hseg 8 -> 1296 tasks, w=3, 12 rows: 36.8 us; hseg 11 -> 976 tasks, w=2, 15 rows: 33.4 us.
-  // With two sources and a sub-wave grid the sources can also be split over the two warps of a CTA (NW = 2): a task
-  // is then one pass long and there are twice as many warps, so the same occupancy is reached with taller segments
-  // (fewer halo rows); the per-row CTA barrier is charged 5 %.
-  (void)want_warps;
-  int hseg = 64, nw = 1;
-  bool srec = true;       // forward records in shared memory; false: the register-record instances (plain GRAD mode only)
-  {
-    const long long sched = (long long)g_num_sms * 4, slots = (long long)g_num_sms * SFM_MINB_SSIM;
-    const long long slots_reg = (long long)g_num_sms * SFM_MINB_SSIM_REG;
-    const bool may_split = grad && !debug && p.raw_disp_mask == 0 && p.S == 2 && !getenv("SFM_SSIM_NOSPLIT");
-    const bool may_reg = grad && !debug && p.raw_disp_mask == 0;
-    double best = 1e300;
-    for (int var = 0; var <= (may_reg ? 1 : 0); ++var)
-      for (int cand = 1; cand <= (may_split ? 2 : 1); ++cand)
-        for (int h = 8; h <= 64; ++h) {
-          long long n = 0;
-          for (int s = 0; s < p.ns; ++s) n += (long long)p.B * ((p.w[s] + SSIM_IW - 1) / SSIM_IW) * ((p.h[s] + h - 1) / h);
-          const long long warps = n * cand;
-          const double rows = 3.0 * ((h + 4 + 2) / 3) * (cand == 1 ? p.S : 1) * (cand == 1 ? 1.0 : 1.05);
-          double cost;
-          if (var == 1) {
-            // register-record instances: 2 warps per scheduler at most, 9 % faster per row; only while the whole grid is
-            // resident at once (above that the shared-memory instances' third warp per scheduler wins: measured at cfg5)
-            if (warps > slots_reg) continue;
-            const long long w = (warps + sched - 1) / sched;
-            cost = 0.91 * rows * (double)w / (w <= 1 ? 0.66 : 0.9);
-          } else if (warps > slots) {
-            cost = rows * 3.0 * (double)((warps + slots - 1) / slots);
-          } else {
-            const long long w = (warps + sched - 1) / sched;
-            cost = rows * (double)w / (w <= 1 ? 0.66 : w == 2 ? 0.9 : 1.0);
-          }
-          if (cost < best || (cost == best && cand == nw)) { best = cost; hseg = h; nw = cand; srec = (var == 0); }
-        }
-  }
-  if (srec && nw == 1) {
-    // Grids of many waves: the time follows the total number of row steps (measured at cfg5: 64 / 86 / 128 rows per
-    // segment -> 934 / 933 / 912 us for 276 / 276 / 270 row steps per strip), so a taller segment -- fewer halo rows --
-    // is taken when it saves at least 1.5 % of the row steps and still leaves three waves of tasks.
-    const long long slots = (long long)g_num_sms * SFM_MINB_SSIM;
-    auto work = [&](int h, long long* n_out) {
-      long long n = 0, wk = 0;
-      for (int s = 0; s < p.ns; ++s) {
-        const long long strips = (long long)p.B * ((p.w[s] + SSIM_IW - 1) / SSIM_IW);
-        const int full = p.h[s] / h, rem = p.h[s] - full * h;
-        n += strips * (full + (rem ? 1 : 0));
-        wk += strips * ((long long)full * (3 * ((h + 4 + 2) / 3)) + (rem ? 3 * ((rem + 4 + 2) / 3) : 0));
-      }
-      *n_out = n;
-      return wk;
-    };
-    long long n0 = 0;
-    long long w0 = work(hseg, &n0);
-    if (n0 > 3 * slots)
-      for (int h2 : {96, 128, 192, 256}) {
-        long long n2 = 0;
-        const long long w2 = work(h2, &n2);
-        if (n2 >= 3 * slots && (double)w2 < 0.985 * (double)w0) { hseg = h2; w0 = w2; }
-      }
-  }
-  {
-    const char* e = getenv("SFM_HSEG");          // development knobs
-    if (e && atoi(e) > 0) hseg = atoi(e);
-    const char* f = getenv("SFM_SSIM_NW");
-    if (f && (atoi(f) == 1 || (atoi(f) == 2 && grad && !debug && p.raw_disp_mask == 0 && p.S == 2))) nw = atoi(f);
-    const char* g = getenv("SFM_SSIM_SREC");
-    if (g && (atoi(g) == 1 || (atoi(g) == 0 && grad && !debug && p.raw_disp_mask == 0))) srec = atoi(g) != 0;
-  }
-  p.hseg = hseg;
-  int total = 0;
-  for (int s = 0; s < SFM_MAX_SCALES; ++s) {
-    p.task_begin[s] = total;
-    if (s < p.ns) {
-      p.nstrip[s] = (p.w[s] + SSIM_IW - 1) / SSIM_IW;
-      p.nseg[s] = (p.h[s] + hseg - 1) / hseg;
-      total += p.B * p.nstrip[s] * p.nseg[s];
-    } else {
-      p.nstrip[s] = p.nseg[s] = 1;
-    }
-  }
-  p.task_begin[SFM_MAX_SCALES] = total;
-  int rc;
-  const bool raw = p.raw_disp_mask != 0;
-  if (nw == 2) {
-    if (srec)
-      rc = accum ? launch_ssim_kernel(sfm_ssim_march_kernel<true, true, false, false, 2, true>, p, stream, 2)
-                 : launch_ssim_kernel(sfm_ssim_march_kernel<true, false, false, false, 2, true>, p, stream, 2);
-    else
-      rc = accum ? launch_ssim_kernel(sfm_ssim_march_kernel<true, true, false, false, 2, false>, p, stream, 2)
-                 : launch_ssim_kernel(sfm_ssim_march_kernel<true, false, false, false, 2, false>, p, stream, 2);
-    if (rc) return rc;
-    return launch_epilogue(p, stream);
-  }
-  if (!srec) {
-    rc = accum ? launch_ssim_kernel(sfm_ssim_march_kernel<true, true, false, false, 1, false>, p, stream)
-               : launch_ssim_kernel(sfm_ssim_march_kernel<true, false, false, false, 1, false>, p, stream);
-    if (rc) return rc;
-    return launch_epilogue(p, stream);
-  }
-#define SFM_SSIM(GR, AC)                                                                                   \
-  rc = raw ? (debug ? launch_ssim_kernel(sfm_ssim_march_kernel<GR, AC, true, true, 1>, p, stream)             \
-                    : launch_ssim_kernel(sfm_ssim_march_kernel<GR, AC, false, true, 1>, p, stream))           \
-           : (debug ? launch_ssim_kernel(sfm_ssim_march_kernel<GR, AC, true, false, 1>, p, stream)            \
-                    : launch_ssim_kernel(sfm_ssim_march_kernel<GR, AC, false, false, 1>, p, stream))
-  if (grad) {
-    if (accum) { SFM_SSIM(true, true); } else { SFM_SSIM(true, false); }
-  } else {
-    SFM_SSIM(false, false);
-  }
-#undef SFM_SSIM
-  if (rc) return rc;
-  return launch_epilogue(p, stream);
-}

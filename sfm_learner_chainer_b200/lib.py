@@ -4,7 +4,7 @@ import ctypes as C
 import os
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-LIB_PATH = os.environ.get('SFM_LIB_PATH') or os.path.join(HERE, 'libsfmloss.so')   # SFM_LIB_PATH: development builds with other compile-time knobs
+LIB_PATH = os.path.join(HERE, 'libsfmloss.so')
 
 SFM_MAX_SCALES = 4
 SFM_MAX_SOURCES = 8

@@ -19,7 +19,7 @@ def _op(flags, **kw):
 
 
 @pytest.mark.parametrize('flags', [dict(smooth_reg=0.1, exp_reg=0.0, ssim_rate=0.15), dict(smooth_reg=0.5, exp_reg=0.2, ssim_rate=0.0),
-                                   dict(smooth_reg=0.3, exp_reg=0.0, ssim_rate=0.0)])
+                                   dict(smooth_reg=0.3, exp_reg=0.0, ssim_rate=0.0), dict(smooth_reg=-0.2, exp_reg=0.0, ssim_rate=0.15)])
 @pytest.mark.parametrize('B,S,H,W,seed', [(2, 2, 64, 208, 80), (1, 4, 40, 72, 81), (4, 2, 128, 416, 82)])
 def test_edge_smooth_vs_oracle(flags, B, S, H, W, seed):
     d = make_snippets(B, S, H, W, seed=seed, rough_disp=bool(seed & 1))

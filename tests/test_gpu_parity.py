@@ -16,6 +16,7 @@ FLAGSETS = {
     'v1_ssim': dict(smooth_reg=0.1, exp_reg=0.0, ssim_rate=0.15),  # experiments/sfm_learner_v1_ssim.yml
     'v1_odom': dict(smooth_reg=0.1, exp_reg=0.2, ssim_rate=0.0),   # experiments/sfm_learner_v1_odom.yml
     'exp_ssim_rate': dict(smooth_reg=0.05, exp_reg=0.3, ssim_rate=0.25),  # exp branch wins, (1-ssim_rate) weight stays
+    'neg_smooth': dict(smooth_reg=-0.1, exp_reg=0.0, ssim_rate=0.15),  # a negative weight enables the term too (sign(d) * wgt)
 }
 
 
