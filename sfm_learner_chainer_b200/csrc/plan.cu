@@ -51,12 +51,20 @@ void plan_l1(SfmStepPlan& q, const SfmDesc* d, int num_sms) {
   q.tasks = task_table(d->B, d->n_scales, hseg, runs, runs, false);
 }
 
+// Instructions a SSIM task of h rows issues per source, in full row steps: it marches h + 4 steps and runs refill + A + B
+// on all of them, C + D on h + 2 and E + F on h (ssim_march.cuh, RowStages).  The stage shares of a full step are
+// those of the SASS of the row loop (tools/sass_loop.py on instances whose loop runs only A + B, or only A..D): 0.33 /
+// 0.22 / 0.45 in the register-record instance, 0.40 / 0.17 / 0.43 in the shared-memory-record one.
+double ssim_task_steps(int h) { return 0.35 * (h + 4) + 0.2 * (h + 2) + 0.45 * h; }
+
 // SSIM marching kernel.  Task height (rows per strip segment), cost model calibrated on B200 (tools/time_graph.py
-// sweeps, DESIGN.md): a task marches 3*ceil((hseg+4)/3) rows per source (4 halo rows, row loop unrolled by three); up to
-// SFM_SSIM_MIN_WARPS single-warp CTAs are resident per SM, i.e. 3 per scheduler.  Above one wave the time is
-// waves x rows; below one wave the busiest scheduler holds w = ceil(tasks / schedulers) warps and runs them at
-// a relative issue efficiency of 0.66 / 0.9 / 1.0 for w = 1 / 2 / 3 (a lone warp cannot hide its own latencies).
-// Example cfg2 (B=4, 128x416): hseg 8 -> 1296 tasks, w=3, 12 rows: 36.8 us; hseg 11 -> 976 tasks, w=2, 15 rows: 33.4 us.
+// sweeps, DESIGN.md): a task costs ssim_task_steps(hseg) row steps per source; up to SFM_SSIM_MIN_WARPS single-warp
+// CTAs are resident per SM, i.e. 3 per scheduler.  Above one wave the time is waves x steps; below one wave the
+// busiest scheduler holds w = ceil(tasks / schedulers) warps and runs them at a relative issue efficiency of
+// 0.66 / 0.9 / 1.0 for w = 1 / 2 / 3 (a lone warp cannot hide its own latencies).
+// Example cfg2 (B=4, 128x416, register records): NW = 2, hseg 19 -> 588 tasks, w = 1, 20.8 steps: cost 44.2;
+// hseg 20 -> 588 tasks, 21.8 steps: 46.3; shared-memory records, hseg 13 -> 824 tasks, w = 2, 14.8 steps: 46.6; NW = 1,
+// hseg 10 -> 1084 tasks, w = 2, 2 x 11.8 steps: 47.7.
 // With two sources and a sub-wave grid the sources can also be split over the two warps of a CTA (NW = 2): a task
 // is then one pass long and there are twice as many warps, so the same occupancy is reached with taller segments
 // (fewer halo rows); the per-row CTA barrier is charged 5 %.
@@ -80,7 +88,7 @@ void plan_ssim(SfmStepPlan& q, const SfmDesc* d, int num_sms) {
       for (int h = 8; h <= 64; ++h) {
         const long long n = task_table(B, ns, h, strips, hs, true).task_begin[SFM_MAX_SCALES];
         const long long warps = n * cand;
-        const double rows = 3.0 * ((h + 4 + 2) / 3) * (cand == 1 ? S : 1) * (cand == 1 ? 1.0 : 1.05);
+        const double rows = ssim_task_steps(h) * (cand == 1 ? S : 1) * (cand == 1 ? 1.0 : 1.05);
         double cost;
         if (var == 1) {
           // register-record instances: 2 warps per scheduler at most, 9 % faster per row; only while the whole grid is
@@ -97,27 +105,29 @@ void plan_ssim(SfmStepPlan& q, const SfmDesc* d, int num_sms) {
         if (cost < best || (cost == best && cand == nw)) { best = cost; hseg = h; nw = cand; srec = (var == 0); }
       }
   if (srec && nw == 1) {
-    // Grids of many waves: the time follows the total number of row steps (measured at cfg5: 64 / 86 / 128 rows per
-    // segment -> 934 / 933 / 912 us for 276 / 276 / 270 row steps per strip), so a taller segment -- fewer halo rows --
-    // is taken when it saves at least 1.5 % of the row steps and still leaves three waves of tasks.
+    // Grids of many waves: the time follows the total number of row steps (measured at cfg5 before the stage schedule
+    // of RowStages: 64 / 86 / 128 rows per segment -> 934 / 933 / 912 us for 276 / 276 / 270 row steps per strip), so
+    // a taller segment -- fewer halo rows, fewer task flushes -- is taken when it saves at least 1 % of the steps and
+    // still leaves three waves of tasks.
     auto work = [&](int h, long long* n_out) {
-      long long n = 0, wk = 0;
+      long long n = 0;
+      double wk = 0.0;
       for (int s = 0; s < ns; ++s) {
         const long long st = (long long)B * strips[s];
         const int full = hs[s] / h, rem = hs[s] - full * h;
         n += st * (full + (rem ? 1 : 0));
-        wk += st * ((long long)full * (3 * ((h + 4 + 2) / 3)) + (rem ? 3 * ((rem + 4 + 2) / 3) : 0));
+        wk += (double)st * (full * ssim_task_steps(h) + (rem ? ssim_task_steps(rem) : 0.0));
       }
       *n_out = n;
       return wk;
     };
     long long n0 = 0;
-    long long w0 = work(hseg, &n0);
+    double w0 = work(hseg, &n0);
     if (n0 > 3 * slots)
       for (int h2 : {96, 128, 192, 256}) {
         long long n2 = 0;
-        const long long w2 = work(h2, &n2);
-        if (n2 >= 3 * slots && (double)w2 < 0.985 * (double)w0) { hseg = h2; w0 = w2; }
+        const double w2 = work(h2, &n2);
+        if (n2 >= 3 * slots && w2 < 0.99 * w0) { hseg = h2; w0 = w2; }
       }
   }
   const int forced_h = test_hook("SFM_HSEG", 0), forced_nw = test_hook("SFM_SSIM_NW", -1);

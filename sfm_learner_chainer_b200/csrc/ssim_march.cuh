@@ -11,8 +11,9 @@
 //   stage E  vertical 3-sums -> dL/dP at (r-2, lane) = A(g_a) + 2P.A(g_s) + T.A(g_c) + L1 part
 //   stage F  sampler / projection backward of pixel (r-2, lane) from its forward record
 // The rings and the two-row delay line of forward records live in registers; the row loop is unrolled
-// three times so that the ring rotation is pure renaming.  No shared memory, no barrier; the only
-// atomics are the per-task flush.  dL/dP accumulates as sum gq, sum gq*depth, sum gq*depth*y per lane
+// three times so that the ring rotation is pure renaming.  Each step runs only the stages whose row is used:
+// C/D from the third step on, E/F from the fifth, no step past r = y1+1 (see RowStages).  No shared memory, no
+// barrier; the only atomics are the per-task flush.  dL/dP accumulates as sum gq, sum gq*depth, sum gq*depth*y per lane
 // (the lane's column x is constant along the march) and is expanded with Kinv before the flush.
 #pragma once
 
@@ -72,6 +73,17 @@ struct Rec {
 
 template <int N>
 struct IC { static constexpr int value = N; };
+
+// The stages one row step runs.  A task of h rows marches h + 4 steps, j = 0 .. h+3 on rows r = y0-2+j; step j blends
+// row r (A, B), takes the SSIM of row r-1 (C, D) and the backward of row r-2 (E, F).  Rows y0-2 .. y1+1 feed the
+// windows of the owned rows, the gradient fields of rows y0-1 .. y1 feed their dL/dP, so C/D are needed from step 2
+// and E/F from step 4 on.  The ring slots those skipped stages would fill are overwritten before any step reads them.
+// The march ends with step h+3: no step runs past row y1+1.
+enum RowStages {
+  ROW_AB,       // steps 0, 1
+  ROW_ABCD,     // steps 2, 3
+  ROW_ALL,      // steps 4 .. h+3
+};
 
 // NW = warps per CTA.  NW == 1: one warp walks the strip segment once per source.  NW == 2 (two sources, small
 // batches): the two warps of a CTA walk the same segment at the same time, one source each, so a task is half as
@@ -153,29 +165,13 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
       s_ptrs_all[wi].gdisp = gdisp;
     }
     __syncwarp();
-    // rings: window row sums (P, P^2, P.T, T, T^2 per channel), gradient-field row sums, forward records
+    // rings: window row sums (P, P^2, P.T, T, T^2 per channel), gradient-field row sums, forward records.  No
+    // initial value: with the stage schedule of RowStages every slot is written before a step reads it.
     V3 hs[3][5], gs[3][3];        // [ring slot][field]: (P, P^2, P.T, T, T^2) and (g_a, g_s, g_c) row sums, three channels each
     Rec rec[3];
     bool mask[3];                                        // all-zero mask of the row's pixel (base_model.py:96)
-    float dq[3];                                         // disparity / target rows fetched ahead
+    float dq[3] = {1.f, 1.f, 1.f};                       // disparity / target rows fetched ahead
     float Tq[3][3];
-#pragma unroll
-    for (int k = 0; k < 3; ++k) {
-#pragma unroll
-      for (int q = 0; q < 5; ++q) hs[k][q] = v3s(0.f);
-#pragma unroll
-      for (int q = 0; q < 3; ++q) gs[k][q] = v3s(0.f);
-      mask[k] = true;
-#pragma unroll
-      for (int c = 0; c < 3; ++c) rec[k].Ix[c] = rec[k].Iy[c] = rec[k].P[c] = rec[k].T[c] = 0.f;
-      rec[k].q0 = rec[k].q1 = rec[k].q2 = rec[k].r = rec[k].depth = rec[k].dsc = 0.f;
-      if (GRAD && SREC) {
-#pragma unroll
-        for (int q = 0; q < 18; ++q) myrec[(k * 18 + q) * 32] = 0.f;
-      }
-      dq[k] = 1.f;
-      Tq[k][0] = Tq[k][1] = Tq[k][2] = 0.f;
-    }
     auto load_dT = [&](int r, float& dd, float* TT) {
       dd = 1.f;
       TT[0] = TT[1] = TT[2] = 0.f;
@@ -188,25 +184,29 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
         TT[2] = __ldg(tb + (o + 2u * geo.plane));
       }
     };
-    // pending row: projected, gathers in flight, consumed by the next step
-    Taps I;
-    float pwa = 0.f, pwb = 0.f, pwc = 0.f, pwd = 0.f, pq0 = 0.f, pq1 = 0.f, pq2 = 0.f, pr = 0.f, pdepth = 0.f, pdsc = 0.f;
+    // pending rows: projected, gathers in flight, consumed by a later step.  The loop keeps one (pend[0], refilled one
+    // row ahead); the head of the register-record instances keeps two, refilled two rows ahead (see the march below)
+    struct Pend {
+      Taps I;
+      float wa, wb, wc, wd, q0, q1, q2, r, depth, dsc;
+    };
+    Pend pend[2];
     float g_old = 0.f;
 
-    // refill: project row r (its disparity was fetched a step earlier), issue its gathers, fetch row r+1's
-    // disparity / target and the partial gdisp of the row whose backward runs in the next step
-    auto refill = [&](auto SLOT, const int r) {
+    // refill: project row r into pending row pn (its disparity was fetched a step earlier), issue its gathers, fetch
+    // row r+1's disparity / target (unless LOAD_NEXT is false) and the partial gdisp of the row whose backward runs next
+    auto refill = [&](auto SLOT, Pend& pn, const int r, auto LOAD_NEXT) {
       constexpr int sl = decltype(SLOT)::value, nx = (sl + 1) % 3;
       const bool in_img = col_in && (r >= 0) && (r < h) && (r < r_end);
       float d = dq[sl], dact = 1.f;
       if (raw) d = sfm_disp_act(d, dact);      // producer-side fusion: pre-activation disparity map (warp-uniform branch)
-      pdepth = rcp_newton(d);
-      if (RAW) pdsc = raw ? pdepth * dact : pdepth;
+      pn.depth = rcp_newton(d);
+      if (RAW) pn.dsc = raw ? pn.depth * dact : pn.depth;
       const float yf = (float)r;
       const float rx = __fadd_rn(__fadd_rn(rxx, __fmul_rn(kk1, yf)), kk2);
       const float ry = __fadd_rn(__fadd_rn(ryx, __fmul_rn(kk4, yf)), kk5);
       const float rz = __fadd_rn(__fadd_rn(rzx, __fmul_rn(kk7, yf)), kk8);
-      const float X = __fmul_rn(pdepth, rx), Y = __fmul_rn(pdepth, ry), Z = __fmul_rn(pdepth, rz);
+      const float X = __fmul_rn(pn.depth, rx), Y = __fmul_rn(pn.depth, ry), Z = __fmul_rn(pn.depth, rz);
       float P[12];
       {
         const float4 a = sP[0], bb = sP[1], c = sP[2];
@@ -216,10 +216,10 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
       }
       PairFwd f;
       pair_project(P, X, Y, Z, geo, f, in_img);
-      pwa = f.wa; pwb = f.wb; pwc = f.wc; pwd = f.wd;
-      pq0 = f.q0; pq1 = f.q1; pq2 = f.q2; pr = f.r;
-      gather_taps(pp->img, geo, f, I);
-      load_dT(r + 1, dq[nx], Tq[nx]);
+      pn.wa = f.wa; pn.wb = f.wb; pn.wc = f.wc; pn.wd = f.wd;
+      pn.q0 = f.q0; pn.q1 = f.q1; pn.q2 = f.q2; pn.r = f.r;
+      gather_taps(pp->img, geo, f, pn.I);
+      if (decltype(LOAD_NEXT)::value) load_dT(r + 1, dq[nx], Tq[nx]);
       if (GRAD && (ACCUM || !first) && writer) {
         const int rf = r - 2;
         g_old = (col_own && rf >= t.y0 && rf < t.y1) ? ld_global(pp->gdisp + (unsigned)(rf * w + xx)) : 0.f;
@@ -234,8 +234,12 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
       }
     };
 
-    auto step = [&](auto PH, const int r) {
+    // step of row r: consumes pending row pend[PQ]; AHEAD = 1 refills row r+1 into it, 2 row r+2, 0 nothing
+    auto step = [&](auto PH, auto ST, auto PQ, auto AHEAD, const int r) {
       constexpr int cur = decltype(PH)::value, pv1 = (cur + 2) % 3, pv2 = (cur + 1) % 3;
+      constexpr int stages = decltype(ST)::value, ahead = decltype(AHEAD)::value;
+      Pend& pa = pend[decltype(PQ)::value];
+      const Taps& I = pa.I;
       const int rf = r - 2;
       const bool do_f = col_own && rf >= t.y0 && rf < t.y1;
       const float g_prev = g_old;
@@ -243,8 +247,8 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
       Rec& rc_ = rec[cur];
       {
         const float* T = Tq[cur];
-        const float w1 = __fmul_rn(pwa, pwc), w2 = __fmul_rn(pwb, pwc);
-        const float w3 = __fmul_rn(pwa, pwd), w4 = __fmul_rn(pwb, pwd);
+        const float w1 = __fmul_rn(pa.wa, pa.wc), w2 = __fmul_rn(pa.wb, pa.wc);
+        const float w3 = __fmul_rn(pa.wa, pa.wd), w4 = __fmul_rn(pa.wb, pa.wd);
         const float P0 = sfm_blend(w1, w2, w3, w4, I.a[0], I.b[0], I.c[0], I.d[0]);
         const float P1 = sfm_blend(w1, w2, w3, w4, I.a[1], I.b[1], I.c[1], I.d[1]);
         const float P2 = sfm_blend(w1, w2, w3, w4, I.a[2], I.b[2], I.c[2], I.d[2]);
@@ -257,12 +261,12 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
         if (GRAD) {
 #pragma unroll
           for (int c = 0; c < 3; ++c) {
-            rc_.Ix[c] = pwc * (I.b[c] - I.a[c]) + pwd * (I.d[c] - I.c[c]);
-            rc_.Iy[c] = pwa * (I.c[c] - I.a[c]) + pwb * (I.d[c] - I.b[c]);
+            rc_.Ix[c] = pa.wc * (I.b[c] - I.a[c]) + pa.wd * (I.d[c] - I.c[c]);
+            rc_.Iy[c] = pa.wa * (I.c[c] - I.a[c]) + pa.wb * (I.d[c] - I.b[c]);
           }
-          rc_.q0 = pq0; rc_.q1 = pq1; rc_.q2 = pq2; rc_.r = pr;
-          rc_.depth = pdepth;
-          rc_.dsc = RAW ? pdsc : pdepth;
+          rc_.q0 = pa.q0; rc_.q1 = pa.q1; rc_.q2 = pa.q2; rc_.r = pa.r;
+          rc_.depth = pa.depth;
+          rc_.dsc = RAW ? pa.dsc : pa.depth;
           if (SREC) {
             float* o = myrec + cur * 18 * 32;
 #pragma unroll
@@ -272,8 +276,8 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
               o[(6 + c) * 32] = rc_.P[c];
               o[(9 + c) * 32] = rc_.T[c];
             }
-            o[12 * 32] = pq0; o[13 * 32] = pq1; o[14 * 32] = pq2; o[15 * 32] = pr; o[16 * 32] = pdepth;
-            if (RAW) o[17 * 32] = pdsc;
+            o[12 * 32] = pa.q0; o[13 * 32] = pa.q1; o[14 * 32] = pa.q2; o[15 * 32] = pa.r; o[16 * 32] = pa.depth;
+            if (RAW) o[17 * 32] = pa.dsc;
           }
         }
         if (DEBUG && own && p.dbg_P[s]) {
@@ -283,8 +287,9 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
           o[2 * (size_t)plane] = P2;
         }
       }
-      // ---------------- refill for row r + 1: its gathers fly while stages B..F of this step run
-      refill(IC<pv2>{}, r + 1);          // slot of row r+1 in the 3-ring == (cur + 1) % 3
+      // ---------------- refill for row r + 1 (r + 2 in the head): its gathers fly while stages B..F of this step run
+      if constexpr (ahead == 1) refill(IC<pv2>{}, pa, r + 1, IC<1>{});     // ring slot of row r+1 == (cur + 1) % 3
+      if constexpr (ahead == 2) refill(IC<pv1>{}, pa, r + 2, IC<1>{});     // ring slot of row r+2 == (cur + 2) % 3
       // Basic-block fence.  The refill has no consumer before the next step, so ptxas' critical-path scheduler
       // otherwise sinks the projection and the four gathers to the end of the step (seen in the SASS; ncu:
       // half of all stall samples were long-scoreboard waits on the taps ~60 instructions after their issue).
@@ -301,6 +306,7 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
         h0[3] = (tl + tv) + tr;
         h0[4] = vfma(tr, tr, vfma(tv, tv, tl * tl));
       }
+      if constexpr (stages != ROW_AB) {
       // ---------------- stage C: SSIM at (rc = r-1, lane) from rows r-2, r-1, r
       const int rc = r - 1;
       V3 g0[3];
@@ -308,7 +314,7 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
         const V3* h0 = hs[cur];
         const V3* h1 = hs[pv1];
         const V3* h2 = hs[pv2];
-        const bool c_in = col_in && (rc >= 0) && (rc < h) && (r >= r_begin + 2);
+        const bool c_in = col_in && (rc >= 0) && (rc < h);
         const bool live_px = c_in && !mask[pv1];
         const bool own_c = col_own && (rc >= t.y0) && (rc < t.y1);
         const float lw = (live_px && own_c) ? 1.f : 0.f;
@@ -350,6 +356,7 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
         V3* gh0 = gs[cur];
 #pragma unroll
         for (int q = 0; q < 3; ++q) gh0[q] = (vshfl_up(g0[q]) + g0[q]) + vshfl_down(g0[q]);
+        if constexpr (stages != ROW_ABCD) {
         // ---------------- stages E + F: dL/dP and the warp backward for pixel (rf = r-2, lane)
         const V3* g1 = gs[pv1];
         const V3* g2 = gs[pv2];
@@ -404,20 +411,53 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
           if (wi == 0) gval = gval - slot[0] * slot[32];
         }
         if (do_f && writer) st_global(gp, gval);
+        }  // E + F
       }
-      }
+      }  // C + D
+      }  // opaque_true
     };
 
-    // prologue: rows r_begin (slot 0) and its lookahead
+    // r_end - r_begin = h + 4 >= 5 steps: the four head steps, then groups of three (ring rotation = renaming) that
+    // leave the loop right after the step of row r_end - 1.  The exits sit inside the loop: a peeled tail after it
+    // (straight-line copies of the step) pushed the shared-memory-record instances past 168 registers.  The stage sets
+    // depend only on the step, so both warps of an NW = 2 CTA meet the per-row barrier of stage F on the same steps.
+    // The head's steps are short, so with one row of gathers in flight each of them waits a whole memory latency.  In
+    // the register-record instances (grids resident at once: every warp is in its head at the same time) the head
+    // keeps two pending rows: rows r_begin and r_begin+1 are gathered together, the head steps refill two rows ahead
+    // and the last one refills nothing, which hands the loop one pending row, pend[0] (cfg2: 25.2 -> 24.7 us).  The
+    // shared-memory-record instances run many waves, where other warps cover the head; there the second pending row
+    // cost 2 % more instructions in the loop (ptxas' allocation) and local-memory spills in the DEBUG instances.
     load_dT(r_begin, dq[0], Tq[0]);
-    refill(IC<0>{}, r_begin);
-    // the row loop always runs whole groups of three steps (ring rotation = renaming); rows past r_end are
-    // out of range everywhere (loads predicated off, nothing owned)
+    if constexpr (!SREC) {
+      load_dT(r_begin + 1, dq[1], Tq[1]);
+      refill(IC<0>{}, pend[0], r_begin, IC<0>{});
+      refill(IC<1>{}, pend[1], r_begin + 1, IC<1>{});
+      step(IC<0>{}, IC<ROW_AB>{}, IC<0>{}, IC<2>{}, r_begin);
+      step(IC<1>{}, IC<ROW_AB>{}, IC<1>{}, IC<2>{}, r_begin + 1);
+      step(IC<2>{}, IC<ROW_ABCD>{}, IC<0>{}, IC<2>{}, r_begin + 2);
+      step(IC<0>{}, IC<ROW_ABCD>{}, IC<1>{}, IC<0>{}, r_begin + 3);
+    } else {
+      refill(IC<0>{}, pend[0], r_begin, IC<1>{});
+      step(IC<0>{}, IC<ROW_AB>{}, IC<0>{}, IC<1>{}, r_begin);
+      step(IC<1>{}, IC<ROW_AB>{}, IC<0>{}, IC<1>{}, r_begin + 1);
+      step(IC<2>{}, IC<ROW_ABCD>{}, IC<0>{}, IC<1>{}, r_begin + 2);
+      step(IC<0>{}, IC<ROW_ABCD>{}, IC<0>{}, IC<1>{}, r_begin + 3);
+    }
 #pragma unroll 1
-    for (int r = r_begin; r < r_end; r += 3) {
-      step(IC<0>{}, r);
-      step(IC<1>{}, r + 1);
-      step(IC<2>{}, r + 2);
+    for (int r = r_begin + 4;; r += 3) {
+      step(IC<1>{}, IC<ROW_ALL>{}, IC<0>{}, IC<1>{}, r);
+      if (r + 1 >= r_end) break;
+      step(IC<2>{}, IC<ROW_ALL>{}, IC<0>{}, IC<1>{}, r + 1);
+      if (r + 2 >= r_end) break;
+      step(IC<0>{}, IC<ROW_ALL>{}, IC<0>{}, IC<1>{}, r + 2);
+      if (r + 3 >= r_end) break;
+    }
+    // The taps of the last refill are dead once the loop is left, so ptxas sinks every step's gathers past the
+    // fence and the exit test into the next step, right in front of their use (the whole gather latency exposed
+    // per row: 10 % / 17 % slower at cfg2 / cfg5).  A use it cannot rule out keeps them live on the way out.
+    if (!opaque_true) {
+#pragma unroll
+      for (int c = 0; c < 3; ++c) pix_part += ((pend[0].I.a[c] + pend[0].I.b[c]) + pend[0].I.c[c]) + pend[0].I.d[c];
     }
     // ---- flush: expand (A, B, C) to dL/dP = sum gq (x) (X, Y, Z, 1) with X = depth*((k0 x + k2) + k1 y) ...
     const bool last = (NW > 1) || (i == S - 1);
