@@ -49,6 +49,9 @@ extern "C" {
 #define SFM_FLAG_EDGE_AWARE_SMOOTH 0x8u /* the smoothness term is compute_disp_smooth(curr_tgt_img, pred_disps[ns])
                                          (base_model.py:144-155), the edge-aware alternative the reference keeps
                                          commented out at its call site (:78-80), instead of compute_smooth_loss */
+#define SFM_FLAG_IMAGE_GRADS 0x10u    /* the workspace also holds fp32 gradient levels of the pyramid (scales >= 1) for
+                                         sfm_loss_forward_backward_images; every other entry point accepts the flag and
+                                         behaves exactly as without it */
 
 /*
  * Problem descriptor.  Mirrors the reference's model flags (base_model.py:37-39:
@@ -112,6 +115,13 @@ typedef struct SfmGrads {
   float* glogits[SFM_MAX_SCALES];
 } SfmGrads;
 
+/* Gradients w.r.t. the two images (sfm_loss_forward_backward_images), same shapes as SfmInputs.tgt / .src:
+ *   gtgt (B,3,H,W), gsrc (B,S,3,H,W).  Either may be NULL (that gradient is not computed), not both. */
+typedef struct SfmImageGrads {
+  float* gtgt;
+  float* gsrc;
+} SfmImageGrads;
+
 /* Optional per-(scale, source) dumps of the warp for stage-level parity tests (may be NULL):
  *   P[s]   (B,S,3,h,w) f32  warped image            (transform.py:189)
  *   u0[s]  (B,S,h,w)   i32  floor(u), v0 likewise   (integer work: must be bit-exact)
@@ -127,7 +137,7 @@ int sfm_version(void);
 const char* sfm_last_error(void);
 
 /* Bytes of device scratch a call needs (image pyramid of the scales >= 1, planar like the inputs; projection
- * tables; fp64 reduction cells).  The caller allocates it (any 256-byte aligned device pointer) and passes it to
+ * tables; fp64 reduction cells; with SFM_FLAG_IMAGE_GRADS also the fp32 gradient levels of the pyramid).  The caller allocates it (any 256-byte aligned device pointer) and passes it to
  * every call with the same descriptor.  Scale 0 is read straight from in->tgt / in->src. */
 size_t sfm_workspace_bytes(const SfmDesc* desc);
 
@@ -153,6 +163,21 @@ int sfm_loss_forward_backward(const SfmDesc* desc, const SfmInputs* in, float* l
 
 /* grads *= *gy (device scalar).  No-op on the device when *gy == 1. */
 int sfm_scale_grads(const SfmDesc* desc, const float* gy, const SfmGrads* grads, void* stream);
+
+/* sfm_loss_forward_backward plus the gradients of the reported total (losses_out[0]) w.r.t. the images, for callers
+ * whose images come out of a differentiable module.  The images are treated as differentiable throughout: the
+ * reference's `.data` on the pyramid (base_model.py:71-72) and on mu_y / sigma_y (:131,:134) are lifted, so igrads is
+ * the derivative of the reported value.  The all-zero mask (:96) is piecewise constant and has derivative 0.
+ * desc->flags must contain SFM_FLAG_IMAGE_GRADS (else SFM_E_INVALID_DESC; the workspace is sized with it); with
+ * SFM_FLAG_EDGE_AWARE_SMOOTH it returns SFM_E_UNSUPPORTED (that term depends on the target image).  Losses, gdisps
+ * and glogits are bitwise those of sfm_loss_forward_backward.  gtgt is bitwise reproducible from run to run; gsrc
+ * is accumulated with fp32 atomics and its last bits vary with their order.  Under snippet sharding (B_global > B)
+ * a shard's image gradients are final. */
+int sfm_loss_forward_backward_images(const SfmDesc* desc, const SfmInputs* in, float* losses_out, const SfmGrads* grads,
+                                     const SfmImageGrads* igrads, void* workspace, void* stream);
+
+/* igrads *= *gy (device scalar), the NULL members skipped.  No-op on the device when *gy == 1. */
+int sfm_scale_image_grads(const SfmDesc* desc, const float* gy, const SfmImageGrads* igrads, void* stream);
 
 /* Profiling hook (bench.py's roofline measurement): while set (non-NULL cudaEvent_t handles), every
  * sfm_loss_* call on this thread records `start` right before and `stop` right after the fused loss

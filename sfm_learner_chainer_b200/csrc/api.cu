@@ -165,7 +165,8 @@ int num_sms() {
 }
 
 int run_loss(const SfmDesc* d, const SfmInputs* in, float* losses_out, const SfmGrads* grads, const float* gy,
-             const SfmDebug* dbg, void* workspace, cudaStream_t st, const SfmPeerDev* peer = nullptr) {
+             const SfmDebug* dbg, void* workspace, cudaStream_t st, const SfmPeerDev* peer = nullptr,
+             const SfmImageGrads* ig = nullptr) {
   int rc = sfm_validate_desc(d);
   if (rc) return rc;
   const bool reuse = (d->flags & SFM_FLAG_REUSE_PYRAMID) != 0;
@@ -186,6 +187,7 @@ int run_loss(const SfmDesc* d, const SfmInputs* in, float* losses_out, const Sfm
   if (m.use_smooth) mode |= SFM_MODE_SMOOTH;
   if (grads) mode |= SFM_MODE_GRAD;
   if (dbg) mode |= SFM_MODE_DEBUG;
+  if (ig) mode |= SFM_MODE_IMG;
   const SfmStepPlan plan = sfm_plan_step(d, mode, num_sms());
   SfmWsLayout L;
   sfm_ws_layout(d, &L);
@@ -219,6 +221,10 @@ int run_loss(const SfmDesc* d, const SfmInputs* in, float* losses_out, const Sfm
     if (dbg) {
       p.dbg_P[s] = dbg->P[s]; p.dbg_u0[s] = dbg->u0[s]; p.dbg_v0[s] = dbg->v0[s]; p.dbg_inb[s] = dbg->inb[s];
     }
+    if (ig) {
+      p.gtgt[s] = !ig->gtgt ? nullptr : s == 0 ? ig->gtgt : (float*)(ws + L.off_gtgt[s]);
+      p.gsrc[s] = !ig->gsrc ? nullptr : s == 0 ? ig->gsrc : (float*)(ws + L.off_gsrc[s]);
+    }
   }
   const bool tables = (d->flags & SFM_FLAG_TABLES_PROVIDED) != 0;
   p.proj = tables ? in->proj : (const float*)(ws + L.off_proj);
@@ -248,6 +254,11 @@ int run_loss(const SfmDesc* d, const SfmInputs* in, float* losses_out, const Sfm
   SfmPrepParams pp = prep_params(d, plan.band, ws, reuse ? nullptr : in->tgt, in->src, in->intrinsics, in->poses,
                                  tables ? nullptr : (float*)(ws + L.off_proj), (float*)(ws + L.off_kinv), true);
   pp.n_mix_region = plan.n_mix_region;
+  if (ig && ig->gsrc) {
+    // the march accumulates the source gradients with reductions: scale 0 and the workspace levels start at 0
+    SFM_CUDA_CHECK(cudaMemsetAsync(ig->gsrc, 0, (size_t)d->B * d->S * 3 * d->H * d->W * sizeof(float), st));
+    if (L.gsrc_bytes) SFM_CUDA_CHECK(cudaMemsetAsync(ws + L.off_gsrc[1], 0, L.gsrc_bytes, st));
+  }
   rc = sfm_launch_prep(pp, &sm, grads ? 2 : 1, st);
   if (rc) return rc;
   return sfm_launch_fused(p, plan, st);
@@ -282,6 +293,36 @@ extern "C" int sfm_loss_forward_backward_peer(const SfmDesc* desc, const SfmInpu
   const SfmPeerDev* dev = sfm_peer_dev(peer);
   if (!dev) { sfm_set_error("sfm_loss_forward_backward_peer: the peer object is not connected (sfm_peer_connect)"); return SFM_E_UNSUPPORTED; }
   return run_loss(desc, in, losses_out, grads, nullptr, nullptr, workspace, (cudaStream_t)stream, dev);
+}
+
+extern "C" int sfm_loss_forward_backward_images(const SfmDesc* desc, const SfmInputs* in, float* losses_out,
+                                                const SfmGrads* grads, const SfmImageGrads* igrads, void* workspace,
+                                                void* stream) {
+  int rc = sfm_validate_desc(desc);
+  if (rc) return rc;
+  if (!(desc->flags & SFM_FLAG_IMAGE_GRADS)) {
+    sfm_set_error("sfm_loss_forward_backward_images: desc->flags lacks SFM_FLAG_IMAGE_GRADS (the workspace must be sized with it)");
+    return SFM_E_INVALID_DESC;
+  }
+  if (desc->flags & SFM_FLAG_EDGE_AWARE_SMOOTH) {
+    sfm_set_error("unsupported: image gradients through the edge-aware smoothness term (SFM_FLAG_EDGE_AWARE_SMOOTH)");
+    return SFM_E_UNSUPPORTED;
+  }
+  if (!igrads || (!igrads->gtgt && !igrads->gsrc)) { sfm_set_error("igrads is NULL or has neither gtgt nor gsrc"); return SFM_E_NULL_POINTER; }
+  if (!losses_out) { sfm_set_error("losses_out is NULL"); return SFM_E_NULL_POINTER; }
+  if (!grads) { sfm_set_error("grads is NULL"); return SFM_E_NULL_POINTER; }
+  return run_loss(desc, in, losses_out, grads, nullptr, nullptr, workspace, (cudaStream_t)stream, nullptr, igrads);
+}
+
+extern "C" int sfm_scale_image_grads(const SfmDesc* desc, const float* gy, const SfmImageGrads* igrads, void* stream) {
+  int rc = sfm_validate_desc(desc);
+  if (rc) return rc;
+  if (!gy) { sfm_set_error("gy is NULL"); return SFM_E_NULL_POINTER; }
+  if (!igrads || (!igrads->gtgt && !igrads->gsrc)) { sfm_set_error("igrads is NULL or has neither gtgt nor gsrc"); return SFM_E_NULL_POINTER; }
+  const long long img = 3ll * desc->H * desc->W;
+  float* ptrs[2] = {igrads->gtgt, igrads->gsrc};
+  const long long counts[2] = {desc->B * img, (long long)desc->B * desc->S * img};
+  return sfm_launch_scale(ptrs, counts, 2, gy, (cudaStream_t)stream);
 }
 
 extern "C" int sfm_scale_grads(const SfmDesc* desc, const float* gy, const SfmGrads* grads, void* stream) {

@@ -40,6 +40,11 @@ struct SfmWsLayout {
   size_t off_acc;                  // double [4 + B*S*ns*12] loss sums (pixel, smooth, exp, ssim) + dL/dP per scale
   size_t off_posevec;              // float  [B][S][6]   6-DoF vectors reduced from the raw `poseout` map (raw_pose_hw > 0)
   size_t off_smpart;               // float  [tasks / 8] loss partials of the smoothness CTAs of the prologue kernel
+  // SFM_FLAG_IMAGE_GRADS: fp32 gradient levels of the pyramid (scales >= 1), sized like it: all source levels back to
+  // back (one memset clears them), then the target levels.  0 without the flag.
+  size_t off_gsrc[SFM_MAX_SCALES];  // float [B*S][3][h][w]
+  size_t off_gtgt[SFM_MAX_SCALES];  // float [B][3][h][w]
+  size_t gsrc_bytes;                // span of the source levels
   size_t acc_doubles;
   size_t total;
 };
@@ -97,6 +102,20 @@ static inline void sfm_ws_layout(const SfmDesc* d, SfmWsLayout* L) {
   off = sfm_align_up(off + (size_t)d->B * d->S * 6 * sizeof(float), 256);
   L->off_smpart = off;
   off = sfm_align_up(off + (size_t)((sfm_smooth_plan(d->B, d->n_scales, d->H, d->W, nullptr) + 7) / 8) * sizeof(float), 256);
+  for (int s = 0; s < SFM_MAX_SCALES; ++s) L->off_gsrc[s] = L->off_gtgt[s] = 0;
+  L->gsrc_bytes = 0;
+  if (d->flags & SFM_FLAG_IMAGE_GRADS) {
+    const size_t g0 = off;
+    for (int s = 1; s < d->n_scales; ++s) {
+      L->off_gsrc[s] = off;
+      off = sfm_align_up(off + (size_t)d->B * d->S * 3 * (d->H >> s) * (d->W >> s) * sizeof(float), 256);
+    }
+    L->gsrc_bytes = off - g0;
+    for (int s = 1; s < d->n_scales; ++s) {
+      L->off_gtgt[s] = off;
+      off = sfm_align_up(off + (size_t)d->B * 3 * (d->H >> s) * (d->W >> s) * sizeof(float), 256);
+    }
+  }
   L->total = off;
 }
 

@@ -120,6 +120,11 @@ struct SfmFusedParams {
   int32_t* dbg_u0[SFM_MAX_SCALES];
   int32_t* dbg_v0[SFM_MAX_SCALES];
   uint8_t* dbg_inb[SFM_MAX_SCALES];
+  // image gradients (sfm_loss_forward_backward_images; nullptr when not wanted): scale 0 = the caller's buffers, scales
+  // >= 1 = the gradient levels in the workspace, pulled back into scale 0 by sfm_launch_image_pullback.  gsrc is
+  // zeroed before the step and accumulated with fp32 reductions; gtgt is owned like gdisp (stored by the first pass).
+  float* gtgt[SFM_MAX_SCALES];      // [B][3][h][w]
+  float* gsrc[SFM_MAX_SCALES];      // [B*S][3][h][w]
 };
 
 // Launch helper: with pdl the kernel is a programmatic dependent launch on the previous kernel of the stream (its
@@ -147,12 +152,16 @@ const SfmPeerDev* sfm_peer_dev(const SfmPeer* q);      // comm.cu; nullptr until
 // counts with: forward records in shared memory (168 registers) / in registers (250 registers).
 constexpr int SFM_SSIM_MIN_WARPS = 12;
 constexpr int SFM_SSIM_REG_MIN_WARPS = 8;
+// image-gradient instances: with the bound of 12 the extra gradient field spilled; with 10 ptxas allocates 168 registers
+// without spilling, so 12 warps per SM are still resident and the cost model stays as it is
+constexpr int SFM_SSIM_IMG_MIN_WARPS = 10;
 
 // Launch plan of one fused step (plan.cu, the whole launch policy).  The marching kernel instance is
-// sfm_l1_march_kernel<exp, grad, accum, debug, raw> or sfm_ssim_march_kernel<grad, accum, debug, raw, nw, srec>.
+// sfm_l1_march_kernel<exp, grad, accum, debug, raw, img> or sfm_ssim_march_kernel<grad, accum, debug, raw, nw, srec, img>.
 struct SfmStepPlan {
   bool ssim;                           // kernel family
   bool exp, grad, accum, debug, raw;   // accum: a smoothness kernel has initialised gdisp
+  bool img;                            // image gradients (grad, !debug; SSIM: nw = 1 with shared-memory records)
   int nw;                              // SSIM: warps per CTA (2: the two sources split over the warps of a CTA)
   bool srec;                           // SSIM: forward records in shared memory (false: in registers)
   bool edge_smooth;                    // the edge-aware smoothness kernel runs between the prologue and the march
@@ -161,7 +170,7 @@ struct SfmStepPlan {
   int band, n_mix_region;              // SfmPrepParams
 };
 // mode bits of the planner
-enum { SFM_MODE_EXP = 1, SFM_MODE_SSIM = 2, SFM_MODE_GRAD = 4, SFM_MODE_DEBUG = 8, SFM_MODE_SMOOTH = 16 };
+enum { SFM_MODE_EXP = 1, SFM_MODE_SSIM = 2, SFM_MODE_GRAD = 4, SFM_MODE_DEBUG = 8, SFM_MODE_SMOOTH = 16, SFM_MODE_IMG = 32 };
 SfmStepPlan sfm_plan_step(const SfmDesc* d, int mode, int num_sms);
 int sfm_plan_band(const SfmDesc* d);
 int sfm_launch_fused(SfmFusedParams& p, const SfmStepPlan& plan, cudaStream_t stream);
@@ -169,3 +178,6 @@ int sfm_launch_edge_smooth(const SfmFusedParams& p, bool grad, cudaStream_t stre
 extern thread_local cudaEvent_t sfm_ev_start, sfm_ev_stop;   // profiling hook (sfm_set_kernel_events)
 
 int sfm_launch_scale(float* const* ptrs, const long long* counts, int n, const float* gy, cudaStream_t stream);
+// adds the gradient levels p.gtgt[s] / p.gsrc[s] (s >= 1) into the full-resolution p.gtgt[0] / p.gsrc[0] through the
+// adjoint of the pyramid (fused_loss.cu); a dependent launch behind the epilogue
+int sfm_launch_image_pullback(const SfmFusedParams& p, int H, int W, cudaStream_t stream);

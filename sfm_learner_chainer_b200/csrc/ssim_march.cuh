@@ -94,9 +94,17 @@ enum RowStages {
 // 168 registers, 3 warps per scheduler) -- the throughput form for grids of several waves.  false: registers (250
 // registers, 2 warps per scheduler, 6 % fewer instructions and a third fewer L1 data-pipe wavefronts) -- faster whenever
 // the whole grid is resident at once anyway (cfg2: 29.3 -> 26.6 us), slower when occupancy counts (cfg5: 933 -> 952 us).
-template <bool GRAD, bool ACCUM, bool DEBUG, bool RAW, int NW, bool SREC = true>
-__global__ void __launch_bounds__(32 * NW, (SREC ? SFM_SSIM_MIN_WARPS : SFM_SSIM_REG_MIN_WARPS) / NW)
+// IMG (GRAD, NW == 1, SREC only): also the image gradients.  With h_a = (dL/dSt) / 2 -- the mirror image of g_a -- and
+// (dL/dStt) / 9 == g_s (d2 holds Spp and Stt with the same factor), dL/dT = 2 A(h_a) + 18 T A(g_s) + 18 P A(g_c) + the
+// L1 part: one more gradient field in the ring.  The task owns gtgt like gdisp (stored by the first source, then
+// accumulated); dL/dP is scattered to the four taps of every in-view pixel with fp32 reductions, from the tap index
+// and the two fractions the forward record carries in three more fields.
+template <bool GRAD, bool ACCUM, bool DEBUG, bool RAW, int NW, bool SREC = true, bool IMG = false>
+__global__ void __launch_bounds__(32 * NW, (IMG ? SFM_SSIM_IMG_MIN_WARPS : SREC ? SFM_SSIM_MIN_WARPS : SFM_SSIM_REG_MIN_WARPS) / NW)
 sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
+  static_assert(!IMG || (GRAD && NW == 1 && SREC), "image gradients: GRAD, one warp per CTA, shared-memory records");
+  constexpr int NREC = IMG ? 21 : 18;                   // fields of a forward record
+  constexpr int NG = IMG ? 4 : 3;                       // gradient fields: g_a, g_s, g_c (, h_a)
   __shared__ float4 sP_all[NW][3];
   __shared__ float sG[(NW > 1) ? 3 * 2 * 32 : 1];       // [ring slot][gdd | dsc][lane] of warp 1's row term
   const int wi = (NW > 1) ? (int)(threadIdx.x >> 5) : 0;
@@ -114,9 +122,11 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
   // two-row delay line of forward records: [slot][field][lane], written in stage A of row r and read back by
   // the same lane in stages E/F two steps later (no synchronisation needed).  In registers these 51 values
   // pushed the kernel over its 168-register budget (17-27 local-memory spills per three rows).
-  __shared__ float sRec[(GRAD && SREC) ? NW * 3 * 18 * 32 : 1];
+  __shared__ float sRec[(GRAD && SREC) ? NW * 3 * NREC * 32 : 1];
+  // IMG: gtgt of the snippet, gsrc of the pass's source (scale s), re-read like s_ptrs
+  __shared__ float* s_img_ptrs[2];
   const int lane = threadIdx.x & 31;
-  float* const myrec = sRec + wi * (3 * 18 * 32) + lane;
+  float* const myrec = sRec + wi * (3 * NREC * 32) + lane;
   const StripTask t = decode_strip(p, blockIdx.x);
   const int s = t.s, b = t.b, h = p.h[s], w = p.w[s], S = p.S;
   const Geo geo = make_geo(p, s);
@@ -163,11 +173,15 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
       s_ptrs_all[wi].tgt = tgt;
       s_ptrs_all[wi].disp = disp;
       s_ptrs_all[wi].gdisp = gdisp;
+      if (IMG) {
+        s_img_ptrs[0] = p.gtgt[s] ? p.gtgt[s] + (size_t)b * 3 * plane : nullptr;
+        s_img_ptrs[1] = p.gsrc[s] ? p.gsrc[s] + ((size_t)b * S + i) * src_img : nullptr;
+      }
     }
     __syncwarp();
     // rings: window row sums (P, P^2, P.T, T, T^2 per channel), gradient-field row sums, forward records.  No
     // initial value: with the stage schedule of RowStages every slot is written before a step reads it.
-    V3 hs[3][5], gs[3][3];        // [ring slot][field]: (P, P^2, P.T, T, T^2) and (g_a, g_s, g_c) row sums, three channels each
+    V3 hs[3][5], gs[3][NG];       // [ring slot][field]: (P, P^2, P.T, T, T^2) and (g_a, g_s, g_c (, h_a)) row sums, three channels each
     Rec rec[3];
     bool mask[3];                                        // all-zero mask of the row's pixel (base_model.py:96)
     float dq[3] = {1.f, 1.f, 1.f};                       // disparity / target rows fetched ahead
@@ -189,6 +203,7 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
     struct Pend {
       Taps I;
       float wa, wb, wc, wd, q0, q1, q2, r, depth, dsc;
+      unsigned idx;                                      // IMG: tap (v0, u0)
     };
     Pend pend[2];
     float g_old = 0.f;
@@ -218,6 +233,7 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
       pair_project(P, X, Y, Z, geo, f, in_img);
       pn.wa = f.wa; pn.wb = f.wb; pn.wc = f.wc; pn.wd = f.wd;
       pn.q0 = f.q0; pn.q1 = f.q1; pn.q2 = f.q2; pn.r = f.r;
+      if (IMG) pn.idx = f.idx;
       gather_taps(pp->img, geo, f, pn.I);
       if (decltype(LOAD_NEXT)::value) load_dT(r + 1, dq[nx], Tq[nx]);
       if (GRAD && (ACCUM || !first) && writer) {
@@ -268,7 +284,7 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
           rc_.depth = pa.depth;
           rc_.dsc = RAW ? pa.dsc : pa.depth;
           if (SREC) {
-            float* o = myrec + cur * 18 * 32;
+            float* o = myrec + cur * NREC * 32;
 #pragma unroll
             for (int c = 0; c < 3; ++c) {
               o[(0 + c) * 32] = rc_.Ix[c];
@@ -278,6 +294,7 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
             }
             o[12 * 32] = pa.q0; o[13 * 32] = pa.q1; o[14 * 32] = pa.q2; o[15 * 32] = pa.r; o[16 * 32] = pa.depth;
             if (RAW) o[17 * 32] = pa.dsc;
+            if (IMG) { o[18 * 32] = __uint_as_float(pa.idx); o[19 * 32] = pa.wb; o[20 * 32] = pa.wd; }
           }
         }
         if (DEBUG && own && p.dbg_P[s]) {
@@ -309,7 +326,7 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
       if constexpr (stages != ROW_AB) {
       // ---------------- stage C: SSIM at (rc = r-1, lane) from rows r-2, r-1, r
       const int rc = r - 1;
-      V3 g0[3];
+      V3 g0[NG];
       {
         const V3* h0 = hs[cur];
         const V3* h1 = hs[pv1];
@@ -349,20 +366,21 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
           g0[0] = vfma(g_n * St, n2 + vneg(n1), (g_d * Sp) * (d2v + vneg(d1v)));   // (dL/dSp) / 2
           g0[1] = g_d * d1v;                                                       // (dL/dSpp) / 9
           g0[2] = g_n * n1;                                                        // (dL/dSpt) / 18
+          if constexpr (IMG) g0[3] = vfma(g_n * Sp, n2 + vneg(n1), (g_d * St) * (d2v + vneg(d1v)));  // (dL/dSt) / 2
         }
       }
       if (GRAD) {
         // ---------------- stage D: row sums of the three gradient fields of row rc
         V3* gh0 = gs[cur];
 #pragma unroll
-        for (int q = 0; q < 3; ++q) gh0[q] = (vshfl_up(g0[q]) + g0[q]) + vshfl_down(g0[q]);
+        for (int q = 0; q < NG; ++q) gh0[q] = (vshfl_up(g0[q]) + g0[q]) + vshfl_down(g0[q]);
         if constexpr (stages != ROW_ABCD) {
         // ---------------- stages E + F: dL/dP and the warp backward for pixel (rf = r-2, lane)
         const V3* g1 = gs[pv1];
         const V3* g2 = gs[pv2];
         Rec rb = rec[pv2];
         if (SREC) {
-          const float* o = myrec + pv2 * 18 * 32;
+          const float* o = myrec + pv2 * NREC * 32;
 #pragma unroll
           for (int c = 0; c < 3; ++c) {
             rb.Ix[c] = o[(0 + c) * 32];
@@ -374,7 +392,7 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
           rb.dsc = RAW ? o[17 * 32] : rb.depth;
         }
         const bool mf = mask[pv2];
-        float gP[3];
+        float gP[3], gT[3];
         {
           const V3 Aa = (g2[0] + g1[0]) + gh0[0];
           const V3 As = (g2[1] + g1[1]) + gh0[1];
@@ -384,10 +402,47 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
           const V3 Pb = v3(rb.P[0], rb.P[1], rb.P[2]), Tb = v3(rb.T[0], rb.T[1], rb.T[2]);
           const V3 gsv = vfma(v3s(18.f), vfma(Tb, Ac, Pb * As), v3s(2.f) * Aa);
           const float gs3[3] = {gsv.a.x, gsv.a.y, gsv.b};
+          float gt3[3] = {0.f, 0.f, 0.f};
+          if constexpr (IMG) {
+            // dL/dT = 2 A(h_a) + 18 T As + 18 P Ac
+            const V3 Ah = (g2[3] + g1[3]) + gh0[3];
+            const V3 gtv = vfma(v3s(18.f), vfma(Pb, Ac, Tb * As), v3s(2.f) * Ah);
+            gt3[0] = gtv.a.x; gt3[1] = gtv.a.y; gt3[2] = gtv.b;
+          }
 #pragma unroll
           for (int c = 0; c < 3; ++c) {
             const float gl1 = mf ? 0.f : sfm_sign_times(rb.P[c] - rb.T[c], wpix);
             gP[c] = do_f ? gs3[c] + gl1 : 0.f;
+            if (IMG) gT[c] = do_f ? gt3[c] - gl1 : 0.f;
+          }
+        }
+        if (IMG && do_f) {
+          float* const volatile* ip = s_img_ptrs;
+          float* gt = ip[0];
+          float* gsrc = ip[1];
+          if (gt) {
+            float* q = gt + (unsigned)(rf * w + xx);
+            if (first) {
+              q[0] = gT[0]; q[geo.plane] = gT[1]; q[2u * geo.plane] = gT[2];
+            } else {
+              q[0] += gT[0]; q[geo.plane] += gT[1]; q[2u * geo.plane] += gT[2];
+            }
+          }
+          if (gsrc && rb.r != 0.f) {
+            // in view: wa = 1 - wb and wc = 1 - wd exactly (wb = u - u0 is exact, and so is the difference)
+            const float* o = myrec + pv2 * NREC * 32;
+            const unsigned idx = __float_as_uint(o[18 * 32]);
+            const float wb = o[19 * 32], wd = o[20 * 32];
+            const float wa = __fsub_rn(1.f, wb), wc = __fsub_rn(1.f, wd);
+            const float w1 = __fmul_rn(wa, wc), w2 = __fmul_rn(wb, wc), w3 = __fmul_rn(wa, wd), w4 = __fmul_rn(wb, wd);
+#pragma unroll
+            for (int c = 0; c < 3; ++c) {
+              float* qc = gsrc + (idx + (unsigned)c * geo.plane);
+              atomicAdd(qc, gP[c] * w1);
+              atomicAdd(qc + 1, gP[c] * w2);
+              atomicAdd(qc + w, gP[c] * w3);
+              atomicAdd(qc + w + 1, gP[c] * w4);
+            }
           }
         }
         // sampler + projection backward (SURVEY A.6); out-of-view pixels have Ix = Iy = 0 and r = 0

@@ -23,10 +23,15 @@ class ViewSynthesisLoss(object):
     kernels then apply disp = 10 * sigmoid(x) + 0.01 (models/disp_net.py:104) and return the gradient
     w.r.t. that map.  raw_pose: `poses` is PoseNet's `poseout` map (B, 6*S, h', w') and the kernels apply
     0.01 * mean over (h', w') (models/pose_net.py:52-53); `gposes` then has the map's shape.
+    image_grads: forward_backward also returns gtgt (B,3,H,W) and gsrc (B,S,3,H,W), the gradients of the reported
+    total w.r.t. the two images (for images that come out of a differentiable module); not with edge_aware_smooth.
     """
 
     def __init__(self, smooth_reg=0.0, exp_reg=0.0, ssim_rate=0.0, n_scales=N_SCALES, B_global=None,
-                 raw_disp_scales=0, raw_pose=False, edge_aware_smooth=False):
+                 raw_disp_scales=0, raw_pose=False, edge_aware_smooth=False, image_grads=False):
+        if image_grads and edge_aware_smooth:
+            raise ValueError('image_grads is not supported together with edge_aware_smooth')
+        self.image_grads = bool(image_grads)
         # edge_aware_smooth: smoothness term = compute_disp_smooth (base_model.py:144-155, commented out at :78-80)
         self.edge_aware_smooth = bool(edge_aware_smooth)
         self.raw_disp_scales = int(raw_disp_scales)
@@ -49,11 +54,14 @@ class ViewSynthesisLoss(object):
     def _desc(self, B, S, H, W, flags=0, raw_pose_hw=0):
         if self.edge_aware_smooth:
             flags |= L.SFM_FLAG_EDGE_AWARE_SMOOTH
+        if self.image_grads:
+            flags |= L.SFM_FLAG_IMAGE_GRADS
         return L.SfmDesc(B, S, H, W, self.n_scales, int(self.B_global or 0), self.smooth_reg, self.exp_reg,
                          self.ssim_rate, flags, self.raw_disp_scales, raw_pose_hw)
 
     def _workspace(self, desc, like):
-        key = (desc.B, desc.S, desc.H, desc.W, desc.n_scales, str(getattr(like, 'device', '')))
+        # the image-gradient flag sizes the workspace; the per-call flags (tables, reused pyramid) do not
+        key = (desc.B, desc.S, desc.H, desc.W, desc.n_scales, desc.flags & L.SFM_FLAG_IMAGE_GRADS, str(getattr(like, 'device', '')))
         ws = self._ws.get(key)
         if ws is None:
             n = self._lib.sfm_workspace_bytes(C.byref(desc))
@@ -167,18 +175,32 @@ class ViewSynthesisLoss(object):
         self._ev_pyramid = D.record_event(tgt)
 
     def forward_backward(self, tgt, src, intrinsics, disps, poses, logits=None, proj=None, kinv=None, reuse_pyramid=False,
-                         peer=None):
+                         peer=None, image_grads=('tgt', 'src')):
         """Single fused pass: -> (losses (5,), dict(gdisps, gposes, glogits)) for upstream gradient 1.
         reuse_pyramid: the workspace already holds this batch's pyramid (build_pyramid).
         peer: a distributed.PeerLossSum -- the batch is sharded by snippet over several GPUs (B_global set) and the
-        epilogue kernel completes the five losses across the ranks over NVLink peer memory."""
+        epilogue kernel completes the five losses across the ranks over NVLink peer memory.
+        With the operator's image_grads the dict also holds gtgt and gsrc (None for an image left out of
+        `image_grads`, a subset of ('tgt', 'src'); an empty one runs the plain pass); not with peer."""
         desc, inp = self._pack(tgt, src, intrinsics, disps, poses, logits, proj, kinv)
         if reuse_pyramid:
             desc.flags |= L.SFM_FLAG_REUSE_PYRAMID
             D.wait_event(tgt, self._ev_pyramid)     # build_pyramid may have run on another stream
         g, out = self._alloc_grads(desc, tgt)
         losses = D.empty(tgt, (5,))
-        if peer is not None:
+        want = set(image_grads) if self.image_grads else set()
+        if want:
+            if peer is not None:
+                raise ValueError('image_grads is not supported with peer')
+            if not want <= {'tgt', 'src'}:
+                raise ValueError("image_grads must be a subset of ('tgt', 'src')")
+            out['gtgt'] = D.empty(tgt, (desc.B, 3, desc.H, desc.W)) if 'tgt' in want else None
+            out['gsrc'] = D.empty(tgt, (desc.B, desc.S, 3, desc.H, desc.W)) if 'src' in want else None
+            ig = L.SfmImageGrads(_vp(out['gtgt']), _vp(out['gsrc']))
+            L.check(self._lib.sfm_loss_forward_backward_images(C.byref(desc), C.byref(inp), _vp(losses), C.byref(g),
+                                                               C.byref(ig), self._workspace(desc, tgt),
+                                                               C.c_void_p(D.current_stream(tgt))))
+        elif peer is not None:
             L.check(self._lib.sfm_loss_forward_backward_peer(C.byref(desc), C.byref(inp), _vp(losses), C.byref(g),
                                                              self._workspace(desc, tgt), peer.handle,
                                                              C.c_void_p(D.current_stream(tgt))))
@@ -202,6 +224,10 @@ class ViewSynthesisLoss(object):
         g.gposes = D.ptr(grads['gposes'])
         L.check(self._lib.sfm_scale_grads(C.byref(desc), _vp(gy), C.byref(g),
                                           C.c_void_p(D.current_stream(grads['gposes']))))
+        if grads.get('gtgt') is not None or grads.get('gsrc') is not None:
+            ig = L.SfmImageGrads(_vp(grads.get('gtgt')), _vp(grads.get('gsrc')))
+            L.check(self._lib.sfm_scale_image_grads(C.byref(desc), _vp(gy), C.byref(ig),
+                                                    C.c_void_p(D.current_stream(grads['gposes']))))
         return grads
 
     def pyramid(self, tgt, src):

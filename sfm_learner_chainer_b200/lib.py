@@ -12,6 +12,7 @@ SFM_FLAG_TABLES_PROVIDED = 0x1
 SFM_FLAG_REUSE_PYRAMID = 0x2
 SFM_FLAG_NO_TMA = 0x4
 SFM_FLAG_EDGE_AWARE_SMOOTH = 0x8
+SFM_FLAG_IMAGE_GRADS = 0x10
 
 SFM_E_INVALID_DESC = -1
 SFM_E_INVALID_SHAPE = -2
@@ -43,6 +44,10 @@ class SfmGrads(C.Structure):
     _fields_ = [('gdisps', _vp * SFM_MAX_SCALES), ('gposes', _vp), ('glogits', _vp * SFM_MAX_SCALES)]
 
 
+class SfmImageGrads(C.Structure):
+    _fields_ = [('gtgt', _vp), ('gsrc', _vp)]
+
+
 class SfmAugment(C.Structure):
     _fields_ = [('out_h', C.c_int32), ('out_w', C.c_int32), ('off_y', C.c_int32), ('off_x', C.c_int32),
                 ('flip', C.c_int32), ('reserved_', C.c_int32), ('x_scaling', C.c_double), ('y_scaling', C.c_double)]
@@ -56,6 +61,7 @@ class SfmDebug(C.Structure):
 # every symbol include/sfmloss.h declares: name -> (restype, argtypes)
 _i = C.c_int
 _D, _I, _G, _Dbg = C.POINTER(SfmDesc), C.POINTER(SfmInputs), C.POINTER(SfmGrads), C.POINTER(SfmDebug)
+_IG = C.POINTER(SfmImageGrads)
 SYMBOLS = {
     'sfm_version': (_i, []),
     'sfm_last_error': (C.c_char_p, []),
@@ -64,6 +70,8 @@ SYMBOLS = {
     'sfm_loss_backward': (_i, [_D, _I, _vp, _G, _vp, _vp]),
     'sfm_loss_forward_backward': (_i, [_D, _I, _vp, _G, _vp, _vp]),
     'sfm_scale_grads': (_i, [_D, _vp, _G, _vp]),
+    'sfm_loss_forward_backward_images': (_i, [_D, _I, _vp, _G, _IG, _vp, _vp]),
+    'sfm_scale_image_grads': (_i, [_D, _vp, _IG, _vp]),
     'sfm_set_kernel_events': (_i, [_vp, _vp]),
     'sfm_pyramid': (_i, [_D, _vp, _vp, _vp, _vp]),
     'sfm_pyramid_export': (_i, [_D, _vp, _i, _vp, _vp, _vp]),

@@ -14,9 +14,13 @@ class _ViewSynthesisLossFn(torch.autograd.Function):
         disps = [p.contiguous() for p in preds[:n_scales]]
         poses = preds[n_scales].contiguous()
         logits = [p.contiguous() for p in preds[n_scales + 1:]] if use_exp else None
-        losses, grads = op.forward_backward(tgt.contiguous(), src.contiguous(), intrinsics.contiguous(),
+        # image gradients (op.image_grads) only for the images autograd asks for; the others are not computed
+        ctx.want_tgt = op.image_grads and ctx.needs_input_grad[1]
+        ctx.want_src = op.image_grads and ctx.needs_input_grad[2]
+        want = tuple(n for n, w in (('tgt', ctx.want_tgt), ('src', ctx.want_src)) if w)
+        losses, grads = op.forward_backward(tgt.detach().contiguous(), src.detach().contiguous(), intrinsics.contiguous(),
                                             [d.detach() for d in disps], poses.detach(),
-                                            [l.detach() for l in logits] if logits else None)
+                                            [l.detach() for l in logits] if logits else None, image_grads=want)
         ctx.op, ctx.grads, ctx.shape = op, grads, tuple(src.shape)
         ctx.n_scales, ctx.use_exp = n_scales, use_exp
         ctx.consumed = False
@@ -39,7 +43,9 @@ class _ViewSynthesisLossFn(torch.autograd.Function):
         out = list(g['gdisps']) + [g['gposes']]
         if ctx.use_exp:
             out += list(g['glogits'])
-        return (None, None, None, None, None, None) + tuple(out)
+        gtgt = g.get('gtgt') if ctx.want_tgt else None
+        gsrc = g.get('gsrc') if ctx.want_src else None
+        return (None, gtgt, gsrc, None, None, None) + tuple(out)
 
 
 def view_synthesis_loss(op, tgt, src, intrinsics, pred_disps, pred_poses, pred_maskes=None):
