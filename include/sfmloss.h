@@ -179,6 +179,20 @@ int sfm_loss_forward_backward_images(const SfmDesc* desc, const SfmInputs* in, f
 /* igrads *= *gy (device scalar), the NULL members skipped.  No-op on the device when *gy == 1. */
 int sfm_scale_image_grads(const SfmDesc* desc, const float* gy, const SfmImageGrads* igrads, void* stream);
 
+/* d(reported total)/d intrinsics (B,n_scales,3,3) times the call's gy, from the dL/dP cells that the last
+ * gradient-producing call (sfm_loss_backward, _forward_backward, _forward_backward_peer, _forward_backward_images)
+ * left in `workspace`: same desc, inputs and stream, before the next call on that workspace.  For callers that learn
+ * their camera.  K_s = intrinsics[:, s] is treated as differentiable in both places the reference uses it: the
+ * projection K4.[R|t] (transform.py:86-88) and pixel2cam's batch_inv(K) (:105).  Per (snippet, scale) it is
+ *   sum_i [ A_i R_i^T + g_i t_i^T - K_s^-T R_i^T K_s^T A_i ],   [A_i | g_i] = dL/dP of source i at scale s,
+ * evaluated in fp64 on the device (a dependent launch; graph-capturable).  Under snippet sharding (B_global > B) a
+ * shard's gradient is final.  With SFM_FLAG_TABLES_PROVIDED it returns SFM_E_UNSUPPORTED: the step then did not build
+ * the projection and K^-1 from the intrinsics. */
+int sfm_intrinsics_grad(const SfmDesc* desc, const SfmInputs* in, const void* workspace, float* gintrinsics, void* stream);
+
+/* gintrinsics *= *gy (device scalar).  No-op on the device when *gy == 1. */
+int sfm_scale_intrinsics_grad(const SfmDesc* desc, const float* gy, float* gintrinsics, void* stream);
+
 /* Profiling hook (bench.py's roofline measurement): while set (non-NULL cudaEvent_t handles), every
  * sfm_loss_* call on this thread records `start` right before and `stop` right after the fused loss
  * kernel, on the call's stream.  Pass NULL, NULL to clear. */

@@ -325,6 +325,37 @@ extern "C" int sfm_scale_image_grads(const SfmDesc* desc, const float* gy, const
   return sfm_launch_scale(ptrs, counts, 2, gy, (cudaStream_t)stream);
 }
 
+extern "C" int sfm_intrinsics_grad(const SfmDesc* desc, const SfmInputs* in, const void* workspace, float* gintrinsics,
+                                   void* stream) {
+  int rc = sfm_validate_desc(desc);
+  if (rc) return rc;
+  if (desc->flags & SFM_FLAG_TABLES_PROVIDED) {
+    sfm_set_error("unsupported: intrinsics gradient with SFM_FLAG_TABLES_PROVIDED (the step did not build proj / kinv from the intrinsics)");
+    return SFM_E_UNSUPPORTED;
+  }
+  if (!in) { sfm_set_error("SfmInputs is NULL"); return SFM_E_NULL_POINTER; }
+  if (!in->intrinsics || !in->poses) { sfm_set_error("intrinsics/poses pointer is NULL"); return SFM_E_NULL_POINTER; }
+  if (!workspace) { sfm_set_error("workspace is NULL"); return SFM_E_NULL_POINTER; }
+  if (((uintptr_t)workspace & 255) != 0) { sfm_set_error("workspace must be 256-byte aligned"); return SFM_E_INVALID_DESC; }
+  if (!gintrinsics) { sfm_set_error("gintrinsics is NULL"); return SFM_E_NULL_POINTER; }
+  SfmWsLayout L;
+  sfm_ws_layout(desc, &L);
+  const char* ws = (const char*)workspace;
+  // the poses as the step saw them: under raw_pose_hw the vectors its prologue reduced into the workspace
+  const float* poses = desc->raw_pose_hw > 0 ? (const float*)(ws + L.off_posevec) : in->poses;
+  return sfm_launch_intrinsics_grad(desc->B, desc->S, desc->n_scales, (const double*)(ws + L.off_acc) + 4, poses, in->intrinsics,
+                                    gintrinsics, (cudaStream_t)stream);
+}
+
+extern "C" int sfm_scale_intrinsics_grad(const SfmDesc* desc, const float* gy, float* gintrinsics, void* stream) {
+  int rc = sfm_validate_desc(desc);
+  if (rc) return rc;
+  if (!gy) { sfm_set_error("gy is NULL"); return SFM_E_NULL_POINTER; }
+  if (!gintrinsics) { sfm_set_error("gintrinsics is NULL"); return SFM_E_NULL_POINTER; }
+  const long long count = (long long)desc->B * desc->n_scales * 9;
+  return sfm_launch_scale(&gintrinsics, &count, 1, gy, (cudaStream_t)stream);
+}
+
 extern "C" int sfm_scale_grads(const SfmDesc* desc, const float* gy, const SfmGrads* grads, void* stream) {
   int rc = sfm_validate_desc(desc);
   if (rc) return rc;

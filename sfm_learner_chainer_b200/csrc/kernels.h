@@ -181,3 +181,7 @@ int sfm_launch_scale(float* const* ptrs, const long long* counts, int n, const f
 // adds the gradient levels p.gtgt[s] / p.gsrc[s] (s >= 1) into the full-resolution p.gtgt[0] / p.gsrc[0] through the
 // adjoint of the pyramid (fused_loss.cu); a dependent launch behind the epilogue
 int sfm_launch_image_pullback(const SfmFusedParams& p, int H, int W, cudaStream_t stream);
+// gintrinsics (B,ns,3,3) from the dL/dP cells (SfmWsLayout::off_acc + 4 doubles) and the poses / intrinsics the step
+// used (fused_loss.cu); a dependent launch behind the step's last kernel
+int sfm_launch_intrinsics_grad(int B, int S, int ns, const double* cells, const float* poses, const float* intrinsics,
+                               float* gintrinsics, cudaStream_t stream);

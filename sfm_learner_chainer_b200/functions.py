@@ -25,13 +25,17 @@ class ViewSynthesisLoss(object):
     0.01 * mean over (h', w') (models/pose_net.py:52-53); `gposes` then has the map's shape.
     image_grads: forward_backward also returns gtgt (B,3,H,W) and gsrc (B,S,3,H,W), the gradients of the reported
     total w.r.t. the two images (for images that come out of a differentiable module); not with edge_aware_smooth.
+    intrinsics_grad: forward_backward and backward also return gintrinsics (B,n_scales,3,3), the gradient of the
+    reported total w.r.t. `intrinsics` (for a camera that is learned); not with caller-supplied proj / kinv.
     """
 
     def __init__(self, smooth_reg=0.0, exp_reg=0.0, ssim_rate=0.0, n_scales=N_SCALES, B_global=None,
-                 raw_disp_scales=0, raw_pose=False, edge_aware_smooth=False, image_grads=False):
+                 raw_disp_scales=0, raw_pose=False, edge_aware_smooth=False, image_grads=False,
+                 intrinsics_grad=False):
         if image_grads and edge_aware_smooth:
             raise ValueError('image_grads is not supported together with edge_aware_smooth')
         self.image_grads = bool(image_grads)
+        self.intrinsics_grad = bool(intrinsics_grad)
         # edge_aware_smooth: smoothness term = compute_disp_smooth (base_model.py:144-155, commented out at :78-80)
         self.edge_aware_smooth = bool(edge_aware_smooth)
         self.raw_disp_scales = int(raw_disp_scales)
@@ -126,6 +130,24 @@ class ViewSynthesisLoss(object):
         g.gposes = D.ptr(gp)
         return g, dict(gdisps=gd, gposes=gp, glogits=gl)
 
+    def _want_intrinsics_grad(self, want, proj, kinv):
+        if not (self.intrinsics_grad and want):
+            return False
+        if proj is not None or kinv is not None:
+            raise ValueError('intrinsics_grad needs the projection tables built from the intrinsics (no proj / kinv)')
+        return True
+
+    def _intrinsics_grad(self, desc, inp, tgt, out, want):
+        """Adds gintrinsics to `out` (None when not requested) from the cells the gradient call just left in the
+        workspace."""
+        if not self.intrinsics_grad:
+            return
+        out['gintrinsics'] = None
+        if want:
+            out['gintrinsics'] = D.empty(tgt, (desc.B, self.n_scales, 3, 3))
+            L.check(self._lib.sfm_intrinsics_grad(C.byref(desc), C.byref(inp), self._workspace(desc, tgt),
+                                                  _vp(out['gintrinsics']), C.c_void_p(D.current_stream(tgt))))
+
     # ---- operators
     def forward(self, tgt, src, intrinsics, disps, poses, logits=None, proj=None, kinv=None, debug=False):
         """-> losses (5,) device array in the order of lib.LOSS_KEYS [, debug dict]."""
@@ -149,12 +171,16 @@ class ViewSynthesisLoss(object):
                                            self._workspace(desc, tgt), C.c_void_p(D.current_stream(tgt))))
         return (losses, dbg) if debug else losses
 
-    def backward(self, tgt, src, intrinsics, disps, poses, logits=None, gy=None, proj=None, kinv=None):
-        """Recomputing backward: -> dict(gdisps, gposes, glogits).  gy: device scalar or None (= 1)."""
+    def backward(self, tgt, src, intrinsics, disps, poses, logits=None, gy=None, proj=None, kinv=None,
+                 intrinsics_grad=True):
+        """Recomputing backward: -> dict(gdisps, gposes, glogits).  gy: device scalar or None (= 1).
+        With the operator's intrinsics_grad the dict also holds gintrinsics (None when `intrinsics_grad` is False)."""
+        want_k = self._want_intrinsics_grad(intrinsics_grad, proj, kinv)
         desc, inp = self._pack(tgt, src, intrinsics, disps, poses, logits, proj, kinv)
         g, out = self._alloc_grads(desc, tgt)
         L.check(self._lib.sfm_loss_backward(C.byref(desc), C.byref(inp), _vp(gy), C.byref(g),
                                             self._workspace(desc, tgt), C.c_void_p(D.current_stream(tgt))))
+        self._intrinsics_grad(desc, inp, tgt, out, want_k)
         return out
 
     def build_pyramid(self, tgt, src):
@@ -175,13 +201,15 @@ class ViewSynthesisLoss(object):
         self._ev_pyramid = D.record_event(tgt)
 
     def forward_backward(self, tgt, src, intrinsics, disps, poses, logits=None, proj=None, kinv=None, reuse_pyramid=False,
-                         peer=None, image_grads=('tgt', 'src')):
+                         peer=None, image_grads=('tgt', 'src'), intrinsics_grad=True):
         """Single fused pass: -> (losses (5,), dict(gdisps, gposes, glogits)) for upstream gradient 1.
         reuse_pyramid: the workspace already holds this batch's pyramid (build_pyramid).
         peer: a distributed.PeerLossSum -- the batch is sharded by snippet over several GPUs (B_global set) and the
         epilogue kernel completes the five losses across the ranks over NVLink peer memory.
         With the operator's image_grads the dict also holds gtgt and gsrc (None for an image left out of
-        `image_grads`, a subset of ('tgt', 'src'); an empty one runs the plain pass); not with peer."""
+        `image_grads`, a subset of ('tgt', 'src'); an empty one runs the plain pass); not with peer.
+        With the operator's intrinsics_grad the dict also holds gintrinsics (None when `intrinsics_grad` is False)."""
+        want_k = self._want_intrinsics_grad(intrinsics_grad, proj, kinv)
         desc, inp = self._pack(tgt, src, intrinsics, disps, poses, logits, proj, kinv)
         if reuse_pyramid:
             desc.flags |= L.SFM_FLAG_REUSE_PYRAMID
@@ -208,6 +236,7 @@ class ViewSynthesisLoss(object):
             L.check(self._lib.sfm_loss_forward_backward(C.byref(desc), C.byref(inp), _vp(losses), C.byref(g),
                                                         self._workspace(desc, tgt),
                                                         C.c_void_p(D.current_stream(tgt))))
+        self._intrinsics_grad(desc, inp, tgt, out, want_k)
         if self._ev_pyramid is not None:
             self._ev_loss = D.record_event(tgt)
         return losses, out
@@ -228,6 +257,9 @@ class ViewSynthesisLoss(object):
             ig = L.SfmImageGrads(_vp(grads.get('gtgt')), _vp(grads.get('gsrc')))
             L.check(self._lib.sfm_scale_image_grads(C.byref(desc), _vp(gy), C.byref(ig),
                                                     C.c_void_p(D.current_stream(grads['gposes']))))
+        if grads.get('gintrinsics') is not None:
+            L.check(self._lib.sfm_scale_intrinsics_grad(C.byref(desc), _vp(gy), _vp(grads['gintrinsics']),
+                                                        C.c_void_p(D.current_stream(grads['gposes']))))
         return grads
 
     def pyramid(self, tgt, src):

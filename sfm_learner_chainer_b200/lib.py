@@ -72,6 +72,8 @@ SYMBOLS = {
     'sfm_scale_grads': (_i, [_D, _vp, _G, _vp]),
     'sfm_loss_forward_backward_images': (_i, [_D, _I, _vp, _G, _IG, _vp, _vp]),
     'sfm_scale_image_grads': (_i, [_D, _vp, _IG, _vp]),
+    'sfm_intrinsics_grad': (_i, [_D, _I, _vp, _vp, _vp]),
+    'sfm_scale_intrinsics_grad': (_i, [_D, _vp, _vp, _vp]),
     'sfm_set_kernel_events': (_i, [_vp, _vp]),
     'sfm_pyramid': (_i, [_D, _vp, _vp, _vp, _vp]),
     'sfm_pyramid_export': (_i, [_D, _vp, _i, _vp, _vp, _vp]),

@@ -18,9 +18,12 @@ class _ViewSynthesisLossFn(torch.autograd.Function):
         ctx.want_tgt = op.image_grads and ctx.needs_input_grad[1]
         ctx.want_src = op.image_grads and ctx.needs_input_grad[2]
         want = tuple(n for n, w in (('tgt', ctx.want_tgt), ('src', ctx.want_src)) if w)
-        losses, grads = op.forward_backward(tgt.detach().contiguous(), src.detach().contiguous(), intrinsics.contiguous(),
-                                            [d.detach() for d in disps], poses.detach(),
-                                            [l.detach() for l in logits] if logits else None, image_grads=want)
+        # likewise the intrinsics gradient (op.intrinsics_grad) only when autograd asks for it
+        ctx.want_k = op.intrinsics_grad and ctx.needs_input_grad[3]
+        losses, grads = op.forward_backward(tgt.detach().contiguous(), src.detach().contiguous(),
+                                            intrinsics.detach().contiguous(), [d.detach() for d in disps], poses.detach(),
+                                            [l.detach() for l in logits] if logits else None, image_grads=want,
+                                            intrinsics_grad=ctx.want_k)
         ctx.op, ctx.grads, ctx.shape = op, grads, tuple(src.shape)
         ctx.n_scales, ctx.use_exp = n_scales, use_exp
         ctx.consumed = False
@@ -45,7 +48,8 @@ class _ViewSynthesisLossFn(torch.autograd.Function):
             out += list(g['glogits'])
         gtgt = g.get('gtgt') if ctx.want_tgt else None
         gsrc = g.get('gsrc') if ctx.want_src else None
-        return (None, gtgt, gsrc, None, None, None) + tuple(out)
+        gk = g.get('gintrinsics') if ctx.want_k else None
+        return (None, gtgt, gsrc, gk, None, None) + tuple(out)
 
 
 def view_synthesis_loss(op, tgt, src, intrinsics, pred_disps, pred_poses, pred_maskes=None):
