@@ -302,6 +302,26 @@ def spatial_transformer_sampler_grad(t, gy, h, w):
     return gu * dt.type((w - 1) / 2.), gv * dt.type((h - 1) / 2.)
 
 
+def sampler_image_adjoint(t, gP, h, w):
+    """Gradient of the sampler w.r.t. its image (float64): every pixel scatters gP_c * w_k to its valid taps; a
+    pixel with no valid tap (out of view by the x2 rule) contributes nothing.  t: the tap record of the forward,
+    gP (N,3,hw) -> (N,3,h*w)."""
+    N = gP.shape[0]
+    u0, v0 = t['u0'].astype(np.int64), t['v0'].astype(np.int64)
+    wa, wb = t['wa'].astype(np.float64), t['wb'].astype(np.float64)
+    wc, wd = t['wc'].astype(np.float64), t['wd'].astype(np.float64)
+    out = np.zeros((N, 3, h * w), np.float64)
+    bi = np.broadcast_to(np.arange(N)[:, None], u0.shape)
+    for du, dv, wk in ((0, 0, wa * wc), (1, 0, wb * wc), (0, 1, wa * wd), (1, 1, wb * wd)):
+        uu, vv = u0 + du, v0 + dv
+        ok = t['any_valid'] & (uu >= 0) & (uu <= w - 1) & (vv >= 0) & (vv <= h - 1)
+        wk = wk.astype(t['wa'].dtype).astype(np.float64)      # the forward rounds the weight products to the image dtype
+        idx = np.where(ok, vv * w + uu, 0)
+        for c in range(3):
+            np.add.at(out[:, c], (bi, idx), np.where(ok, wk * gP[:, c], 0.0))
+    return out
+
+
 def sampler_interp_forward(x, grid):
     """models/spational_transformer_sampler_interp.py:32-78 -- the repo-local
     sampler (unused by the live path): grid in PIXEL units, indices clamped to
@@ -411,6 +431,23 @@ def resize_images(x, out_shape):
     V0, U0 = v0[:, None], u0[None, :]
     return ((w1 * x[:, :, V0, U0] + w2 * x[:, :, V0, U0 + 1])
             + w3 * x[:, :, V0 + 1, U0]) + w4 * x[:, :, V0 + 1, U0 + 1]
+
+
+def resize_images_adjoint(gy, in_shape, dtype=np.float32):
+    """Adjoint of resize_images (float64): gy (B,C,oh,ow) -> (B,C,H,W).  The tap weights are the forward's, float64
+    products rounded to `dtype`.  The identity when the sizes agree (scale 0)."""
+    B, C, oh, ow = gy.shape
+    H, W = in_shape
+    if (oh, ow) == (H, W):
+        return gy.astype(np.float64)
+    u0, ua, ub = resize_axis_tables(W, ow)
+    v0, va, vb = resize_axis_tables(H, oh)
+    gx = np.zeros((B, C, H, W), np.float64)
+    V0, U0 = np.broadcast_arrays(v0[:, None], u0[None, :])
+    for wv, wu, dv, du in ((va, ua, 0, 0), (va, ub, 0, 1), (vb, ua, 1, 0), (vb, ub, 1, 1)):
+        wk = (wv[:, None] * wu[None, :]).astype(dtype).astype(np.float64)
+        np.add.at(gx.transpose(2, 3, 0, 1), (V0 + dv, U0 + du), (wk * gy).transpose(2, 3, 0, 1))
+    return gx
 
 
 # --------------------------------------------------------------------------
@@ -546,9 +583,36 @@ def _pose_backward(vec, K_scales, dP_scales):
     return g.astype(dt), dT
 
 
+def intrinsics_grad(intrinsics, poses, dP):
+    """d total / d intrinsics from the dL/dP cells -> (B,n_scales,3,3) float64.  intrinsics (B,n_scales,3,3), poses
+    (B,S,6) as the loss used them, dP (B,S,n_scales,3,4).
+
+    K enters the projection P = K4 . [R|t] (transform.py:86-88) and pixel2cam's batch_inv(K) (:105).  Per pixel
+    q = K (R c + t) with c = depth K^-1 pix, so with the cells dL/dP = [A_i | g_i] (A_i = sum gq (x) c, g_i = sum gq):
+
+        dL/dK_s = sum_i [ A_i R_i^T + g_i t_i^T - K_s^-T R_i^T K_s^T A_i ]
+
+    R_i = (Rx . Ry) . Rz of the clipped angles with sin / cos rounded to the working dtype and t_i unclipped, as
+    `_pose_backward` has them; K^-1 and the sum in float64."""
+    B, S, ns = dP.shape[:3]
+    K = intrinsics.astype(np.float64)
+    Ki = np.linalg.inv(K)
+    out = np.zeros((B, ns, 3, 3), np.float64)
+    for i in range(S):
+        _, c, s = euler_sincos(poses[:, i, :3])
+        xm, ym, zm = [m.astype(np.float64) for m in _rot_mats(c, s)]
+        R = ((xm @ ym) @ zm)[:, None]                                    # (B,1,3,3)
+        t = poses[:, i, 3:].astype(np.float64)[:, None]                  # (B,1,3)
+        A, g = dP[:, i, :, :, :3], dP[:, i, :, :, 3]
+        RT = np.swapaxes(R, -1, -2)
+        out += A @ RT + g[..., :, None] * t[..., None, :]
+        out -= np.swapaxes(Ki, -1, -2) @ RT @ np.swapaxes(K, -1, -2) @ A
+    return out
+
+
 def sfm_loss(tgt, src, intrinsics, disps, poses, logits, cfg,
              want_grads=True, proj_override=None, kinv_override=None,
-             want_debug=False):
+             want_debug=False, want_image_grads=False, want_intrinsics_grad=False):
     """SFMLearner.__call__ loss loop (base_model.py:57-124) + its backward.
 
     tgt (B,3,H,W); src (B,S,3,H,W); intrinsics (B,n_scales,3,3);
@@ -556,7 +620,20 @@ def sfm_loss(tgt, src, intrinsics, disps, poses, logits, cfg,
     or None.  Returns (losses dict, grads dict or None, debug dict).
     `cfg.B_global` (default B) is the batch size every F.mean divides by, so a
     shard of a larger batch yields partial sums that add up to the full loss.
+
+    Opt-in gradients (both need `want_grads`), added to the grads dict in float64:
+    * want_image_grads: gtgt (B,3,H,W) and gsrc (B,S,3,H,W).  The images are
+      treated as differentiable throughout (the reference's `.data` on the
+      pyramid, base_model.py:71-72, and on mu_y / sigma_y, :131, :134, are
+      lifted), so they are the derivative of the reported total; the all-zero
+      mask (:96) is piecewise constant.  Not with the edge-aware smoothness term.
+    * want_intrinsics_grad: dP (B,S,n_scales,3,4), the dL/dP cells the pose
+      chain starts from, and gintrinsics (B,n_scales,3,3) (`intrinsics_grad`).
     """
+    if (want_image_grads or want_intrinsics_grad) and not want_grads:
+        raise ValueError('image and intrinsics gradients need want_grads')
+    if want_image_grads and cfg.smooth_reg and cfg.edge_aware_smooth:
+        raise ValueError('image gradients through the edge-aware smoothness term are not supported')
     dt = tgt.dtype
     B, S, _, H, W = src.shape
     Bg = cfg.B_global if cfg.B_global else B
@@ -570,6 +647,9 @@ def sfm_loss(tgt, src, intrinsics, disps, poses, logits, cfg,
     gdisp = [np.zeros(d.shape, np.float64) for d in disps]
     glogits = [np.zeros(l.shape, np.float64) for l in logits] if (use_exp and logits is not None) else None
     dP_all = [[None] * ns_total for _ in range(S)]
+    if want_image_grads:
+        gtgt = np.zeros(tgt.shape, np.float64)
+        gsrc = np.zeros(src.shape, np.float64)
     debug = dict(P=[], u0=[], v0=[], inb=[], tgt_pyr=[], src_pyr=[])
 
     for ns in range(ns_total):
@@ -627,6 +707,9 @@ def sfm_loss(tgt, src, intrinsics, disps, poses, logits, cfg,
         Kinv = kinv_override[:, ns] if kinv_override is not None else batch_inv3(K)
         ray, cam = pixel2cam(depth, Kinv, h, w)
         g_depth = np.zeros((B, hw_n), np.float64)
+        if want_image_grads:
+            gT = np.zeros((B, 3, h, w), np.float64)
+            gS = np.zeros((B, S, 3, h, w), np.float64)
         dbgP, dbgu, dbgv, dbgi = [], [], [], []
         for i in range(S):
             img = cur_src[:, 3 * i:3 * i + 3]
@@ -664,24 +747,31 @@ def sfm_loss(tgt, src, intrinsics, disps, poses, logits, cfg,
                 pixel_loss += _fsum(err) / n_pix3
                 if want_grads:
                     gP += sgn * ((1 - ssim_rate) / n_pix3)
-                if use_ssim:
-                    st = ssim_terms(P, cur_tgt)
-                    e = np.clip(st['raw'], 0, 1) * (1 - m)
-                    ssim_loss += _fsum(e) / n_pix3
-                    if want_grads:
-                        raw = st['raw'].astype(np.float64)
-                        a, my = st['a'].astype(np.float64), st['my'].astype(np.float64)
-                        n1, n2 = st['n1'].astype(np.float64), st['n2'].astype(np.float64)
-                        d1, d2 = st['d1'].astype(np.float64), st['d2'].astype(np.float64)
-                        n, d = st['n'].astype(np.float64), st['d'].astype(np.float64)
-                        g_e = (ssim_rate / n_pix3) * (1 - m) * ((raw >= 0) & (raw <= 1))
-                        g_n = -g_e / (2 * d)
-                        g_d = g_e * n / (2 * d * d)
-                        g_a = g_n * (2 * my * n2 - 2 * my * n1) + g_d * (2 * a * d2 - 2 * a * d1)
-                        g_s = g_d * d1
-                        g_c = 2 * g_n * n1
-                        gP += (avg_pool3(g_a) + 2 * P.astype(np.float64) * avg_pool3(g_s)
-                               + cur_tgt.astype(np.float64) * avg_pool3(g_c))
+            if want_image_grads:
+                gT -= gP                                        # the L1 part: d|P - T| / dT = -d|P - T| / dP
+            if use_ssim:
+                st = ssim_terms(P, cur_tgt)
+                e = np.clip(st['raw'], 0, 1) * (1 - m)
+                ssim_loss += _fsum(e) / n_pix3
+                if want_grads:
+                    raw = st['raw'].astype(np.float64)
+                    a, my = st['a'].astype(np.float64), st['my'].astype(np.float64)
+                    n1, n2 = st['n1'].astype(np.float64), st['n2'].astype(np.float64)
+                    d1, d2 = st['d1'].astype(np.float64), st['d2'].astype(np.float64)
+                    n, d = st['n'].astype(np.float64), st['d'].astype(np.float64)
+                    g_e = (ssim_rate / n_pix3) * (1 - m) * ((raw >= 0) & (raw <= 1))
+                    g_n = -g_e / (2 * d)
+                    g_d = g_e * n / (2 * d * d)
+                    g_a = g_n * (2 * my * n2 - 2 * my * n1) + g_d * (2 * a * d2 - 2 * a * d1)
+                    g_s = g_d * d1
+                    g_c = 2 * g_n * n1
+                    Pd, Td = P.astype(np.float64), cur_tgt.astype(np.float64)
+                    As, Ac = avg_pool3(g_s), avg_pool3(g_c)
+                    gP += avg_pool3(g_a) + 2 * Pd * As + Td * Ac
+                    if want_image_grads:
+                        # avg_pool3 is its own adjoint; g_my mirrors g_a
+                        g_my = g_n * (2 * a * n2 - 2 * a * n1) + g_d * (2 * my * d2 - 2 * my * d1)
+                        gT += avg_pool3(g_my) + 2 * Td * As + Pd * Ac
             if want_grads:
                 # sampler -> grid -> q -> cam/proj  (A.6)
                 gyf = gP.reshape(B, 3, hw_n)
@@ -703,6 +793,11 @@ def sfm_loss(tgt, src, intrinsics, disps, poses, logits, cfg,
                 g_depth += np.sum(g_cam * ray.astype(np.float64), axis=1)
                 cam4 = np.concatenate([cam.astype(np.float64), np.ones((B, 1, hw_n))], axis=1)
                 dP_all[i][ns] = np.einsum('nkp,njp->nkj', g_q, cam4)
+                if want_image_grads:
+                    gS[:, i] = sampler_image_adjoint(t, gyf, h, w).reshape(B, 3, h, w)
+        if want_image_grads:
+            gtgt += resize_images_adjoint(gT, (H, W), dt)
+            gsrc += resize_images_adjoint(gS.reshape(B, 3 * S, h, w), (H, W), dt).reshape(src.shape)
         if want_debug:
             debug['P'].append(np.stack(dbgP, 1))
             debug['u0'].append(np.stack(dbgu, 1))
@@ -725,6 +820,11 @@ def sfm_loss(tgt, src, intrinsics, disps, poses, logits, cfg,
         grads = dict(gdisp=[g.astype(dt) for g in gdisp], gpose=gpose,
                      glogits=[g.astype(dt) for g in glogits] if glogits is not None else None,
                      dT=dT_all)
+        if want_image_grads:
+            grads.update(gtgt=gtgt, gsrc=gsrc)
+        if want_intrinsics_grad:
+            dP = np.stack([np.stack(dP_all[i], 1) for i in range(S)], 1)
+            grads.update(dP=dP, gintrinsics=intrinsics_grad(intrinsics, poses, dP))
     return losses, grads, debug
 
 
@@ -761,7 +861,8 @@ def pose_from_raw(x, n_sources):
 def sfm_loss_raw(tgt, src, intrinsics, disps_in, poses_in, logits, cfg, raw_disp_scales=0, raw_pose=False, **kw):
     """sfm_loss with the seam included: scales in the bit mask `raw_disp_scales` take the pre-activation
     `dispout` map, `raw_pose` takes the `poseout` map (B, 6*S, h', w').  Gradients are returned w.r.t. what was
-    passed in (chain rule through disp_activation / pose_from_raw)."""
+    passed in (chain rule through disp_activation / pose_from_raw).  The opt-in gradients of sfm_loss pass through
+    as they are: gintrinsics is built from the reduced pose vectors."""
     S = src.shape[1]
     disps, dacts = [], []
     for s, d in enumerate(disps_in):

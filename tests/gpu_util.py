@@ -30,6 +30,36 @@ def oracle_tables(O, d, n_scales=4):
     return proj, kinv
 
 
+FLAGSETS = {
+    'cfg1': dict(smooth_reg=0.0, exp_reg=0.0, ssim_rate=0.0),
+    'cfg2': dict(smooth_reg=0.1, exp_reg=0.0, ssim_rate=0.15),
+    'cfg4': dict(smooth_reg=0.1, exp_reg=0.2, ssim_rate=0.0),
+}
+
+
+def make_op(flags, **kw):
+    from sfm_learner_chainer_b200 import ViewSynthesisLoss
+    return ViewSynthesisLoss(flags['smooth_reg'], flags['exp_reg'], flags['ssim_rate'], **kw)
+
+
+def op_args(g, flags):
+    """The loss arguments from a dict of inputs (device tensors or host arrays); logits only with the
+    explainability term."""
+    return (g['tgt'], g['src'], g['intrinsics'], g['disps'], g['poses'], g['logits'] if flags['exp_reg'] else None)
+
+
+def check_same_as_plain(l, g, lp, gp, ns, exp):
+    """Losses, gdisps, glogits of an operator with an opt-in gradient bitwise those of the operator without it; gposes
+    to the order of the fp64 atomics (they vary from run to run in either operator)."""
+    np.testing.assert_array_equal(host(l), host(lp))
+    for s in range(ns):
+        np.testing.assert_array_equal(host(g['gdisps'][s]), host(gp['gdisps'][s]))
+        if exp:
+            np.testing.assert_array_equal(host(g['glogits'][s]), host(gp['glogits'][s]))
+    np.testing.assert_allclose(host(g['gposes']), host(gp['gposes']), rtol=1e-5, atol=1e-6 * np.abs(host(gp['gposes'])).max())
+    assert 'gintrinsics' not in gp
+
+
 def assert_grad_close(got, ref, rtol=1e-4, atol_rel=5e-5, what=''):
     """fp32 gradient bar of the north star: rtol 1e-4, plus an absolute floor relative to the largest
     reference entry (sums with different association, fp64 atomics)."""

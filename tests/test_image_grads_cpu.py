@@ -1,19 +1,18 @@
 """-m "not gpu": image gradients of the fused loss (d total / d tgt_img, d total / d src_imgs).
 
-The oracle's analytic gtgt / gsrc (tests/image_grad_oracle.py) are checked against torch fp64 autograd through an independent restatement of the
-image-dependent part of the forward (the projection grid does not depend on the images and is taken from the oracle),
-against central differences of the oracle itself, and the resize adjoint against <Rx, y> = <x, R^T y>.  The C ABI
-additions are checked for their argument errors without a device."""
+The oracle's analytic gtgt / gsrc (O.sfm_loss(want_image_grads=True)) are checked against torch fp64 autograd through
+an independent restatement of the forward (tests/torch_restatement.py), against central differences of the oracle
+itself, and the resize adjoint against <Rx, y> = <x, R^T y>.  The C ABI additions are checked for their argument
+errors without a device."""
 import ctypes as C
 
 import numpy as np
 import pytest
 import torch
-import torch.nn.functional as F
 
 from oracle import sfm_oracle as O
 from sfm_learner_chainer_b200.synthetic import make_snippets
-from tests import image_grad_oracle as IO
+from tests.torch_restatement import torch_total
 
 FLAGS = {
     'l1': dict(smooth_reg=0.1, exp_reg=0.0, ssim_rate=0.0),
@@ -27,48 +26,6 @@ def _data(B, S, H, W, ns, harsh, seed=0):
     return d
 
 
-def _torch_total(d, cfg, tgt, src):
-    """(1 - r) * pixel + r * ssim of base_model.py:64-118 with the images as torch leaves; the terms that do not
-    depend on the images (smoothness, explainability regulariser) are left out."""
-    B, S, _, H, W = d['src'].shape
-    Bg = B
-    use_exp = bool(cfg.exp_reg)
-    use_ssim = not use_exp and bool(cfg.ssim_rate)
-    rate = cfg.ssim_rate or 0.0
-    pixel = ssim = 0.0
-    for ns in range(cfg.n_scales):
-        h, w = H >> ns, W >> ns
-        if ns == 0:
-            ct, cs = tgt, src.reshape(B, 3 * S, H, W)
-        else:
-            ct = F.interpolate(tgt, size=(h, w), mode='bilinear', align_corners=True)
-            cs = F.interpolate(src.reshape(B, 3 * S, H, W), size=(h, w), mode='bilinear', align_corners=True)
-        depth = 1.0 / d['disps'][ns].reshape(B, h * w)
-        K = d['intrinsics'][:, ns]
-        _, cam = O.pixel2cam(depth, O.batch_inv3(K), h, w)
-        n3 = Bg * 3 * h * w
-        for i in range(S):
-            gr = O.cam2pixel(cam, O.proj_tgt_to_src(d['poses'][:, i], K), h, w)
-            grid = torch.from_numpy(np.stack([gr['xn'], gr['yn']], -1).reshape(B, h, w, 2))
-            P = F.grid_sample(cs[:, 3 * i:3 * i + 3], grid, mode='bilinear', padding_mode='zeros', align_corners=True)
-            m = (P == 0).all(dim=1, keepdim=True).detach()
-            err = torch.where(m, torch.zeros_like(P), (P - ct).abs())
-            if use_exp:
-                sg = torch.sigmoid(torch.from_numpy(d['logits'][ns][:, i:i + 1]))
-                pixel = pixel + (err * sg).sum() / n3
-            else:
-                pixel = pixel + err.sum() / n3
-            if use_ssim:
-                pool = lambda x: F.avg_pool2d(x, 3, 1, 1, count_include_pad=True)
-                a, my = pool(P), pool(ct)
-                sx, sy, sxy = pool(P * P) - a * a, pool(ct * ct) - my * my, pool(P * ct) - a * my
-                n = (2 * a * my + O.SSIM_C1) * (2 * sxy + O.SSIM_C2)
-                dd = (a * a + my * my + O.SSIM_C1) * (sx + sy + O.SSIM_C2)
-                e = torch.clamp((1 - n / dd) / 2, 0, 1) * (~m)
-                ssim = ssim + e.sum() / n3
-    return (1 - rate) * pixel + rate * ssim
-
-
 @pytest.mark.parametrize('flags', sorted(FLAGS))
 @pytest.mark.parametrize('S', [1, 2, 4])
 @pytest.mark.parametrize('ns', [1, 4])
@@ -76,10 +33,10 @@ def _torch_total(d, cfg, tgt, src):
 def test_oracle_image_grads_match_torch_autograd(flags, S, ns, harsh):
     d = _data(2, S, 32, 64, ns, harsh, seed=S + 10 * ns)
     cfg = O.LossConfig(n_scales=ns, **FLAGS[flags])
-    L, G, _ = IO.sfm_loss_with_image_grads(d['tgt'], d['src'], d['intrinsics'], d['disps'], d['poses'], d['logits'], cfg)
+    L, G, _ = O.sfm_loss(d['tgt'], d['src'], d['intrinsics'], d['disps'], d['poses'], d['logits'], cfg, want_image_grads=True)
     tgt = torch.from_numpy(d['tgt']).requires_grad_(True)
     src = torch.from_numpy(d['src']).requires_grad_(True)
-    tot = _torch_total(d, cfg, tgt, src)
+    tot = torch_total(d, cfg, tgt, src, torch.from_numpy(d['intrinsics']))
     tot.backward()
     # the restatement leaves out only image-independent terms
     np.testing.assert_allclose(tot.item(), L['total_loss'] - L['smooth_loss'] - L['exp_loss'], rtol=1e-9, atol=1e-12)
@@ -99,7 +56,7 @@ def test_oracle_image_grads_central_differences(flags):
     def total(tgt, src):
         return O.sfm_loss(tgt, src, d['intrinsics'], d['disps'], d['poses'], d['logits'], cfg, want_grads=False)[0]['total_loss']
 
-    _, G, _ = IO.sfm_loss_with_image_grads(d['tgt'], d['src'], d['intrinsics'], d['disps'], d['poses'], d['logits'], cfg)
+    _, G, _ = O.sfm_loss(d['tgt'], d['src'], d['intrinsics'], d['disps'], d['poses'], d['logits'], cfg, want_image_grads=True)
     rs = np.random.RandomState(1)
     eps = 1e-6
     mid = total(d['tgt'], d['src'])
@@ -131,7 +88,7 @@ def test_resize_adjoint_is_the_transpose():
         x = rs.standard_normal((2, 3, H, W))
         y = rs.standard_normal((2, 3, h, w))
         lhs = np.sum(O.resize_images(x, (h, w)) * y)
-        rhs = np.sum(x * IO.resize_images_adjoint(y, (H, W), np.float64))
+        rhs = np.sum(x * O.resize_images_adjoint(y, (H, W), np.float64))
         assert abs(lhs - rhs) <= 1e-12 * (abs(lhs) + np.sum(np.abs(x)) * np.abs(y).max())
 
 

@@ -1,6 +1,7 @@
 """Property tests of the oracle (SURVEY section 4, T4) with hypothesis: randomised small shapes, poses and flag sets.
 They pin the semantics the multi-GPU decomposition and the kernels' task decomposition rely on."""
 import numpy as np
+import pytest
 from hypothesis import given, settings, strategies as st
 
 from oracle import sfm_oracle as O
@@ -62,3 +63,14 @@ def test_out_of_view_poses_give_zero_photometric_terms(H, W, seed):
     L, G, _ = _loss(d, O.LossConfig(smooth_reg=0.0, exp_reg=0.0, ssim_rate=0.15))
     assert L['pixel_loss'] == 0 and L['ssim_loss'] == 0 and L['total_loss'] == 0
     assert np.all(G['gpose'] == 0) and all(np.all(g == 0) for g in G['gdisp'])
+
+
+def test_opt_in_gradient_argument_errors():
+    d = make_snippets(2, 2, 32, 32, seed=5)
+    for kw in (dict(want_image_grads=True), dict(want_intrinsics_grad=True)):
+        with pytest.raises(ValueError):
+            _loss(d, O.LossConfig(**FLAGS[1]), want_grads=False, **kw)
+    with pytest.raises(ValueError):
+        _loss(d, O.LossConfig(**FLAGS[3]), want_image_grads=True)
+    _, G, _ = _loss(d, O.LossConfig(**FLAGS[3]), want_intrinsics_grad=True)
+    assert G['gintrinsics'].shape == (2, 4, 3, 3) and 'gtgt' not in G
