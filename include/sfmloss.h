@@ -52,6 +52,9 @@ extern "C" {
 #define SFM_FLAG_IMAGE_GRADS 0x10u    /* the workspace also holds fp32 gradient levels of the pyramid (scales >= 1) for
                                          sfm_loss_forward_backward_images; every other entry point accepts the flag and
                                          behaves exactly as without it */
+#define SFM_FLAG_SNIPPET_TERMS 0x20u  /* the workspace also holds 4 fp64 loss cells per snippet and one float per smoothness
+                                         task for sfm_loss_snippets; every other entry point accepts the flag and behaves
+                                         exactly as without it */
 
 /*
  * Problem descriptor.  Mirrors the reference's model flags (base_model.py:37-39:
@@ -192,6 +195,19 @@ int sfm_intrinsics_grad(const SfmDesc* desc, const SfmInputs* in, const void* wo
 
 /* gintrinsics *= *gy (device scalar).  No-op on the device when *gy == 1. */
 int sfm_scale_intrinsics_grad(const SfmDesc* desc, const float* gy, float* gintrinsics, void* stream);
+
+/* Per-snippet weights and per-snippet loss values (sfm_loss_snippets).  Every term of the loss is a sum over the
+ * snippets, total = sum_b l_b with the 1/B_global means inside each l_b, so the weighted loss sum_b w_b * l_b is linear
+ * in the weights and d total / d w_b = l_b[0].  Weights held in device memory let one captured CUDA graph run batches
+ * with fewer real snippets: pad to the captured B with copies of a real snippet, keep B_global = B and pass
+ * w_b = B / B_real for the real snippets and 0 for the padding.  Any float is accepted (0 and negative ones included);
+ * a non-finite weight propagates. */
+typedef struct SfmSnippetTerms {
+  const float* weights;  /* (B) device: w_b, or NULL = all 1 */
+  float* losses;         /* (B,5) device: l_b = total, pixel, smooth, exp, ssim of snippet b (unweighted, with the
+                            1/B_global means), or NULL */
+} SfmSnippetTerms;
+
 
 /* Profiling hook (bench.py's roofline measurement): while set (non-NULL cudaEvent_t handles), every
  * sfm_loss_* call on this thread records `start` right before and `stop` right after the fused loss
@@ -337,6 +353,16 @@ int sfm_peer_connect(SfmPeer* peer, const void* all_handles);
 int sfm_peer_destroy(SfmPeer* peer);
 int sfm_loss_forward_backward_peer(const SfmDesc* desc, const SfmInputs* in, float* losses_out, const SfmGrads* grads,
                                    void* workspace, SfmPeer* peer, void* stream);
+
+/* losses_out = sum_b w_b * l_b (under `peer`: summed over the ranks as sfm_loss_forward_backward_peer does), and every
+ * gradient is that of losses_out[0].  grads == NULL: forward only.  igrads: as sfm_loss_forward_backward_images (needs
+ * SFM_FLAG_IMAGE_GRADS and grads; not with SFM_FLAG_EDGE_AWARE_SMOOTH).  peer: as sfm_loss_forward_backward_peer (may be
+ * NULL); terms->losses stays per rank.  A non-NULL member of `terms` needs SFM_FLAG_SNIPPET_TERMS in desc->flags (else
+ * SFM_E_INVALID_DESC); terms == NULL or both members NULL is the plain step of the same grads / igrads / peer.  The
+ * weighted sums run in fp64 in a fixed snippet order; with all weights 1 the gradients are bitwise those of the plain
+ * step and the losses agree to rounding.  sfm_intrinsics_grad after this call returns the weighted gradient. */
+int sfm_loss_snippets(const SfmDesc* desc, const SfmInputs* in, const SfmSnippetTerms* terms, float* losses_out,
+                      const SfmGrads* grads, const SfmImageGrads* igrads, void* workspace, SfmPeer* peer, void* stream);
 
 #ifdef __cplusplus
 }

@@ -166,7 +166,7 @@ int num_sms() {
 
 int run_loss(const SfmDesc* d, const SfmInputs* in, float* losses_out, const SfmGrads* grads, const float* gy,
              const SfmDebug* dbg, void* workspace, cudaStream_t st, const SfmPeerDev* peer = nullptr,
-             const SfmImageGrads* ig = nullptr) {
+             const SfmImageGrads* ig = nullptr, const SfmSnippetTerms* snip = nullptr) {
   int rc = sfm_validate_desc(d);
   if (rc) return rc;
   const bool reuse = (d->flags & SFM_FLAG_REUSE_PYRAMID) != 0;
@@ -251,6 +251,18 @@ int run_loss(const SfmDesc* d, const SfmInputs* in, float* losses_out, const Sfm
   sm.part = (float*)(ws + L.off_smpart);
   p.sm_part = sm.part;
   p.n_sm_part = sm.n_ctas;
+  if (snip) {
+    // per-snippet terms: the smoothness tasks write per-task losses instead of CTA partials (the epilogue sums each
+    // snippet's tasks), every other loss partial goes to its snippet's cells
+    p.snip_w = snip->weights;
+    p.snip_losses = snip->losses;
+    p.snip_cell0 = (int)L.snip_cell0;
+    p.n_sm_part = 0;
+    sm.snip_w = snip->weights;
+    sm.task_part = (float*)(ws + L.off_smtask);
+    p.sm_part = sm.task_part;
+    p.sm_hseg = sm.n_ctas > 0 ? sm.hseg : 0;
+  }
   SfmPrepParams pp = prep_params(d, plan.band, ws, reuse ? nullptr : in->tgt, in->src, in->intrinsics, in->poses,
                                  tables ? nullptr : (float*)(ws + L.off_proj), (float*)(ws + L.off_kinv), true);
   pp.n_mix_region = plan.n_mix_region;
@@ -259,7 +271,7 @@ int run_loss(const SfmDesc* d, const SfmInputs* in, float* losses_out, const Sfm
     SFM_CUDA_CHECK(cudaMemsetAsync(ig->gsrc, 0, (size_t)d->B * d->S * 3 * d->H * d->W * sizeof(float), st));
     if (L.gsrc_bytes) SFM_CUDA_CHECK(cudaMemsetAsync(ws + L.off_gsrc[1], 0, L.gsrc_bytes, st));
   }
-  rc = sfm_launch_prep(pp, &sm, grads ? 2 : 1, st);
+  rc = sfm_launch_prep(pp, &sm, (grads ? 2 : 1) + (snip ? 2 : 0), st);
   if (rc) return rc;
   return sfm_launch_fused(p, plan, st);
 }
@@ -312,6 +324,38 @@ extern "C" int sfm_loss_forward_backward_images(const SfmDesc* desc, const SfmIn
   if (!losses_out) { sfm_set_error("losses_out is NULL"); return SFM_E_NULL_POINTER; }
   if (!grads) { sfm_set_error("grads is NULL"); return SFM_E_NULL_POINTER; }
   return run_loss(desc, in, losses_out, grads, nullptr, nullptr, workspace, (cudaStream_t)stream, nullptr, igrads);
+}
+
+extern "C" int sfm_loss_snippets(const SfmDesc* desc, const SfmInputs* in, const SfmSnippetTerms* terms, float* losses_out,
+                                 const SfmGrads* grads, const SfmImageGrads* igrads, void* workspace, SfmPeer* peer,
+                                 void* stream) {
+  int rc = sfm_validate_desc(desc);
+  if (rc) return rc;
+  const bool snip = terms && (terms->weights || terms->losses);
+  if (snip && !(desc->flags & SFM_FLAG_SNIPPET_TERMS)) {
+    sfm_set_error("sfm_loss_snippets: desc->flags lacks SFM_FLAG_SNIPPET_TERMS (the workspace must be sized with it)");
+    return SFM_E_INVALID_DESC;
+  }
+  if (igrads) {
+    if (!(desc->flags & SFM_FLAG_IMAGE_GRADS)) {
+      sfm_set_error("sfm_loss_snippets: igrads given but desc->flags lacks SFM_FLAG_IMAGE_GRADS (the workspace must be sized with it)");
+      return SFM_E_INVALID_DESC;
+    }
+    if (desc->flags & SFM_FLAG_EDGE_AWARE_SMOOTH) {
+      sfm_set_error("unsupported: image gradients through the edge-aware smoothness term (SFM_FLAG_EDGE_AWARE_SMOOTH)");
+      return SFM_E_UNSUPPORTED;
+    }
+    if (!igrads->gtgt && !igrads->gsrc) { sfm_set_error("igrads has neither gtgt nor gsrc"); return SFM_E_NULL_POINTER; }
+    if (!grads) { sfm_set_error("sfm_loss_snippets: igrads needs grads"); return SFM_E_NULL_POINTER; }
+  }
+  if (!losses_out) { sfm_set_error("losses_out is NULL"); return SFM_E_NULL_POINTER; }
+  const SfmPeerDev* dev = nullptr;
+  if (peer && !(dev = sfm_peer_dev(peer))) {
+    sfm_set_error("sfm_loss_snippets: the peer object is not connected (sfm_peer_connect)");
+    return SFM_E_UNSUPPORTED;
+  }
+  return run_loss(desc, in, losses_out, grads, nullptr, nullptr, workspace, (cudaStream_t)stream, dev, igrads,
+                  snip ? terms : nullptr);
 }
 
 extern "C" int sfm_scale_image_grads(const SfmDesc* desc, const float* gy, const SfmImageGrads* igrads, void* stream) {

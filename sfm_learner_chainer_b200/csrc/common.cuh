@@ -37,9 +37,12 @@ struct SfmWsLayout {
   size_t off_src[SFM_MAX_SCALES];  // float [B*S][3][h][w]
   size_t off_proj;                 // float  [B][S][ns][12]  3x4 projection K4.T
   size_t off_kinv;                 // float  [B][ns][9]
-  size_t off_acc;                  // double [4 + B*S*ns*12] loss sums (pixel, smooth, exp, ssim) + dL/dP per scale
+  size_t off_acc;                  // double [4 + B*S*ns*12 (+ 4*B)] loss sums (pixel, smooth, exp, ssim) + dL/dP per scale
+                                   // (+ with SFM_FLAG_SNIPPET_TERMS the four loss sums of every snippet, at snip_cell0)
+  size_t snip_cell0;               // index of snippet 0's pixel cell in the fp64 cells (0 without the flag)
   size_t off_posevec;              // float  [B][S][6]   6-DoF vectors reduced from the raw `poseout` map (raw_pose_hw > 0)
   size_t off_smpart;               // float  [tasks / 8] loss partials of the smoothness CTAs of the prologue kernel
+  size_t off_smtask;               // SFM_FLAG_SNIPPET_TERMS: float [tasks] loss of every smoothness task (0 without the flag)
   // SFM_FLAG_IMAGE_GRADS: fp32 gradient levels of the pyramid (scales >= 1), sized like it: all source levels back to
   // back (one memset clears them), then the target levels.  0 without the flag.
   size_t off_gsrc[SFM_MAX_SCALES];  // float [B*S][3][h][w]
@@ -95,13 +98,24 @@ static inline void sfm_ws_layout(const SfmDesc* d, SfmWsLayout* L) {
   L->off_kinv = off;
   off = sfm_align_up(off + (size_t)d->B * d->n_scales * 9 * sizeof(float), 256);
   L->acc_doubles = 4 + (size_t)d->B * d->S * d->n_scales * 12;
+  L->snip_cell0 = 0;
+  if (d->flags & SFM_FLAG_SNIPPET_TERMS) {
+    L->snip_cell0 = L->acc_doubles;
+    L->acc_doubles += 4 * (size_t)d->B;
+  }
   L->off_acc = off;
   off += L->acc_doubles * sizeof(double);
   off = sfm_align_up(off, 256);
   L->off_posevec = off;
   off = sfm_align_up(off + (size_t)d->B * d->S * 6 * sizeof(float), 256);
   L->off_smpart = off;
-  off = sfm_align_up(off + (size_t)((sfm_smooth_plan(d->B, d->n_scales, d->H, d->W, nullptr) + 7) / 8) * sizeof(float), 256);
+  const int n_sm_tasks = sfm_smooth_plan(d->B, d->n_scales, d->H, d->W, nullptr);
+  off = sfm_align_up(off + (size_t)((n_sm_tasks + 7) / 8) * sizeof(float), 256);
+  L->off_smtask = 0;
+  if (d->flags & SFM_FLAG_SNIPPET_TERMS) {
+    L->off_smtask = off;
+    off = sfm_align_up(off + (size_t)n_sm_tasks * sizeof(float), 256);
+  }
   for (int s = 0; s < SFM_MAX_SCALES; ++s) L->off_gsrc[s] = L->off_gtgt[s] = 0;
   L->gsrc_bytes = 0;
   if (d->flags & SFM_FLAG_IMAGE_GRADS) {

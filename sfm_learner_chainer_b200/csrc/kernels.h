@@ -40,9 +40,13 @@ struct SfmSmoothParams {
   const float* gy;
   unsigned raw_disp_mask;
   float* part;       // [n_ctas] loss partials (workspace)
+  // per-snippet terms (sm_mode 3 / 4): the gradient factor of snippet b is gy * snip_w[b] (snip_w nullptr: gy), and each
+  // task t writes its loss to task_part[t] instead of the CTA partial (a CTA's tasks may belong to different snippets)
+  const float* snip_w;
+  float* task_part;
 };
 
-// sm_mode: 0 = no smoothness tasks, 1 = loss only, 2 = loss + gdisp
+// sm_mode: 0 = no smoothness tasks, 1 = loss only, 2 = loss + gdisp; 3 / 4 = 1 / 2 with per-task losses (task_part)
 int sfm_launch_prep(const SfmPrepParams& p, const SfmSmoothParams* sm, int sm_mode, cudaStream_t stream);
 int sfm_launch_ingest_u8(int B, int S, int H, int W, int ns, const uint8_t* frames, const float* K_in, const SfmAugment* aug,
                          float* tgt, float* src, float* K_out, cudaStream_t stream);   // ingest.cu
@@ -99,7 +103,7 @@ struct SfmFusedParams {
   unsigned raw_disp_mask;   // bit s: disp[s] is pre-activation, gdisp[s] the gradient w.r.t. it
   const float* gy;          // upstream gradient (device scalar) or nullptr
   double* acc;              // [4 + B*S*ns*12]
-  const float* sm_part;     // loss partials of the smoothness CTAs of the prologue kernel
+  const float* sm_part;     // loss partials of the smoothness CTAs of the prologue kernel (per-snippet terms: of its tasks)
   int n_sm_part;
   SfmPeerDev peer;          // nranks > 0: losses_out receives the sums over all ranks (epilogue kernel)
   float* losses_out;        // [5] or nullptr
@@ -125,6 +129,15 @@ struct SfmFusedParams {
   // zeroed before the step and accumulated with fp32 reductions; gtgt is owned like gdisp (stored by the first pass).
   float* gtgt[SFM_MAX_SCALES];      // [B][3][h][w]
   float* gsrc[SFM_MAX_SCALES];      // [B*S][3][h][w]
+  // per-snippet terms (sfm_loss_snippets; snip_cell0 == 0 when off).  The gradient factor of snippet b's tasks is
+  // gy * snip_w[b] (snip_w nullptr: gy); its loss partials go to cells acc[snip_cell0 + 4b + k] (pixel, smooth, exp, ssim)
+  // instead of acc[k], and the epilogue forms losses_out = sum_b w_b * cells_b and the rows snip_losses[b][5]
+  const float* snip_w;
+  float* snip_losses;               // [B][5] or nullptr
+  int snip_cell0;
+  // per-snippet terms: segment height of the prologue's smoothness tasks, whose losses sm_part then holds one per task
+  // (0: no such tasks).  Their order is the planner's (plan_smooth): per scale, per snippet, strips x segments.
+  int sm_hseg;
 };
 
 // Launch helper: with pdl the kernel is a programmatic dependent launch on the previous kernel of the stream (its

@@ -35,7 +35,8 @@ struct PrepRow {
 // latter spread evenly over the first R = n_mix_region blocks (block i < R is a smoothness CTA when
 // floor((i+1) n_sm / R) > floor(i n_sm / R)): the long, issue-bound smoothness CTAs start early and the short,
 // memory-bound pyramid CTAs fill the SMs around them and run on alone at the end.
-// SM: 0 = no smoothness tasks, 1 = loss only, 2 = loss and gdisp.  No early programmatic-launch trigger: the dependent
+// SM: 0 = no smoothness tasks, 1 = loss only, 2 = loss and gdisp; 3 / 4 = 1 / 2 with per-task losses instead of the CTA
+// partial (a CTA's tasks may belong to different snippets).  No early programmatic-launch trigger: the dependent
 // fused kernel's CTAs would pile up on whichever SMs are free first (measured, see the launch policy notes in DESIGN.md).
 template <int SM>
 __global__ void __launch_bounds__(kPrepThreads) sfm_prep_kernel(const __grid_constant__ SfmPrepParams p,
@@ -96,6 +97,10 @@ __global__ void __launch_bounds__(kPrepThreads) sfm_prep_kernel(const __grid_con
       __shared__ float s_part[kPrepThreads / 32];
       const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
       const int t = k0 * (kPrepThreads / 32) + warp;
+      if (SM >= 3) {
+        if (t < sm.n_tasks) sfm_smooth_task<SM == 4, true>(sm, t, lane);
+        return;
+      }
       float loss = (t < sm.n_tasks) ? sfm_smooth_task<SM == 2>(sm, t, lane) : 0.f;
       loss = sfm_warp_sum(loss);
       if (lane == 0) s_part[warp] = loss;
@@ -209,7 +214,8 @@ int sfm_launch_prep(const SfmPrepParams& p_in, const SfmSmoothParams* sm_in, int
   p.n_tail_blocks = (int)((n_tail + kPrepThreads - 1) / kPrepThreads);
   const unsigned grid = (unsigned)(p.n_tail_blocks + p.n_pyr_blocks + (sm_mode ? sm.n_ctas : 0));
   if (grid == 0) return 0;                        // e.g. sfm_pyramid with a single scale: nothing to build
-  const auto kernel = sm_mode == 2 ? sfm_prep_kernel<2> : sm_mode == 1 ? sfm_prep_kernel<1> : sfm_prep_kernel<0>;
+  const auto kernel = sm_mode == 4 ? sfm_prep_kernel<4> : sm_mode == 3 ? sfm_prep_kernel<3> : sm_mode == 2 ? sfm_prep_kernel<2>
+                    : sm_mode == 1 ? sfm_prep_kernel<1> : sfm_prep_kernel<0>;
   SFM_CUDA_CHECK(sfm_launch_kernel(kernel, grid, kPrepThreads, stream, false, p, sm));
   return 0;
 }

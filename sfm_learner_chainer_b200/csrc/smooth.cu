@@ -27,7 +27,8 @@ namespace {
 // gather form: its right / down differences give the loss terms it owns, and together with the left / up ones
 // the gradient, so there is no scatter and no atomic on gdisp.  Needs the pyramid, so unlike the second-order
 // kernel above it starts after the prep kernel.
-template <bool GRAD>
+// SNIP: per-snippet terms (gradient factor gy * w_b, the loss to snippet b's smooth cell), an instance of its own.
+template <bool GRAD, bool SNIP>
 __global__ void __launch_bounds__(256) sfm_edge_smooth_kernel(const __grid_constant__ SfmFusedParams p) {
   const int s = blockIdx.y % p.ns, b = blockIdx.y / p.ns;
   const int h = p.h[s], w = p.w[s], plane = h * w;
@@ -36,7 +37,8 @@ __global__ void __launch_bounds__(256) sfm_edge_smooth_kernel(const __grid_const
   const float* __restrict__ T = p.tgt_pl[s] + (size_t)b * 3 * plane;      // planar (3, h, w)
   float* __restrict__ G = GRAD ? p.gdisp[s] + (size_t)b * plane : nullptr;
   const float kx = p.sm_ex[s], ky = p.sm_ey[s];
-  const float gyv = (GRAD && p.gy) ? __ldg(p.gy) : 1.f;
+  float gyv = (GRAD && p.gy) ? __ldg(p.gy) : 1.f;
+  if (SNIP && GRAD && p.snip_w) gyv *= __ldg(p.snip_w + b);
   cudaGridDependencySynchronize();          // pyramid and loss cells (prep kernel)
   auto disp_at = [&](int i, float& f) {
     const float v = __ldg(D + i);
@@ -80,7 +82,7 @@ __global__ void __launch_bounds__(256) sfm_edge_smooth_kernel(const __grid_const
   if (threadIdx.x == 0) {
     float t = 0.f;
     for (int k = 0; k < 8; ++k) t += part[k];
-    if (t != 0.f) atomicAdd(p.acc + 1, (double)t);
+    if (t != 0.f) atomicAdd(p.acc + (SNIP ? p.snip_cell0 + 4 * (size_t)b + 1 : 1), (double)t);
   }
 }
 
@@ -89,6 +91,8 @@ __global__ void __launch_bounds__(256) sfm_edge_smooth_kernel(const __grid_const
 int sfm_launch_edge_smooth(const SfmFusedParams& p, bool grad, cudaStream_t stream) {
   const int per = (p.h[0] * p.w[0] + 255) / 256;
   const dim3 grid((unsigned)(per > 32 ? 32 : per), (unsigned)(p.B * p.ns));
-  SFM_CUDA_CHECK(sfm_launch_kernel(grad ? sfm_edge_smooth_kernel<true> : sfm_edge_smooth_kernel<false>, grid, 256, stream, true, p));
+  const auto kernel = p.snip_cell0 ? (grad ? sfm_edge_smooth_kernel<true, true> : sfm_edge_smooth_kernel<false, true>)
+                                    : (grad ? sfm_edge_smooth_kernel<true, false> : sfm_edge_smooth_kernel<false, false>);
+  SFM_CUDA_CHECK(sfm_launch_kernel(kernel, grid, 256, stream, true, p));
   return 0;
 }

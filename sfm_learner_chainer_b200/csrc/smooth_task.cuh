@@ -10,10 +10,12 @@ namespace {
 
 constexpr int SM_IW = SFM_SMOOTH_IW;         // interior columns per strip
 
-// -> this lane's part of the task's loss (to be summed over the warp by the caller)
-template <bool GRAD>
+// -> this lane's part of the task's loss (to be summed over the warp by the caller).  SNIP: the warp writes the task's loss
+// to p.task_part[t] instead and 0 is returned.
+template <bool GRAD, bool SNIP = false>
 __device__ __forceinline__ float sfm_smooth_task(const SfmSmoothParams& p, int t, const int lane) {
   // ---- task decode (uniform): strips x row segments of every (snippet, scale)
+  const int t_task = t;
   int s = 0;
 #pragma unroll
   for (int q = 1; q < SFM_MAX_SCALES; ++q)
@@ -31,7 +33,8 @@ __device__ __forceinline__ float sfm_smooth_task(const SfmSmoothParams& p, int t
   const float* __restrict__ D = p.disp[s] + (size_t)b * h * w;
   float* __restrict__ G = GRAD ? p.gdisp[s] + (size_t)b * h * w : nullptr;
   const float k_dx2 = p.k_dx2[s], k_mix = p.k_mix[s], k_dy2 = p.k_dy2[s];
-  const float gyv = (GRAD && p.gy) ? __ldg(p.gy) : 1.f;
+  float gyv = (GRAD && p.gy) ? __ldg(p.gy) : 1.f;
+  if (SNIP && GRAD && p.snip_w) gyv *= __ldg(p.snip_w + b);
   const bool x_dx2 = col_in && (xx <= w - 3);          // dx2(., xx) exists
   const bool x_mix = col_in && (xx <= w - 2);          // cell (., xx) exists
   float loss = 0.f;
@@ -91,6 +94,11 @@ __device__ __forceinline__ float sfm_smooth_task(const SfmSmoothParams& p, int t
     sy4 = sy3; sy3 = sy2;
     n3 = n2; n2 = n1;
     gx2 = gx1; gx1 = gx0;
+  }
+  if (SNIP) {
+    loss = sfm_warp_sum(loss);
+    if (lane == 0) p.task_part[t_task] = loss;
+    return 0.f;
   }
   return loss;
 }

@@ -99,7 +99,8 @@ enum RowStages {
 // L1 part: one more gradient field in the ring.  The task owns gtgt like gdisp (stored by the first source, then
 // accumulated); dL/dP is scattered to the four taps of every in-view pixel with fp32 reductions, from the tap index
 // and the two fractions the forward record carries in three more fields.
-template <bool GRAD, bool ACCUM, bool DEBUG, bool RAW, int NW, bool SREC = true, bool IMG = false>
+// SNIP: per-snippet terms, as in sfm_l1_march_kernel.
+template <bool GRAD, bool ACCUM, bool DEBUG, bool RAW, int NW, bool SREC = true, bool IMG = false, bool SNIP = false>
 __global__ void __launch_bounds__(32 * NW, (IMG ? SFM_SSIM_IMG_MIN_WARPS : SREC ? SFM_SSIM_MIN_WARPS : SFM_SSIM_REG_MIN_WARPS) / NW)
 sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
   static_assert(!IMG || (GRAD && NW == 1 && SREC), "image gradients: GRAD, one warp per CTA, shared-memory records");
@@ -133,7 +134,8 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
   const int xx = t.x0 - 2 + lane;                       // this lane's image column (may be outside)
   const bool col_in = (xx >= 0) && (xx < w);
   const bool col_own = (lane >= 2) && (lane < 2 + SFM_SSIM_IW) && (xx < w);
-  const float gyv = p.gy ? __ldg(p.gy) : 1.f;
+  float gyv = p.gy ? __ldg(p.gy) : 1.f;
+  if (SNIP && p.snip_w) gyv *= __ldg(p.snip_w + b);        // per-snippet weight
   const float inv_n3 = p.inv_n3[s];
   const float wpix = gyv * (1.f - p.ssim_rate) * inv_n3;
   const float wssim = gyv * p.ssim_rate * inv_n3;
@@ -528,7 +530,7 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
           acc[k * 4 + 3] = accC[k];
         }
       }
-      flush_dP(p, acc, b, i, s, lane, last ? pix_part * inv_n3 : 0.f, last ? ssim_part * inv_n3 : 0.f, 0.f, 0, 3, -1, GRAD);
+      flush_dP<SNIP>(p, acc, b, i, s, lane, last ? pix_part * inv_n3 : 0.f, last ? ssim_part * inv_n3 : 0.f, 0.f, 0, 3, -1, GRAD);
     }
   }
 }

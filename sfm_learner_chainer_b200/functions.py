@@ -27,15 +27,23 @@ class ViewSynthesisLoss(object):
     total w.r.t. the two images (for images that come out of a differentiable module); not with edge_aware_smooth.
     intrinsics_grad: forward_backward and backward also return gintrinsics (B,n_scales,3,3), the gradient of the
     reported total w.r.t. `intrinsics` (for a camera that is learned); not with caller-supplied proj / kinv.
+    snippet_terms: forward and forward_backward take `snippet_weights` (B,) float32 device array w (None = all 1) and
+    also return the per-snippet losses (B,5) l_b = total, pixel, smooth, exp, ssim of snippet b (unweighted, with the
+    1/B_global means); the five losses are then sum_b w_b * l_b and every gradient is that of their total.  The
+    weights are device data, so a CUDA graph captured for B snippets can run a batch of B_real < B: fill the padding
+    with copies of a real snippet (a zero disparity gives NaN, and NaN * 0 is NaN), keep B_global = B and pass
+    w_b = B / B_real for the real snippets and 0 for the padding; that gives the loss and gradients of the B_real batch
+    up to rounding.  d total / d w_b = l_b[0] (the torch adapter returns it as the weights' gradient).
     """
 
     def __init__(self, smooth_reg=0.0, exp_reg=0.0, ssim_rate=0.0, n_scales=N_SCALES, B_global=None,
                  raw_disp_scales=0, raw_pose=False, edge_aware_smooth=False, image_grads=False,
-                 intrinsics_grad=False):
+                 intrinsics_grad=False, snippet_terms=False):
         if image_grads and edge_aware_smooth:
             raise ValueError('image_grads is not supported together with edge_aware_smooth')
         self.image_grads = bool(image_grads)
         self.intrinsics_grad = bool(intrinsics_grad)
+        self.snippet_terms = bool(snippet_terms)
         # edge_aware_smooth: smoothness term = compute_disp_smooth (base_model.py:144-155, commented out at :78-80)
         self.edge_aware_smooth = bool(edge_aware_smooth)
         self.raw_disp_scales = int(raw_disp_scales)
@@ -60,12 +68,15 @@ class ViewSynthesisLoss(object):
             flags |= L.SFM_FLAG_EDGE_AWARE_SMOOTH
         if self.image_grads:
             flags |= L.SFM_FLAG_IMAGE_GRADS
+        if self.snippet_terms:
+            flags |= L.SFM_FLAG_SNIPPET_TERMS
         return L.SfmDesc(B, S, H, W, self.n_scales, int(self.B_global or 0), self.smooth_reg, self.exp_reg,
                          self.ssim_rate, flags, self.raw_disp_scales, raw_pose_hw)
 
     def _workspace(self, desc, like):
-        # the image-gradient flag sizes the workspace; the per-call flags (tables, reused pyramid) do not
-        key = (desc.B, desc.S, desc.H, desc.W, desc.n_scales, desc.flags & L.SFM_FLAG_IMAGE_GRADS, str(getattr(like, 'device', '')))
+        # the image-gradient and snippet-terms flags size the workspace; the per-call flags (tables, reused pyramid) do not
+        key = (desc.B, desc.S, desc.H, desc.W, desc.n_scales, desc.flags & (L.SFM_FLAG_IMAGE_GRADS | L.SFM_FLAG_SNIPPET_TERMS),
+               str(getattr(like, 'device', '')))
         ws = self._ws.get(key)
         if ws is None:
             n = self._lib.sfm_workspace_bytes(C.byref(desc))
@@ -148,11 +159,33 @@ class ViewSynthesisLoss(object):
             L.check(self._lib.sfm_intrinsics_grad(C.byref(desc), C.byref(inp), self._workspace(desc, tgt),
                                                   _vp(out['gintrinsics']), C.c_void_p(D.current_stream(tgt))))
 
+    def _snippet_terms(self, desc, tgt, snippet_weights):
+        """-> (SfmSnippetTerms or None, snippet losses (B,5) or None)."""
+        if not self.snippet_terms:
+            if snippet_weights is not None:
+                raise ValueError('snippet_weights needs ViewSynthesisLoss(snippet_terms=True)')
+            return None, None
+        if snippet_weights is not None:
+            D.check_array(snippet_weights, 'snippet_weights', (desc.B,))
+        rows = D.empty(tgt, (desc.B, 5))
+        return L.SfmSnippetTerms(_vp(snippet_weights), _vp(rows)), rows
+
     # ---- operators
-    def forward(self, tgt, src, intrinsics, disps, poses, logits=None, proj=None, kinv=None, debug=False):
-        """-> losses (5,) device array in the order of lib.LOSS_KEYS [, debug dict]."""
+    def forward(self, tgt, src, intrinsics, disps, poses, logits=None, proj=None, kinv=None, debug=False,
+                snippet_weights=None):
+        """-> losses (5,) device array in the order of lib.LOSS_KEYS [, debug dict].
+        With the operator's snippet_terms: -> (losses, snippet losses (B,5)), losses = sum_b w_b * l_b."""
+        if debug and self.snippet_terms:
+            raise ValueError('debug dumps are not available on an operator with snippet_terms')
         desc, inp = self._pack(tgt, src, intrinsics, disps, poses, logits, proj, kinv)
         losses = D.empty(tgt, (5,))
+        if self.snippet_terms:
+            terms, rows = self._snippet_terms(desc, tgt, snippet_weights)
+            L.check(self._lib.sfm_loss_snippets(C.byref(desc), C.byref(inp), C.byref(terms), _vp(losses), None, None,
+                                                self._workspace(desc, tgt), None, C.c_void_p(D.current_stream(tgt))))
+            return losses, rows
+        if snippet_weights is not None:
+            raise ValueError('snippet_weights needs ViewSynthesisLoss(snippet_terms=True)')
         dbg_struct, dbg = None, None
         if debug:
             B, S, H, W = desc.B, desc.S, desc.H, desc.W
@@ -201,14 +234,17 @@ class ViewSynthesisLoss(object):
         self._ev_pyramid = D.record_event(tgt)
 
     def forward_backward(self, tgt, src, intrinsics, disps, poses, logits=None, proj=None, kinv=None, reuse_pyramid=False,
-                         peer=None, image_grads=('tgt', 'src'), intrinsics_grad=True):
+                         peer=None, image_grads=('tgt', 'src'), intrinsics_grad=True, snippet_weights=None):
         """Single fused pass: -> (losses (5,), dict(gdisps, gposes, glogits)) for upstream gradient 1.
         reuse_pyramid: the workspace already holds this batch's pyramid (build_pyramid).
         peer: a distributed.PeerLossSum -- the batch is sharded by snippet over several GPUs (B_global set) and the
         epilogue kernel completes the five losses across the ranks over NVLink peer memory.
         With the operator's image_grads the dict also holds gtgt and gsrc (None for an image left out of
-        `image_grads`, a subset of ('tgt', 'src'); an empty one runs the plain pass); not with peer.
-        With the operator's intrinsics_grad the dict also holds gintrinsics (None when `intrinsics_grad` is False)."""
+        `image_grads`, a subset of ('tgt', 'src'); an empty one runs the plain pass).
+        With the operator's intrinsics_grad the dict also holds gintrinsics (None when `intrinsics_grad` is False).
+        With the operator's snippet_terms: snippet_weights (B,) (None = all 1; under peer the local shard's) weight the
+        snippets, the losses are sum_b w_b * l_b, every gradient is that of their total, and the dict also holds
+        snippet_losses (B,5), this shard's rows l_b."""
         want_k = self._want_intrinsics_grad(intrinsics_grad, proj, kinv)
         desc, inp = self._pack(tgt, src, intrinsics, disps, poses, logits, proj, kinv)
         if reuse_pyramid:
@@ -216,26 +252,21 @@ class ViewSynthesisLoss(object):
             D.wait_event(tgt, self._ev_pyramid)     # build_pyramid may have run on another stream
         g, out = self._alloc_grads(desc, tgt)
         losses = D.empty(tgt, (5,))
+        terms, rows = self._snippet_terms(desc, tgt, snippet_weights)
+        if rows is not None:
+            out['snippet_losses'] = rows
+        ig = None
         want = set(image_grads) if self.image_grads else set()
         if want:
-            if peer is not None:
-                raise ValueError('image_grads is not supported with peer')
             if not want <= {'tgt', 'src'}:
                 raise ValueError("image_grads must be a subset of ('tgt', 'src')")
             out['gtgt'] = D.empty(tgt, (desc.B, 3, desc.H, desc.W)) if 'tgt' in want else None
             out['gsrc'] = D.empty(tgt, (desc.B, desc.S, 3, desc.H, desc.W)) if 'src' in want else None
             ig = L.SfmImageGrads(_vp(out['gtgt']), _vp(out['gsrc']))
-            L.check(self._lib.sfm_loss_forward_backward_images(C.byref(desc), C.byref(inp), _vp(losses), C.byref(g),
-                                                               C.byref(ig), self._workspace(desc, tgt),
-                                                               C.c_void_p(D.current_stream(tgt))))
-        elif peer is not None:
-            L.check(self._lib.sfm_loss_forward_backward_peer(C.byref(desc), C.byref(inp), _vp(losses), C.byref(g),
-                                                             self._workspace(desc, tgt), peer.handle,
-                                                             C.c_void_p(D.current_stream(tgt))))
-        else:
-            L.check(self._lib.sfm_loss_forward_backward(C.byref(desc), C.byref(inp), _vp(losses), C.byref(g),
-                                                        self._workspace(desc, tgt),
-                                                        C.c_void_p(D.current_stream(tgt))))
+        # one entry point for every combination of image gradients, peer sum and snippet terms
+        L.check(self._lib.sfm_loss_snippets(C.byref(desc), C.byref(inp), C.byref(terms) if terms else None, _vp(losses),
+                                            C.byref(g), C.byref(ig) if ig else None, self._workspace(desc, tgt),
+                                            peer.handle if peer is not None else None, C.c_void_p(D.current_stream(tgt))))
         self._intrinsics_grad(desc, inp, tgt, out, want_k)
         if self._ev_pyramid is not None:
             self._ev_loss = D.record_event(tgt)

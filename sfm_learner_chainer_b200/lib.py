@@ -13,6 +13,7 @@ SFM_FLAG_REUSE_PYRAMID = 0x2
 SFM_FLAG_NO_TMA = 0x4
 SFM_FLAG_EDGE_AWARE_SMOOTH = 0x8
 SFM_FLAG_IMAGE_GRADS = 0x10
+SFM_FLAG_SNIPPET_TERMS = 0x20
 
 SFM_E_INVALID_DESC = -1
 SFM_E_INVALID_SHAPE = -2
@@ -48,6 +49,10 @@ class SfmImageGrads(C.Structure):
     _fields_ = [('gtgt', _vp), ('gsrc', _vp)]
 
 
+class SfmSnippetTerms(C.Structure):
+    _fields_ = [('weights', _vp), ('losses', _vp)]
+
+
 class SfmAugment(C.Structure):
     _fields_ = [('out_h', C.c_int32), ('out_w', C.c_int32), ('off_y', C.c_int32), ('off_x', C.c_int32),
                 ('flip', C.c_int32), ('reserved_', C.c_int32), ('x_scaling', C.c_double), ('y_scaling', C.c_double)]
@@ -62,6 +67,7 @@ class SfmDebug(C.Structure):
 _i = C.c_int
 _D, _I, _G, _Dbg = C.POINTER(SfmDesc), C.POINTER(SfmInputs), C.POINTER(SfmGrads), C.POINTER(SfmDebug)
 _IG = C.POINTER(SfmImageGrads)
+_ST = C.POINTER(SfmSnippetTerms)
 SYMBOLS = {
     'sfm_version': (_i, []),
     'sfm_last_error': (C.c_char_p, []),
@@ -104,6 +110,7 @@ SYMBOLS = {
     'sfm_peer_connect': (_i, [_vp, _vp]),
     'sfm_peer_destroy': (_i, [_vp]),
     'sfm_loss_forward_backward_peer': (_i, [_D, _I, _vp, _G, _vp, _vp, _vp]),
+    'sfm_loss_snippets': (_i, [_D, _I, _ST, _vp, _G, _IG, _vp, _vp, _vp]),
 }
 
 _lib = None

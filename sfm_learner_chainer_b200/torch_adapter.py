@@ -10,7 +10,7 @@ from .functions import ViewSynthesisLoss
 
 class _ViewSynthesisLossFn(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, op, tgt, src, intrinsics, n_scales, use_exp, *preds):
+    def forward(ctx, op, tgt, src, intrinsics, weights, n_scales, use_exp, *preds):
         disps = [p.contiguous() for p in preds[:n_scales]]
         poses = preds[n_scales].contiguous()
         logits = [p.contiguous() for p in preds[n_scales + 1:]] if use_exp else None
@@ -23,16 +23,24 @@ class _ViewSynthesisLossFn(torch.autograd.Function):
         losses, grads = op.forward_backward(tgt.detach().contiguous(), src.detach().contiguous(),
                                             intrinsics.detach().contiguous(), [d.detach() for d in disps], poses.detach(),
                                             [l.detach() for l in logits] if logits else None, image_grads=want,
-                                            intrinsics_grad=ctx.want_k)
+                                            intrinsics_grad=ctx.want_k,
+                                            snippet_weights=weights.detach().contiguous() if weights is not None else None)
         ctx.op, ctx.grads, ctx.shape = op, grads, tuple(src.shape)
         ctx.n_scales, ctx.use_exp = n_scales, use_exp
         ctx.consumed = False
+        if op.snippet_terms:
+            # d total / d w_b = l_b[0]: the weights' gradient needs the rows alone
+            ctx.want_w = weights is not None and ctx.needs_input_grad[4]
+            ctx.rows = grads['snippet_losses']
+            ctx.mark_non_differentiable(losses, ctx.rows)
+            return losses[0].clone(), losses, ctx.rows
+        ctx.want_w = False
         ctx.mark_non_differentiable(losses)
         return losses[0].clone(), losses
 
     @staticmethod
     @torch.autograd.function.once_differentiable
-    def backward(ctx, gy, _g_losses):
+    def backward(ctx, gy, *_g_rest):
         # The gradients were produced by the forward's fused pass and are rescaled IN PLACE by the upstream gradient;
         # a second backward through the same node (retain_graph=True) would rescale them again, so it is refused.
         if ctx.consumed:
@@ -42,6 +50,7 @@ class _ViewSynthesisLossFn(torch.autograd.Function):
         B, S, _, H, W = ctx.shape
         g = ctx.grads
         gy = gy.to(torch.float32).reshape(1).contiguous()
+        gw = gy * ctx.rows[:, 0] if ctx.want_w else None
         ctx.op.scale_grads(g, gy, B, S, H, W)            # no-op on the device when gy == 1
         out = list(g['gdisps']) + [g['gposes']]
         if ctx.use_exp:
@@ -49,17 +58,22 @@ class _ViewSynthesisLossFn(torch.autograd.Function):
         gtgt = g.get('gtgt') if ctx.want_tgt else None
         gsrc = g.get('gsrc') if ctx.want_src else None
         gk = g.get('gintrinsics') if ctx.want_k else None
-        return (None, gtgt, gsrc, gk, None, None) + tuple(out)
+        return (None, gtgt, gsrc, gk, gw, None, None) + tuple(out)
 
 
-def view_synthesis_loss(op, tgt, src, intrinsics, pred_disps, pred_poses, pred_maskes=None):
+def view_synthesis_loss(op, tgt, src, intrinsics, pred_disps, pred_poses, pred_maskes=None, snippet_weights=None):
     """-> (total_loss scalar tensor with grad_fn, losses (5,) tensor [total, pixel, smooth, exp, ssim]).
 
     pred_poses: (B,S,6) tensor or a tuple of S (B,6) tensors as PoseNet returns them (pose_net.py:52-54).
+    With op.snippet_terms: -> (total, losses, snippet_losses (B,5)); snippet_weights (B,) (None = all 1) weight the
+    snippets, total = sum_b w_b * snippet_losses[b, 0], the other inputs' gradients are the weighted ones, and weights
+    that require grad receive gy * snippet_losses[:, 0].  See ViewSynthesisLoss for padding a captured batch.
     """
     assert isinstance(op, ViewSynthesisLoss)
+    if snippet_weights is not None and not op.snippet_terms:
+        raise ValueError('snippet_weights needs ViewSynthesisLoss(snippet_terms=True)')
     if isinstance(pred_poses, (tuple, list)):
         pred_poses = torch.stack(list(pred_poses), dim=1)
     use_exp = op.use_exp
     preds = list(pred_disps) + [pred_poses] + (list(pred_maskes) if use_exp else [])
-    return _ViewSynthesisLossFn.apply(op, tgt, src, intrinsics, op.n_scales, use_exp, *preds)
+    return _ViewSynthesisLossFn.apply(op, tgt, src, intrinsics, snippet_weights, op.n_scales, use_exp, *preds)

@@ -1,12 +1,13 @@
-"""Step time of the fused loss with and without one opt-in gradient: image_grads (ViewSynthesisLoss(image_grads=True))
-or intrinsics_grad (ViewSynthesisLoss(intrinsics_grad=True)).
+"""Step time of the fused loss with and without one opt-in option: image_grads (ViewSynthesisLoss(image_grads=True)),
+intrinsics_grad (ViewSynthesisLoss(intrinsics_grad=True)) or snippet_terms (ViewSynthesisLoss(snippet_terms=True) with
+per-snippet weights, returning the per-snippet losses).
 
 For each config the step (forward_backward on device tensors) is captured four times into one CUDA graph and the graph
 is replayed; the two variants alternate, and the median over the repeats is reported per step.  Prints one JSON line
 per config and writes them all, with the card name and its power limit, to the file given as the first argument.
 The last column is the relative overhead for image_grads and the added microseconds for intrinsics_grad (the cost of
-one extra dependent launch, sfm_intrinsics_grad_kernel).
-usage: python tools/time_opt_in_grads.py OUT.json {image_grads,intrinsics_grad} [cfg ...]"""
+one extra dependent launch, sfm_intrinsics_grad_kernel) and for snippet_terms.
+usage: python tools/time_opt_in_grads.py OUT.json {image_grads,intrinsics_grad,snippet_terms} [cfg ...]"""
 import json
 import os
 import subprocess
@@ -24,6 +25,7 @@ STEPS_PER_GRAPH = 4
 LAST_COLUMN = {
     'image_grads': ('overhead', lambda p, q: round(q / p - 1.0, 4)),
     'intrinsics_grad': ('extra_us', lambda p, q: round(q - p, 2)),
+    'snippet_terms': ('extra_us', lambda p, q: round(q - p, 2)),
 }
 
 
@@ -33,17 +35,17 @@ def card():
     return q
 
 
-def make_graph(op, args):
+def make_graph(op, args, **kw):
     side = torch.cuda.Stream()
     graph = torch.cuda.CUDAGraph()
     with torch.cuda.stream(side):
         for _ in range(3):
-            losses, _ = op.forward_backward(*args)
+            losses, _ = op.forward_backward(*args, **kw)
         side.synchronize()
         assert torch.isfinite(losses).all()
         with torch.cuda.graph(graph, stream=side):
             for _ in range(STEPS_PER_GRAPH):
-                op.forward_backward(*args)
+                op.forward_backward(*args, **kw)
     torch.cuda.synchronize()
     return graph
 
@@ -75,7 +77,11 @@ def main():
                 [dev(x) for x in d['logits']] if c['exp_reg'] else None)
         # the operators own the workspaces the graphs write: they live as long as the graphs
         ops = {'plain': ViewSynthesisLoss(**flags), option: ViewSynthesisLoss(**{option: True}, **flags)}
-        graphs = {k: make_graph(op, args) for k, op in ops.items()}
+        # snippet_terms: weights of a padded batch (the last snippet weighs 0)
+        w = torch.full((c['B'],), 1.0, device='cuda')
+        w[-1] = 0.0
+        kw = {option: dict(snippet_weights=w)} if option == 'snippet_terms' else {}
+        graphs = {k: make_graph(op, args, **kw.get(k, {})) for k, op in ops.items()}
         replays = 10 if name == 'cfg5' else 200
         t = {k: [] for k in graphs}
         for _ in range(7):
