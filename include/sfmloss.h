@@ -364,6 +364,37 @@ int sfm_loss_forward_backward_peer(const SfmDesc* desc, const SfmInputs* in, flo
 int sfm_loss_snippets(const SfmDesc* desc, const SfmInputs* in, const SfmSnippetTerms* terms, float* losses_out,
                       const SfmGrads* grads, const SfmImageGrads* igrads, void* workspace, SfmPeer* peer, void* stream);
 
+/* Per-pixel weights and per-pixel loss maps (sfm_loss_weighted).  M_s = weights[s] is a (B,S,h_s,w_s) array laid out
+ * like logits[s]; it multiplies the per-pixel photometric terms of source i at scale s, broadcast over the 3 channels,
+ * and the means keep their denominators B_global*3*h*w (as the explainability weighting does):
+ *   pixel_loss += mean(E * sigma(l) * M)   (exp branch; mean(E * M) otherwise)
+ *   ssim_loss  += mean(clip((1 - SSIM) / 2, 0, 1) * (1 - m_zero) * M)
+ * The smoothness term and the explainability regulariser are not weighted.  Every gradient (gdisps, gposes, glogits and
+ * the dL/dP cells, hence sfm_intrinsics_grad) is that of the weighted total.  The loss is linear in M, so the map
+ *   losses[s][b,i,y,x] = d losses_out[0] / d M
+ *     = w_b * [ (1 - ssim_rate) * sigma(l) * sum_c E_c + ssim_rate * sum_c clip(raw_c, 0, 1) * (1 - m_zero) ] / (B_global*3*h_s*w_s)
+ * (sigma = 1 without the exp branch, the SSIM part only when SSIM runs, w_b the snippet weight or 1) is each pixel's
+ * share of the photometric loss: sum M * map = (1 - ssim_rate) * pixel + ssim_rate * ssim.  Uses: validity or semantic
+ * masks (moving objects, the ego-vehicle, rectification borders, sky), per-source confidence maps, learned weight maps
+ * (their gradient is the map), and per-pixel loss maps for validation and outlier search.  Any float weight is
+ * accepted, 0 and negative ones included; a non-finite weight propagates.  The maps are written with plain stores, each
+ * pixel once: bitwise reproducible from run to run. */
+typedef struct SfmPixelTerms {
+  const float* weights[SFM_MAX_SCALES];  /* (B,S,h_s,w_s) device, or NULL = 1 at that scale */
+  float* losses[SFM_MAX_SCALES];         /* (B,S,h_s,w_s) device: d losses_out[0] / d weights, or NULL */
+} SfmPixelTerms;
+
+/* sfm_loss_snippets with per-pixel terms.  pix == NULL, or every member of the scales < n_scales NULL, is exactly
+ * sfm_loss_snippets of the other arguments (members of scales >= n_scales are ignored).  Maps may be requested with or
+ * without weights and with or without grads (grads == NULL: forward only, the validation use).  Composes with snippet
+ * terms, the peer sum (the maps stay per rank), raw disparity / pose, edge-aware smoothness, SFM_FLAG_TABLES_PROVIDED,
+ * SFM_FLAG_REUSE_PYRAMID and sfm_intrinsics_grad afterwards.  Per-pixel terms together with igrads return
+ * SFM_E_UNSUPPORTED.  With all weights 1 (or NULL) the losses are bitwise those of the step without per-pixel terms run
+ * with the same plan, and so are gdisps and glogits without SSIM (with SSIM gdisps agree to the last bits). */
+int sfm_loss_weighted(const SfmDesc* desc, const SfmInputs* in, const SfmSnippetTerms* terms, const SfmPixelTerms* pix,
+                      float* losses_out, const SfmGrads* grads, const SfmImageGrads* igrads, void* workspace, SfmPeer* peer,
+                      void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -166,7 +166,7 @@ int num_sms() {
 
 int run_loss(const SfmDesc* d, const SfmInputs* in, float* losses_out, const SfmGrads* grads, const float* gy,
              const SfmDebug* dbg, void* workspace, cudaStream_t st, const SfmPeerDev* peer = nullptr,
-             const SfmImageGrads* ig = nullptr, const SfmSnippetTerms* snip = nullptr) {
+             const SfmImageGrads* ig = nullptr, const SfmSnippetTerms* snip = nullptr, const SfmPixelTerms* pix = nullptr) {
   int rc = sfm_validate_desc(d);
   if (rc) return rc;
   const bool reuse = (d->flags & SFM_FLAG_REUSE_PYRAMID) != 0;
@@ -188,6 +188,7 @@ int run_loss(const SfmDesc* d, const SfmInputs* in, float* losses_out, const Sfm
   if (grads) mode |= SFM_MODE_GRAD;
   if (dbg) mode |= SFM_MODE_DEBUG;
   if (ig) mode |= SFM_MODE_IMG;
+  if (pix) mode |= SFM_MODE_PIX;
   const SfmStepPlan plan = sfm_plan_step(d, mode, num_sms());
   SfmWsLayout L;
   sfm_ws_layout(d, &L);
@@ -224,6 +225,10 @@ int run_loss(const SfmDesc* d, const SfmInputs* in, float* losses_out, const Sfm
     if (ig) {
       p.gtgt[s] = !ig->gtgt ? nullptr : s == 0 ? ig->gtgt : (float*)(ws + L.off_gtgt[s]);
       p.gsrc[s] = !ig->gsrc ? nullptr : s == 0 ? ig->gsrc : (float*)(ws + L.off_gsrc[s]);
+    }
+    if (pix) {
+      p.pix_w[s] = pix->weights[s];
+      p.pix_map[s] = pix->losses[s];
     }
   }
   const bool tables = (d->flags & SFM_FLAG_TABLES_PROVIDED) != 0;
@@ -329,6 +334,12 @@ extern "C" int sfm_loss_forward_backward_images(const SfmDesc* desc, const SfmIn
 extern "C" int sfm_loss_snippets(const SfmDesc* desc, const SfmInputs* in, const SfmSnippetTerms* terms, float* losses_out,
                                  const SfmGrads* grads, const SfmImageGrads* igrads, void* workspace, SfmPeer* peer,
                                  void* stream) {
+  return sfm_loss_weighted(desc, in, terms, nullptr, losses_out, grads, igrads, workspace, peer, stream);
+}
+
+extern "C" int sfm_loss_weighted(const SfmDesc* desc, const SfmInputs* in, const SfmSnippetTerms* terms, const SfmPixelTerms* pix,
+                                 float* losses_out, const SfmGrads* grads, const SfmImageGrads* igrads, void* workspace,
+                                 SfmPeer* peer, void* stream) {
   int rc = sfm_validate_desc(desc);
   if (rc) return rc;
   const bool snip = terms && (terms->weights || terms->losses);
@@ -348,6 +359,12 @@ extern "C" int sfm_loss_snippets(const SfmDesc* desc, const SfmInputs* in, const
     if (!igrads->gtgt && !igrads->gsrc) { sfm_set_error("igrads has neither gtgt nor gsrc"); return SFM_E_NULL_POINTER; }
     if (!grads) { sfm_set_error("sfm_loss_snippets: igrads needs grads"); return SFM_E_NULL_POINTER; }
   }
+  bool pixel = false;                  // per-pixel terms: some member of a scale < n_scales is set
+  for (int s = 0; pix && s < desc->n_scales; ++s) pixel = pixel || pix->weights[s] || pix->losses[s];
+  if (pixel && igrads) {
+    sfm_set_error("unsupported: per-pixel terms (SfmPixelTerms) together with image gradients (igrads)");
+    return SFM_E_UNSUPPORTED;
+  }
   if (!losses_out) { sfm_set_error("losses_out is NULL"); return SFM_E_NULL_POINTER; }
   const SfmPeerDev* dev = nullptr;
   if (peer && !(dev = sfm_peer_dev(peer))) {
@@ -355,7 +372,7 @@ extern "C" int sfm_loss_snippets(const SfmDesc* desc, const SfmInputs* in, const
     return SFM_E_UNSUPPORTED;
   }
   return run_loss(desc, in, losses_out, grads, nullptr, nullptr, workspace, (cudaStream_t)stream, dev, igrads,
-                  snip ? terms : nullptr);
+                  snip ? terms : nullptr, pixel ? pix : nullptr);
 }
 
 extern "C" int sfm_scale_image_grads(const SfmDesc* desc, const float* gy, const SfmImageGrads* igrads, void* stream) {

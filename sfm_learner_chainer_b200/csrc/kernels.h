@@ -138,6 +138,11 @@ struct SfmFusedParams {
   // per-snippet terms: segment height of the prologue's smoothness tasks, whose losses sm_part then holds one per task
   // (0: no such tasks).  Their order is the planner's (plan_smooth): per scale, per snippet, strips x segments.
   int sm_hseg;
+  // per-pixel terms (sfm_loss_weighted; nullptr when off), [B][S][h][w] per scale like logits.  pix_w[s] multiplies the
+  // photometric terms of every (pixel, source) at scale s (nullptr: 1); pix_map[s] receives d losses_out[0] / d pix_w.
+  // Appended last, so that no member the other kernels read moves.
+  const float* pix_w[SFM_MAX_SCALES];
+  float* pix_map[SFM_MAX_SCALES];
 };
 
 // Launch helper: with pdl the kernel is a programmatic dependent launch on the previous kernel of the stream (its
@@ -170,11 +175,13 @@ constexpr int SFM_SSIM_REG_MIN_WARPS = 8;
 constexpr int SFM_SSIM_IMG_MIN_WARPS = 10;
 
 // Launch plan of one fused step (plan.cu, the whole launch policy).  The marching kernel instance is
-// sfm_l1_march_kernel<exp, grad, accum, debug, raw, img> or sfm_ssim_march_kernel<grad, accum, debug, raw, nw, srec, img>.
+// sfm_l1_march_kernel<exp, grad, accum, debug, raw, img, snip, pix> or
+// sfm_ssim_march_kernel<grad, accum, debug, raw, nw, srec, img, snip, pix>.
 struct SfmStepPlan {
   bool ssim;                           // kernel family
   bool exp, grad, accum, debug, raw;   // accum: a smoothness kernel has initialised gdisp
   bool img;                            // image gradients (grad, !debug; SSIM: nw = 1 with shared-memory records)
+  bool pix;                            // per-pixel terms (!debug, !img; SSIM: nw = 1 with shared-memory records)
   int nw;                              // SSIM: warps per CTA (2: the two sources split over the warps of a CTA)
   bool srec;                           // SSIM: forward records in shared memory (false: in registers)
   bool edge_smooth;                    // the edge-aware smoothness kernel runs between the prologue and the march
@@ -183,7 +190,8 @@ struct SfmStepPlan {
   int band, n_mix_region;              // SfmPrepParams
 };
 // mode bits of the planner
-enum { SFM_MODE_EXP = 1, SFM_MODE_SSIM = 2, SFM_MODE_GRAD = 4, SFM_MODE_DEBUG = 8, SFM_MODE_SMOOTH = 16, SFM_MODE_IMG = 32 };
+enum { SFM_MODE_EXP = 1, SFM_MODE_SSIM = 2, SFM_MODE_GRAD = 4, SFM_MODE_DEBUG = 8, SFM_MODE_SMOOTH = 16, SFM_MODE_IMG = 32,
+       SFM_MODE_PIX = 64 };
 SfmStepPlan sfm_plan_step(const SfmDesc* d, int mode, int num_sms);
 int sfm_plan_band(const SfmDesc* d);
 int sfm_launch_fused(SfmFusedParams& p, const SfmStepPlan& plan, cudaStream_t stream);

@@ -75,8 +75,9 @@ void plan_ssim(SfmStepPlan& q, const SfmDesc* d, int num_sms) {
     hs[s] = d->H >> s;
     strips[s] = ((d->W >> s) + SFM_SSIM_IW - 1) / SFM_SSIM_IW;
   }
-  // the register-record and source-split instances exist for the plain gradient mode only (no image gradients)
-  const bool may_reg = q.grad && !q.debug && !q.raw && !q.img;
+  // the register-record and source-split instances exist for the plain gradient mode only (no image gradients, no
+  // per-pixel terms)
+  const bool may_reg = q.grad && !q.debug && !q.raw && !q.img && !q.pix;
   const bool may_split = may_reg && S == 2;
   int hseg = 64, nw = 1;
   bool srec = true;
@@ -182,6 +183,7 @@ SfmStepPlan sfm_plan_step(const SfmDesc* d, int mode, int num_sms) {
   q.grad = (mode & SFM_MODE_GRAD) != 0;
   q.debug = (mode & SFM_MODE_DEBUG) != 0;
   q.img = q.grad && !q.debug && (mode & SFM_MODE_IMG) != 0;
+  q.pix = !q.debug && !q.img && (mode & SFM_MODE_PIX) != 0;
   q.raw = d->raw_disp_scales != 0;
   const bool smooth = (mode & SFM_MODE_SMOOTH) != 0;
   q.accum = q.grad && smooth;

@@ -100,11 +100,18 @@ enum RowStages {
 // accumulated); dL/dP is scattered to the four taps of every in-view pixel with fp32 reductions, from the tap index
 // and the two fractions the forward record carries in three more fields.
 // SNIP: per-snippet terms, as in sfm_l1_march_kernel.
-template <bool GRAD, bool ACCUM, bool DEBUG, bool RAW, int NW, bool SREC = true, bool IMG = false, bool SNIP = false>
+// PIX (NW == 1, SREC, no IMG / DEBUG): per-pixel terms.  The weight M of a pixel is loaded with its taps and is needed at
+// three lags: stage A of row r (the L1 loss partial), row r-1 (lw of the SSIM loss and wl of the gradient fields: a
+// one-step register carry) and row r-2 (the L1 part of dL/dP in stage F: one more field of the forward record).  Stage C
+// stores the map wpix * esum + wssim * sum_c sat(raw_c) = d total / d M of the owned pixels of row r-1, whose esum is
+// carried one step like its weight.  M = 1 multiplies exactly: unit weights give bitwise the plain step.
+template <bool GRAD, bool ACCUM, bool DEBUG, bool RAW, int NW, bool SREC = true, bool IMG = false, bool SNIP = false,
+          bool PIX = false>
 __global__ void __launch_bounds__(32 * NW, (IMG ? SFM_SSIM_IMG_MIN_WARPS : SREC ? SFM_SSIM_MIN_WARPS : SFM_SSIM_REG_MIN_WARPS) / NW)
 sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
   static_assert(!IMG || (GRAD && NW == 1 && SREC), "image gradients: GRAD, one warp per CTA, shared-memory records");
-  constexpr int NREC = IMG ? 21 : 18;                   // fields of a forward record
+  static_assert(!PIX || (NW == 1 && SREC && !IMG && !DEBUG), "per-pixel terms: one warp per CTA, shared-memory records");
+  constexpr int NREC = IMG ? 21 : PIX ? 19 : 18;        // fields of a forward record
   constexpr int NG = IMG ? 4 : 3;                       // gradient fields: g_a, g_s, g_c (, h_a)
   __shared__ float4 sP_all[NW][3];
   __shared__ float sG[(NW > 1) ? 3 * 2 * 32 : 1];       // [ring slot][gdd | dsc][lane] of warp 1's row term
@@ -126,6 +133,8 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
   __shared__ float sRec[(GRAD && SREC) ? NW * 3 * NREC * 32 : 1];
   // IMG: gtgt of the snippet, gsrc of the pass's source (scale s), re-read like s_ptrs
   __shared__ float* s_img_ptrs[2];
+  // PIX: weight and map of the pass's source (scale s), re-read like s_ptrs
+  __shared__ float* s_pix_ptrs[2];
   const int lane = threadIdx.x & 31;
   float* const myrec = sRec + wi * (3 * NREC * 32) + lane;
   const StripTask t = decode_strip(p, blockIdx.x);
@@ -179,6 +188,10 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
         s_img_ptrs[0] = p.gtgt[s] ? p.gtgt[s] + (size_t)b * 3 * plane : nullptr;
         s_img_ptrs[1] = p.gsrc[s] ? p.gsrc[s] + ((size_t)b * S + i) * src_img : nullptr;
       }
+      if (PIX) {
+        s_pix_ptrs[0] = p.pix_w[s] ? const_cast<float*>(p.pix_w[s]) + ((size_t)b * S + i) * plane : nullptr;
+        s_pix_ptrs[1] = p.pix_map[s] ? p.pix_map[s] + ((size_t)b * S + i) * plane : nullptr;
+      }
     }
     __syncwarp();
     // rings: window row sums (P, P^2, P.T, T, T^2 per channel), gradient-field row sums, forward records.  No
@@ -206,9 +219,11 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
       Taps I;
       float wa, wb, wc, wd, q0, q1, q2, r, depth, dsc;
       unsigned idx;                                      // IMG: tap (v0, u0)
+      float mw;                                          // PIX: per-pixel weight
     };
     Pend pend[2];
     float g_old = 0.f;
+    float w_lag1 = 1.f, e_lag1 = 0.f;                    // PIX: weight and L1 sum of the row before the current one
 
     // refill: project row r into pending row pn (its disparity was fetched a step earlier), issue its gathers, fetch
     // row r+1's disparity / target (unless LOAD_NEXT is false) and the partial gdisp of the row whose backward runs next
@@ -237,6 +252,11 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
       pn.q0 = f.q0; pn.q1 = f.q1; pn.q2 = f.q2; pn.r = f.r;
       if (IMG) pn.idx = f.idx;
       gather_taps(pp->img, geo, f, pn.I);
+      if (PIX) {
+        float* const volatile* pq = s_pix_ptrs;
+        const float* wq = pq[0];
+        pn.mw = (in_img && wq) ? __ldg(wq + (unsigned)(r * w + xx)) : 1.f;
+      }
       if (decltype(LOAD_NEXT)::value) load_dT(r + 1, dq[nx], Tq[nx]);
       if (GRAD && (ACCUM || !first) && writer) {
         const int rf = r - 2;
@@ -261,6 +281,8 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
       const int rf = r - 2;
       const bool do_f = col_own && rf >= t.y0 && rf < t.y1;
       const float g_prev = g_old;
+      const float m_cur = PIX ? pa.mw : 1.f;             // weight of row r (pa is refilled below)
+      float e_cur = 0.f;
       // ---------------- stage A: blend pixel (r, lane) from the taps gathered during the previous step
       Rec& rc_ = rec[cur];
       {
@@ -272,7 +294,12 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
         const float P2 = sfm_blend(w1, w2, w3, w4, I.a[2], I.b[2], I.c[2], I.d[2]);
         const bool m = (P0 == 0.f) && (P1 == 0.f) && (P2 == 0.f);               // true outside the image / view
         const bool own = col_own && (r >= t.y0) && (r < t.y1);
-        pix_part += (own && !m) ? (fabsf(P0 - T[0]) + fabsf(P1 - T[1]) + fabsf(P2 - T[2])) : 0.f;
+        if (PIX) {
+          e_cur = m ? 0.f : (fabsf(P0 - T[0]) + fabsf(P1 - T[1]) + fabsf(P2 - T[2]));
+          pix_part += own ? e_cur * m_cur : 0.f;
+        } else {
+          pix_part += (own && !m) ? (fabsf(P0 - T[0]) + fabsf(P1 - T[1]) + fabsf(P2 - T[2])) : 0.f;
+        }
         mask[cur] = m;
         rc_.P[0] = P0; rc_.P[1] = P1; rc_.P[2] = P2;
         rc_.T[0] = T[0]; rc_.T[1] = T[1]; rc_.T[2] = T[2];
@@ -297,6 +324,7 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
             o[12 * 32] = pa.q0; o[13 * 32] = pa.q1; o[14 * 32] = pa.q2; o[15 * 32] = pa.r; o[16 * 32] = pa.depth;
             if (RAW) o[17 * 32] = pa.dsc;
             if (IMG) { o[18 * 32] = __uint_as_float(pa.idx); o[19 * 32] = pa.wb; o[20 * 32] = pa.wd; }
+            if (PIX) o[18 * 32] = m_cur;
           }
         }
         if (DEBUG && own && p.dbg_P[s]) {
@@ -336,7 +364,7 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
         const bool c_in = col_in && (rc >= 0) && (rc < h);
         const bool live_px = c_in && !mask[pv1];
         const bool own_c = col_own && (rc >= t.y0) && (rc < t.y1);
-        const float lw = (live_px && own_c) ? 1.f : 0.f;
+        const float lw = (live_px && own_c) ? (PIX ? w_lag1 : 1.f) : 0.f;
         // window sums: Sp = 9a, Spp = 9 A(P^2), Spt = 9 A(PT), St = 9 my, Stt = 9 A(T^2)
         const V3 Sp = (h2[0] + h1[0]) + h0[0];
         const V3 Spp = (h2[1] + h1[1]) + h0[1];
@@ -354,13 +382,19 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
         const V3 rd = v3(rcp_approx(dd.a.x), rcp_approx(dd.a.y), rcp_approx(dd.b));
         const V3 q = n * rd;                          // SSIM
         const V3 raw = vfma(v3s(-0.5f), q, v3s(0.5f));
-        ssim_part = fmaf((__saturatef(raw.a.x) + __saturatef(raw.a.y)) + __saturatef(raw.b), lw, ssim_part);
+        const float sat3 = (__saturatef(raw.a.x) + __saturatef(raw.a.y)) + __saturatef(raw.b);
+        ssim_part = fmaf(sat3, lw, ssim_part);
+        if (PIX) {
+          float* const volatile* pq = s_pix_ptrs;
+          float* mq = pq[1];
+          if (own_c && c_in && mq) st_global(mq + (unsigned)(rc * w + xx), live_px ? wpix * e_lag1 + wssim * sat3 : 0.f);
+        }
         if (GRAD) {
           // d raw / d(Sp, Spp, Spt) with n, d in the 81x units (SURVEY A.7 rescaled):
           //   g_n = dL/dn = -0.5 w / d ; g_d = dL/dd = 0.5 w n / d^2
           //   dn/dSp = 2 St (n2 - n1) ; dn/dSpt = 18 n1 ; dd/dSp = 2 Sp (d2 - d1) ; dd/dSpp = 9 d1
           // F.clip passes gradient inside [0, 1]
-          const float wl = live_px ? -0.5f * wssim : 0.f;
+          const float wl = live_px ? (PIX ? -0.5f * wssim * w_lag1 : -0.5f * wssim) : 0.f;
           const V3 wv = v3((raw.a.x >= 0.f && raw.a.x <= 1.f) ? wl : 0.f, (raw.a.y >= 0.f && raw.a.y <= 1.f) ? wl : 0.f,
                            (raw.b >= 0.f && raw.b <= 1.f) ? wl : 0.f);
           const V3 g_n = wv * rd;
@@ -394,6 +428,7 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
           rb.dsc = RAW ? o[17 * 32] : rb.depth;
         }
         const bool mf = mask[pv2];
+        const float wpf = PIX ? wpix * (SREC ? myrec[pv2 * NREC * 32 + 18 * 32] : 1.f) : wpix;   // PIX: weight of row rf
         float gP[3], gT[3];
         {
           const V3 Aa = (g2[0] + g1[0]) + gh0[0];
@@ -413,7 +448,7 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
           }
 #pragma unroll
           for (int c = 0; c < 3; ++c) {
-            const float gl1 = mf ? 0.f : sfm_sign_times(rb.P[c] - rb.T[c], wpix);
+            const float gl1 = mf ? 0.f : sfm_sign_times(rb.P[c] - rb.T[c], wpf);
             gP[c] = do_f ? gs3[c] + gl1 : 0.f;
             if (IMG) gT[c] = do_f ? gt3[c] - gl1 : 0.f;
           }
@@ -472,6 +507,7 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
       }
       }  // C + D
       }  // opaque_true
+      if (PIX) { w_lag1 = m_cur; e_lag1 = e_cur; }
     };
 
     // r_end - r_begin = h + 4 >= 5 steps: the four head steps, then groups of three (ring rotation = renaming) that

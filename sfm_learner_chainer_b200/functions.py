@@ -34,13 +34,24 @@ class ViewSynthesisLoss(object):
     with copies of a real snippet (a zero disparity gives NaN, and NaN * 0 is NaN), keep B_global = B and pass
     w_b = B / B_real for the real snippets and 0 for the padding; that gives the loss and gradients of the B_real batch
     up to rounding.  d total / d w_b = l_b[0] (the torch adapter returns it as the weights' gradient).
+    pixel_terms: forward and forward_backward take `pixel_weights`, a list of n_scales float32 device arrays
+    (B,S,h_s,w_s) laid out like the logits, or None entries (None = all 1), and also return the per-pixel loss maps
+    (a list of n_scales (B,S,h_s,w_s) arrays).  M_s multiplies the photometric terms of every (pixel, source) at scale s
+    (the means keep their denominators; the smoothness and explainability regularisers are not weighted), every gradient
+    is that of the weighted total, and the map is d total / d M: each pixel's share of the photometric loss
+    (sum M * map = (1 - ssim_rate) * pixel + ssim_rate * ssim).  Masks of moving objects, the ego-vehicle or sky, and
+    learned weight maps (whose gradient is the map) go in here; a forward call with maps is the validation use.  Not
+    with image_grads.
     """
 
     def __init__(self, smooth_reg=0.0, exp_reg=0.0, ssim_rate=0.0, n_scales=N_SCALES, B_global=None,
                  raw_disp_scales=0, raw_pose=False, edge_aware_smooth=False, image_grads=False,
-                 intrinsics_grad=False, snippet_terms=False):
+                 intrinsics_grad=False, snippet_terms=False, pixel_terms=False):
         if image_grads and edge_aware_smooth:
             raise ValueError('image_grads is not supported together with edge_aware_smooth')
+        if image_grads and pixel_terms:
+            raise ValueError('image_grads is not supported together with pixel_terms')
+        self.pixel_terms = bool(pixel_terms)
         self.image_grads = bool(image_grads)
         self.intrinsics_grad = bool(intrinsics_grad)
         self.snippet_terms = bool(snippet_terms)
@@ -170,22 +181,51 @@ class ViewSynthesisLoss(object):
         rows = D.empty(tgt, (desc.B, 5))
         return L.SfmSnippetTerms(_vp(snippet_weights), _vp(rows)), rows
 
+    def _pixel_terms(self, desc, tgt, pixel_weights):
+        """-> (SfmPixelTerms or None, per-pixel loss maps (list of n_scales (B,S,h,w)) or None)."""
+        if not self.pixel_terms:
+            if pixel_weights is not None:
+                raise ValueError('pixel_weights needs ViewSynthesisLoss(pixel_terms=True)')
+            return None, None
+        ns = self.n_scales
+        if pixel_weights is None:
+            pixel_weights = [None] * ns
+        if len(pixel_weights) != ns:
+            raise ValueError('pixel_weights must hold %d entries (one per scale, None = 1), got %d' % (ns, len(pixel_weights)))
+        pt = L.SfmPixelTerms()
+        maps = []
+        for s in range(ns):
+            shape = (desc.B, desc.S, desc.H >> s, desc.W >> s)
+            if pixel_weights[s] is not None:
+                D.check_array(pixel_weights[s], 'pixel_weights[%d]' % s, shape)
+                pt.weights[s] = D.ptr(pixel_weights[s])
+            maps.append(D.empty(tgt, shape))
+            pt.losses[s] = D.ptr(maps[s])
+        return pt, maps
+
     # ---- operators
     def forward(self, tgt, src, intrinsics, disps, poses, logits=None, proj=None, kinv=None, debug=False,
-                snippet_weights=None):
+                snippet_weights=None, pixel_weights=None):
         """-> losses (5,) device array in the order of lib.LOSS_KEYS [, debug dict].
-        With the operator's snippet_terms: -> (losses, snippet losses (B,5)), losses = sum_b w_b * l_b."""
-        if debug and self.snippet_terms:
-            raise ValueError('debug dumps are not available on an operator with snippet_terms')
+        With the operator's snippet_terms: -> (losses, snippet losses (B,5)), losses = sum_b w_b * l_b.
+        With the operator's pixel_terms the per-pixel loss maps (list of n_scales (B,S,h,w)) are appended as the last
+        element: (losses, maps) or (losses, snippet losses, maps)."""
+        if debug and (self.snippet_terms or self.pixel_terms):
+            raise ValueError('debug dumps are not available on an operator with snippet_terms or pixel_terms')
         desc, inp = self._pack(tgt, src, intrinsics, disps, poses, logits, proj, kinv)
         losses = D.empty(tgt, (5,))
-        if self.snippet_terms:
+        if self.snippet_terms or self.pixel_terms:
             terms, rows = self._snippet_terms(desc, tgt, snippet_weights)
-            L.check(self._lib.sfm_loss_snippets(C.byref(desc), C.byref(inp), C.byref(terms), _vp(losses), None, None,
+            pt, maps = self._pixel_terms(desc, tgt, pixel_weights)
+            L.check(self._lib.sfm_loss_weighted(C.byref(desc), C.byref(inp), C.byref(terms) if terms else None,
+                                                C.byref(pt) if pt else None, _vp(losses), None, None,
                                                 self._workspace(desc, tgt), None, C.c_void_p(D.current_stream(tgt))))
-            return losses, rows
+            out = (losses,) + ((rows,) if self.snippet_terms else ()) + ((maps,) if self.pixel_terms else ())
+            return out
         if snippet_weights is not None:
             raise ValueError('snippet_weights needs ViewSynthesisLoss(snippet_terms=True)')
+        if pixel_weights is not None:
+            raise ValueError('pixel_weights needs ViewSynthesisLoss(pixel_terms=True)')
         dbg_struct, dbg = None, None
         if debug:
             B, S, H, W = desc.B, desc.S, desc.H, desc.W
@@ -234,7 +274,8 @@ class ViewSynthesisLoss(object):
         self._ev_pyramid = D.record_event(tgt)
 
     def forward_backward(self, tgt, src, intrinsics, disps, poses, logits=None, proj=None, kinv=None, reuse_pyramid=False,
-                         peer=None, image_grads=('tgt', 'src'), intrinsics_grad=True, snippet_weights=None):
+                         peer=None, image_grads=('tgt', 'src'), intrinsics_grad=True, snippet_weights=None,
+                         pixel_weights=None):
         """Single fused pass: -> (losses (5,), dict(gdisps, gposes, glogits)) for upstream gradient 1.
         reuse_pyramid: the workspace already holds this batch's pyramid (build_pyramid).
         peer: a distributed.PeerLossSum -- the batch is sharded by snippet over several GPUs (B_global set) and the
@@ -244,7 +285,10 @@ class ViewSynthesisLoss(object):
         With the operator's intrinsics_grad the dict also holds gintrinsics (None when `intrinsics_grad` is False).
         With the operator's snippet_terms: snippet_weights (B,) (None = all 1; under peer the local shard's) weight the
         snippets, the losses are sum_b w_b * l_b, every gradient is that of their total, and the dict also holds
-        snippet_losses (B,5), this shard's rows l_b."""
+        snippet_losses (B,5), this shard's rows l_b.
+        With the operator's pixel_terms: pixel_weights (list of n_scales (B,S,h,w) or None entries) weight the
+        photometric terms per (pixel, source), and the dict also holds pixel_losses, the maps d total / d weights
+        (this shard's, under peer)."""
         want_k = self._want_intrinsics_grad(intrinsics_grad, proj, kinv)
         desc, inp = self._pack(tgt, src, intrinsics, disps, poses, logits, proj, kinv)
         if reuse_pyramid:
@@ -255,6 +299,9 @@ class ViewSynthesisLoss(object):
         terms, rows = self._snippet_terms(desc, tgt, snippet_weights)
         if rows is not None:
             out['snippet_losses'] = rows
+        pt, maps = self._pixel_terms(desc, tgt, pixel_weights)
+        if maps is not None:
+            out['pixel_losses'] = maps
         ig = None
         want = set(image_grads) if self.image_grads else set()
         if want:
@@ -263,10 +310,11 @@ class ViewSynthesisLoss(object):
             out['gtgt'] = D.empty(tgt, (desc.B, 3, desc.H, desc.W)) if 'tgt' in want else None
             out['gsrc'] = D.empty(tgt, (desc.B, desc.S, 3, desc.H, desc.W)) if 'src' in want else None
             ig = L.SfmImageGrads(_vp(out['gtgt']), _vp(out['gsrc']))
-        # one entry point for every combination of image gradients, peer sum and snippet terms
-        L.check(self._lib.sfm_loss_snippets(C.byref(desc), C.byref(inp), C.byref(terms) if terms else None, _vp(losses),
-                                            C.byref(g), C.byref(ig) if ig else None, self._workspace(desc, tgt),
-                                            peer.handle if peer is not None else None, C.c_void_p(D.current_stream(tgt))))
+        # one entry point for every combination of image gradients, peer sum, snippet and per-pixel terms
+        L.check(self._lib.sfm_loss_weighted(C.byref(desc), C.byref(inp), C.byref(terms) if terms else None,
+                                            C.byref(pt) if pt else None, _vp(losses), C.byref(g), C.byref(ig) if ig else None,
+                                            self._workspace(desc, tgt), peer.handle if peer is not None else None,
+                                            C.c_void_p(D.current_stream(tgt))))
         self._intrinsics_grad(desc, inp, tgt, out, want_k)
         if self._ev_pyramid is not None:
             self._ev_loss = D.record_event(tgt)

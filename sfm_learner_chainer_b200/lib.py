@@ -53,6 +53,10 @@ class SfmSnippetTerms(C.Structure):
     _fields_ = [('weights', _vp), ('losses', _vp)]
 
 
+class SfmPixelTerms(C.Structure):
+    _fields_ = [('weights', _vp * SFM_MAX_SCALES), ('losses', _vp * SFM_MAX_SCALES)]
+
+
 class SfmAugment(C.Structure):
     _fields_ = [('out_h', C.c_int32), ('out_w', C.c_int32), ('off_y', C.c_int32), ('off_x', C.c_int32),
                 ('flip', C.c_int32), ('reserved_', C.c_int32), ('x_scaling', C.c_double), ('y_scaling', C.c_double)]
@@ -68,6 +72,7 @@ _i = C.c_int
 _D, _I, _G, _Dbg = C.POINTER(SfmDesc), C.POINTER(SfmInputs), C.POINTER(SfmGrads), C.POINTER(SfmDebug)
 _IG = C.POINTER(SfmImageGrads)
 _ST = C.POINTER(SfmSnippetTerms)
+_PT = C.POINTER(SfmPixelTerms)
 SYMBOLS = {
     'sfm_version': (_i, []),
     'sfm_last_error': (C.c_char_p, []),
@@ -111,6 +116,7 @@ SYMBOLS = {
     'sfm_peer_destroy': (_i, [_vp]),
     'sfm_loss_forward_backward_peer': (_i, [_D, _I, _vp, _G, _vp, _vp, _vp]),
     'sfm_loss_snippets': (_i, [_D, _I, _ST, _vp, _G, _IG, _vp, _vp, _vp]),
+    'sfm_loss_weighted': (_i, [_D, _I, _ST, _PT, _vp, _G, _IG, _vp, _vp, _vp]),
 }
 
 _lib = None

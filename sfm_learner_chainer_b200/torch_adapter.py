@@ -10,7 +10,8 @@ from .functions import ViewSynthesisLoss
 
 class _ViewSynthesisLossFn(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, op, tgt, src, intrinsics, weights, n_scales, use_exp, *preds):
+    def forward(ctx, op, tgt, src, intrinsics, weights, n_scales, use_exp, n_pred, *rest):
+        preds, pix_w = rest[:n_pred], rest[n_pred:]      # pix_w: n_scales per-pixel weights (or None) with op.pixel_terms
         disps = [p.contiguous() for p in preds[:n_scales]]
         poses = preds[n_scales].contiguous()
         logits = [p.contiguous() for p in preds[n_scales + 1:]] if use_exp else None
@@ -24,19 +25,25 @@ class _ViewSynthesisLossFn(torch.autograd.Function):
                                             intrinsics.detach().contiguous(), [d.detach() for d in disps], poses.detach(),
                                             [l.detach() for l in logits] if logits else None, image_grads=want,
                                             intrinsics_grad=ctx.want_k,
-                                            snippet_weights=weights.detach().contiguous() if weights is not None else None)
+                                            snippet_weights=weights.detach().contiguous() if weights is not None else None,
+                                            **(dict(pixel_weights=[w.detach().contiguous() if w is not None else None
+                                                                   for w in pix_w]) if op.pixel_terms else {}))
         ctx.op, ctx.grads, ctx.shape = op, grads, tuple(src.shape)
         ctx.n_scales, ctx.use_exp = n_scales, use_exp
         ctx.consumed = False
+        outs = [losses]
+        ctx.want_w = False
         if op.snippet_terms:
             # d total / d w_b = l_b[0]: the weights' gradient needs the rows alone
             ctx.want_w = weights is not None and ctx.needs_input_grad[4]
             ctx.rows = grads['snippet_losses']
-            ctx.mark_non_differentiable(losses, ctx.rows)
-            return losses[0].clone(), losses, ctx.rows
-        ctx.want_w = False
-        ctx.mark_non_differentiable(losses)
-        return losses[0].clone(), losses
+            outs.append(ctx.rows)
+        # likewise d total / d M_s = the per-pixel loss map of scale s
+        ctx.maps = grads.get('pixel_losses') or []
+        ctx.want_pw = [w is not None and ctx.needs_input_grad[8 + n_pred + s] for s, w in enumerate(pix_w)]
+        outs += ctx.maps
+        ctx.mark_non_differentiable(*outs)
+        return (losses[0].clone(),) + tuple(outs)
 
     @staticmethod
     @torch.autograd.function.once_differentiable
@@ -58,22 +65,38 @@ class _ViewSynthesisLossFn(torch.autograd.Function):
         gtgt = g.get('gtgt') if ctx.want_tgt else None
         gsrc = g.get('gsrc') if ctx.want_src else None
         gk = g.get('gintrinsics') if ctx.want_k else None
-        return (None, gtgt, gsrc, gk, gw, None, None) + tuple(out)
+        gpw = tuple(gy * m if want else None for m, want in zip(ctx.maps, ctx.want_pw))
+        return (None, gtgt, gsrc, gk, gw, None, None, None) + tuple(out) + gpw
 
 
-def view_synthesis_loss(op, tgt, src, intrinsics, pred_disps, pred_poses, pred_maskes=None, snippet_weights=None):
+def view_synthesis_loss(op, tgt, src, intrinsics, pred_disps, pred_poses, pred_maskes=None, snippet_weights=None,
+                        pixel_weights=None):
     """-> (total_loss scalar tensor with grad_fn, losses (5,) tensor [total, pixel, smooth, exp, ssim]).
 
     pred_poses: (B,S,6) tensor or a tuple of S (B,6) tensors as PoseNet returns them (pose_net.py:52-54).
     With op.snippet_terms: -> (total, losses, snippet_losses (B,5)); snippet_weights (B,) (None = all 1) weight the
     snippets, total = sum_b w_b * snippet_losses[b, 0], the other inputs' gradients are the weighted ones, and weights
     that require grad receive gy * snippet_losses[:, 0].  See ViewSynthesisLoss for padding a captured batch.
+    With op.pixel_terms: pixel_weights (list of n_scales (B,S,h,w) tensors or None entries; None = all 1) weight the
+    photometric terms per (pixel, source), and pixel_losses (list of n_scales maps d total / d weights) is appended to
+    the returned tuple; weights that require grad receive gy * pixel_losses[s].
     """
     assert isinstance(op, ViewSynthesisLoss)
     if snippet_weights is not None and not op.snippet_terms:
         raise ValueError('snippet_weights needs ViewSynthesisLoss(snippet_terms=True)')
+    if pixel_weights is not None and not op.pixel_terms:
+        raise ValueError('pixel_weights needs ViewSynthesisLoss(pixel_terms=True)')
+    pix_w = []
+    if op.pixel_terms:
+        pix_w = list(pixel_weights) if pixel_weights is not None else [None] * op.n_scales
+        if len(pix_w) != op.n_scales:
+            raise ValueError('pixel_weights must hold %d entries (one per scale, None = 1)' % op.n_scales)
     if isinstance(pred_poses, (tuple, list)):
         pred_poses = torch.stack(list(pred_poses), dim=1)
     use_exp = op.use_exp
     preds = list(pred_disps) + [pred_poses] + (list(pred_maskes) if use_exp else [])
-    return _ViewSynthesisLossFn.apply(op, tgt, src, intrinsics, snippet_weights, op.n_scales, use_exp, *preds)
+    res = _ViewSynthesisLossFn.apply(op, tgt, src, intrinsics, snippet_weights, op.n_scales, use_exp, len(preds), *preds, *pix_w)
+    if not op.pixel_terms:
+        return res
+    k = len(res) - op.n_scales
+    return tuple(res[:k]) + (list(res[k:]),)

@@ -1,13 +1,14 @@
 """Step time of the fused loss with and without one opt-in option: image_grads (ViewSynthesisLoss(image_grads=True)),
-intrinsics_grad (ViewSynthesisLoss(intrinsics_grad=True)) or snippet_terms (ViewSynthesisLoss(snippet_terms=True) with
-per-snippet weights, returning the per-snippet losses).
+intrinsics_grad (ViewSynthesisLoss(intrinsics_grad=True)), snippet_terms (ViewSynthesisLoss(snippet_terms=True) with
+per-snippet weights, returning the per-snippet losses) or pixel_terms (ViewSynthesisLoss(pixel_terms=True) with random
+per-pixel weights in [0, 1] at every scale, returning the per-pixel loss maps).
 
 For each config the step (forward_backward on device tensors) is captured four times into one CUDA graph and the graph
 is replayed; the two variants alternate, and the median over the repeats is reported per step.  Prints one JSON line
 per config and writes them all, with the card name and its power limit, to the file given as the first argument.
 The last column is the relative overhead for image_grads and the added microseconds for intrinsics_grad (the cost of
-one extra dependent launch, sfm_intrinsics_grad_kernel) and for snippet_terms.
-usage: python tools/time_opt_in_grads.py OUT.json {image_grads,intrinsics_grad,snippet_terms} [cfg ...]"""
+one extra dependent launch, sfm_intrinsics_grad_kernel) and for snippet_terms, the relative overhead for pixel_terms.
+usage: python tools/time_opt_in_grads.py OUT.json {image_grads,intrinsics_grad,snippet_terms,pixel_terms} [cfg ...]"""
 import json
 import os
 import subprocess
@@ -26,6 +27,7 @@ LAST_COLUMN = {
     'image_grads': ('overhead', lambda p, q: round(q / p - 1.0, 4)),
     'intrinsics_grad': ('extra_us', lambda p, q: round(q - p, 2)),
     'snippet_terms': ('extra_us', lambda p, q: round(q - p, 2)),
+    'pixel_terms': ('overhead', lambda p, q: round(q / p - 1.0, 4)),
 }
 
 
@@ -81,6 +83,11 @@ def main():
         w = torch.full((c['B'],), 1.0, device='cuda')
         w[-1] = 0.0
         kw = {option: dict(snippet_weights=w)} if option == 'snippet_terms' else {}
+        if option == 'pixel_terms':
+            # pixel_terms: a weight in [0, 1] for every (pixel, source) of every scale; the maps are always returned
+            gen = torch.Generator(device='cuda').manual_seed(0)
+            pw = [torch.rand((c['B'], c['S'], c['H'] >> s, c['W'] >> s), device='cuda', generator=gen) for s in range(4)]
+            kw = {option: dict(pixel_weights=pw)}
         graphs = {k: make_graph(op, args, **kw.get(k, {})) for k, op in ops.items()}
         replays = 10 if name == 'cfg5' else 200
         t = {k: [] for k in graphs}
