@@ -55,6 +55,9 @@ extern "C" {
 #define SFM_FLAG_SNIPPET_TERMS 0x20u  /* the workspace also holds 4 fp64 loss cells per snippet and one float per smoothness
                                          task for sfm_loss_snippets; every other entry point accepts the flag and behaves
                                          exactly as without it */
+#define SFM_FLAG_MIN_REPROJECTION 0x40u /* the workspace also holds B*S*sum_s h_s*w_s floats, the per-(pixel, source) error /
+                                         weight planes of sfm_loss_min_reprojection; every other entry point accepts the
+                                         flag and behaves exactly as without it */
 
 /*
  * Problem descriptor.  Mirrors the reference's model flags (base_model.py:37-39:
@@ -394,6 +397,55 @@ typedef struct SfmPixelTerms {
 int sfm_loss_weighted(const SfmDesc* desc, const SfmInputs* in, const SfmSnippetTerms* terms, const SfmPixelTerms* pix,
                       float* losses_out, const SfmGrads* grads, const SfmImageGrads* igrads, void* workspace, SfmPeer* peer,
                       void* stream);
+
+/* Per-pixel minimum reprojection and auto-masking over the source views (Godard et al., "Digging Into Self-Supervised
+ * Monocular Depth Estimation", ICCV 2019), sfm_loss_min_reprojection.  The reference's photometric loss is a mean over
+ * the source views of every (pixel, source) error; here each target pixel is scored on the one source that explains it
+ * best, so a pixel occluded in one source is scored on a source where it is visible, and (auto-masking) a pixel is
+ * dropped when an UNWARPED source already matches the target at least as well (a static camera, objects that move with
+ * the camera).  Per scale s, snippet b, target pixel p, source i, with r = ssim_rate:
+ *   reprojection error  e_i(p) = (1 - r) * sum_c E_c + r * sum_c clip((1 - SSIM_c) / 2, 0, 1) * (1 - m)
+ *                       the per-pixel map of sfm_loss_weighted without its 1/(B_global*3*h*w) factor, without gy and
+ *                       without snippet weights; the SSIM part only when SSIM runs (ssim_rate != 0).
+ *   candidates          source i is a candidate at p only where its all-zero mask m (base_model.py:96) is 0; every
+ *                       out-of-view pixel is masked (the x2 rule makes the warped value exactly 0).  A masked source is
+ *                       NOT a candidate with error 0 (it would always win).
+ *   identity error      e_id_i(p): the same formula with the warped image replaced by source i's own pyramid level at p
+ *                       (scale 0: the caller's tensor), no mask, the same 3x3 zero-padded windows as the reference SSIM.
+ *   selection           sel(p) = -2 when p has no candidate; else i* = argmin over the candidates of e_i(p), ties to the
+ *                       lowest index; with automask, sel(p) = -1 when e_i*(p) >= min_i e_id_i(p) (a strict < keeps the
+ *                       pixel), else sel(p) = i*.  The selection uses neither snippet weights nor gy, so a negative
+ *                       snippet weight cannot turn the minimum into a maximum.
+ *   loss                the loss of sfm_loss_weighted with the one-hot weights M_i(p) = [sel(p) = i].  The means keep their
+ *                       denominators, so the photometric part is the mean over the pixels of the per-pixel minimum;
+ *                       losses_out[1] (pixel) and [4] (ssim) are the L1 and SSIM parts of the chosen terms; smoothness
+ *                       (either kind) is unchanged.  Every gradient (gdisps, gposes, the dL/dP cells, hence
+ *                       sfm_intrinsics_grad afterwards) is that of this total; the selection is piecewise constant and
+ *                       has derivative 0.
+ * Auto-masked pixels contribute 0 to the reported value, as the paper's mask mu does.  Monodepth2's code instead adds the
+ * identity error of those pixels to the reported value; that part carries no disparity, pose or intrinsics gradient, so
+ * the gradients are the same either way and only the reported value differs.
+ * Computed in two marches on the device (graph-capturable): a forward march writes every e_i into the workspace planes,
+ * a select kernel computes the identity errors and turns the planes into the one-hot weights, and the march of
+ * sfm_loss_weighted runs with them. */
+typedef struct SfmMinReprojection {
+  int32_t automask;                       /* != 0: auto-masking on */
+  int32_t reserved_;                      /* 0 (else SFM_E_INVALID_DESC) */
+  int8_t* selection[SFM_MAX_SCALES];      /* (B,h_s,w_s) device: sel(p) in {-2, -1, 0 .. S-1}, or NULL */
+} SfmMinReprojection;
+
+/* sfm_loss_snippets with minimum reprojection (and auto-masking) over the sources.  desc->flags must contain
+ * SFM_FLAG_MIN_REPROJECTION (else SFM_E_INVALID_DESC; the workspace is sized with it), mr must not be NULL and
+ * desc->ssim_rate must lie in [0, 1] (else SFM_E_INVALID_DESC: the selection needs a non-negative error).  grads == NULL:
+ * forward only (the losses and the selection, the validation use).  Composes with snippet terms (their weights apply to
+ * the loss, not to the selection), the peer sum (the selection stays per rank), raw disparity / pose, edge-aware
+ * smoothness, SFM_FLAG_TABLES_PROVIDED, SFM_FLAG_REUSE_PYRAMID and sfm_intrinsics_grad afterwards.  The explainability
+ * branch (exp_reg != 0) returns SFM_E_UNSUPPORTED: auto-masking replaces it, and sigma(l) would enter the selection.
+ * Image gradients and caller per-pixel weights (SfmPixelTerms) have no argument here, as per-pixel terms exclude image
+ * gradients in sfm_loss_weighted. */
+int sfm_loss_min_reprojection(const SfmDesc* desc, const SfmInputs* in, const SfmSnippetTerms* terms,
+                              const SfmMinReprojection* mr, float* losses_out, const SfmGrads* grads, void* workspace,
+                              SfmPeer* peer, void* stream);
 
 #ifdef __cplusplus
 }

@@ -166,7 +166,8 @@ int num_sms() {
 
 int run_loss(const SfmDesc* d, const SfmInputs* in, float* losses_out, const SfmGrads* grads, const float* gy,
              const SfmDebug* dbg, void* workspace, cudaStream_t st, const SfmPeerDev* peer = nullptr,
-             const SfmImageGrads* ig = nullptr, const SfmSnippetTerms* snip = nullptr, const SfmPixelTerms* pix = nullptr) {
+             const SfmImageGrads* ig = nullptr, const SfmSnippetTerms* snip = nullptr, const SfmPixelTerms* pix = nullptr,
+             const SfmMinReprojection* mr = nullptr) {
   int rc = sfm_validate_desc(d);
   if (rc) return rc;
   const bool reuse = (d->flags & SFM_FLAG_REUSE_PYRAMID) != 0;
@@ -189,6 +190,7 @@ int run_loss(const SfmDesc* d, const SfmInputs* in, float* losses_out, const Sfm
   if (dbg) mode |= SFM_MODE_DEBUG;
   if (ig) mode |= SFM_MODE_IMG;
   if (pix) mode |= SFM_MODE_PIX;
+  if (mr) mode |= SFM_MODE_PIX | SFM_MODE_MINREP;
   const SfmStepPlan plan = sfm_plan_step(d, mode, num_sms());
   SfmWsLayout L;
   sfm_ws_layout(d, &L);
@@ -230,6 +232,7 @@ int run_loss(const SfmDesc* d, const SfmInputs* in, float* losses_out, const Sfm
       p.pix_w[s] = pix->weights[s];
       p.pix_map[s] = pix->losses[s];
     }
+    if (mr) p.pix_w[s] = (const float*)(ws + L.off_mrw[s]);   // the one-hot weights, made by the select kernel
   }
   const bool tables = (d->flags & SFM_FLAG_TABLES_PROVIDED) != 0;
   p.proj = tables ? in->proj : (const float*)(ws + L.off_proj);
@@ -278,6 +281,12 @@ int run_loss(const SfmDesc* d, const SfmInputs* in, float* losses_out, const Sfm
   }
   rc = sfm_launch_prep(pp, &sm, (grads ? 2 : 1) + (snip ? 2 : 0), st);
   if (rc) return rc;
+  if (mr) {
+    SfmMinRepArgs a{};
+    a.automask = mr->automask != 0 ? 1 : 0;
+    for (int s = 0; s < d->n_scales; ++s) a.selection[s] = mr->selection[s];
+    return sfm_launch_fused(p, plan, st, &a);
+  }
   return sfm_launch_fused(p, plan, st);
 }
 
@@ -373,6 +382,41 @@ extern "C" int sfm_loss_weighted(const SfmDesc* desc, const SfmInputs* in, const
   }
   return run_loss(desc, in, losses_out, grads, nullptr, nullptr, workspace, (cudaStream_t)stream, dev, igrads,
                   snip ? terms : nullptr, pixel ? pix : nullptr);
+}
+
+extern "C" int sfm_loss_min_reprojection(const SfmDesc* desc, const SfmInputs* in, const SfmSnippetTerms* terms,
+                                         const SfmMinReprojection* mr, float* losses_out, const SfmGrads* grads, void* workspace,
+                                         SfmPeer* peer, void* stream) {
+  int rc = sfm_validate_desc(desc);
+  if (rc) return rc;
+  if (!(desc->flags & SFM_FLAG_MIN_REPROJECTION)) {
+    sfm_set_error("sfm_loss_min_reprojection: desc->flags lacks SFM_FLAG_MIN_REPROJECTION (the workspace must be sized with it)");
+    return SFM_E_INVALID_DESC;
+  }
+  if (!(desc->ssim_rate >= 0.f && desc->ssim_rate <= 1.f)) {
+    sfm_set_error("sfm_loss_min_reprojection: ssim_rate=%g outside [0, 1] (the selection needs a non-negative error)",
+                  (double)desc->ssim_rate);
+    return SFM_E_INVALID_DESC;
+  }
+  if (desc->exp_reg != 0.f) {
+    sfm_set_error("unsupported: minimum reprojection together with the explainability branch (exp_reg != 0)");
+    return SFM_E_UNSUPPORTED;
+  }
+  if (!mr) { sfm_set_error("SfmMinReprojection is NULL"); return SFM_E_NULL_POINTER; }
+  if (mr->reserved_ != 0) { sfm_set_error("SfmMinReprojection.reserved_ must be 0"); return SFM_E_INVALID_DESC; }
+  const bool snip = terms && (terms->weights || terms->losses);
+  if (snip && !(desc->flags & SFM_FLAG_SNIPPET_TERMS)) {
+    sfm_set_error("sfm_loss_min_reprojection: desc->flags lacks SFM_FLAG_SNIPPET_TERMS (the workspace must be sized with it)");
+    return SFM_E_INVALID_DESC;
+  }
+  if (!losses_out) { sfm_set_error("losses_out is NULL"); return SFM_E_NULL_POINTER; }
+  const SfmPeerDev* dev = nullptr;
+  if (peer && !(dev = sfm_peer_dev(peer))) {
+    sfm_set_error("sfm_loss_min_reprojection: the peer object is not connected (sfm_peer_connect)");
+    return SFM_E_UNSUPPORTED;
+  }
+  return run_loss(desc, in, losses_out, grads, nullptr, nullptr, workspace, (cudaStream_t)stream, dev, nullptr,
+                  snip ? terms : nullptr, nullptr, mr);
 }
 
 extern "C" int sfm_scale_image_grads(const SfmDesc* desc, const float* gy, const SfmImageGrads* igrads, void* stream) {

@@ -48,6 +48,9 @@ struct SfmWsLayout {
   size_t off_gsrc[SFM_MAX_SCALES];  // float [B*S][3][h][w]
   size_t off_gtgt[SFM_MAX_SCALES];  // float [B][3][h][w]
   size_t gsrc_bytes;                // span of the source levels
+  // SFM_FLAG_MIN_REPROJECTION: per-(pixel, source) error planes of the forward march, turned into the one-hot weights
+  // by the select kernel.  0 without the flag.
+  size_t off_mrw[SFM_MAX_SCALES];   // float [B][S][h][w]
   size_t acc_doubles;
   size_t total;
 };
@@ -128,6 +131,13 @@ static inline void sfm_ws_layout(const SfmDesc* d, SfmWsLayout* L) {
     for (int s = 1; s < d->n_scales; ++s) {
       L->off_gtgt[s] = off;
       off = sfm_align_up(off + (size_t)d->B * 3 * (d->H >> s) * (d->W >> s) * sizeof(float), 256);
+    }
+  }
+  for (int s = 0; s < SFM_MAX_SCALES; ++s) L->off_mrw[s] = 0;
+  if (d->flags & SFM_FLAG_MIN_REPROJECTION) {
+    for (int s = 0; s < d->n_scales; ++s) {
+      L->off_mrw[s] = off;
+      off = sfm_align_up(off + (size_t)d->B * d->S * (d->H >> s) * (d->W >> s) * sizeof(float), 256);
     }
   }
   L->total = off;

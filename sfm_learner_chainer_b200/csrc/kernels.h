@@ -143,6 +143,9 @@ struct SfmFusedParams {
   // Appended last, so that no member the other kernels read moves.
   const float* pix_w[SFM_MAX_SCALES];
   float* pix_map[SFM_MAX_SCALES];
+  // what pix_map receives for a masked or out-of-view (pixel, source): 0 (its share of the loss), or a negative marker in
+  // the forward march of sfm_loss_min_reprojection, whose select kernel must tell "masked" from "error 0"
+  float pix_map_masked;
 };
 
 // Launch helper: with pdl the kernel is a programmatic dependent launch on the previous kernel of the stream (its
@@ -182,6 +185,9 @@ struct SfmStepPlan {
   bool exp, grad, accum, debug, raw;   // accum: a smoothness kernel has initialised gdisp
   bool img;                            // image gradients (grad, !debug; SSIM: nw = 1 with shared-memory records)
   bool pix;                            // per-pixel terms (!debug, !img; SSIM: nw = 1 with shared-memory records)
+  bool minrep;                         // minimum reprojection (pix): a forward per-pixel march with the task table pre_tasks
+                                       // and the select kernel run ahead of the march of this plan
+  SfmTaskTable pre_tasks;
   int nw;                              // SSIM: warps per CTA (2: the two sources split over the warps of a CTA)
   bool srec;                           // SSIM: forward records in shared memory (false: in registers)
   bool edge_smooth;                    // the edge-aware smoothness kernel runs between the prologue and the march
@@ -191,10 +197,16 @@ struct SfmStepPlan {
 };
 // mode bits of the planner
 enum { SFM_MODE_EXP = 1, SFM_MODE_SSIM = 2, SFM_MODE_GRAD = 4, SFM_MODE_DEBUG = 8, SFM_MODE_SMOOTH = 16, SFM_MODE_IMG = 32,
-       SFM_MODE_PIX = 64 };
+       SFM_MODE_PIX = 64, SFM_MODE_MINREP = 128 };
 SfmStepPlan sfm_plan_step(const SfmDesc* d, int mode, int num_sms);
 int sfm_plan_band(const SfmDesc* d);
-int sfm_launch_fused(SfmFusedParams& p, const SfmStepPlan& plan, cudaStream_t stream);
+// Minimum reprojection (sfm_loss_min_reprojection): the planes p.pix_w[s] are written by the forward march and turned
+// into the one-hot weights by the select kernel, which also writes the optional selection maps.
+struct SfmMinRepArgs {
+  int automask;
+  int8_t* selection[SFM_MAX_SCALES];
+};
+int sfm_launch_fused(SfmFusedParams& p, const SfmStepPlan& plan, cudaStream_t stream, const SfmMinRepArgs* mr = nullptr);
 int sfm_launch_edge_smooth(const SfmFusedParams& p, bool grad, cudaStream_t stream);   // smooth.cu
 extern thread_local cudaEvent_t sfm_ev_start, sfm_ev_stop;   // profiling hook (sfm_set_kernel_events)
 

@@ -184,6 +184,7 @@ SfmStepPlan sfm_plan_step(const SfmDesc* d, int mode, int num_sms) {
   q.debug = (mode & SFM_MODE_DEBUG) != 0;
   q.img = q.grad && !q.debug && (mode & SFM_MODE_IMG) != 0;
   q.pix = !q.debug && !q.img && (mode & SFM_MODE_PIX) != 0;
+  q.minrep = q.pix && (mode & SFM_MODE_MINREP) != 0;
   q.raw = d->raw_disp_scales != 0;
   const bool smooth = (mode & SFM_MODE_SMOOTH) != 0;
   q.accum = q.grad && smooth;
@@ -192,6 +193,14 @@ SfmStepPlan sfm_plan_step(const SfmDesc* d, int mode, int num_sms) {
   q.srec = true;
   if (q.ssim) plan_ssim(q, d, num_sms);
   else plan_l1(q, d, num_sms);
+  if (q.minrep) {
+    // the forward march ahead of the select kernel: the per-pixel instance of the forward mode, planned as such
+    SfmStepPlan f = q;
+    f.grad = f.accum = false;
+    if (f.ssim) plan_ssim(f, d, num_sms);
+    else plan_l1(f, d, num_sms);
+    q.pre_tasks = f.tasks;
+  }
   if (smooth && !q.edge_smooth) plan_smooth(q.smooth, d);
   // the long, issue-bound smoothness CTAs are spread over the first 75 % of the pyramid + smoothness blocks: they start
   // early and the short, memory-bound pyramid CTAs fill the SMs around them and run on alone at the end

@@ -104,7 +104,8 @@ enum RowStages {
 // three lags: stage A of row r (the L1 loss partial), row r-1 (lw of the SSIM loss and wl of the gradient fields: a
 // one-step register carry) and row r-2 (the L1 part of dL/dP in stage F: one more field of the forward record).  Stage C
 // stores the map wpix * esum + wssim * sum_c sat(raw_c) = d total / d M of the owned pixels of row r-1, whose esum is
-// carried one step like its weight.  M = 1 multiplies exactly: unit weights give bitwise the plain step.
+// carried one step like its weight (p.pix_map_masked for masked pixels).  M = 1 multiplies exactly: unit weights give
+// bitwise the plain step.
 template <bool GRAD, bool ACCUM, bool DEBUG, bool RAW, int NW, bool SREC = true, bool IMG = false, bool SNIP = false,
           bool PIX = false>
 __global__ void __launch_bounds__(32 * NW, (IMG ? SFM_SSIM_IMG_MIN_WARPS : SREC ? SFM_SSIM_MIN_WARPS : SFM_SSIM_REG_MIN_WARPS) / NW)
@@ -387,7 +388,7 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
         if (PIX) {
           float* const volatile* pq = s_pix_ptrs;
           float* mq = pq[1];
-          if (own_c && c_in && mq) st_global(mq + (unsigned)(rc * w + xx), live_px ? wpix * e_lag1 + wssim * sat3 : 0.f);
+          if (own_c && c_in && mq) st_global(mq + (unsigned)(rc * w + xx), live_px ? wpix * e_lag1 + wssim * sat3 : p.pix_map_masked);
         }
         if (GRAD) {
           // d raw / d(Sp, Spp, Spt) with n, d in the 81x units (SURVEY A.7 rescaled):

@@ -10,7 +10,8 @@ def _torch():
     import torch
     if not _NP2TORCH:
         _NP2TORCH.update({np.dtype('float32'): torch.float32, np.dtype('int32'): torch.int32,
-                          np.dtype('uint8'): torch.uint8, np.dtype('float64'): torch.float64})
+                          np.dtype('uint8'): torch.uint8, np.dtype('float64'): torch.float64,
+                          np.dtype('int8'): torch.int8})
     return torch
 
 

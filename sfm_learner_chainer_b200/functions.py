@@ -42,15 +42,30 @@ class ViewSynthesisLoss(object):
     (sum M * map = (1 - ssim_rate) * pixel + ssim_rate * ssim).  Masks of moving objects, the ego-vehicle or sky, and
     learned weight maps (whose gradient is the map) go in here; a forward call with maps is the validation use.  Not
     with image_grads.
+    min_reprojection: Monodepth2's per-pixel minimum reprojection (each target pixel is scored on the source view with
+    the smallest error, masked sources excluded) and, with automask, its auto-masking (a pixel is dropped when an
+    unwarped source matches the target at least as well); see sfm_loss_min_reprojection in include/sfmloss.h for the
+    exact rules.  forward and forward_backward also return the selection maps (a list of n_scales (B,h_s,w_s) int8
+    arrays: the chosen source, -1 auto-masked, -2 no candidate), appended like the pixel maps / as `selection`.  Not
+    with exp_reg, image_grads or pixel_terms; ssim_rate must lie in [0, 1].
     """
 
     def __init__(self, smooth_reg=0.0, exp_reg=0.0, ssim_rate=0.0, n_scales=N_SCALES, B_global=None,
                  raw_disp_scales=0, raw_pose=False, edge_aware_smooth=False, image_grads=False,
-                 intrinsics_grad=False, snippet_terms=False, pixel_terms=False):
+                 intrinsics_grad=False, snippet_terms=False, pixel_terms=False, min_reprojection=False, automask=True):
         if image_grads and edge_aware_smooth:
             raise ValueError('image_grads is not supported together with edge_aware_smooth')
         if image_grads and pixel_terms:
             raise ValueError('image_grads is not supported together with pixel_terms')
+        if min_reprojection:
+            if image_grads or pixel_terms:
+                raise ValueError('min_reprojection is not supported together with image_grads or pixel_terms')
+            if float(exp_reg or 0.0) != 0.0:
+                raise ValueError('min_reprojection is not supported together with the explainability branch (exp_reg)')
+            if not 0.0 <= float(ssim_rate or 0.0) <= 1.0:
+                raise ValueError('min_reprojection needs ssim_rate in [0, 1]')
+        self.min_reprojection = bool(min_reprojection)
+        self.automask = bool(automask)
         self.pixel_terms = bool(pixel_terms)
         self.image_grads = bool(image_grads)
         self.intrinsics_grad = bool(intrinsics_grad)
@@ -81,12 +96,16 @@ class ViewSynthesisLoss(object):
             flags |= L.SFM_FLAG_IMAGE_GRADS
         if self.snippet_terms:
             flags |= L.SFM_FLAG_SNIPPET_TERMS
+        if self.min_reprojection:
+            flags |= L.SFM_FLAG_MIN_REPROJECTION
         return L.SfmDesc(B, S, H, W, self.n_scales, int(self.B_global or 0), self.smooth_reg, self.exp_reg,
                          self.ssim_rate, flags, self.raw_disp_scales, raw_pose_hw)
 
     def _workspace(self, desc, like):
-        # the image-gradient and snippet-terms flags size the workspace; the per-call flags (tables, reused pyramid) do not
-        key = (desc.B, desc.S, desc.H, desc.W, desc.n_scales, desc.flags & (L.SFM_FLAG_IMAGE_GRADS | L.SFM_FLAG_SNIPPET_TERMS),
+        # the image-gradient, snippet-terms and min-reprojection flags size the workspace; the per-call flags (tables,
+        # reused pyramid) do not
+        sizing = L.SFM_FLAG_IMAGE_GRADS | L.SFM_FLAG_SNIPPET_TERMS | L.SFM_FLAG_MIN_REPROJECTION
+        key = (desc.B, desc.S, desc.H, desc.W, desc.n_scales, desc.flags & sizing,
                str(getattr(like, 'device', '')))
         ws = self._ws.get(key)
         if ws is None:
@@ -203,17 +222,39 @@ class ViewSynthesisLoss(object):
             pt.losses[s] = D.ptr(maps[s])
         return pt, maps
 
+    def _min_reprojection(self, desc, tgt):
+        """-> (SfmMinReprojection or None, selection maps (list of n_scales (B,h,w) int8) or None)."""
+        if not self.min_reprojection:
+            return None, None
+        mr = L.SfmMinReprojection()
+        mr.automask = 1 if self.automask else 0
+        sel = []
+        for s in range(self.n_scales):
+            sel.append(D.empty(tgt, (desc.B, desc.H >> s, desc.W >> s), 'int8'))
+            mr.selection[s] = D.ptr(sel[s])
+        return mr, sel
+
     # ---- operators
     def forward(self, tgt, src, intrinsics, disps, poses, logits=None, proj=None, kinv=None, debug=False,
                 snippet_weights=None, pixel_weights=None):
         """-> losses (5,) device array in the order of lib.LOSS_KEYS [, debug dict].
         With the operator's snippet_terms: -> (losses, snippet losses (B,5)), losses = sum_b w_b * l_b.
         With the operator's pixel_terms the per-pixel loss maps (list of n_scales (B,S,h,w)) are appended as the last
-        element: (losses, maps) or (losses, snippet losses, maps)."""
-        if debug and (self.snippet_terms or self.pixel_terms):
-            raise ValueError('debug dumps are not available on an operator with snippet_terms or pixel_terms')
+        element: (losses, maps) or (losses, snippet losses, maps).
+        With the operator's min_reprojection the selection maps (list of n_scales (B,h,w) int8) are appended likewise."""
+        if debug and (self.snippet_terms or self.pixel_terms or self.min_reprojection):
+            raise ValueError('debug dumps are not available on an operator with snippet_terms, pixel_terms or min_reprojection')
         desc, inp = self._pack(tgt, src, intrinsics, disps, poses, logits, proj, kinv)
         losses = D.empty(tgt, (5,))
+        if self.min_reprojection:
+            terms, rows = self._snippet_terms(desc, tgt, snippet_weights)
+            if pixel_weights is not None:
+                raise ValueError('pixel_weights needs ViewSynthesisLoss(pixel_terms=True)')
+            mr, sel = self._min_reprojection(desc, tgt)
+            L.check(self._lib.sfm_loss_min_reprojection(C.byref(desc), C.byref(inp), C.byref(terms) if terms else None,
+                                                        C.byref(mr), _vp(losses), None, self._workspace(desc, tgt), None,
+                                                        C.c_void_p(D.current_stream(tgt))))
+            return (losses,) + ((rows,) if self.snippet_terms else ()) + (sel,)
         if self.snippet_terms or self.pixel_terms:
             terms, rows = self._snippet_terms(desc, tgt, snippet_weights)
             pt, maps = self._pixel_terms(desc, tgt, pixel_weights)
@@ -288,7 +329,9 @@ class ViewSynthesisLoss(object):
         snippet_losses (B,5), this shard's rows l_b.
         With the operator's pixel_terms: pixel_weights (list of n_scales (B,S,h,w) or None entries) weight the
         photometric terms per (pixel, source), and the dict also holds pixel_losses, the maps d total / d weights
-        (this shard's, under peer)."""
+        (this shard's, under peer).
+        With the operator's min_reprojection the dict also holds selection (list of n_scales (B,h,w) int8; this
+        shard's, under peer)."""
         want_k = self._want_intrinsics_grad(intrinsics_grad, proj, kinv)
         desc, inp = self._pack(tgt, src, intrinsics, disps, poses, logits, proj, kinv)
         if reuse_pyramid:
@@ -302,6 +345,16 @@ class ViewSynthesisLoss(object):
         pt, maps = self._pixel_terms(desc, tgt, pixel_weights)
         if maps is not None:
             out['pixel_losses'] = maps
+        if self.min_reprojection:
+            mr, out['selection'] = self._min_reprojection(desc, tgt)
+            L.check(self._lib.sfm_loss_min_reprojection(C.byref(desc), C.byref(inp), C.byref(terms) if terms else None,
+                                                        C.byref(mr), _vp(losses), C.byref(g), self._workspace(desc, tgt),
+                                                        peer.handle if peer is not None else None,
+                                                        C.c_void_p(D.current_stream(tgt))))
+            self._intrinsics_grad(desc, inp, tgt, out, want_k)
+            if self._ev_pyramid is not None:
+                self._ev_loss = D.record_event(tgt)
+            return losses, out
         ig = None
         want = set(image_grads) if self.image_grads else set()
         if want:

@@ -14,6 +14,7 @@ SFM_FLAG_NO_TMA = 0x4
 SFM_FLAG_EDGE_AWARE_SMOOTH = 0x8
 SFM_FLAG_IMAGE_GRADS = 0x10
 SFM_FLAG_SNIPPET_TERMS = 0x20
+SFM_FLAG_MIN_REPROJECTION = 0x40
 
 SFM_E_INVALID_DESC = -1
 SFM_E_INVALID_SHAPE = -2
@@ -57,6 +58,10 @@ class SfmPixelTerms(C.Structure):
     _fields_ = [('weights', _vp * SFM_MAX_SCALES), ('losses', _vp * SFM_MAX_SCALES)]
 
 
+class SfmMinReprojection(C.Structure):
+    _fields_ = [('automask', C.c_int32), ('reserved_', C.c_int32), ('selection', _vp * SFM_MAX_SCALES)]
+
+
 class SfmAugment(C.Structure):
     _fields_ = [('out_h', C.c_int32), ('out_w', C.c_int32), ('off_y', C.c_int32), ('off_x', C.c_int32),
                 ('flip', C.c_int32), ('reserved_', C.c_int32), ('x_scaling', C.c_double), ('y_scaling', C.c_double)]
@@ -73,6 +78,7 @@ _D, _I, _G, _Dbg = C.POINTER(SfmDesc), C.POINTER(SfmInputs), C.POINTER(SfmGrads)
 _IG = C.POINTER(SfmImageGrads)
 _ST = C.POINTER(SfmSnippetTerms)
 _PT = C.POINTER(SfmPixelTerms)
+_MR = C.POINTER(SfmMinReprojection)
 SYMBOLS = {
     'sfm_version': (_i, []),
     'sfm_last_error': (C.c_char_p, []),
@@ -117,6 +123,7 @@ SYMBOLS = {
     'sfm_loss_forward_backward_peer': (_i, [_D, _I, _vp, _G, _vp, _vp, _vp]),
     'sfm_loss_snippets': (_i, [_D, _I, _ST, _vp, _G, _IG, _vp, _vp, _vp]),
     'sfm_loss_weighted': (_i, [_D, _I, _ST, _PT, _vp, _G, _IG, _vp, _vp, _vp]),
+    'sfm_loss_min_reprojection': (_i, [_D, _I, _ST, _MR, _vp, _G, _vp, _vp, _vp]),
 }
 
 _lib = None

@@ -42,6 +42,7 @@ class _ViewSynthesisLossFn(torch.autograd.Function):
         ctx.maps = grads.get('pixel_losses') or []
         ctx.want_pw = [w is not None and ctx.needs_input_grad[8 + n_pred + s] for s, w in enumerate(pix_w)]
         outs += ctx.maps
+        outs += grads.get('selection') or []      # min_reprojection: the selection maps, non-differentiable
         ctx.mark_non_differentiable(*outs)
         return (losses[0].clone(),) + tuple(outs)
 
@@ -80,6 +81,8 @@ def view_synthesis_loss(op, tgt, src, intrinsics, pred_disps, pred_poses, pred_m
     With op.pixel_terms: pixel_weights (list of n_scales (B,S,h,w) tensors or None entries; None = all 1) weight the
     photometric terms per (pixel, source), and pixel_losses (list of n_scales maps d total / d weights) is appended to
     the returned tuple; weights that require grad receive gy * pixel_losses[s].
+    With op.min_reprojection: the selection maps (list of n_scales (B,h,w) int8 tensors: the chosen source, -1
+    auto-masked, -2 no candidate) are appended to the returned tuple; they are not differentiable.
     """
     assert isinstance(op, ViewSynthesisLoss)
     if snippet_weights is not None and not op.snippet_terms:
@@ -96,7 +99,7 @@ def view_synthesis_loss(op, tgt, src, intrinsics, pred_disps, pred_poses, pred_m
     use_exp = op.use_exp
     preds = list(pred_disps) + [pred_poses] + (list(pred_maskes) if use_exp else [])
     res = _ViewSynthesisLossFn.apply(op, tgt, src, intrinsics, snippet_weights, op.n_scales, use_exp, len(preds), *preds, *pix_w)
-    if not op.pixel_terms:
+    if not (op.pixel_terms or op.min_reprojection):
         return res
     k = len(res) - op.n_scales
     return tuple(res[:k]) + (list(res[k:]),)

@@ -1,14 +1,18 @@
 """Step time of the fused loss with and without one opt-in option: image_grads (ViewSynthesisLoss(image_grads=True)),
 intrinsics_grad (ViewSynthesisLoss(intrinsics_grad=True)), snippet_terms (ViewSynthesisLoss(snippet_terms=True) with
-per-snippet weights, returning the per-snippet losses) or pixel_terms (ViewSynthesisLoss(pixel_terms=True) with random
-per-pixel weights in [0, 1] at every scale, returning the per-pixel loss maps).
+per-snippet weights, returning the per-snippet losses), pixel_terms (ViewSynthesisLoss(pixel_terms=True) with random
+per-pixel weights in [0, 1] at every scale, returning the per-pixel loss maps) or min_reprojection
+(ViewSynthesisLoss(min_reprojection=True), auto-masking on, returning the selection maps; not with the explainability
+branch, so its default configs are cfg1, cfg2 and cfg5).
 
 For each config the step (forward_backward on device tensors) is captured four times into one CUDA graph and the graph
 is replayed; the two variants alternate, and the median over the repeats is reported per step.  Prints one JSON line
 per config and writes them all, with the card name and its power limit, to the file given as the first argument.
 The last column is the relative overhead for image_grads and the added microseconds for intrinsics_grad (the cost of
-one extra dependent launch, sfm_intrinsics_grad_kernel) and for snippet_terms, the relative overhead for pixel_terms.
-usage: python tools/time_opt_in_grads.py OUT.json {image_grads,intrinsics_grad,snippet_terms,pixel_terms} [cfg ...]"""
+one extra dependent launch, sfm_intrinsics_grad_kernel) and for snippet_terms, the relative overhead for pixel_terms and
+min_reprojection.
+usage: python tools/time_opt_in_grads.py OUT.json {image_grads,intrinsics_grad,snippet_terms,pixel_terms,min_reprojection}
+       [cfg ...]"""
 import json
 import os
 import subprocess
@@ -28,6 +32,7 @@ LAST_COLUMN = {
     'intrinsics_grad': ('extra_us', lambda p, q: round(q - p, 2)),
     'snippet_terms': ('extra_us', lambda p, q: round(q - p, 2)),
     'pixel_terms': ('overhead', lambda p, q: round(q / p - 1.0, 4)),
+    'min_reprojection': ('overhead', lambda p, q: round(q / p - 1.0, 4)),
 }
 
 
@@ -67,7 +72,7 @@ def main():
     if len(sys.argv) < 3 or sys.argv[2] not in LAST_COLUMN:
         sys.exit(__doc__)
     out, option = sys.argv[1:3]
-    names = sys.argv[3:] or ['cfg1', 'cfg2', 'cfg4', 'cfg5']
+    names = sys.argv[3:] or (['cfg1', 'cfg2', 'cfg5'] if option == 'min_reprojection' else ['cfg1', 'cfg2', 'cfg4', 'cfg5'])
     torch.cuda.set_device(0)
     rows = []
     for name in names:
