@@ -58,6 +58,10 @@ extern "C" {
 #define SFM_FLAG_MIN_REPROJECTION 0x40u /* the workspace also holds B*S*sum_s h_s*w_s floats, the per-(pixel, source) error /
                                          weight planes of sfm_loss_min_reprojection; every other entry point accepts the
                                          flag and behaves exactly as without it */
+#define SFM_FLAG_FULL_RES_MULTISCALE 0x80u /* Monodepth2's full-resolution multi-scale loss (Godard et al., ICCV 2019, §3
+                                         "multi-scale estimation"): the photometric terms of every scale are computed at
+                                         full resolution on the upsampled disparity; see "Full-resolution multi-scale"
+                                         below.  Changes the loss and sizes the workspace */
 
 /*
  * Problem descriptor.  Mirrors the reference's model flags (base_model.py:37-39:
@@ -446,6 +450,46 @@ typedef struct SfmMinReprojection {
 int sfm_loss_min_reprojection(const SfmDesc* desc, const SfmInputs* in, const SfmSnippetTerms* terms,
                               const SfmMinReprojection* mr, float* losses_out, const SfmGrads* grads, void* workspace,
                               SfmPeer* peer, void* stream);
+
+/* Full-resolution multi-scale (SFM_FLAG_FULL_RES_MULTISCALE; Monodepth2, Godard et al., ICCV 2019, §3).  Low-resolution
+ * photometric terms produce holes and texture-copy artefacts, so every coarse disparity is upsampled to the input size
+ * and its photometric terms are computed there.  With the flag, for every scale s < n_scales:
+ *   upsampling     U_s(d) = d_s upsampled to (H, W) with the fp32 arithmetic of torch's
+ *                  F.interpolate(d, size=(H, W), mode='bilinear', align_corners=False): scale = (float)h_s / H,
+ *                  src = max((Y + 0.5f) * scale - 0.5f, 0), y0 = (int)src, y1 = y0 + (y0 < h_s - 1), l1 = src - y0,
+ *                  l0 = 1 - l1, the same for x, value ly0 * (lx0 * d[y0,x0] + lx1 * d[y0,x1]) + ly1 * (lx0 * d[y1,x0] +
+ *                  lx1 * d[y1,x1]).  scale is h_s / H, not 2^-s (they differ when H is not a multiple of 2^s).  Scale 0 is
+ *                  the identity and is never copied.
+ *   photometric    the terms of scale s are those of scale 0 with disps[0] replaced by U_s(d_s): warped with
+ *                  K_0 = intrinsics[:, 0] and the caller's tgt / src, over H x W pixels, means over B_global*3*H*W, the
+ *                  same mask, SSIM windows and x2 out-of-view rule.
+ *   smoothness     (second-order, or edge-aware with the target pyramid level) stays on d_s at its native resolution
+ *                  with its smooth_reg / 2^s weight, unchanged.
+ *   loss           the scales are summed as the reference does; Monodepth2's 1 / num_scales is a constant the caller
+ *                  applies.
+ *   gradients      those of this total: gdisps[s] = U_s^T(d total / d U_s(d_s)) + the smoothness gradient, at
+ *                  (B,1,h_s,w_s); gposes through K_0 at every scale.  The adjoint is a gather without atomics, so gdisps
+ *                  are bitwise reproducible from run to run.
+ *   raw disparity  with bit s >= 1 of raw_disp_scales the activation is applied at native resolution before the
+ *                  upsampling (Monodepth2's order) and gdisps[s] is multiplied by its derivative at the native pixel.
+ *                  Bit 0 is unchanged.
+ *   shapes         every per-scale map of the photometric terms grows to H x W: SfmPixelTerms weights and maps (B,S,H,W),
+ *                  the selections of sfm_loss_min_reprojection (B,H,W), the debug dumps (B,S,3,H,W) / (B,S,H,W), and the
+ *                  min-reprojection workspace planes.
+ *   intrinsics     keeps its (B,n_scales,3,3) shape; only [:, 0] is read by the photometric terms.  With
+ *                  SFM_FLAG_TABLES_PROVIDED the caller's proj / kinv must be those of K_0 at every scale.
+ *                  sfm_intrinsics_grad after such a step returns the sum over the scales at [:, 0] and zeros at [:, 1:].
+ * Supported: sfm_loss_forward (with debug dumps), _backward, _forward_backward, _peer, sfm_loss_snippets,
+ * sfm_loss_weighted, sfm_loss_min_reprojection (with automask, the Monodepth2 configuration), SFM_FLAG_REUSE_PYRAMID,
+ * SFM_FLAG_TABLES_PROVIDED, edge-aware smoothness, raw pose and CUDA-graph capture.  SFM_E_UNSUPPORTED: exp_reg != 0 (the
+ * logits live at scale resolution, and auto-masking replaces the branch), image gradients
+ * (sfm_loss_forward_backward_images, igrads) and sfm_host_ctx_create.  n_scales == 1 with the flag is the step without it.
+ * The workspace holds B*H*W floats per scale >= 1 for the upsampled disparity and as many for its gradient, and a copy
+ * of K_0 per scale.
+ *
+ * sfm_upsample_disparity: the upsampling U on its own (the device code the step uses), x (N,1,h,w) -> y (N,1,H,W),
+ * for tests and callers that want the upsampled maps. */
+int sfm_upsample_disparity(int N, int h, int w, int H, int W, const float* x, float* y, void* stream);
 
 #ifdef __cplusplus
 }

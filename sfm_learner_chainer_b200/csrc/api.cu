@@ -182,6 +182,16 @@ int run_loss(const SfmDesc* d, const SfmInputs* in, float* losses_out, const Sfm
     return SFM_E_NO_DEVICE;
   }
   const Modes m = modes_of(d);
+  const bool fr = sfm_full_res(d);
+  if (fr && m.use_exp) {
+    sfm_set_error("unsupported: SFM_FLAG_FULL_RES_MULTISCALE together with the explainability branch (exp_reg != 0): the logits "
+                  "live at scale resolution");
+    return SFM_E_UNSUPPORTED;
+  }
+  if (fr && ig) {
+    sfm_set_error("unsupported: image gradients together with SFM_FLAG_FULL_RES_MULTISCALE");
+    return SFM_E_UNSUPPORTED;
+  }
   int mode = 0;
   if (m.use_exp) mode |= SFM_MODE_EXP;
   if (m.use_ssim) mode |= SFM_MODE_SSIM;
@@ -200,7 +210,7 @@ int run_loss(const SfmDesc* d, const SfmInputs* in, float* losses_out, const Sfm
   p.B = d->B; p.S = d->S; p.ns = d->n_scales;
   const double Bg = (double)(d->B_global > 0 ? d->B_global : d->B);
   for (int s = 0; s < d->n_scales; ++s) {
-    const int h = d->H >> s, w = d->W >> s;
+    const int h = d->H >> s, w = d->W >> s;           // native size: the smoothness terms
     p.h[s] = h; p.w[s] = w;
     p.tgt_pl[s] = s == 0 ? in->tgt : (const float*)(ws + L.off_tgt[s]);
     p.src_pl[s] = s == 0 ? in->src : (const float*)(ws + L.off_src[s]);
@@ -208,16 +218,12 @@ int run_loss(const SfmDesc* d, const SfmInputs* in, float* losses_out, const Sfm
     p.logits[s] = m.use_exp ? in->logits[s] : nullptr;
     p.gdisp[s] = grads ? grads->gdisps[s] : nullptr;
     p.glogits[s] = (grads && m.use_exp) ? grads->glogits[s] : nullptr;
-    p.inv_n3[s] = (float)(1.0 / (Bg * 3.0 * h * w));
-    p.inv_n1[s] = (float)(1.0 / (Bg * h * w));
     const double wgt = (double)d->smooth_reg / (double)(1 << s);
     p.sm_dx2[s] = (float)(wgt / (Bg * h * (w - 2)));
     p.sm_mix[s] = (float)(wgt / (Bg * (h - 1) * (w - 1)));
     p.sm_dy2[s] = (float)(wgt / (Bg * (h - 2) * w));
     p.sm_ex[s] = (float)(wgt / (Bg * h * (w - 1)));
     p.sm_ey[s] = (float)(wgt / (Bg * (h - 1) * w));
-    p.hwf[s] = (float)((w - 1) / 2.0);
-    p.hhf[s] = (float)((h - 1) / 2.0);
     sm.disp[s] = p.disp[s];
     sm.gdisp[s] = p.gdisp[s];
     sm.k_dx2[s] = p.sm_dx2[s]; sm.k_mix[s] = p.sm_mix[s]; sm.k_dy2[s] = p.sm_dy2[s];
@@ -234,10 +240,18 @@ int run_loss(const SfmDesc* d, const SfmInputs* in, float* losses_out, const Sfm
     }
     if (mr) p.pix_w[s] = (const float*)(ws + L.off_mrw[s]);   // the one-hot weights, made by the select kernel
   }
+  auto photometric_consts = [&](int s) {              // from the size of the photometric terms of scale s
+    const int h = p.h[s], w = p.w[s];
+    p.inv_n3[s] = (float)(1.0 / (Bg * 3.0 * h * w));
+    p.inv_n1[s] = (float)(1.0 / (Bg * h * w));
+    p.hwf[s] = (float)((w - 1) / 2.0);
+    p.hhf[s] = (float)((h - 1) / 2.0);
+  };
+  for (int s = 0; s < d->n_scales; ++s) photometric_consts(s);
   const bool tables = (d->flags & SFM_FLAG_TABLES_PROVIDED) != 0;
   p.proj = tables ? in->proj : (const float*)(ws + L.off_proj);
   p.kinv = tables ? in->kinv : (const float*)(ws + L.off_kinv);
-  p.intrinsics = in->intrinsics;
+  p.intrinsics = fr ? (const float*)(ws + L.off_k0) : in->intrinsics;
   p.poses = d->raw_pose_hw > 0 ? (const float*)(ws + L.off_posevec) : in->poses;
   p.raw_pose_hw = d->raw_pose_hw;
   p.raw_disp_mask = d->raw_disp_scales;
@@ -255,7 +269,7 @@ int run_loss(const SfmDesc* d, const SfmInputs* in, float* losses_out, const Sfm
   // prologue kernel: pyramid + tables + cell reset and, in the same grid, the second-order smoothness tasks (the
   // edge-aware variant reads the pyramid and is launched by sfm_launch_fused after it)
   sm.gy = gy;
-  sm.raw_disp_mask = p.raw_disp_mask;
+  sm.raw_disp_mask = d->raw_disp_scales;
   sm.part = (float*)(ws + L.off_smpart);
   p.sm_part = sm.part;
   p.n_sm_part = sm.n_ctas;
@@ -271,7 +285,37 @@ int run_loss(const SfmDesc* d, const SfmInputs* in, float* losses_out, const Sfm
     p.sm_part = sm.task_part;
     p.sm_hseg = sm.n_ctas > 0 ? sm.hseg : 0;
   }
-  SfmPrepParams pp = prep_params(d, plan.band, ws, reuse ? nullptr : in->tgt, in->src, in->intrinsics, in->poses,
+  // SFM_FLAG_FULL_RES_MULTISCALE: `native` keeps the scales as the smoothness kernels see them, and every scale >= 1 of
+  // the photometric step becomes a full-resolution scale (the caller's images, U_s(d_s) and its gradient plane in the
+  // workspace, the activation already applied by the upsample kernel); the tables are built from the K_0 copy
+  SfmFusedParams native;
+  SfmFullRes f{};
+  if (fr) {
+    native = p;
+    f.B = d->B; f.ns = d->n_scales; f.H = d->H; f.W = d->W;
+    f.raw_disp_mask = d->raw_disp_scales;
+    f.intrinsics = in->intrinsics;
+    f.k0 = (float*)(ws + L.off_k0);
+    f.zero_gup = plan.accum ? 1 : 0;
+    f.accum = plan.accum ? 1 : 0;
+    for (int s = 1; s < d->n_scales; ++s) {
+      f.h[s] = p.h[s]; f.w[s] = p.w[s];
+      f.disp[s] = in->disps[s];
+      f.gdisp[s] = p.gdisp[s];
+      f.up[s] = (float*)(ws + L.off_up[s]);
+      f.gup[s] = grads ? (float*)(ws + L.off_gup[s]) : nullptr;
+      p.h[s] = d->H; p.w[s] = d->W;
+      p.tgt_pl[s] = in->tgt;
+      p.src_pl[s] = in->src;
+      p.disp[s] = f.up[s];
+      p.gdisp[s] = f.gup[s];
+      photometric_consts(s);
+    }
+    p.raw_disp_mask = d->raw_disp_scales & 1u;
+  }
+  // under SFM_FLAG_FULL_RES_MULTISCALE only the edge-aware smoothness reads the pyramid
+  const bool pyramid = !reuse && (!fr || plan.edge_smooth);
+  SfmPrepParams pp = prep_params(d, plan.band, ws, pyramid ? in->tgt : nullptr, in->src, p.intrinsics, in->poses,
                                  tables ? nullptr : (float*)(ws + L.off_proj), (float*)(ws + L.off_kinv), true);
   pp.n_mix_region = plan.n_mix_region;
   if (ig && ig->gsrc) {
@@ -279,15 +323,17 @@ int run_loss(const SfmDesc* d, const SfmInputs* in, float* losses_out, const Sfm
     SFM_CUDA_CHECK(cudaMemsetAsync(ig->gsrc, 0, (size_t)d->B * d->S * 3 * d->H * d->W * sizeof(float), st));
     if (L.gsrc_bytes) SFM_CUDA_CHECK(cudaMemsetAsync(ws + L.off_gsrc[1], 0, L.gsrc_bytes, st));
   }
+  if (fr && (rc = sfm_launch_full_res_upsample(f, st))) return rc;
   rc = sfm_launch_prep(pp, &sm, (grads ? 2 : 1) + (snip ? 2 : 0), st);
   if (rc) return rc;
+  SfmMinRepArgs a{};
   if (mr) {
-    SfmMinRepArgs a{};
     a.automask = mr->automask != 0 ? 1 : 0;
     for (int s = 0; s < d->n_scales; ++s) a.selection[s] = mr->selection[s];
-    return sfm_launch_fused(p, plan, st, &a);
   }
-  return sfm_launch_fused(p, plan, st);
+  rc = sfm_launch_fused(p, plan, st, mr ? &a : nullptr, fr ? &native : nullptr);
+  if (rc || !fr || !grads) return rc;
+  return sfm_launch_full_res_adjoint(f, st);
 }
 
 }  // namespace
@@ -334,6 +380,10 @@ extern "C" int sfm_loss_forward_backward_images(const SfmDesc* desc, const SfmIn
     sfm_set_error("unsupported: image gradients through the edge-aware smoothness term (SFM_FLAG_EDGE_AWARE_SMOOTH)");
     return SFM_E_UNSUPPORTED;
   }
+  if (desc->flags & SFM_FLAG_FULL_RES_MULTISCALE) {
+    sfm_set_error("unsupported: image gradients together with SFM_FLAG_FULL_RES_MULTISCALE");
+    return SFM_E_UNSUPPORTED;
+  }
   if (!igrads || (!igrads->gtgt && !igrads->gsrc)) { sfm_set_error("igrads is NULL or has neither gtgt nor gsrc"); return SFM_E_NULL_POINTER; }
   if (!losses_out) { sfm_set_error("losses_out is NULL"); return SFM_E_NULL_POINTER; }
   if (!grads) { sfm_set_error("grads is NULL"); return SFM_E_NULL_POINTER; }
@@ -363,6 +413,10 @@ extern "C" int sfm_loss_weighted(const SfmDesc* desc, const SfmInputs* in, const
     }
     if (desc->flags & SFM_FLAG_EDGE_AWARE_SMOOTH) {
       sfm_set_error("unsupported: image gradients through the edge-aware smoothness term (SFM_FLAG_EDGE_AWARE_SMOOTH)");
+      return SFM_E_UNSUPPORTED;
+    }
+    if (desc->flags & SFM_FLAG_FULL_RES_MULTISCALE) {
+      sfm_set_error("unsupported: image gradients together with SFM_FLAG_FULL_RES_MULTISCALE");
       return SFM_E_UNSUPPORTED;
     }
     if (!igrads->gtgt && !igrads->gsrc) { sfm_set_error("igrads has neither gtgt nor gsrc"); return SFM_E_NULL_POINTER; }
@@ -448,8 +502,13 @@ extern "C" int sfm_intrinsics_grad(const SfmDesc* desc, const SfmInputs* in, con
   const char* ws = (const char*)workspace;
   // the poses as the step saw them: under raw_pose_hw the vectors its prologue reduced into the workspace
   const float* poses = desc->raw_pose_hw > 0 ? (const float*)(ws + L.off_posevec) : in->poses;
-  return sfm_launch_intrinsics_grad(desc->B, desc->S, desc->n_scales, (const double*)(ws + L.off_acc) + 4, poses, in->intrinsics,
-                                    gintrinsics, (cudaStream_t)stream);
+  // under SFM_FLAG_FULL_RES_MULTISCALE every scale's projection was built from K_0 (the step's copy in the workspace), so
+  // the per-scale gradients are folded into [:, 0]
+  const bool fr = sfm_full_res(desc);
+  rc = sfm_launch_intrinsics_grad(desc->B, desc->S, desc->n_scales, (const double*)(ws + L.off_acc) + 4, poses,
+                                  fr ? (const float*)(ws + L.off_k0) : in->intrinsics, gintrinsics, (cudaStream_t)stream);
+  if (rc || !fr) return rc;
+  return sfm_launch_intrinsics_fold(desc->B, desc->n_scales, gintrinsics, (cudaStream_t)stream);
 }
 
 extern "C" int sfm_scale_intrinsics_grad(const SfmDesc* desc, const float* gy, float* gintrinsics, void* stream) {
@@ -550,6 +609,15 @@ extern "C" int sfm_disp_activation(long long n, const float* x, float* disp, flo
   return sfm_launch_disp_activation(n, x, disp, dact, (cudaStream_t)stream);
 }
 
+extern "C" int sfm_upsample_disparity(int N, int h, int w, int H, int W, const float* x, float* y, void* stream) {
+  if (N < 1 || h < 1 || w < 1 || h > H || w > W || (long long)N * H * W >= (1ll << 31)) {
+    sfm_set_error("sfm_upsample_disparity: invalid shape N=%d %dx%d -> %dx%d", N, h, w, H, W);
+    return SFM_E_INVALID_SHAPE;
+  }
+  if (!x || !y) { sfm_set_error("sfm_upsample_disparity: null pointer"); return SFM_E_NULL_POINTER; }
+  return sfm_launch_upsample_stage(N, h, w, H, W, x, y, (cudaStream_t)stream);
+}
+
 extern "C" int sfm_pose_reduce(int B, int S, int hw, const float* x, float* poses_out, void* stream) {
   if (B < 1 || S < 1 || S > SFM_MAX_SOURCES) { sfm_set_error("sfm_pose_reduce: invalid B=%d S=%d", B, S); return SFM_E_INVALID_DESC; }
   if (hw < 1 || hw > 128) { sfm_set_error("sfm_pose_reduce: unsupported hw=%d (1..128)", hw); return SFM_E_UNSUPPORTED; }
@@ -594,6 +662,10 @@ extern "C" int sfm_host_ctx_create(const SfmDesc* desc, SfmHostCtx** ctx_out) {
   int rc = sfm_validate_desc(desc);
   if (rc) return rc;
   if (!ctx_out) { sfm_set_error("ctx_out is NULL"); return SFM_E_NULL_POINTER; }
+  if (desc->flags & SFM_FLAG_FULL_RES_MULTISCALE) {
+    sfm_set_error("unsupported: the host-buffer path with SFM_FLAG_FULL_RES_MULTISCALE");
+    return SFM_E_UNSUPPORTED;
+  }
   int ndev = 0;
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
     sfm_set_error("no CUDA device: libsfmloss has no CPU fallback");

@@ -51,6 +51,12 @@ struct SfmWsLayout {
   // SFM_FLAG_MIN_REPROJECTION: per-(pixel, source) error planes of the forward march, turned into the one-hot weights
   // by the select kernel.  0 without the flag.
   size_t off_mrw[SFM_MAX_SCALES];   // float [B][S][h][w]
+  // SFM_FLAG_FULL_RES_MULTISCALE with n_scales > 1: the upsampled disparity and its gradient of every scale >= 1 at full
+  // resolution, and K_0 replicated over the scales (what the prologue's tables, the epilogue's pose chain and
+  // sfm_intrinsics_grad read).  0 otherwise.
+  size_t off_up[SFM_MAX_SCALES];    // float [B][H][W]
+  size_t off_gup[SFM_MAX_SCALES];   // float [B][H][W]
+  size_t off_k0;                    // float [B][ns][9]
   size_t acc_doubles;
   size_t total;
 };
@@ -83,6 +89,12 @@ static inline int sfm_smooth_plan(int B, int ns, int H, int W, int* hseg_out) {
   if (hseg_out) *hseg_out = hseg;
   return (int)n;
 }
+
+// SFM_FLAG_FULL_RES_MULTISCALE with more than one scale: the photometric terms of every scale run at full resolution
+static inline bool sfm_full_res(const SfmDesc* d) { return (d->flags & SFM_FLAG_FULL_RES_MULTISCALE) && d->n_scales > 1; }
+// image size of the photometric terms of scale s: (H >> s, W >> s), or (H, W) at every scale with the flag
+static inline int sfm_step_h(const SfmDesc* d, int s) { return sfm_full_res(d) ? d->H : d->H >> s; }
+static inline int sfm_step_w(const SfmDesc* d, int s) { return sfm_full_res(d) ? d->W : d->W >> s; }
 
 static inline void sfm_ws_layout(const SfmDesc* d, SfmWsLayout* L) {
   size_t off = 0;
@@ -137,8 +149,21 @@ static inline void sfm_ws_layout(const SfmDesc* d, SfmWsLayout* L) {
   if (d->flags & SFM_FLAG_MIN_REPROJECTION) {
     for (int s = 0; s < d->n_scales; ++s) {
       L->off_mrw[s] = off;
-      off = sfm_align_up(off + (size_t)d->B * d->S * (d->H >> s) * (d->W >> s) * sizeof(float), 256);
+      off = sfm_align_up(off + (size_t)d->B * d->S * sfm_step_h(d, s) * sfm_step_w(d, s) * sizeof(float), 256);
     }
+  }
+  for (int s = 0; s < SFM_MAX_SCALES; ++s) L->off_up[s] = L->off_gup[s] = 0;
+  L->off_k0 = 0;
+  if (sfm_full_res(d)) {
+    const size_t plane = (size_t)d->B * d->H * d->W * sizeof(float);
+    for (int s = 1; s < d->n_scales; ++s) {
+      L->off_up[s] = off;
+      off = sfm_align_up(off + plane, 256);
+      L->off_gup[s] = off;
+      off = sfm_align_up(off + plane, 256);
+    }
+    L->off_k0 = off;
+    off = sfm_align_up(off + (size_t)d->B * d->n_scales * 9 * sizeof(float), 256);
   }
   L->total = off;
 }

@@ -206,7 +206,10 @@ struct SfmMinRepArgs {
   int automask;
   int8_t* selection[SFM_MAX_SCALES];
 };
-int sfm_launch_fused(SfmFusedParams& p, const SfmStepPlan& plan, cudaStream_t stream, const SfmMinRepArgs* mr = nullptr);
+// native: with SFM_FLAG_FULL_RES_MULTISCALE, the parameters of the native-resolution scales (dims, disparity, gradient,
+// pyramid, raw bits), read by the edge-aware smoothness kernel and by the epilogue's layout of the smoothness tasks
+int sfm_launch_fused(SfmFusedParams& p, const SfmStepPlan& plan, cudaStream_t stream, const SfmMinRepArgs* mr = nullptr,
+                     const SfmFusedParams* native = nullptr);
 int sfm_launch_edge_smooth(const SfmFusedParams& p, bool grad, cudaStream_t stream);   // smooth.cu
 extern thread_local cudaEvent_t sfm_ev_start, sfm_ev_stop;   // profiling hook (sfm_set_kernel_events)
 
@@ -218,3 +221,29 @@ int sfm_launch_image_pullback(const SfmFusedParams& p, int H, int W, cudaStream_
 // used (fused_loss.cu); a dependent launch behind the step's last kernel
 int sfm_launch_intrinsics_grad(int B, int S, int ns, const double* cells, const float* poses, const float* intrinsics,
                                float* gintrinsics, cudaStream_t stream);
+
+// Full-resolution multi-scale (SFM_FLAG_FULL_RES_MULTISCALE, full_res.cu): the scales >= 1 of the step are full-resolution
+// scales whose disparity up[s] = U_s(disp[s]) and gradient gup[s] live in the workspace.
+struct SfmFullRes {
+  int B, ns, H, W;
+  int h[SFM_MAX_SCALES], w[SFM_MAX_SCALES];   // native sizes
+  const float* disp[SFM_MAX_SCALES];          // the caller's maps (pre-activation for the raw bits)
+  float* gdisp[SFM_MAX_SCALES];               // the caller's gradients (nullptr: forward only)
+  float* up[SFM_MAX_SCALES];                  // [B][H][W], s >= 1
+  float* gup[SFM_MAX_SCALES];                 // [B][H][W], s >= 1 (nullptr: forward only)
+  unsigned raw_disp_mask;                     // the caller's raw bits (only s >= 1 are read)
+  const float* intrinsics;                    // the caller's (B, ns, 3, 3)
+  float* k0;                                  // (B, ns, 3, 3): K_0 at every scale
+  int zero_gup;                               // the march accumulates into gup: the upsample kernel zeroes it
+  int accum;                                  // a smoothness kernel wrote gdisp: the adjoint adds to it
+};
+struct SfmUpGrid {
+  int blk_begin[SFM_MAX_SCALES + 1];          // adjoint blocks of scale s: [blk_begin[s], blk_begin[s+1])
+};
+// first in the step's chain, without PDL: U_s(d_s), the zeroed gradient planes and the K_0 copy
+int sfm_launch_full_res_upsample(const SfmFullRes& f, cudaStream_t stream);
+// last, a dependent launch behind the epilogue: gdisp[s] (+)= U_s^T(gup[s]) (times d disp / d x for the raw bits)
+int sfm_launch_full_res_adjoint(const SfmFullRes& f, cudaStream_t stream);
+// gintrinsics[:, 0] = sum over the scales, [:, 1:] = 0; a dependent launch behind the intrinsics-gradient kernel
+int sfm_launch_intrinsics_fold(int B, int ns, float* gintrinsics, cudaStream_t stream);
+int sfm_launch_upsample_stage(int N, int h, int w, int H, int W, const float* x, float* y, cudaStream_t stream);

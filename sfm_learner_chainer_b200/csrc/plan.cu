@@ -42,7 +42,7 @@ SfmTaskTable task_table(int B, int ns, int hseg, const int* nstrip, const int* r
 // (~12 per scheduler), but not below 4 runs, where the prologue / flush of a task dominates (measured).
 void plan_l1(SfmStepPlan& q, const SfmDesc* d, int num_sms) {
   int runs[SFM_MAX_SCALES];
-  for (int s = 0; s < d->n_scales; ++s) runs[s] = ((d->H >> s) * (d->W >> s) + 31) / 32;
+  for (int s = 0; s < d->n_scales; ++s) runs[s] = (sfm_step_h(d, s) * sfm_step_w(d, s) + 31) / 32;
   const long long want_warps = (long long)num_sms * 4 * 12;
   int hseg = 32;
   while (task_table(d->B, d->n_scales, hseg, runs, runs, false).task_begin[SFM_MAX_SCALES] < want_warps && hseg > 4) hseg >>= 1;
@@ -72,8 +72,8 @@ void plan_ssim(SfmStepPlan& q, const SfmDesc* d, int num_sms) {
   const int B = d->B, S = d->S, ns = d->n_scales;
   int hs[SFM_MAX_SCALES], strips[SFM_MAX_SCALES];
   for (int s = 0; s < ns; ++s) {
-    hs[s] = d->H >> s;
-    strips[s] = ((d->W >> s) + SFM_SSIM_IW - 1) / SFM_SSIM_IW;
+    hs[s] = sfm_step_h(d, s);
+    strips[s] = (sfm_step_w(d, s) + SFM_SSIM_IW - 1) / SFM_SSIM_IW;
   }
   // the register-record and source-split instances exist for the plain gradient mode only (no image gradients, no
   // per-pixel terms)
@@ -185,7 +185,8 @@ SfmStepPlan sfm_plan_step(const SfmDesc* d, int mode, int num_sms) {
   q.img = q.grad && !q.debug && (mode & SFM_MODE_IMG) != 0;
   q.pix = !q.debug && !q.img && (mode & SFM_MODE_PIX) != 0;
   q.minrep = q.pix && (mode & SFM_MODE_MINREP) != 0;
-  q.raw = d->raw_disp_scales != 0;
+  // under SFM_FLAG_FULL_RES_MULTISCALE the upsample kernel activates the raw scales >= 1 and the march sees bit 0 only
+  q.raw = (sfm_full_res(d) ? d->raw_disp_scales & 1u : d->raw_disp_scales) != 0;
   const bool smooth = (mode & SFM_MODE_SMOOTH) != 0;
   q.accum = q.grad && smooth;
   q.edge_smooth = smooth && (d->flags & SFM_FLAG_EDGE_AWARE_SMOOTH);
@@ -205,7 +206,8 @@ SfmStepPlan sfm_plan_step(const SfmDesc* d, int mode, int num_sms) {
   // the long, issue-bound smoothness CTAs are spread over the first 75 % of the pyramid + smoothness blocks: they start
   // early and the short, memory-bound pyramid CTAs fill the SMs around them and run on alone at the end
   q.band = sfm_plan_band(d);
-  const bool pyramid = !(d->flags & SFM_FLAG_REUSE_PYRAMID) && d->n_scales > 1;
+  // under SFM_FLAG_FULL_RES_MULTISCALE only the edge-aware smoothness reads the pyramid; without it the prologue has none
+  const bool pyramid = !(d->flags & SFM_FLAG_REUSE_PYRAMID) && d->n_scales > 1 && (!sfm_full_res(d) || q.edge_smooth);
   const long long mix = ((long long)(pyramid ? pyramid_ctas(d, q.band) : 0) + q.smooth.n_ctas) * 75 / 100;
   q.n_mix_region = (int)(mix < q.smooth.n_ctas ? q.smooth.n_ctas : mix);
   return q;

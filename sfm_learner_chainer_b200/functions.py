@@ -48,11 +48,24 @@ class ViewSynthesisLoss(object):
     exact rules.  forward and forward_backward also return the selection maps (a list of n_scales (B,h_s,w_s) int8
     arrays: the chosen source, -1 auto-masked, -2 no candidate), appended like the pixel maps / as `selection`.  Not
     with exp_reg, image_grads or pixel_terms; ssim_rate must lie in [0, 1].
+    full_res_multiscale: Monodepth2's full-resolution multi-scale loss: every coarse disparity is upsampled bilinearly
+    to (H, W) (align_corners=False) and the photometric terms of every scale are computed there with intrinsics[:, 0],
+    while the smoothness term stays at the scale's own resolution; see SFM_FLAG_FULL_RES_MULTISCALE in include/sfmloss.h.
+    The scales are summed (Monodepth2's 1 / num_scales is the caller's).  The gradients keep the native shapes; the
+    per-pixel weights and maps, the selection maps and the debug dumps are (.., H, W) at every scale, and gintrinsics
+    holds the whole gradient at [:, 0].  Not with exp_reg or image_grads.
     """
 
     def __init__(self, smooth_reg=0.0, exp_reg=0.0, ssim_rate=0.0, n_scales=N_SCALES, B_global=None,
                  raw_disp_scales=0, raw_pose=False, edge_aware_smooth=False, image_grads=False,
-                 intrinsics_grad=False, snippet_terms=False, pixel_terms=False, min_reprojection=False, automask=True):
+                 intrinsics_grad=False, snippet_terms=False, pixel_terms=False, min_reprojection=False, automask=True,
+                 full_res_multiscale=False):
+        if full_res_multiscale:
+            if image_grads:
+                raise ValueError('full_res_multiscale is not supported together with image_grads')
+            if float(exp_reg or 0.0) != 0.0:
+                raise ValueError('full_res_multiscale is not supported together with the explainability branch (exp_reg)')
+        self.full_res_multiscale = bool(full_res_multiscale)
         if image_grads and edge_aware_smooth:
             raise ValueError('image_grads is not supported together with edge_aware_smooth')
         if image_grads and pixel_terms:
@@ -98,13 +111,16 @@ class ViewSynthesisLoss(object):
             flags |= L.SFM_FLAG_SNIPPET_TERMS
         if self.min_reprojection:
             flags |= L.SFM_FLAG_MIN_REPROJECTION
+        if self.full_res_multiscale:
+            flags |= L.SFM_FLAG_FULL_RES_MULTISCALE
         return L.SfmDesc(B, S, H, W, self.n_scales, int(self.B_global or 0), self.smooth_reg, self.exp_reg,
                          self.ssim_rate, flags, self.raw_disp_scales, raw_pose_hw)
 
     def _workspace(self, desc, like):
-        # the image-gradient, snippet-terms and min-reprojection flags size the workspace; the per-call flags (tables,
-        # reused pyramid) do not
-        sizing = L.SFM_FLAG_IMAGE_GRADS | L.SFM_FLAG_SNIPPET_TERMS | L.SFM_FLAG_MIN_REPROJECTION
+        # the image-gradient, snippet-terms, min-reprojection and full-resolution flags size the workspace; the per-call
+        # flags (tables, reused pyramid) do not
+        sizing = (L.SFM_FLAG_IMAGE_GRADS | L.SFM_FLAG_SNIPPET_TERMS | L.SFM_FLAG_MIN_REPROJECTION
+                  | L.SFM_FLAG_FULL_RES_MULTISCALE)
         key = (desc.B, desc.S, desc.H, desc.W, desc.n_scales, desc.flags & sizing,
                str(getattr(like, 'device', '')))
         ws = self._ws.get(key)
@@ -157,6 +173,12 @@ class ViewSynthesisLoss(object):
             inp.proj, inp.kinv = _vp(proj), _vp(kinv)
             flags |= L.SFM_FLAG_TABLES_PROVIDED
         return self._desc(B, S, H, W, flags, raw_pose_hw), inp
+
+    def _step_hw(self, desc, s):
+        """(h, w) of the photometric terms of scale s: the scale's own size, or (H, W) with full_res_multiscale."""
+        if self.full_res_multiscale:
+            return desc.H, desc.W
+        return desc.H >> s, desc.W >> s
 
     def _alloc_grads(self, desc, tgt):
         B, S, H, W = desc.B, desc.S, desc.H, desc.W
@@ -214,7 +236,7 @@ class ViewSynthesisLoss(object):
         pt = L.SfmPixelTerms()
         maps = []
         for s in range(ns):
-            shape = (desc.B, desc.S, desc.H >> s, desc.W >> s)
+            shape = (desc.B, desc.S) + self._step_hw(desc, s)
             if pixel_weights[s] is not None:
                 D.check_array(pixel_weights[s], 'pixel_weights[%d]' % s, shape)
                 pt.weights[s] = D.ptr(pixel_weights[s])
@@ -230,7 +252,7 @@ class ViewSynthesisLoss(object):
         mr.automask = 1 if self.automask else 0
         sel = []
         for s in range(self.n_scales):
-            sel.append(D.empty(tgt, (desc.B, desc.H >> s, desc.W >> s), 'int8'))
+            sel.append(D.empty(tgt, (desc.B,) + self._step_hw(desc, s), 'int8'))
             mr.selection[s] = D.ptr(sel[s])
         return mr, sel
 
@@ -273,7 +295,7 @@ class ViewSynthesisLoss(object):
             dbg_struct = L.SfmDebug()
             dbg = dict(P=[], u0=[], v0=[], inb=[])
             for s in range(self.n_scales):
-                h, w = H >> s, W >> s
+                h, w = self._step_hw(desc, s)
                 dbg['P'].append(D.empty(tgt, (B, S, 3, h, w)))
                 dbg['u0'].append(D.empty(tgt, (B, S, h, w), 'int32'))
                 dbg['v0'].append(D.empty(tgt, (B, S, h, w), 'int32'))
@@ -500,6 +522,18 @@ def disp_activation(x, want_dact=False):
     dact = D.empty(x, tuple(x.shape)) if want_dact else None
     L.check(L.load().sfm_disp_activation(n, _vp(x), _vp(disp), _vp(dact), C.c_void_p(D.current_stream(x))))
     return (disp, dact) if want_dact else disp
+
+
+def upsample_disparity(x, H, W):
+    """F.interpolate(x, size=(H, W), mode='bilinear', align_corners=False) of disparity maps x (N,1,h,w) in the fp32
+    arithmetic the full-resolution multi-scale step uses (the same device code).  -> (N,1,H,W)."""
+    D.check_array(x, 'x')
+    if len(x.shape) != 4 or x.shape[1] != 1:
+        raise ValueError('x must be (N, 1, h, w)')
+    N, _, h, w = [int(v) for v in x.shape]
+    y = D.empty(x, (N, 1, int(H), int(W)))
+    L.check(L.load().sfm_upsample_disparity(N, h, w, int(H), int(W), _vp(x), _vp(y), C.c_void_p(D.current_stream(x))))
+    return y
 
 
 def pose_reduce(x, n_sources):

@@ -15,6 +15,7 @@ SFM_FLAG_EDGE_AWARE_SMOOTH = 0x8
 SFM_FLAG_IMAGE_GRADS = 0x10
 SFM_FLAG_SNIPPET_TERMS = 0x20
 SFM_FLAG_MIN_REPROJECTION = 0x40
+SFM_FLAG_FULL_RES_MULTISCALE = 0x80
 
 SFM_E_INVALID_DESC = -1
 SFM_E_INVALID_SHAPE = -2
@@ -100,6 +101,7 @@ SYMBOLS = {
     'sfm_eval_depth': (_i, [_i, _i, _i, _i, _i, _vp, _vp, _vp, C.c_float, C.c_float, _vp, _vp, _vp]),
     'sfm_disp_activation': (_i, [C.c_longlong, _vp, _vp, _vp, _vp]),
     'sfm_pose_reduce': (_i, [_i, _i, _i, _vp, _vp, _vp]),
+    'sfm_upsample_disparity': (_i, [_i, _i, _i, _i, _i, _vp, _vp, _vp]),
     'sfm_warp_forward': (_i, [_i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     'sfm_warp_backward_scratch_bytes': (C.c_size_t, [_i]),
     'sfm_warp_backward': (_i, [_i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),

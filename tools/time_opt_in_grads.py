@@ -3,16 +3,18 @@ intrinsics_grad (ViewSynthesisLoss(intrinsics_grad=True)), snippet_terms (ViewSy
 per-snippet weights, returning the per-snippet losses), pixel_terms (ViewSynthesisLoss(pixel_terms=True) with random
 per-pixel weights in [0, 1] at every scale, returning the per-pixel loss maps) or min_reprojection
 (ViewSynthesisLoss(min_reprojection=True), auto-masking on, returning the selection maps; not with the explainability
-branch, so its default configs are cfg1, cfg2 and cfg5).
+branch, so its default configs are cfg1, cfg2 and cfg5), full_res_multiscale (ViewSynthesisLoss(full_res_multiscale=True),
+Monodepth2's full-resolution photometric terms at every scale; default configs cfg1, cfg2 and cfg5) or
+full_res_min_reprojection (min_reprojection with and without full_res_multiscale; default configs cfg2 and cfg5).
 
 For each config the step (forward_backward on device tensors) is captured four times into one CUDA graph and the graph
 is replayed; the two variants alternate, and the median over the repeats is reported per step.  Prints one JSON line
 per config and writes them all, with the card name and its power limit, to the file given as the first argument.
 The last column is the relative overhead for image_grads and the added microseconds for intrinsics_grad (the cost of
 one extra dependent launch, sfm_intrinsics_grad_kernel) and for snippet_terms, the relative overhead for pixel_terms and
-min_reprojection.
-usage: python tools/time_opt_in_grads.py OUT.json {image_grads,intrinsics_grad,snippet_terms,pixel_terms,min_reprojection}
-       [cfg ...]"""
+min_reprojection, full_res_multiscale and full_res_min_reprojection.
+usage: python tools/time_opt_in_grads.py OUT.json {image_grads,intrinsics_grad,snippet_terms,pixel_terms,min_reprojection,
+       full_res_multiscale,full_res_min_reprojection} [cfg ...]"""
 import json
 import os
 import subprocess
@@ -33,7 +35,13 @@ LAST_COLUMN = {
     'snippet_terms': ('extra_us', lambda p, q: round(q - p, 2)),
     'pixel_terms': ('overhead', lambda p, q: round(q / p - 1.0, 4)),
     'min_reprojection': ('overhead', lambda p, q: round(q / p - 1.0, 4)),
+    'full_res_multiscale': ('overhead', lambda p, q: round(q / p - 1.0, 4)),
+    'full_res_min_reprojection': ('overhead', lambda p, q: round(q / p - 1.0, 4)),
 }
+# operator options of the two variants where they are not (nothing, {option: True})
+VARIANTS = {'full_res_min_reprojection': (dict(min_reprojection=True), dict(min_reprojection=True, full_res_multiscale=True))}
+DEFAULT_CONFIGS = {'min_reprojection': ['cfg1', 'cfg2', 'cfg5'], 'full_res_multiscale': ['cfg1', 'cfg2', 'cfg5'],
+                   'full_res_min_reprojection': ['cfg2', 'cfg5']}
 
 
 def card():
@@ -72,7 +80,7 @@ def main():
     if len(sys.argv) < 3 or sys.argv[2] not in LAST_COLUMN:
         sys.exit(__doc__)
     out, option = sys.argv[1:3]
-    names = sys.argv[3:] or (['cfg1', 'cfg2', 'cfg5'] if option == 'min_reprojection' else ['cfg1', 'cfg2', 'cfg4', 'cfg5'])
+    names = sys.argv[3:] or DEFAULT_CONFIGS.get(option, ['cfg1', 'cfg2', 'cfg4', 'cfg5'])
     torch.cuda.set_device(0)
     rows = []
     for name in names:
@@ -83,7 +91,8 @@ def main():
         args = (dev(d['tgt']), dev(d['src']), dev(d['intrinsics']), [dev(x) for x in d['disps']], dev(d['poses']),
                 [dev(x) for x in d['logits']] if c['exp_reg'] else None)
         # the operators own the workspaces the graphs write: they live as long as the graphs
-        ops = {'plain': ViewSynthesisLoss(**flags), option: ViewSynthesisLoss(**{option: True}, **flags)}
+        base_kw, option_kw = VARIANTS.get(option, ({}, {option: True}))
+        ops = {'plain': ViewSynthesisLoss(**base_kw, **flags), option: ViewSynthesisLoss(**option_kw, **flags)}
         # snippet_terms: weights of a padded batch (the last snippet weighs 0)
         w = torch.full((c['B'],), 1.0, device='cuda')
         w[-1] = 0.0
