@@ -62,6 +62,11 @@ extern "C" {
                                          "multi-scale estimation"): the photometric terms of every scale are computed at
                                          full resolution on the upsampled disparity; see "Full-resolution multi-scale"
                                          below.  Changes the loss and sizes the workspace */
+#define SFM_FLAG_MEAN_NORM_SMOOTH 0x100u /* Monodepth2's mean-normalised smoothness: the smoothness term of every scale is
+                                         evaluated on d_s / (mean(d_s) + 1e-7); see "Mean-normalised smoothness" below.
+                                         Changes the loss and sizes the workspace */
+#define SFM_FLAG_EDGE_MEAN_ABS 0x200u /* with SFM_FLAG_EDGE_AWARE_SMOOTH: Monodepth2's edge weight exp(-mean_c |dI_c|) instead
+                                         of the reference's exp(-|mean_c dI_c|) (else SFM_E_INVALID_DESC) */
 
 /*
  * Problem descriptor.  Mirrors the reference's model flags (base_model.py:37-39:
@@ -490,6 +495,33 @@ int sfm_loss_min_reprojection(const SfmDesc* desc, const SfmInputs* in, const Sf
  * sfm_upsample_disparity: the upsampling U on its own (the device code the step uses), x (N,1,h,w) -> y (N,1,H,W),
  * for tests and callers that want the upsampled maps. */
 int sfm_upsample_disparity(int N, int h, int w, int H, int W, const float* x, float* y, void* stream);
+
+/* Mean-normalised smoothness (SFM_FLAG_MEAN_NORM_SMOOTH; Monodepth2, Godard et al., ICCV 2019, after Wang et al., CVPR
+ * 2018).  Without it the smoothness term rewards shrinking the disparity; dividing by the mean removes that degenerate
+ * solution.  With the flag, for every snippet b and scale s < n_scales:
+ *   mean           m_bs = mean of the activated disparity d_s of snippet b over its native h_s x w_s plane (the raw bits of
+ *                  raw_disp_scales are activated first; under SFM_FLAG_FULL_RES_MULTISCALE the native plane, not the
+ *                  upsampled one, as Monodepth2 does), accumulated in a fixed order.
+ *   smoothness     the term of either kind (second-order, or edge-aware with either edge weight) is evaluated on
+ *                  d_s / (m_bs + 1e-7), with its smooth_reg / 2^s and 1 / B_global factors unchanged.  Every such term is
+ *                  positively homogeneous of degree 1 in d, so with r_bs = 1 / (m_bs + 1e-7) and L_bs the unnormalised term
+ *                  the loss is r_bs * L_bs and its disparity gradient r_bs * dL_bs/dd_j - r_bs^2 * L_bs / (h_s * w_s), times
+ *                  d disp / d x at the pixel for a raw bit, times gy and the snippet weight.
+ *   photometric    untouched.
+ * Composes with every entry point of the fused step (sfm_loss_forward, _backward, _forward_backward, _peer,
+ * sfm_loss_snippets, sfm_loss_weighted, sfm_loss_min_reprojection with or without SFM_FLAG_FULL_RES_MULTISCALE,
+ * sfm_intrinsics_grad afterwards, CUDA-graph capture) and, with second-order smoothness, sfm_loss_forward_backward_images.
+ * The means are per snippet, so snippet sharding needs no communication.  No float atomics feed the result: gdisps stay
+ * bitwise reproducible from run to run.  smooth_reg == 0 with the flag is the step without it.  sfm_host_ctx_create
+ * returns SFM_E_UNSUPPORTED with this flag or SFM_FLAG_EDGE_MEAN_ABS.
+ * Workspace: with the flag it also holds B*n_scales*32 floats of disparity partials, as many of edge-aware loss partials,
+ * B floats of per-snippet smoothness losses and (unless SFM_FLAG_SNIPPET_TERMS already holds it) the per-task loss array
+ * of the second-order term; each array 256-byte aligned.  Without the flag the workspace is unchanged.
+ *
+ * Edge weight (SFM_FLAG_EDGE_MEAN_ABS, needs SFM_FLAG_EDGE_AWARE_SMOOTH): exp(-((|D0| + |D1|) + |D2|) / 3) with D_c the
+ * neighbour difference of channel c of the target image, Monodepth2's form, instead of exp(-|((D0 + D1) + D2) / 3|).  The
+ * two differ where the channel differences have opposite signs.  The weight depends on the image range: Monodepth2's
+ * images are in [0, 1], the reference's in [-1, 1]. */
 
 #ifdef __cplusplus
 }

@@ -64,6 +64,10 @@ int sfm_validate_desc(const SfmDesc* d) {
     sfm_set_error("unsupported SfmDesc: raw_pose_hw > 0 together with SFM_FLAG_TABLES_PROVIDED (the tables are built from the reduced poses)");
     return SFM_E_UNSUPPORTED;
   }
+  if ((d->flags & SFM_FLAG_EDGE_MEAN_ABS) && !(d->flags & SFM_FLAG_EDGE_AWARE_SMOOTH)) {
+    sfm_set_error("invalid SfmDesc: SFM_FLAG_EDGE_MEAN_ABS needs SFM_FLAG_EDGE_AWARE_SMOOTH");
+    return SFM_E_INVALID_DESC;
+  }
   if (!(d->smooth_reg == d->smooth_reg) || !(d->exp_reg == d->exp_reg) || !(d->ssim_rate == d->ssim_rate)) {
     sfm_set_error("invalid SfmDesc: NaN loss weight");
     return SFM_E_INVALID_DESC;
@@ -285,6 +289,49 @@ int run_loss(const SfmDesc* d, const SfmInputs* in, float* losses_out, const Sfm
     p.sm_part = sm.task_part;
     p.sm_hseg = sm.n_ctas > 0 ? sm.hseg : 0;
   }
+  // SFM_FLAG_MEAN_NORM_SMOOTH: the smoothness writers leave the loss of every (snippet, scale) in fixed slots -- the
+  // prologue's per-task losses, or the edge-aware kernel's per-CTA partials -- and the fix-up kernel writes the
+  // normalised loss where the epilogue reads the smoothness: into the snippets' smooth cells, or as its partials
+  const bool mean_norm = (d->flags & SFM_FLAG_MEAN_NORM_SMOOTH) && m.use_smooth;
+  SfmMeanNorm mn{};
+  if (mean_norm) {
+    mn.B = d->B; mn.ns = d->n_scales;
+    const int chunks = (d->H * d->W + 2047) / 2048;
+    mn.chunks = chunks < SFM_MN_SLOTS ? chunks : SFM_MN_SLOTS;
+    for (int s = 0; s < d->n_scales; ++s) {
+      mn.h[s] = p.h[s]; mn.w[s] = p.w[s];
+      mn.disp[s] = in->disps[s];
+      mn.gdisp[s] = p.gdisp[s];
+    }
+    mn.raw_disp_mask = d->raw_disp_scales;
+    mn.gy = gy;
+    mn.snip_w = snip ? snip->weights : nullptr;
+    mn.mean_part = (float*)(ws + L.off_mnmean);
+    if (plan.edge_smooth) {
+      mn.edge_slots = (float*)(ws + L.off_mnedge);
+      mn.loss_part = mn.edge_slots;
+      for (int s = 0; s < d->n_scales; ++s) {
+        mn.loss_off[s] = s * SFM_MN_SLOTS;
+        mn.loss_stride[s] = d->n_scales * SFM_MN_SLOTS;
+        mn.loss_cnt[s] = sfm_edge_smooth_ctas(p.h[0] * p.w[0]);
+      }
+    } else {
+      sm.task_part = (float*)(ws + L.off_smtask);
+      mn.loss_part = sm.task_part;
+      for (int s = 0; s < d->n_scales; ++s) {
+        mn.loss_off[s] = sm.tile_begin[s];
+        mn.loss_stride[s] = mn.loss_cnt[s] = sm.tiles_x[s] * sm.tiles_y[s];
+      }
+    }
+    mn.snip_loss = (float*)(ws + L.off_mnloss);
+    if (snip) {
+      mn.snip_cell = p.acc + L.snip_cell0 + 1;
+      p.sm_hseg = 0;
+    } else {
+      p.sm_part = mn.snip_loss;
+      p.n_sm_part = d->B;
+    }
+  }
   // SFM_FLAG_FULL_RES_MULTISCALE: `native` keeps the scales as the smoothness kernels see them, and every scale >= 1 of
   // the photometric step becomes a full-resolution scale (the caller's images, U_s(d_s) and its gradient plane in the
   // workspace, the activation already applied by the upsample kernel); the tables are built from the K_0 copy
@@ -324,14 +371,15 @@ int run_loss(const SfmDesc* d, const SfmInputs* in, float* losses_out, const Sfm
     if (L.gsrc_bytes) SFM_CUDA_CHECK(cudaMemsetAsync(ws + L.off_gsrc[1], 0, L.gsrc_bytes, st));
   }
   if (fr && (rc = sfm_launch_full_res_upsample(f, st))) return rc;
-  rc = sfm_launch_prep(pp, &sm, (grads ? 2 : 1) + (snip ? 2 : 0), st);
+  rc = sfm_launch_prep(pp, &sm, (grads ? 2 : 1) + ((snip || mean_norm) ? 2 : 0), st);
   if (rc) return rc;
   SfmMinRepArgs a{};
   if (mr) {
     a.automask = mr->automask != 0 ? 1 : 0;
     for (int s = 0; s < d->n_scales; ++s) a.selection[s] = mr->selection[s];
   }
-  rc = sfm_launch_fused(p, plan, st, mr ? &a : nullptr, fr ? &native : nullptr);
+  rc = sfm_launch_fused(p, plan, st, mr ? &a : nullptr, fr ? &native : nullptr, mean_norm ? &mn : nullptr,
+                        (d->flags & SFM_FLAG_EDGE_MEAN_ABS) != 0);
   if (rc || !fr || !grads) return rc;
   return sfm_launch_full_res_adjoint(f, st);
 }
@@ -664,6 +712,10 @@ extern "C" int sfm_host_ctx_create(const SfmDesc* desc, SfmHostCtx** ctx_out) {
   if (!ctx_out) { sfm_set_error("ctx_out is NULL"); return SFM_E_NULL_POINTER; }
   if (desc->flags & SFM_FLAG_FULL_RES_MULTISCALE) {
     sfm_set_error("unsupported: the host-buffer path with SFM_FLAG_FULL_RES_MULTISCALE");
+    return SFM_E_UNSUPPORTED;
+  }
+  if (desc->flags & (SFM_FLAG_MEAN_NORM_SMOOTH | SFM_FLAG_EDGE_MEAN_ABS)) {
+    sfm_set_error("unsupported: the host-buffer path with SFM_FLAG_MEAN_NORM_SMOOTH or SFM_FLAG_EDGE_MEAN_ABS");
     return SFM_E_UNSUPPORTED;
   }
   int ndev = 0;

@@ -57,6 +57,11 @@ struct SfmWsLayout {
   size_t off_up[SFM_MAX_SCALES];    // float [B][H][W]
   size_t off_gup[SFM_MAX_SCALES];   // float [B][H][W]
   size_t off_k0;                    // float [B][ns][9]
+  // SFM_FLAG_MEAN_NORM_SMOOTH: per-CTA disparity sums and edge-aware loss partials of every (snippet, scale), and the
+  // normalised smoothness loss of every snippet.  0 without the flag (which also allocates off_smtask).
+  size_t off_mnmean;                // float [B][ns][SFM_MN_SLOTS]
+  size_t off_mnedge;                // float [B][ns][SFM_MN_SLOTS]
+  size_t off_mnloss;                // float [B]
   size_t acc_doubles;
   size_t total;
 };
@@ -88,6 +93,14 @@ static inline int sfm_smooth_plan(int B, int ns, int H, int W, int* hseg_out) {
   }
   if (hseg_out) *hseg_out = hseg;
   return (int)n;
+}
+
+// SFM_FLAG_MEAN_NORM_SMOOTH: CTAs per (snippet, scale) of the edge-aware smoothness kernel and per snippet of the
+// mean-normalisation kernels, each writing one partial slot
+#define SFM_MN_SLOTS 32
+static inline int sfm_edge_smooth_ctas(int plane0) {
+  const int per = (plane0 + 255) / 256;
+  return per > SFM_MN_SLOTS ? SFM_MN_SLOTS : per;
 }
 
 // SFM_FLAG_FULL_RES_MULTISCALE with more than one scale: the photometric terms of every scale run at full resolution
@@ -127,7 +140,7 @@ static inline void sfm_ws_layout(const SfmDesc* d, SfmWsLayout* L) {
   const int n_sm_tasks = sfm_smooth_plan(d->B, d->n_scales, d->H, d->W, nullptr);
   off = sfm_align_up(off + (size_t)((n_sm_tasks + 7) / 8) * sizeof(float), 256);
   L->off_smtask = 0;
-  if (d->flags & SFM_FLAG_SNIPPET_TERMS) {
+  if (d->flags & (SFM_FLAG_SNIPPET_TERMS | SFM_FLAG_MEAN_NORM_SMOOTH)) {
     L->off_smtask = off;
     off = sfm_align_up(off + (size_t)n_sm_tasks * sizeof(float), 256);
   }
@@ -164,6 +177,16 @@ static inline void sfm_ws_layout(const SfmDesc* d, SfmWsLayout* L) {
     }
     L->off_k0 = off;
     off = sfm_align_up(off + (size_t)d->B * d->n_scales * 9 * sizeof(float), 256);
+  }
+  L->off_mnmean = L->off_mnedge = L->off_mnloss = 0;
+  if (d->flags & SFM_FLAG_MEAN_NORM_SMOOTH) {
+    const size_t slots = (size_t)d->B * d->n_scales * SFM_MN_SLOTS * sizeof(float);
+    L->off_mnmean = off;
+    off = sfm_align_up(off + slots, 256);
+    L->off_mnedge = off;
+    off = sfm_align_up(off + slots, 256);
+    L->off_mnloss = off;
+    off = sfm_align_up(off + (size_t)d->B * sizeof(float), 256);
   }
   L->total = off;
 }

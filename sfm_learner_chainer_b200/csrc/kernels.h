@@ -206,11 +206,35 @@ struct SfmMinRepArgs {
   int automask;
   int8_t* selection[SFM_MAX_SCALES];
 };
+// Mean-normalised smoothness (SFM_FLAG_MEAN_NORM_SMOOTH, mean_norm.cu), per snippet b and native scale s: the sum kernel
+// writes the per-CTA sums of the activated disparity, the fix-up kernel reduces them and the smoothness loss partials
+// of (b, s) in a fixed order into m_bs and L_bs, stores the snippet's normalised loss sum_s L_bs / (m_bs + 1e-7) and, in
+// gradient steps, rewrites the smoothness gradient in place as r G - gy w_b r^2 L_bs / (h w) f (r = 1 / (m_bs + 1e-7)).
+struct SfmMeanNorm {
+  int B, ns, chunks;                          // chunks: CTAs per snippet of both kernels (<= SFM_MN_SLOTS)
+  int h[SFM_MAX_SCALES], w[SFM_MAX_SCALES];   // native sizes
+  const float* disp[SFM_MAX_SCALES];          // the caller's maps (pre-activation for the raw bits)
+  float* gdisp[SFM_MAX_SCALES];               // the caller's gradients, holding the smoothness gradient (nullptr: forward)
+  unsigned raw_disp_mask;
+  const float* gy;                            // device scalar or nullptr (1)
+  const float* snip_w;                        // (B) snippet weights or nullptr
+  float* mean_part;                           // [B][ns][SFM_MN_SLOTS]
+  // loss partials of (b, s): loss_part[loss_off[s] + b * loss_stride[s] + k], k < loss_cnt[s]
+  const float* loss_part;
+  float* edge_slots;                          // edge-aware smoothness: where that kernel writes them (== loss_part)
+  int loss_off[SFM_MAX_SCALES], loss_stride[SFM_MAX_SCALES], loss_cnt[SFM_MAX_SCALES];
+  float* snip_loss;                           // [B] normalised loss of every snippet (the epilogue's smoothness partials)
+  double* snip_cell;                          // per-snippet terms: snippet b's smooth cell at snip_cell[4 b] (else nullptr)
+};
+int sfm_launch_mean_norm_sum(const SfmMeanNorm& m, cudaStream_t stream);   // a dependent launch behind the prologue
+int sfm_launch_mean_norm_fix(const SfmMeanNorm& m, bool grad, cudaStream_t stream);   // behind the smoothness writers
 // native: with SFM_FLAG_FULL_RES_MULTISCALE, the parameters of the native-resolution scales (dims, disparity, gradient,
-// pyramid, raw bits), read by the edge-aware smoothness kernel and by the epilogue's layout of the smoothness tasks
+// pyramid, raw bits), read by the edge-aware smoothness kernel and by the epilogue's layout of the smoothness tasks.
+// mn: SFM_FLAG_MEAN_NORM_SMOOTH with a smoothness term (nullptr otherwise); edge_mean_abs: SFM_FLAG_EDGE_MEAN_ABS
 int sfm_launch_fused(SfmFusedParams& p, const SfmStepPlan& plan, cudaStream_t stream, const SfmMinRepArgs* mr = nullptr,
-                     const SfmFusedParams* native = nullptr);
-int sfm_launch_edge_smooth(const SfmFusedParams& p, bool grad, cudaStream_t stream);   // smooth.cu
+                     const SfmFusedParams* native = nullptr, const SfmMeanNorm* mn = nullptr, bool edge_mean_abs = false);
+// smooth.cu; slots (SFM_FLAG_MEAN_NORM_SMOOTH): the per-CTA loss partials [B][ns][SFM_MN_SLOTS] instead of the cells
+int sfm_launch_edge_smooth(const SfmFusedParams& p, bool grad, bool mean_abs, float* slots, cudaStream_t stream);
 extern thread_local cudaEvent_t sfm_ev_start, sfm_ev_stop;   // profiling hook (sfm_set_kernel_events)
 
 int sfm_launch_scale(float* const* ptrs, const long long* counts, int n, const float* gy, cudaStream_t stream);

@@ -28,8 +28,12 @@ namespace {
 // the gradient, so there is no scatter and no atomic on gdisp.  Needs the pyramid, so unlike the second-order
 // kernel above it starts after the prep kernel.
 // SNIP: per-snippet terms (gradient factor gy * w_b, the loss to snippet b's smooth cell), an instance of its own.
-template <bool GRAD, bool SNIP>
-__global__ void __launch_bounds__(256) sfm_edge_smooth_kernel(const __grid_constant__ SfmFusedParams p) {
+// MEAN_ABS (SFM_FLAG_EDGE_MEAN_ABS): Monodepth2's weight exp(-mean_c |i_dx|).  SLOTS (SFM_FLAG_MEAN_NORM_SMOOTH): the CTA
+// writes its loss partial to slots[blockIdx.y][blockIdx.x] instead of adding it to a cell, so that the mean
+// normalisation (mean_norm.cu) reads the loss of every (snippet, scale) in a fixed order; the gradient factor is
+// gy * w_b whenever snippet weights are given.
+template <bool GRAD, bool SNIP, bool MEAN_ABS = false, bool SLOTS = false>
+__global__ void __launch_bounds__(256) sfm_edge_smooth_kernel(const __grid_constant__ SfmFusedParams p, float* slots) {
   const int s = blockIdx.y % p.ns, b = blockIdx.y / p.ns;
   const int h = p.h[s], w = p.w[s], plane = h * w;
   const bool raw = (p.raw_disp_mask >> s) & 1u;
@@ -38,7 +42,7 @@ __global__ void __launch_bounds__(256) sfm_edge_smooth_kernel(const __grid_const
   float* __restrict__ G = GRAD ? p.gdisp[s] + (size_t)b * plane : nullptr;
   const float kx = p.sm_ex[s], ky = p.sm_ey[s];
   float gyv = (GRAD && p.gy) ? __ldg(p.gy) : 1.f;
-  if (SNIP && GRAD && p.snip_w) gyv *= __ldg(p.snip_w + b);
+  if ((SNIP || SLOTS) && GRAD && p.snip_w) gyv *= __ldg(p.snip_w + b);
   cudaGridDependencySynchronize();          // pyramid and loss cells (prep kernel)
   auto disp_at = [&](int i, float& f) {
     const float v = __ldg(D + i);
@@ -48,7 +52,12 @@ __global__ void __launch_bounds__(256) sfm_edge_smooth_kernel(const __grid_const
   // exp(-|mean_c (b - a)|): F.mean over the three channels = ((d0 + d1) + d2) / 3, F.absolute, F.exp
   struct Px { float x, y, z; };
   auto tex = [&](int i) { Px v; v.x = __ldg(T + i); v.y = __ldg(T + plane + i); v.z = __ldg(T + 2 * plane + i); return v; };
+  // MEAN_ABS: exp(-((|b0 - a0| + |b1 - a1|) + |b2 - a2|) / 3)
   auto edge = [&](const Px& a, const Px& c) {
+    if (MEAN_ABS) {
+      const float m = __fdiv_rn(__fadd_rn(__fadd_rn(fabsf(__fsub_rn(c.x, a.x)), fabsf(__fsub_rn(c.y, a.y))), fabsf(__fsub_rn(c.z, a.z))), 3.f);
+      return expf(-m);
+    }
     const float m = __fdiv_rn(__fadd_rn(__fadd_rn(__fsub_rn(c.x, a.x), __fsub_rn(c.y, a.y)), __fsub_rn(c.z, a.z)), 3.f);
     return expf(-fabsf(m));
   };
@@ -82,17 +91,23 @@ __global__ void __launch_bounds__(256) sfm_edge_smooth_kernel(const __grid_const
   if (threadIdx.x == 0) {
     float t = 0.f;
     for (int k = 0; k < 8; ++k) t += part[k];
-    if (t != 0.f) atomicAdd(p.acc + (SNIP ? p.snip_cell0 + 4 * (size_t)b + 1 : 1), (double)t);
+    if (SLOTS) slots[(size_t)blockIdx.y * SFM_MN_SLOTS + blockIdx.x] = t;
+    else if (t != 0.f) atomicAdd(p.acc + (SNIP ? p.snip_cell0 + 4 * (size_t)b + 1 : 1), (double)t);
   }
 }
 
 }  // namespace
 
-int sfm_launch_edge_smooth(const SfmFusedParams& p, bool grad, cudaStream_t stream) {
-  const int per = (p.h[0] * p.w[0] + 255) / 256;
-  const dim3 grid((unsigned)(per > 32 ? 32 : per), (unsigned)(p.B * p.ns));
-  const auto kernel = p.snip_cell0 ? (grad ? sfm_edge_smooth_kernel<true, true> : sfm_edge_smooth_kernel<false, true>)
-                                    : (grad ? sfm_edge_smooth_kernel<true, false> : sfm_edge_smooth_kernel<false, false>);
-  SFM_CUDA_CHECK(sfm_launch_kernel(kernel, grid, 256, stream, true, p));
+int sfm_launch_edge_smooth(const SfmFusedParams& p, bool grad, bool mean_abs, float* slots, cudaStream_t stream) {
+  const dim3 grid((unsigned)sfm_edge_smooth_ctas(p.h[0] * p.w[0]), (unsigned)(p.B * p.ns));
+  auto kernel = p.snip_cell0 ? (grad ? sfm_edge_smooth_kernel<true, true> : sfm_edge_smooth_kernel<false, true>)
+                             : (grad ? sfm_edge_smooth_kernel<true, false> : sfm_edge_smooth_kernel<false, false>);
+  if (slots)
+    kernel = mean_abs ? (grad ? sfm_edge_smooth_kernel<true, false, true, true> : sfm_edge_smooth_kernel<false, false, true, true>)
+                      : (grad ? sfm_edge_smooth_kernel<true, false, false, true> : sfm_edge_smooth_kernel<false, false, false, true>);
+  else if (mean_abs)
+    kernel = p.snip_cell0 ? (grad ? sfm_edge_smooth_kernel<true, true, true> : sfm_edge_smooth_kernel<false, true, true>)
+                          : (grad ? sfm_edge_smooth_kernel<true, false, true> : sfm_edge_smooth_kernel<false, false, true>);
+  SFM_CUDA_CHECK(sfm_launch_kernel(kernel, grid, 256, stream, true, p, slots));
   return 0;
 }

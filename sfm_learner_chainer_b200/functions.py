@@ -54,12 +54,21 @@ class ViewSynthesisLoss(object):
     The scales are summed (Monodepth2's 1 / num_scales is the caller's).  The gradients keep the native shapes; the
     per-pixel weights and maps, the selection maps and the debug dumps are (.., H, W) at every scale, and gintrinsics
     holds the whole gradient at [:, 0].  Not with exp_reg or image_grads.
+    mean_norm_smooth: Monodepth2's mean-normalised smoothness: the smoothness term of every scale (either kind) is
+    evaluated on disp / (mean(disp) + 1e-7), the mean per snippet and scale over the native plane of the activated
+    disparity; see SFM_FLAG_MEAN_NORM_SMOOTH in include/sfmloss.h.  The photometric terms are untouched.
+    edge_mean_abs: with edge_aware_smooth, Monodepth2's edge weight exp(-mean_c |dI_c|) instead of the reference's
+    exp(-|mean_c dI_c|).
     """
 
     def __init__(self, smooth_reg=0.0, exp_reg=0.0, ssim_rate=0.0, n_scales=N_SCALES, B_global=None,
                  raw_disp_scales=0, raw_pose=False, edge_aware_smooth=False, image_grads=False,
                  intrinsics_grad=False, snippet_terms=False, pixel_terms=False, min_reprojection=False, automask=True,
-                 full_res_multiscale=False):
+                 full_res_multiscale=False, mean_norm_smooth=False, edge_mean_abs=False):
+        if edge_mean_abs and not edge_aware_smooth:
+            raise ValueError('edge_mean_abs needs edge_aware_smooth')
+        self.mean_norm_smooth = bool(mean_norm_smooth)
+        self.edge_mean_abs = bool(edge_mean_abs)
         if full_res_multiscale:
             if image_grads:
                 raise ValueError('full_res_multiscale is not supported together with image_grads')
@@ -113,14 +122,18 @@ class ViewSynthesisLoss(object):
             flags |= L.SFM_FLAG_MIN_REPROJECTION
         if self.full_res_multiscale:
             flags |= L.SFM_FLAG_FULL_RES_MULTISCALE
+        if self.mean_norm_smooth:
+            flags |= L.SFM_FLAG_MEAN_NORM_SMOOTH
+        if self.edge_mean_abs:
+            flags |= L.SFM_FLAG_EDGE_MEAN_ABS
         return L.SfmDesc(B, S, H, W, self.n_scales, int(self.B_global or 0), self.smooth_reg, self.exp_reg,
                          self.ssim_rate, flags, self.raw_disp_scales, raw_pose_hw)
 
     def _workspace(self, desc, like):
-        # the image-gradient, snippet-terms, min-reprojection and full-resolution flags size the workspace; the per-call
-        # flags (tables, reused pyramid) do not
+        # the image-gradient, snippet-terms, min-reprojection, full-resolution and mean-normalisation flags size the
+        # workspace; the per-call flags (tables, reused pyramid) do not
         sizing = (L.SFM_FLAG_IMAGE_GRADS | L.SFM_FLAG_SNIPPET_TERMS | L.SFM_FLAG_MIN_REPROJECTION
-                  | L.SFM_FLAG_FULL_RES_MULTISCALE)
+                  | L.SFM_FLAG_FULL_RES_MULTISCALE | L.SFM_FLAG_MEAN_NORM_SMOOTH)
         key = (desc.B, desc.S, desc.H, desc.W, desc.n_scales, desc.flags & sizing,
                str(getattr(like, 'device', '')))
         ws = self._ws.get(key)

@@ -5,16 +5,22 @@ per-pixel weights in [0, 1] at every scale, returning the per-pixel loss maps) o
 (ViewSynthesisLoss(min_reprojection=True), auto-masking on, returning the selection maps; not with the explainability
 branch, so its default configs are cfg1, cfg2 and cfg5), full_res_multiscale (ViewSynthesisLoss(full_res_multiscale=True),
 Monodepth2's full-resolution photometric terms at every scale; default configs cfg1, cfg2 and cfg5) or
-full_res_min_reprojection (min_reprojection with and without full_res_multiscale; default configs cfg2 and cfg5).
+full_res_min_reprojection (min_reprojection with and without full_res_multiscale; default configs cfg2 and cfg5),
+mean_norm_smooth (ViewSynthesisLoss(mean_norm_smooth=True), Monodepth2's mean-normalised second-order smoothness),
+mean_norm_smooth_edge (the same with edge-aware smoothness on both sides), edge_mean_abs (edge-aware smoothness with and
+without Monodepth2's edge weight) or monodepth2 (full_res_multiscale + min_reprojection + edge-aware smoothness with and
+without mean_norm_smooth + edge_mean_abs: Monodepth2's whole loss against the same step with the reference's smoothness);
+the last four have default configs cfg2 and cfg5.
 
 For each config the step (forward_backward on device tensors) is captured four times into one CUDA graph and the graph
 is replayed; the two variants alternate, and the median over the repeats is reported per step.  Prints one JSON line
 per config and writes them all, with the card name and its power limit, to the file given as the first argument.
 The last column is the relative overhead for image_grads and the added microseconds for intrinsics_grad (the cost of
 one extra dependent launch, sfm_intrinsics_grad_kernel) and for snippet_terms, the relative overhead for pixel_terms and
-min_reprojection, full_res_multiscale and full_res_min_reprojection.
+min_reprojection, full_res_multiscale and full_res_min_reprojection, and the added microseconds for the last four.
 usage: python tools/time_opt_in_grads.py OUT.json {image_grads,intrinsics_grad,snippet_terms,pixel_terms,min_reprojection,
-       full_res_multiscale,full_res_min_reprojection} [cfg ...]"""
+       full_res_multiscale,full_res_min_reprojection,mean_norm_smooth,mean_norm_smooth_edge,edge_mean_abs,monodepth2}
+       [cfg ...]"""
 import json
 import os
 import subprocess
@@ -37,11 +43,21 @@ LAST_COLUMN = {
     'min_reprojection': ('overhead', lambda p, q: round(q / p - 1.0, 4)),
     'full_res_multiscale': ('overhead', lambda p, q: round(q / p - 1.0, 4)),
     'full_res_min_reprojection': ('overhead', lambda p, q: round(q / p - 1.0, 4)),
+    'mean_norm_smooth': ('extra_us', lambda p, q: round(q - p, 2)),
+    'mean_norm_smooth_edge': ('extra_us', lambda p, q: round(q - p, 2)),
+    'edge_mean_abs': ('extra_us', lambda p, q: round(q - p, 2)),
+    'monodepth2': ('extra_us', lambda p, q: round(q - p, 2)),
 }
+EDGE = dict(edge_aware_smooth=True)
+MONODEPTH2 = dict(full_res_multiscale=True, min_reprojection=True, edge_aware_smooth=True)
 # operator options of the two variants where they are not (nothing, {option: True})
-VARIANTS = {'full_res_min_reprojection': (dict(min_reprojection=True), dict(min_reprojection=True, full_res_multiscale=True))}
+VARIANTS = {'full_res_min_reprojection': (dict(min_reprojection=True), dict(min_reprojection=True, full_res_multiscale=True)),
+            'mean_norm_smooth_edge': (EDGE, dict(EDGE, mean_norm_smooth=True)),
+            'edge_mean_abs': (EDGE, dict(EDGE, edge_mean_abs=True)),
+            'monodepth2': (MONODEPTH2, dict(MONODEPTH2, mean_norm_smooth=True, edge_mean_abs=True))}
 DEFAULT_CONFIGS = {'min_reprojection': ['cfg1', 'cfg2', 'cfg5'], 'full_res_multiscale': ['cfg1', 'cfg2', 'cfg5'],
-                   'full_res_min_reprojection': ['cfg2', 'cfg5']}
+                   'full_res_min_reprojection': ['cfg2', 'cfg5'], 'mean_norm_smooth': ['cfg2', 'cfg5'],
+                   'mean_norm_smooth_edge': ['cfg2', 'cfg5'], 'edge_mean_abs': ['cfg2', 'cfg5'], 'monodepth2': ['cfg2', 'cfg5']}
 
 
 def card():
