@@ -67,6 +67,9 @@ extern "C" {
                                          Changes the loss and sizes the workspace */
 #define SFM_FLAG_EDGE_MEAN_ABS 0x200u /* with SFM_FLAG_EDGE_AWARE_SMOOTH: Monodepth2's edge weight exp(-mean_c |dI_c|) instead
                                          of the reference's exp(-|mean_c dI_c|) (else SFM_E_INVALID_DESC) */
+#define SFM_FLAG_BORDER_PADDING 0x400u /* Monodepth2's image borders: border-clamped sampling without the out-of-view mask
+                                         and reflection-padded SSIM windows; see "Border padding" below.  Changes the
+                                         loss; does not size the workspace */
 
 /*
  * Problem descriptor.  Mirrors the reference's model flags (base_model.py:37-39:
@@ -522,6 +525,28 @@ int sfm_upsample_disparity(int N, int h, int w, int H, int W, const float* x, fl
  * neighbour difference of channel c of the target image, Monodepth2's form, instead of exp(-|((D0 + D1) + D2) / 3|).  The
  * two differ where the channel differences have opposite signs.  The weight depends on the image range: Monodepth2's
  * images are in [0, 1], the reference's in [-1, 1]. */
+
+/* Border padding (SFM_FLAG_BORDER_PADDING; Monodepth2, Godard et al., ICCV 2019: F.grid_sample(..., padding_mode="border")
+ * with the align-corners mapping, and the SSIM module's ReflectionPad2d(1) + AvgPool2d(3, 1)).  The reference zero-pads
+ * and masks pixels that leave the view; Monodepth2 scores them against the clamped border.  With the flag:
+ *   coordinates    the projection chain is unchanged up to xn, yn (the same 1e-10 and individually rounded fp32
+ *                  operations); the x2 rule is skipped.  u = clamp(((xn+1)*(w-1))/2, 0, w-1), v likewise.
+ *   sampling       bilinear with taps u0 = min(floor(u), w-2), weight u - u0 on u0+1, the same for v: every tap is inside
+ *                  the image (at u = w-1 the value is 1 * I[w-1] + 0 * I[w-2]).
+ *   gradient       d u / d xn = (w-1)/2 for 0 < ((xn+1)*(w-1))/2 < w-1 strictly, 0 otherwise (torch's
+ *                  clip_coordinates_set_grad, equality at either end included); v likewise.
+ *   mask           no all-zero mask.  Only a pixel whose projection is degenerate -- |z| outside [2^-58, 2^126], or a
+ *                  non-finite xn or yn -- is masked: value 0, gradient 0, pix_map_masked in the per-pixel maps and no
+ *                  candidate of the minimum reprojection.
+ *   SSIM           the 3x3 windows of the warped image and of the target use reflection padding by one pixel (row /
+ *                  column -1 is 1, h / w is h-2 / w-2), still divided by 9; the backward is the adjoint of that padding.
+ *                  The identity error of sfm_loss_min_reprojection uses the same windows.
+ *   unchanged      means and denominators, the smoothness term (either kind, any normalisation), the loss rows, the
+ *                  intrinsics gradient and the peer sum.
+ * Supported: sfm_loss_forward (without debug dumps), _backward, _forward_backward, _peer, sfm_loss_snippets,
+ * sfm_loss_weighted, sfm_loss_min_reprojection, SFM_FLAG_FULL_RES_MULTISCALE, mean-normalised and edge-aware smoothness,
+ * raw disparity and pose, SFM_FLAG_REUSE_PYRAMID, SFM_FLAG_TABLES_PROVIDED, sfm_intrinsics_grad afterwards and CUDA-graph
+ * capture.  SFM_E_UNSUPPORTED: exp_reg != 0, image gradients, debug dumps and sfm_host_ctx_create. */
 
 #ifdef __cplusplus
 }

@@ -174,6 +174,13 @@ int run_loss(const SfmDesc* d, const SfmInputs* in, float* losses_out, const Sfm
              const SfmMinReprojection* mr = nullptr) {
   int rc = sfm_validate_desc(d);
   if (rc) return rc;
+  // SFM_FLAG_BORDER_PADDING runs the per-pixel instances (weights and maps NULL unless the caller passed them)
+  const bool border = (d->flags & SFM_FLAG_BORDER_PADDING) != 0;
+  if (border && (modes_of(d).use_exp || ig || dbg)) {
+    sfm_set_error("unsupported: SFM_FLAG_BORDER_PADDING together with %s", modes_of(d).use_exp ? "the explainability branch (exp_reg != 0)"
+                  : ig ? "image gradients" : "debug dumps");
+    return SFM_E_UNSUPPORTED;
+  }
   const bool reuse = (d->flags & SFM_FLAG_REUSE_PYRAMID) != 0;
   rc = check_inputs(d, in, true);      // the images are always needed: scale 0 is read from the caller's tensors
   if (rc) return rc;
@@ -205,6 +212,7 @@ int run_loss(const SfmDesc* d, const SfmInputs* in, float* losses_out, const Sfm
   if (ig) mode |= SFM_MODE_IMG;
   if (pix) mode |= SFM_MODE_PIX;
   if (mr) mode |= SFM_MODE_PIX | SFM_MODE_MINREP;
+  if (border) mode |= SFM_MODE_PIX | SFM_MODE_BORDER;
   const SfmStepPlan plan = sfm_plan_step(d, mode, num_sms());
   SfmWsLayout L;
   sfm_ws_layout(d, &L);
@@ -716,6 +724,10 @@ extern "C" int sfm_host_ctx_create(const SfmDesc* desc, SfmHostCtx** ctx_out) {
   }
   if (desc->flags & (SFM_FLAG_MEAN_NORM_SMOOTH | SFM_FLAG_EDGE_MEAN_ABS)) {
     sfm_set_error("unsupported: the host-buffer path with SFM_FLAG_MEAN_NORM_SMOOTH or SFM_FLAG_EDGE_MEAN_ABS");
+    return SFM_E_UNSUPPORTED;
+  }
+  if (desc->flags & SFM_FLAG_BORDER_PADDING) {
+    sfm_set_error("unsupported: the host-buffer path with SFM_FLAG_BORDER_PADDING");
     return SFM_E_UNSUPPORTED;
   }
   int ndev = 0;

@@ -178,13 +178,14 @@ constexpr int SFM_SSIM_REG_MIN_WARPS = 8;
 constexpr int SFM_SSIM_IMG_MIN_WARPS = 10;
 
 // Launch plan of one fused step (plan.cu, the whole launch policy).  The marching kernel instance is
-// sfm_l1_march_kernel<exp, grad, accum, debug, raw, img, snip, pix> or
-// sfm_ssim_march_kernel<grad, accum, debug, raw, nw, srec, img, snip, pix>.
+// sfm_l1_march_kernel<exp, grad, accum, debug, raw, img, snip, pix, border> or
+// sfm_ssim_march_kernel<grad, accum, debug, raw, nw, srec, img, snip, pix, border>.
 struct SfmStepPlan {
   bool ssim;                           // kernel family
   bool exp, grad, accum, debug, raw;   // accum: a smoothness kernel has initialised gdisp
   bool img;                            // image gradients (grad, !debug; SSIM: nw = 1 with shared-memory records)
   bool pix;                            // per-pixel terms (!debug, !img; SSIM: nw = 1 with shared-memory records)
+  bool border;                         // SFM_FLAG_BORDER_PADDING (pix, !exp): border-clamped sampler, reflection-padded SSIM
   bool minrep;                         // minimum reprojection (pix): a forward per-pixel march with the task table pre_tasks
                                        // and the select kernel run ahead of the march of this plan
   SfmTaskTable pre_tasks;
@@ -197,7 +198,7 @@ struct SfmStepPlan {
 };
 // mode bits of the planner
 enum { SFM_MODE_EXP = 1, SFM_MODE_SSIM = 2, SFM_MODE_GRAD = 4, SFM_MODE_DEBUG = 8, SFM_MODE_SMOOTH = 16, SFM_MODE_IMG = 32,
-       SFM_MODE_PIX = 64, SFM_MODE_MINREP = 128 };
+       SFM_MODE_PIX = 64, SFM_MODE_MINREP = 128, SFM_MODE_BORDER = 256 };
 SfmStepPlan sfm_plan_step(const SfmDesc* d, int mode, int num_sms);
 int sfm_plan_band(const SfmDesc* d);
 // Minimum reprojection (sfm_loss_min_reprojection): the planes p.pix_w[s] are written by the forward march and turned

@@ -19,15 +19,22 @@ struct SfmSelectGrid {
   int blk_begin[SFM_MAX_SCALES + 1];
 };
 
-// target pixel (b, y, x) of scale s, three channels; 0 outside the image (the zero padding of the reference's SSIM pool)
+// target pixel (b, y, x) of scale s, three channels; 0 outside the image (the zero padding of the reference's SSIM pool),
+// or with BORDER the pixel reflected at the border (y = -1 reads row 1, y = h row h-2; the callers stay within one pixel)
+template <bool BORDER = false>
 __device__ __forceinline__ V3 sel_tap(const float* __restrict__ img, int plane, int h, int w, int y, int x) {
+  if (BORDER) {
+    y = (y < 0) ? -y : (y >= h) ? 2 * (h - 1) - y : y;
+    x = (x < 0) ? -x : (x >= w) ? 2 * (w - 1) - x : x;
+  }
   if (y < 0 || y >= h || x < 0 || x >= w) return v3s(0.f);
   const float* q = img + y * w + x;
   return v3(__ldg(q), __ldg(q + plane), __ldg(q + 2 * plane));
 }
 
-// SSIM: the identity error includes the clipped SSIM term of the same 3x3 zero-padded windows as the march
-template <bool SSIM>
+// SSIM: the identity error includes the clipped SSIM term of the same 3x3 zero-padded windows as the march.  BORDER
+// (SFM_FLAG_BORDER_PADDING): the windows are reflection-padded, as the march's are.
+template <bool SSIM, bool BORDER = false>
 __global__ void __launch_bounds__(kSelectThreads) sfm_min_reprojection_select_kernel(const __grid_constant__ SfmFusedParams p,
                                                                                      const SfmSelectGrid g, const SfmMinRepArgs a) {
   int s = 0;
@@ -70,7 +77,7 @@ __global__ void __launch_bounds__(kSelectThreads) sfm_min_reprojection_select_ke
 #pragma unroll
       for (int r = 0; r < 3; ++r)
 #pragma unroll
-        for (int c = 0; c < 3; ++c) tq[r][c] = sel_tap(T, plane, h, w, y - 1 + r, x - 1 + c);
+        for (int c = 0; c < 3; ++c) tq[r][c] = sel_tap<BORDER>(T, plane, h, w, y - 1 + r, x - 1 + c);
       // the march's association: row sums (l + c) + r, window sums (row y-1 + row y) + row y+1
       V3 hT[3], hTT[3];
 #pragma unroll
@@ -90,7 +97,7 @@ __global__ void __launch_bounds__(kSelectThreads) sfm_min_reprojection_select_ke
 #pragma unroll
         for (int r = 0; r < 3; ++r)
 #pragma unroll
-          for (int c = 0; c < 3; ++c) pq[r][c] = sel_tap(P, plane, h, w, y - 1 + r, x - 1 + c);
+          for (int c = 0; c < 3; ++c) pq[r][c] = sel_tap<BORDER>(P, plane, h, w, y - 1 + r, x - 1 + c);
       } else {
         pq[1][1] = sel_tap(P, plane, h, w, y, x);
       }

@@ -106,12 +106,20 @@ enum RowStages {
 // stores the map wpix * esum + wssim * sum_c sat(raw_c) = d total / d M of the owned pixels of row r-1, whose esum is
 // carried one step like its weight (p.pix_map_masked for masked pixels).  M = 1 multiplies exactly: unit weights give
 // bitwise the plain step.
+// BORDER (PIX): SFM_FLAG_BORDER_PADDING.  The sampler is pair_project_border, the mask the degenerate projection (r == 0),
+// and the windows use reflection padding by one pixel (Monodepth2's ReflectionPad2d(1) + AvgPool2d(3, 1)): a lane whose
+// column is -1 or w warps column 1 or w-2 (its ray, disparity, target), a step whose row is -1 or h row 1 or h-2.  They
+// own no gradient and centre no window (do_f, c_in stay false); columns -2 / w+1 and rows -2 / h+1 stay dead, as they
+// feed only windows outside the image.  The adjoint of the padding folds the window terms of column 0 / w-1 twice into
+// column 1 / w-2 (stage D: 2 up + self + down, up + self + 2 down) and those of row 0 / h-1 into row 1 / h-2 (stage E),
+// whose product is the 2-D adjoint; both test the image column / row, so a halo or a task boundary anywhere is fine.
 template <bool GRAD, bool ACCUM, bool DEBUG, bool RAW, int NW, bool SREC = true, bool IMG = false, bool SNIP = false,
-          bool PIX = false>
+          bool PIX = false, bool BORDER = false>
 __global__ void __launch_bounds__(32 * NW, (IMG ? SFM_SSIM_IMG_MIN_WARPS : SREC ? SFM_SSIM_MIN_WARPS : SFM_SSIM_REG_MIN_WARPS) / NW)
 sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
   static_assert(!IMG || (GRAD && NW == 1 && SREC), "image gradients: GRAD, one warp per CTA, shared-memory records");
   static_assert(!PIX || (NW == 1 && SREC && !IMG && !DEBUG), "per-pixel terms: one warp per CTA, shared-memory records");
+  static_assert(!BORDER || PIX, "border padding: per-pixel instances");
   constexpr int NREC = IMG ? 21 : PIX ? 19 : 18;        // fields of a forward record
   constexpr int NG = IMG ? 4 : 3;                       // gradient fields: g_a, g_s, g_c (, h_a)
   __shared__ float4 sP_all[NW][3];
@@ -144,6 +152,10 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
   const int xx = t.x0 - 2 + lane;                       // this lane's image column (may be outside)
   const bool col_in = (xx >= 0) && (xx < w);
   const bool col_own = (lane >= 2) && (lane < 2 + SFM_SSIM_IW) && (xx < w);
+  // BORDER: the column this lane warps (reflected at -1 and w; recomputed where used, which keeps the instances with
+  // a pre-activation disparity within 168 registers) and whether it warps one at all
+  auto xs_of = [&]() { return (xx == -1) ? 1 : (xx == w) ? w - 2 : xx; };
+  const bool col_ld = BORDER ? (xx >= -1 && xx <= w) : col_in;
   float gyv = p.gy ? __ldg(p.gy) : 1.f;
   if (SNIP && p.snip_w) gyv *= __ldg(p.snip_w + b);        // per-snippet weight
   const float inv_n3 = p.inv_n3[s];
@@ -156,7 +168,7 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
   cudaTriggerProgrammaticLaunchCompletion();           // lets the epilogue's CTAs become resident while this grid drains (after the
                                                        // wait: the epilogue reads the prologue's smoothness partials ahead of its own wait)
   const float* __restrict__ kinvp = p.kinv + ((size_t)b * p.ns + s) * 9;
-  const float xf = (float)xx;
+  const float xf = (float)(BORDER ? xs_of() : xx);
   const bool raw = RAW && ((p.raw_disp_mask >> s) & 1u);    // RAW: some scale takes the pre-activation disparity map
   const float kk0 = __ldg(kinvp + 0), kk1 = __ldg(kinvp + 1), kk2 = __ldg(kinvp + 2);
   const float kk3 = __ldg(kinvp + 3), kk4 = __ldg(kinvp + 4), kk5 = __ldg(kinvp + 5);
@@ -205,7 +217,17 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
     auto load_dT = [&](int r, float& dd, float* TT) {
       dd = 1.f;
       TT[0] = TT[1] = TT[2] = 0.f;
-      if (col_in && (r >= 0) && (r < h) && (r < r_end)) {
+      if constexpr (BORDER) {
+        if (col_ld && (r >= -1) && (r <= h) && (r < r_end)) {
+          const int rs = (r == -1) ? 1 : (r == h) ? h - 2 : r;
+          const unsigned o = (unsigned)(rs * w + xs_of());
+          const float* tb = pp->tgt;
+          dd = __ldg(pp->disp + o);
+          TT[0] = __ldg(tb + o);
+          TT[1] = __ldg(tb + (o + geo.plane));
+          TT[2] = __ldg(tb + (o + 2u * geo.plane));
+        }
+      } else if (col_in && (r >= 0) && (r < h) && (r < r_end)) {
         const unsigned o = (unsigned)(r * w + xx);
         const float* tb = pp->tgt;
         dd = __ldg(pp->disp + o);
@@ -230,12 +252,14 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
     // row r+1's disparity / target (unless LOAD_NEXT is false) and the partial gdisp of the row whose backward runs next
     auto refill = [&](auto SLOT, Pend& pn, const int r, auto LOAD_NEXT) {
       constexpr int sl = decltype(SLOT)::value, nx = (sl + 1) % 3;
-      const bool in_img = col_in && (r >= 0) && (r < h) && (r < r_end);
+      int rs = r;                                        // BORDER: the row warped
+      if constexpr (BORDER) rs = (r == -1) ? 1 : (r == h) ? h - 2 : r;
+      const bool in_img = BORDER ? col_ld && (r >= -1) && (r <= h) && (r < r_end) : col_in && (r >= 0) && (r < h) && (r < r_end);
       float d = dq[sl], dact = 1.f;
       if (raw) d = sfm_disp_act(d, dact);      // producer-side fusion: pre-activation disparity map (warp-uniform branch)
       pn.depth = rcp_newton(d);
       if (RAW) pn.dsc = raw ? pn.depth * dact : pn.depth;
-      const float yf = (float)r;
+      const float yf = (float)(BORDER ? rs : r);
       const float rx = __fadd_rn(__fadd_rn(rxx, __fmul_rn(kk1, yf)), kk2);
       const float ry = __fadd_rn(__fadd_rn(ryx, __fmul_rn(kk4, yf)), kk5);
       const float rz = __fadd_rn(__fadd_rn(rzx, __fmul_rn(kk7, yf)), kk8);
@@ -248,15 +272,18 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
         P[8] = c.x; P[9] = c.y; P[10] = c.z; P[11] = c.w;
       }
       PairFwd f;
-      pair_project(P, X, Y, Z, geo, f, in_img);
+      [[maybe_unused]] unsigned du = 1u, dvw = 0u;
+      if constexpr (BORDER) pair_project_border(P, X, Y, Z, geo, f, du, dvw, in_img);
+      else pair_project(P, X, Y, Z, geo, f, in_img);
       pn.wa = f.wa; pn.wb = f.wb; pn.wc = f.wc; pn.wd = f.wd;
       pn.q0 = f.q0; pn.q1 = f.q1; pn.q2 = f.q2; pn.r = f.r;
       if (IMG) pn.idx = f.idx;
-      gather_taps(pp->img, geo, f, pn.I);
+      if constexpr (BORDER) gather_taps_border(pp->img, geo, f, du, dvw, pn.I);
+      else gather_taps(pp->img, geo, f, pn.I);
       if (PIX) {
         float* const volatile* pq = s_pix_ptrs;
         const float* wq = pq[0];
-        pn.mw = (in_img && wq) ? __ldg(wq + (unsigned)(r * w + xx)) : 1.f;
+        pn.mw = (in_img && wq) ? __ldg(wq + (BORDER ? (unsigned)(rs * w + xs_of()) : (unsigned)(r * w + xx))) : 1.f;
       }
       if (decltype(LOAD_NEXT)::value) load_dT(r + 1, dq[nx], Tq[nx]);
       if (GRAD && (ACCUM || !first) && writer) {
@@ -293,7 +320,8 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
         const float P0 = sfm_blend(w1, w2, w3, w4, I.a[0], I.b[0], I.c[0], I.d[0]);
         const float P1 = sfm_blend(w1, w2, w3, w4, I.a[1], I.b[1], I.c[1], I.d[1]);
         const float P2 = sfm_blend(w1, w2, w3, w4, I.a[2], I.b[2], I.c[2], I.d[2]);
-        const bool m = (P0 == 0.f) && (P1 == 0.f) && (P2 == 0.f);               // true outside the image / view
+        const bool m = BORDER ? (pa.r == 0.f)                                     // degenerate or dead
+                              : (P0 == 0.f) && (P1 == 0.f) && (P2 == 0.f);         // true outside the image / view
         const bool own = col_own && (r >= t.y0) && (r < t.y1);
         if (PIX) {
           e_cur = m ? 0.f : (fabsf(P0 - T[0]) + fabsf(P1 - T[1]) + fabsf(P2 - T[2]));
@@ -410,7 +438,12 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
         // ---------------- stage D: row sums of the three gradient fields of row rc
         V3* gh0 = gs[cur];
 #pragma unroll
-        for (int q = 0; q < NG; ++q) gh0[q] = (vshfl_up(g0[q]) + g0[q]) + vshfl_down(g0[q]);
+        for (int q = 0; q < NG; ++q) {
+          // BORDER: the adjoint of the column reflection (column 1 / w-2 also holds the windows of column 0 / w-1)
+          if constexpr (BORDER)
+            gh0[q] = vfma(v3s(xx == w - 2 ? 2.f : 1.f), vshfl_down(g0[q]), vfma(v3s(xx == 1 ? 2.f : 1.f), vshfl_up(g0[q]), g0[q]));
+          else gh0[q] = (vshfl_up(g0[q]) + g0[q]) + vshfl_down(g0[q]);
+        }
         if constexpr (stages != ROW_ABCD) {
         // ---------------- stages E + F: dL/dP and the warp backward for pixel (rf = r-2, lane)
         const V3* g1 = gs[pv1];
@@ -432,9 +465,19 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
         const float wpf = PIX ? wpix * (SREC ? myrec[pv2 * NREC * 32 + 18 * 32] : 1.f) : wpix;   // PIX: weight of row rf
         float gP[3], gT[3];
         {
-          const V3 Aa = (g2[0] + g1[0]) + gh0[0];
-          const V3 As = (g2[1] + g1[1]) + gh0[1];
-          const V3 Ac = (g2[2] + g1[2]) + gh0[2];
+          V3 Aa, As, Ac;
+          if constexpr (BORDER) {
+            // the adjoint of the row reflection: row 1 also holds the windows of row 0 as row -1, row h-2 those of
+            // row h-1 as row h
+            const V3 f2 = v3s(rf == 1 ? 2.f : 1.f), f0 = v3s(rf == h - 2 ? 2.f : 1.f);
+            Aa = vfma(f0, gh0[0], vfma(f2, g2[0], g1[0]));
+            As = vfma(f0, gh0[1], vfma(f2, g2[1], g1[1]));
+            Ac = vfma(f0, gh0[2], vfma(f2, g2[2], g1[2]));
+          } else {
+            Aa = (g2[0] + g1[0]) + gh0[0];
+            As = (g2[1] + g1[1]) + gh0[1];
+            Ac = (g2[2] + g1[2]) + gh0[2];
+          }
           // dL/dP = sum over the 3x3 windows containing the pixel of dL/dSp + 2P dL/dSpp + T dL/dSpt
           //       = 2 Aa + 18 P As + 18 T Ac
           const V3 Pb = v3(rb.P[0], rb.P[1], rb.P[2]), Tb = v3(rb.T[0], rb.T[1], rb.T[2]);

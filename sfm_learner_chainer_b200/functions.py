@@ -59,14 +59,24 @@ class ViewSynthesisLoss(object):
     disparity; see SFM_FLAG_MEAN_NORM_SMOOTH in include/sfmloss.h.  The photometric terms are untouched.
     edge_mean_abs: with edge_aware_smooth, Monodepth2's edge weight exp(-mean_c |dI_c|) instead of the reference's
     exp(-|mean_c dI_c|).
+    border_padding: Monodepth2's image borders: the warp samples with border clamping (grid_sample's
+    padding_mode="border", align-corners mapping, no x2 rule) and masks only pixels whose projection is degenerate, and
+    the SSIM windows use reflection padding by one pixel; see SFM_FLAG_BORDER_PADDING in include/sfmloss.h.  Not with
+    exp_reg, image_grads or debug dumps.
     """
 
     def __init__(self, smooth_reg=0.0, exp_reg=0.0, ssim_rate=0.0, n_scales=N_SCALES, B_global=None,
                  raw_disp_scales=0, raw_pose=False, edge_aware_smooth=False, image_grads=False,
                  intrinsics_grad=False, snippet_terms=False, pixel_terms=False, min_reprojection=False, automask=True,
-                 full_res_multiscale=False, mean_norm_smooth=False, edge_mean_abs=False):
+                 full_res_multiscale=False, mean_norm_smooth=False, edge_mean_abs=False, border_padding=False):
         if edge_mean_abs and not edge_aware_smooth:
             raise ValueError('edge_mean_abs needs edge_aware_smooth')
+        if border_padding:
+            if image_grads:
+                raise ValueError('border_padding is not supported together with image_grads')
+            if float(exp_reg or 0.0) != 0.0:
+                raise ValueError('border_padding is not supported together with the explainability branch (exp_reg)')
+        self.border_padding = bool(border_padding)
         self.mean_norm_smooth = bool(mean_norm_smooth)
         self.edge_mean_abs = bool(edge_mean_abs)
         if full_res_multiscale:
@@ -126,6 +136,8 @@ class ViewSynthesisLoss(object):
             flags |= L.SFM_FLAG_MEAN_NORM_SMOOTH
         if self.edge_mean_abs:
             flags |= L.SFM_FLAG_EDGE_MEAN_ABS
+        if self.border_padding:
+            flags |= L.SFM_FLAG_BORDER_PADDING
         return L.SfmDesc(B, S, H, W, self.n_scales, int(self.B_global or 0), self.smooth_reg, self.exp_reg,
                          self.ssim_rate, flags, self.raw_disp_scales, raw_pose_hw)
 
@@ -277,8 +289,9 @@ class ViewSynthesisLoss(object):
         With the operator's pixel_terms the per-pixel loss maps (list of n_scales (B,S,h,w)) are appended as the last
         element: (losses, maps) or (losses, snippet losses, maps).
         With the operator's min_reprojection the selection maps (list of n_scales (B,h,w) int8) are appended likewise."""
-        if debug and (self.snippet_terms or self.pixel_terms or self.min_reprojection):
-            raise ValueError('debug dumps are not available on an operator with snippet_terms, pixel_terms or min_reprojection')
+        if debug and (self.snippet_terms or self.pixel_terms or self.min_reprojection or self.border_padding):
+            raise ValueError('debug dumps are not available on an operator with snippet_terms, pixel_terms, min_reprojection '
+                             'or border_padding')
         desc, inp = self._pack(tgt, src, intrinsics, disps, poses, logits, proj, kinv)
         losses = D.empty(tgt, (5,))
         if self.min_reprojection:

@@ -18,6 +18,7 @@ SFM_FLAG_MIN_REPROJECTION = 0x40
 SFM_FLAG_FULL_RES_MULTISCALE = 0x80
 SFM_FLAG_MEAN_NORM_SMOOTH = 0x100
 SFM_FLAG_EDGE_MEAN_ABS = 0x200
+SFM_FLAG_BORDER_PADDING = 0x400
 
 SFM_E_INVALID_DESC = -1
 SFM_E_INVALID_SHAPE = -2

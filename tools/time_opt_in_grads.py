@@ -10,16 +10,20 @@ mean_norm_smooth (ViewSynthesisLoss(mean_norm_smooth=True), Monodepth2's mean-no
 mean_norm_smooth_edge (the same with edge-aware smoothness on both sides), edge_mean_abs (edge-aware smoothness with and
 without Monodepth2's edge weight) or monodepth2 (full_res_multiscale + min_reprojection + edge-aware smoothness with and
 without mean_norm_smooth + edge_mean_abs: Monodepth2's whole loss against the same step with the reference's smoothness);
-the last four have default configs cfg2 and cfg5.
+the last four have default configs cfg2 and cfg5.  border_padding (ViewSynthesisLoss(border_padding=True), Monodepth2's
+image borders) and monodepth2_border (Monodepth2's whole loss, as the second variant of monodepth2, with and without
+border_padding) have default configs cfg2 and cfg5 too.
 
 For each config the step (forward_backward on device tensors) is captured four times into one CUDA graph and the graph
 is replayed; the two variants alternate, and the median over the repeats is reported per step.  Prints one JSON line
 per config and writes them all, with the card name and its power limit, to the file given as the first argument.
 The last column is the relative overhead for image_grads and the added microseconds for intrinsics_grad (the cost of
 one extra dependent launch, sfm_intrinsics_grad_kernel) and for snippet_terms, the relative overhead for pixel_terms and
-min_reprojection, full_res_multiscale and full_res_min_reprojection, and the added microseconds for the last four.
+min_reprojection, full_res_multiscale and full_res_min_reprojection, the added microseconds for the next four and the
+relative overhead for border_padding and monodepth2_border.
 usage: python tools/time_opt_in_grads.py OUT.json {image_grads,intrinsics_grad,snippet_terms,pixel_terms,min_reprojection,
-       full_res_multiscale,full_res_min_reprojection,mean_norm_smooth,mean_norm_smooth_edge,edge_mean_abs,monodepth2}
+       full_res_multiscale,full_res_min_reprojection,mean_norm_smooth,mean_norm_smooth_edge,edge_mean_abs,monodepth2,
+       border_padding,monodepth2_border}
        [cfg ...]"""
 import json
 import os
@@ -47,17 +51,22 @@ LAST_COLUMN = {
     'mean_norm_smooth_edge': ('extra_us', lambda p, q: round(q - p, 2)),
     'edge_mean_abs': ('extra_us', lambda p, q: round(q - p, 2)),
     'monodepth2': ('extra_us', lambda p, q: round(q - p, 2)),
+    'border_padding': ('overhead', lambda p, q: round(q / p - 1.0, 4)),
+    'monodepth2_border': ('overhead', lambda p, q: round(q / p - 1.0, 4)),
 }
 EDGE = dict(edge_aware_smooth=True)
 MONODEPTH2 = dict(full_res_multiscale=True, min_reprojection=True, edge_aware_smooth=True)
+MONODEPTH2_SMOOTH = dict(MONODEPTH2, mean_norm_smooth=True, edge_mean_abs=True)
 # operator options of the two variants where they are not (nothing, {option: True})
 VARIANTS = {'full_res_min_reprojection': (dict(min_reprojection=True), dict(min_reprojection=True, full_res_multiscale=True)),
             'mean_norm_smooth_edge': (EDGE, dict(EDGE, mean_norm_smooth=True)),
             'edge_mean_abs': (EDGE, dict(EDGE, edge_mean_abs=True)),
-            'monodepth2': (MONODEPTH2, dict(MONODEPTH2, mean_norm_smooth=True, edge_mean_abs=True))}
+            'monodepth2': (MONODEPTH2, MONODEPTH2_SMOOTH),
+            'monodepth2_border': (MONODEPTH2_SMOOTH, dict(MONODEPTH2_SMOOTH, border_padding=True))}
 DEFAULT_CONFIGS = {'min_reprojection': ['cfg1', 'cfg2', 'cfg5'], 'full_res_multiscale': ['cfg1', 'cfg2', 'cfg5'],
                    'full_res_min_reprojection': ['cfg2', 'cfg5'], 'mean_norm_smooth': ['cfg2', 'cfg5'],
-                   'mean_norm_smooth_edge': ['cfg2', 'cfg5'], 'edge_mean_abs': ['cfg2', 'cfg5'], 'monodepth2': ['cfg2', 'cfg5']}
+                   'mean_norm_smooth_edge': ['cfg2', 'cfg5'], 'edge_mean_abs': ['cfg2', 'cfg5'], 'monodepth2': ['cfg2', 'cfg5'],
+                   'border_padding': ['cfg2', 'cfg5'], 'monodepth2_border': ['cfg2', 'cfg5']}
 
 
 def card():
