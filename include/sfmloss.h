@@ -70,6 +70,13 @@ extern "C" {
 #define SFM_FLAG_BORDER_PADDING 0x400u /* Monodepth2's image borders: border-clamped sampling without the out-of-view mask
                                          and reflection-padded SSIM windows; see "Border padding" below.  Changes the
                                          loss; does not size the workspace */
+#define SFM_FLAG_AXISANGLE_POSE 0x800u /* Monodepth2's pose: `poses` rows are (v0, v1, v2, tx, ty, tz), an axis-angle
+                                         vector and a translation, instead of the Euler vector; see "Axis-angle pose"
+                                         below.  Does not size the workspace */
+#define SFM_FLAG_POSE_INVERT_SHIFT 16   /* flags bits 16..23: with SFM_FLAG_AXISANGLE_POSE, bit 16 + i inverts the
+                                         transform of source i (Monodepth2's frame ids < 0) */
+#define SFM_FLAG_POSE_INVERT(i) (1u << (SFM_FLAG_POSE_INVERT_SHIFT + (i)))
+#define SFM_FLAG_POSE_INVERT_MASK (0xffu << SFM_FLAG_POSE_INVERT_SHIFT)
 
 /*
  * Problem descriptor.  Mirrors the reference's model flags (base_model.py:37-39:
@@ -547,6 +554,26 @@ int sfm_upsample_disparity(int N, int h, int w, int H, int W, const float* x, fl
  * sfm_loss_weighted, sfm_loss_min_reprojection, SFM_FLAG_FULL_RES_MULTISCALE, mean-normalised and edge-aware smoothness,
  * raw disparity and pose, SFM_FLAG_REUSE_PYRAMID, SFM_FLAG_TABLES_PROVIDED, sfm_intrinsics_grad afterwards and CUDA-graph
  * capture.  SFM_E_UNSUPPORTED: exp_reg != 0, image gradients, debug dumps and sfm_host_ctx_create. */
+
+/* Axis-angle pose (SFM_FLAG_AXISANGLE_POSE; Monodepth2, Godard et al., ICCV 2019: layers.py rot_from_axisangle,
+ * get_translation_matrix and transformation_from_parameters, followed literally).  Monodepth2's PoseDecoder emits
+ * 0.01 * mean over its output map, which is what raw_pose_hw applies, so its raw `poseout` map composes unchanged.
+ * For a pose row (v, t):
+ *   rotation       theta = |v|_2, a = v / (theta + 1e-7), c = cos theta, s = sin theta, C = 1 - c,
+ *                  R = C a a^T + s [a]_x + c I, entry by entry as rot_from_axisangle; no angle clipping.  For theta below
+ *                  ~1e-7 R is not exactly orthonormal, as in Monodepth2.
+ *   transform      T = [R | t], or with bit 16 + i of flags (SFM_FLAG_POSE_INVERT(i)) for source i, T = [R^T | -R^T t]
+ *                  (Monodepth2 runs the pose network on the swapped pair for a source that precedes the target and
+ *                  inverts the result: frame ids [0, -1, 1] with sources [-1, +1] give the mask 0b01).
+ *   evaluation     theta, a, sin / cos, R and -R^T t in fp64, each operation individually rounded; R and t rounded to
+ *                  fp32 once; P_s = K4_s . T as for the Euler pose (the same fp32 order and non-finite guard).
+ *   gradient       gposes is the derivative of this formula in fp64, with torch's convention d theta / d v = 0 at
+ *                  theta = 0.  With SFM_FLAG_TABLES_PROVIDED gposes goes through this chain, as it goes through the
+ *                  Euler chain without the flag.  sfm_intrinsics_grad uses the R and t of the transform (fp32-rounded,
+ *                  inverted where the mask says so).
+ * An invert bit without SFM_FLAG_AXISANGLE_POSE, or for a source >= S, is SFM_E_INVALID_DESC.  The flag works with every
+ * fused entry point, sfm_build_tables, sfm_intrinsics_grad, raw pose maps and CUDA-graph capture; sfm_host_ctx_create
+ * returns SFM_E_UNSUPPORTED.  The stage warp (sfm_warp_forward / sfm_warp_backward) has no descriptor and stays Euler. */
 
 #ifdef __cplusplus
 }

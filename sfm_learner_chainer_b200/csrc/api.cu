@@ -68,6 +68,15 @@ int sfm_validate_desc(const SfmDesc* d) {
     sfm_set_error("invalid SfmDesc: SFM_FLAG_EDGE_MEAN_ABS needs SFM_FLAG_EDGE_AWARE_SMOOTH");
     return SFM_E_INVALID_DESC;
   }
+  const unsigned inv = (d->flags & SFM_FLAG_POSE_INVERT_MASK) >> SFM_FLAG_POSE_INVERT_SHIFT;
+  if (inv && !(d->flags & SFM_FLAG_AXISANGLE_POSE)) {
+    sfm_set_error("invalid SfmDesc: pose inversion bits 0x%x need SFM_FLAG_AXISANGLE_POSE", inv);
+    return SFM_E_INVALID_DESC;
+  }
+  if (inv >> d->S) {
+    sfm_set_error("invalid SfmDesc: pose inversion bits 0x%x name a source >= S=%d", inv, d->S);
+    return SFM_E_INVALID_DESC;
+  }
   if (!(d->smooth_reg == d->smooth_reg) || !(d->exp_reg == d->exp_reg) || !(d->ssim_rate == d->ssim_rate)) {
     sfm_set_error("invalid SfmDesc: NaN loss weight");
     return SFM_E_INVALID_DESC;
@@ -266,6 +275,7 @@ int run_loss(const SfmDesc* d, const SfmInputs* in, float* losses_out, const Sfm
   p.intrinsics = fr ? (const float*)(ws + L.off_k0) : in->intrinsics;
   p.poses = d->raw_pose_hw > 0 ? (const float*)(ws + L.off_posevec) : in->poses;
   p.raw_pose_hw = d->raw_pose_hw;
+  p.pose_flags = d->flags & (SFM_FLAG_AXISANGLE_POSE | SFM_FLAG_POSE_INVERT_MASK);
   p.raw_disp_mask = d->raw_disp_scales;
   p.gy = gy;
   p.acc = (double*)(ws + L.off_acc);
@@ -379,7 +389,7 @@ int run_loss(const SfmDesc* d, const SfmInputs* in, float* losses_out, const Sfm
     if (L.gsrc_bytes) SFM_CUDA_CHECK(cudaMemsetAsync(ws + L.off_gsrc[1], 0, L.gsrc_bytes, st));
   }
   if (fr && (rc = sfm_launch_full_res_upsample(f, st))) return rc;
-  rc = sfm_launch_prep(pp, &sm, (grads ? 2 : 1) + ((snip || mean_norm) ? 2 : 0), st);
+  rc = sfm_launch_prep(pp, &sm, (grads ? 2 : 1) + ((snip || mean_norm) ? 2 : 0), st, p.pose_flags);
   if (rc) return rc;
   SfmMinRepArgs a{};
   if (mr) {
@@ -562,7 +572,9 @@ extern "C" int sfm_intrinsics_grad(const SfmDesc* desc, const SfmInputs* in, con
   // the per-scale gradients are folded into [:, 0]
   const bool fr = sfm_full_res(desc);
   rc = sfm_launch_intrinsics_grad(desc->B, desc->S, desc->n_scales, (const double*)(ws + L.off_acc) + 4, poses,
-                                  fr ? (const float*)(ws + L.off_k0) : in->intrinsics, gintrinsics, (cudaStream_t)stream);
+                                  fr ? (const float*)(ws + L.off_k0) : in->intrinsics, (desc->flags & SFM_FLAG_AXISANGLE_POSE) ? 1 : 0,
+                                  (desc->flags & SFM_FLAG_POSE_INVERT_MASK) >> SFM_FLAG_POSE_INVERT_SHIFT, gintrinsics,
+                                  (cudaStream_t)stream);
   if (rc || !fr) return rc;
   return sfm_launch_intrinsics_fold(desc->B, desc->n_scales, gintrinsics, (cudaStream_t)stream);
 }
@@ -628,7 +640,7 @@ extern "C" int sfm_build_tables(const SfmDesc* desc, const float* poses, const f
   if (rc) return rc;
   if (!poses || !intrinsics || !proj_out || !kinv_out) { sfm_set_error("sfm_build_tables: null pointer"); return SFM_E_NULL_POINTER; }
   const SfmPrepParams p = prep_params(desc, sfm_plan_band(desc), nullptr, nullptr, nullptr, intrinsics, poses, proj_out, kinv_out, false);
-  return sfm_launch_prep(p, nullptr, 0, (cudaStream_t)stream);
+  return sfm_launch_prep(p, nullptr, 0, (cudaStream_t)stream, desc->flags & (SFM_FLAG_AXISANGLE_POSE | SFM_FLAG_POSE_INVERT_MASK));
 }
 
 extern "C" int sfm_ingest_u8(int B, int S, int H, int W, int n_scales, const uint8_t* frames, const float* K_in,
@@ -728,6 +740,10 @@ extern "C" int sfm_host_ctx_create(const SfmDesc* desc, SfmHostCtx** ctx_out) {
   }
   if (desc->flags & SFM_FLAG_BORDER_PADDING) {
     sfm_set_error("unsupported: the host-buffer path with SFM_FLAG_BORDER_PADDING");
+    return SFM_E_UNSUPPORTED;
+  }
+  if (desc->flags & SFM_FLAG_AXISANGLE_POSE) {
+    sfm_set_error("unsupported: the host-buffer path with SFM_FLAG_AXISANGLE_POSE");
     return SFM_E_UNSUPPORTED;
   }
   int ndev = 0;

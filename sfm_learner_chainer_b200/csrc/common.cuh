@@ -226,6 +226,21 @@ __device__ __forceinline__ void sfm_rot_mats(const float* c, const float* s, flo
   X[0] = 1.f; X[1] = 0.f; X[2] = 0.f; X[3] = 0.f; X[4] = c[0]; X[5] = -s[0]; X[6] = 0.f; X[7] = s[0]; X[8] = c[0];
 }
 
+// proj (3x4) = K . [R | t], canonical order, no FMA (transform.py:86-88)
+__device__ __forceinline__ void sfm_proj_from_rt(const float* K, const float* R, const float* t, float* P) {
+#pragma unroll
+  for (int r = 0; r < 3; ++r) {
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      float t0 = (j < 3) ? R[0 * 3 + j] : t[0];
+      float t1 = (j < 3) ? R[1 * 3 + j] : t[1];
+      float t2 = (j < 3) ? R[2 * 3 + j] : t[2];
+      P[r * 4 + j] =
+          __fadd_rn(__fadd_rn(__fmul_rn(K[r * 3 + 0], t0), __fmul_rn(K[r * 3 + 1], t1)), __fmul_rn(K[r * 3 + 2], t2));
+    }
+  }
+}
+
 // proj (3x4) = K . [R | t]   with R = (Rx.Ry).Rz    (transform.py:27-39, 52-58, 86-88)
 __device__ __forceinline__ void sfm_build_proj(const float* pose, const float* K, float* P) {
   float c[3], s[3], X[9], Y[9], Z[9], XY[9], R[9];
@@ -233,16 +248,97 @@ __device__ __forceinline__ void sfm_build_proj(const float* pose, const float* K
   sfm_rot_mats(c, s, X, Y, Z);
   sfm_mm3(X, Y, XY);
   sfm_mm3(XY, Z, R);
+  sfm_proj_from_rt(K, R, pose + 3, P);
+}
+
+// ---- Monodepth2's axis-angle pose (SFM_FLAG_AXISANGLE_POSE; layers.py rot_from_axisangle, get_translation_matrix,
+// transformation_from_parameters).  The prologue's tables, the epilogue's pose chain and the intrinsics gradient share
+// these functions, so all three see the same transform.  The forward runs in fp64 with every operation individually
+// rounded (no contraction), in the order tests/axisangle_oracle.py repeats.
+struct SfmAxisAngle {
+  double th, c, s;   // theta = |v|, cos theta, sin theta
+  double a[3];       // v / (theta + 1e-7)
+  double R[9];       // rot_from_axisangle(v), row major, before any inversion
+};
+
+__device__ __forceinline__ void sfm_axisangle_rot(const float* pose, SfmAxisAngle& q) {
+  const double v0 = pose[0], v1 = pose[1], v2 = pose[2];
+  q.th = __dsqrt_rn(__dadd_rn(__dadd_rn(__dmul_rn(v0, v0), __dmul_rn(v1, v1)), __dmul_rn(v2, v2)));
+  const double den = __dadd_rn(q.th, 1e-7);
+  const double x = __ddiv_rn(v0, den), y = __ddiv_rn(v1, den), z = __ddiv_rn(v2, den);
+  q.a[0] = x; q.a[1] = y; q.a[2] = z;
+  sincos(q.th, &q.s, &q.c);
+  const double C = __dsub_rn(1.0, q.c);
+  const double xs = __dmul_rn(x, q.s), ys = __dmul_rn(y, q.s), zs = __dmul_rn(z, q.s);
+  const double xC = __dmul_rn(x, C), yC = __dmul_rn(y, C), zC = __dmul_rn(z, C);
+  const double xyC = __dmul_rn(x, yC), yzC = __dmul_rn(y, zC), zxC = __dmul_rn(z, xC);
+  q.R[0] = __dadd_rn(__dmul_rn(x, xC), q.c); q.R[1] = __dsub_rn(xyC, zs); q.R[2] = __dadd_rn(zxC, ys);
+  q.R[3] = __dadd_rn(xyC, zs); q.R[4] = __dadd_rn(__dmul_rn(y, yC), q.c); q.R[5] = __dsub_rn(yzC, xs);
+  q.R[6] = __dsub_rn(zxC, ys); q.R[7] = __dadd_rn(yzC, xs); q.R[8] = __dadd_rn(__dmul_rn(z, zC), q.c);
+}
+
+// the transform's rotation and translation rounded to fp32: [R | t], or inverted [R^T | -R^T t] with
+// (R^T t)_j = ((R_0j t_0 + R_1j t_1) + R_2j t_2) from the fp64 R
+__device__ __forceinline__ void sfm_axisangle_transform(const SfmAxisAngle& q, const float* t, bool inv, float* Rt, float* tt) {
+#pragma unroll
+  for (int u = 0; u < 3; ++u)
+#pragma unroll
+    for (int v = 0; v < 3; ++v) Rt[u * 3 + v] = (float)(inv ? q.R[v * 3 + u] : q.R[u * 3 + v]);
+#pragma unroll
+  for (int j = 0; j < 3; ++j) {
+    const double m = __dadd_rn(__dadd_rn(__dmul_rn(q.R[0 * 3 + j], (double)t[0]), __dmul_rn(q.R[1 * 3 + j], (double)t[1])),
+                               __dmul_rn(q.R[2 * 3 + j], (double)t[2]));
+    tt[j] = inv ? (float)(-m) : t[j];
+  }
+}
+
+// proj (3x4) = K . T of the axis-angle pose (6 floats)
+__device__ __forceinline__ void sfm_build_proj_axisangle(const float* pose, bool inv, const float* K, float* P) {
+  SfmAxisAngle q;
+  sfm_axisangle_rot(pose, q);
+  float R[9], t[3];
+  sfm_axisangle_transform(q, pose + 3, inv, R, t);
+  sfm_proj_from_rt(K, R, t, P);
+}
+
+// dL/dpose (6) from dL/dT (3x4, fp64) of the axis-angle transform, in fp64 from the quantities of sfm_axisangle_rot.
+// G_R = dL/dR: G3 (not inverted) or G3^T - t g^T (inverted), dL/dt = g or -R g, with [G3 | g] = dT.  Then
+//   dL/da   = C (G_R + G_R^T) a + s (G_R[2,1] - G_R[1,2], G_R[0,2] - G_R[2,0], G_R[1,0] - G_R[0,1])
+//   dL/dth  = sum G_R o (s a a^T + c [a]_x - s I)
+//   dL/dv   = dL/da / (th + 1e-7) + (dL/dth - (dL/da . v) / (th + 1e-7)^2) v / th      (last term 0 at th = 0)
+__device__ __forceinline__ void sfm_axisangle_backward(const SfmAxisAngle& q, const float* pose, bool inv, const double* dT,
+                                                       float* gpose) {
+  double G[9], gt[3];
+  const double t[3] = {pose[3], pose[4], pose[5]};
 #pragma unroll
   for (int r = 0; r < 3; ++r) {
 #pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      float t0 = (j < 3) ? R[0 * 3 + j] : pose[3];
-      float t1 = (j < 3) ? R[1 * 3 + j] : pose[4];
-      float t2 = (j < 3) ? R[2 * 3 + j] : pose[5];
-      P[r * 4 + j] =
-          __fadd_rn(__fadd_rn(__fmul_rn(K[r * 3 + 0], t0), __fmul_rn(K[r * 3 + 1], t1)), __fmul_rn(K[r * 3 + 2], t2));
-    }
+    for (int c = 0; c < 3; ++c) G[r * 3 + c] = inv ? dT[c * 4 + r] - t[r] * dT[c * 4 + 3] : dT[r * 4 + c];
+    gt[r] = inv ? -(q.R[r * 3 + 0] * dT[3] + q.R[r * 3 + 1] * dT[7] + q.R[r * 3 + 2] * dT[11]) : dT[r * 4 + 3];
+  }
+  const double* a = q.a;
+  const double C = 1.0 - q.c;
+  double ga[3];
+#pragma unroll
+  for (int k = 0; k < 3; ++k)
+    ga[k] = C * ((G[k * 3 + 0] + G[0 * 3 + k]) * a[0] + (G[k * 3 + 1] + G[1 * 3 + k]) * a[1] + (G[k * 3 + 2] + G[2 * 3 + k]) * a[2]);
+  ga[0] += q.s * (G[7] - G[5]);
+  ga[1] += q.s * (G[2] - G[6]);
+  ga[2] += q.s * (G[3] - G[1]);
+  // [a]_x = [[0, -a2, a1], [a2, 0, -a0], [-a1, a0, 0]]
+  double gth = q.c * (a[1] * (G[2] - G[6]) + a[2] * (G[3] - G[1]) + a[0] * (G[7] - G[5])) - q.s * (G[0] + G[4] + G[8]);
+#pragma unroll
+  for (int u = 0; u < 3; ++u)
+#pragma unroll
+    for (int v = 0; v < 3; ++v) gth += q.s * G[u * 3 + v] * a[u] * a[v];
+  const double v[3] = {pose[0], pose[1], pose[2]};
+  const double den = q.th + 1e-7;
+  const double gav = ga[0] * v[0] + ga[1] * v[1] + ga[2] * v[2];
+  const double k = q.th > 0.0 ? (gth - gav / (den * den)) / q.th : 0.0;
+#pragma unroll
+  for (int j = 0; j < 3; ++j) {
+    gpose[j] = (float)(ga[j] / den + k * v[j]);
+    gpose[3 + j] = (float)gt[j];
   }
 }
 

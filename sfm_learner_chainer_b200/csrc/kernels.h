@@ -46,8 +46,10 @@ struct SfmSmoothParams {
   float* task_part;
 };
 
-// sm_mode: 0 = no smoothness tasks, 1 = loss only, 2 = loss + gdisp; 3 / 4 = 1 / 2 with per-task losses (task_part)
-int sfm_launch_prep(const SfmPrepParams& p, const SfmSmoothParams* sm, int sm_mode, cudaStream_t stream);
+// sm_mode: 0 = no smoothness tasks, 1 = loss only, 2 = loss + gdisp; 3 / 4 = 1 / 2 with per-task losses (task_part).
+// pose_flags: desc->flags & (SFM_FLAG_AXISANGLE_POSE | SFM_FLAG_POSE_INVERT_MASK); with the first bit the tables are
+// built from Monodepth2's axis-angle pose by instances of their own, so that the Euler instances keep the parent's code
+int sfm_launch_prep(const SfmPrepParams& p, const SfmSmoothParams* sm, int sm_mode, cudaStream_t stream, unsigned pose_flags = 0);
 int sfm_launch_ingest_u8(int B, int S, int H, int W, int ns, const uint8_t* frames, const float* K_in, const SfmAugment* aug,
                          float* tgt, float* src, float* K_out, cudaStream_t stream);   // ingest.cu
 size_t sfm_eval_scratch_bytes_impl(int B, int Hg, int Wg);                                  // eval.cu
@@ -146,6 +148,10 @@ struct SfmFusedParams {
   // what pix_map receives for a masked or out-of-view (pixel, source): 0 (its share of the loss), or a negative marker in
   // the forward march of sfm_loss_min_reprojection, whose select kernel must tell "masked" from "error 0"
   float pix_map_masked;
+  // desc->flags & (SFM_FLAG_AXISANGLE_POSE | SFM_FLAG_POSE_INVERT_MASK): with the first bit the epilogue instances of the
+  // axis-angle pose run its chain, bit 16 + i inverting source i's (the march reads only the tables).  One word, so that
+  // it takes the struct's tail padding and no kernel parameter behind the struct moves
+  unsigned pose_flags;
 };
 
 // Launch helper: with pdl the kernel is a programmatic dependent launch on the previous kernel of the stream (its
@@ -244,8 +250,9 @@ int sfm_launch_scale(float* const* ptrs, const long long* counts, int n, const f
 int sfm_launch_image_pullback(const SfmFusedParams& p, int H, int W, cudaStream_t stream);
 // gintrinsics (B,ns,3,3) from the dL/dP cells (SfmWsLayout::off_acc + 4 doubles) and the poses / intrinsics the step
 // used (fused_loss.cu); a dependent launch behind the step's last kernel
+// (pose_aa / pose_inv: SFM_FLAG_AXISANGLE_POSE and the inversion mask, bit i for source i)
 int sfm_launch_intrinsics_grad(int B, int S, int ns, const double* cells, const float* poses, const float* intrinsics,
-                               float* gintrinsics, cudaStream_t stream);
+                               int pose_aa, unsigned pose_inv, float* gintrinsics, cudaStream_t stream);
 
 // Full-resolution multi-scale (SFM_FLAG_FULL_RES_MULTISCALE, full_res.cu): the scales >= 1 of the step are full-resolution
 // scales whose disparity up[s] = U_s(disp[s]) and gradient gup[s] live in the workspace.

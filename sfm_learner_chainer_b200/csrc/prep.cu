@@ -38,9 +38,12 @@ struct PrepRow {
 // SM: 0 = no smoothness tasks, 1 = loss only, 2 = loss and gdisp; 3 / 4 = 1 / 2 with per-task losses instead of the CTA
 // partial (a CTA's tasks may belong to different snippets).  No early programmatic-launch trigger: the dependent
 // fused kernel's CTAs would pile up on whichever SMs are free first (measured, see the launch policy notes in DESIGN.md).
-template <int SM>
+// AA: SFM_FLAG_AXISANGLE_POSE, the tables of Monodepth2's axis-angle pose, bit i of pose_inv inverting source i's.  Its
+// own instances: the inlined fp64 chain changes the register allocation of the whole kernel, so the Euler instances keep
+// the parent's code (and pose_inv, the trailing argument, is not read there).
+template <int SM, bool AA>
 __global__ void __launch_bounds__(kPrepThreads) sfm_prep_kernel(const __grid_constant__ SfmPrepParams p,
-                                                                const __grid_constant__ SfmSmoothParams sm) {
+                                                                const __grid_constant__ SfmSmoothParams sm, unsigned pose_inv) {
   int blk = blockIdx.x;
   if (blk < p.n_tail_blocks) {
     // ---- tables + accumulator reset (a handful of leading CTAs)
@@ -62,7 +65,10 @@ __global__ void __launch_bounds__(kPrepThreads) sfm_prep_kernel(const __grid_con
       } else {
         for (int k = 0; k < 6; ++k) pose[k] = p.poses[((size_t)b * p.S + i) * 6 + k];
       }
-      sfm_build_proj(pose, K, P);
+      if constexpr (AA)
+        sfm_build_proj_axisangle(pose, (pose_inv >> i) & 1u, K, P);
+      else
+        sfm_build_proj(pose, K, P);
       // A non-finite pose or intrinsic would make every pixel of this (snippet, source) pair project to NaN: out of view
       // by the strict test of transform.py:128-131, but with NaN in the backward's 0 * P products.  Such a pair gets a
       // finite projection that sends every pixel out of view instead (q = (1e30, 1e30, 1)): losses and gradients of the
@@ -205,7 +211,17 @@ __global__ void sfm_pose_reduce_kernel(const float* __restrict__ x, float* __res
 
 }  // namespace
 
-int sfm_launch_prep(const SfmPrepParams& p_in, const SfmSmoothParams* sm_in, int sm_mode, cudaStream_t stream) {
+template <bool AA>
+int launch_prep(const SfmPrepParams& p, const SfmSmoothParams& sm, int sm_mode, unsigned grid, unsigned pose_inv,
+                cudaStream_t stream) {
+  const auto kernel = sm_mode == 4 ? sfm_prep_kernel<4, AA> : sm_mode == 3 ? sfm_prep_kernel<3, AA> : sm_mode == 2 ? sfm_prep_kernel<2, AA>
+                    : sm_mode == 1 ? sfm_prep_kernel<1, AA> : sfm_prep_kernel<0, AA>;
+  SFM_CUDA_CHECK(sfm_launch_kernel(kernel, grid, kPrepThreads, stream, false, p, sm, pose_inv));
+  return 0;
+}
+
+int sfm_launch_prep(const SfmPrepParams& p_in, const SfmSmoothParams* sm_in, int sm_mode, cudaStream_t stream,
+                    unsigned pose_flags) {
   SfmPrepParams p = p_in;
   const SfmSmoothParams sm = sm_in ? *sm_in : SfmSmoothParams{};
   if (sm.n_ctas <= 0) sm_mode = 0;
@@ -214,10 +230,9 @@ int sfm_launch_prep(const SfmPrepParams& p_in, const SfmSmoothParams* sm_in, int
   p.n_tail_blocks = (int)((n_tail + kPrepThreads - 1) / kPrepThreads);
   const unsigned grid = (unsigned)(p.n_tail_blocks + p.n_pyr_blocks + (sm_mode ? sm.n_ctas : 0));
   if (grid == 0) return 0;                        // e.g. sfm_pyramid with a single scale: nothing to build
-  const auto kernel = sm_mode == 4 ? sfm_prep_kernel<4> : sm_mode == 3 ? sfm_prep_kernel<3> : sm_mode == 2 ? sfm_prep_kernel<2>
-                    : sm_mode == 1 ? sfm_prep_kernel<1> : sfm_prep_kernel<0>;
-  SFM_CUDA_CHECK(sfm_launch_kernel(kernel, grid, kPrepThreads, stream, false, p, sm));
-  return 0;
+  const unsigned inv = (pose_flags & SFM_FLAG_POSE_INVERT_MASK) >> SFM_FLAG_POSE_INVERT_SHIFT;
+  return (p.build_tables && (pose_flags & SFM_FLAG_AXISANGLE_POSE)) ? launch_prep<true>(p, sm, sm_mode, grid, inv, stream)
+                                                                    : launch_prep<false>(p, sm, sm_mode, grid, 0u, stream);
 }
 
 int sfm_launch_disp_activation(long long n, const float* x, float* disp, float* dact, cudaStream_t stream) {

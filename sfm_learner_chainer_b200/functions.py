@@ -63,12 +63,26 @@ class ViewSynthesisLoss(object):
     padding_mode="border", align-corners mapping, no x2 rule) and masks only pixels whose projection is degenerate, and
     the SSIM windows use reflection padding by one pixel; see SFM_FLAG_BORDER_PADDING in include/sfmloss.h.  Not with
     exp_reg, image_grads or debug dumps.
+    axisangle_pose: Monodepth2's pose parametrisation: every `poses` row is (v0, v1, v2, tx, ty, tz), an axis-angle
+    vector and a translation, turned into [R | t] as Monodepth2's transformation_from_parameters does (no angle
+    clipping); gposes is the gradient w.r.t. those rows.  invert_sources: tuple of source indices whose transform is
+    inverted, [R^T | -R^T t] (Monodepth2 inverts the pose of every source that precedes the target: frame ids
+    [0, -1, 1] give invert_sources=(0,)); needs axisangle_pose and is checked against S at call time.  See
+    SFM_FLAG_AXISANGLE_POSE in include/sfmloss.h.
     """
 
     def __init__(self, smooth_reg=0.0, exp_reg=0.0, ssim_rate=0.0, n_scales=N_SCALES, B_global=None,
                  raw_disp_scales=0, raw_pose=False, edge_aware_smooth=False, image_grads=False,
                  intrinsics_grad=False, snippet_terms=False, pixel_terms=False, min_reprojection=False, automask=True,
-                 full_res_multiscale=False, mean_norm_smooth=False, edge_mean_abs=False, border_padding=False):
+                 full_res_multiscale=False, mean_norm_smooth=False, edge_mean_abs=False, border_padding=False,
+                 axisangle_pose=False, invert_sources=()):
+        invert_sources = tuple(int(i) for i in (invert_sources or ()))
+        if invert_sources and not axisangle_pose:
+            raise ValueError('invert_sources needs axisangle_pose')
+        if any(i < 0 for i in invert_sources):
+            raise ValueError('invert_sources must hold source indices >= 0, got %r' % (invert_sources,))
+        self.axisangle_pose = bool(axisangle_pose)
+        self.invert_sources = invert_sources
         if edge_mean_abs and not edge_aware_smooth:
             raise ValueError('edge_mean_abs needs edge_aware_smooth')
         if border_padding:
@@ -138,6 +152,12 @@ class ViewSynthesisLoss(object):
             flags |= L.SFM_FLAG_EDGE_MEAN_ABS
         if self.border_padding:
             flags |= L.SFM_FLAG_BORDER_PADDING
+        if self.axisangle_pose:
+            flags |= L.SFM_FLAG_AXISANGLE_POSE
+            for i in self.invert_sources:
+                if i >= S:
+                    raise ValueError('invert_sources names source %d, but there are S=%d sources' % (i, S))
+                flags |= 1 << (L.SFM_FLAG_POSE_INVERT_SHIFT + i)
         return L.SfmDesc(B, S, H, W, self.n_scales, int(self.B_global or 0), self.smooth_reg, self.exp_reg,
                          self.ssim_rate, flags, self.raw_disp_scales, raw_pose_hw)
 

@@ -19,6 +19,8 @@ SFM_FLAG_FULL_RES_MULTISCALE = 0x80
 SFM_FLAG_MEAN_NORM_SMOOTH = 0x100
 SFM_FLAG_EDGE_MEAN_ABS = 0x200
 SFM_FLAG_BORDER_PADDING = 0x400
+SFM_FLAG_AXISANGLE_POSE = 0x800
+SFM_FLAG_POSE_INVERT_SHIFT = 16          # flags bit 16 + i: invert the transform of source i
 
 SFM_E_INVALID_DESC = -1
 SFM_E_INVALID_SHAPE = -2
