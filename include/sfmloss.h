@@ -73,6 +73,10 @@ extern "C" {
 #define SFM_FLAG_AXISANGLE_POSE 0x800u /* Monodepth2's pose: `poses` rows are (v0, v1, v2, tx, ty, tz), an axis-angle
                                          vector and a translation, instead of the Euler vector; see "Axis-angle pose"
                                          below.  Does not size the workspace */
+#define SFM_FLAG_GEOMETRY_CONSISTENCY 0x1000u /* the workspace also holds the self-discovered mask planes and the per-pixel
+                                         map planes of sfm_loss_geometry (B*S*sum_s h_s*w_s floats each); see "Geometry
+                                         consistency" below.  Every other entry point accepts the flag and behaves exactly
+                                         as without it */
 #define SFM_FLAG_POSE_INVERT_SHIFT 16   /* flags bits 16..23: with SFM_FLAG_AXISANGLE_POSE, bit 16 + i inverts the
                                          transform of source i (Monodepth2's frame ids < 0) */
 #define SFM_FLAG_POSE_INVERT(i) (1u << (SFM_FLAG_POSE_INVERT_SHIFT + (i)))
@@ -574,6 +578,60 @@ int sfm_upsample_disparity(int N, int h, int w, int H, int W, const float* x, fl
  * An invert bit without SFM_FLAG_AXISANGLE_POSE, or for a source >= S, is SFM_E_INVALID_DESC.  The flag works with every
  * fused entry point, sfm_build_tables, sfm_intrinsics_grad, raw pose maps and CUDA-graph capture; sfm_host_ctx_create
  * returns SFM_E_UNSUPPORTED.  The stage warp (sfm_warp_forward / sfm_warp_backward) has no descriptor and stays Euler. */
+
+/* Geometry consistency (SC-SfMLearner: Bian et al., "Unsupervised Scale-consistent Depth and Ego-motion Learning from
+ * Monocular Video", NeurIPS 2019), sfm_loss_geometry.  Without it the depth and pose of SfM-Learner drift in scale from
+ * snippet to snippet; the term ties the depth of the target to the predicted depth of every source frame.  Per scale s,
+ * snippet b, target pixel p and source i:
+ *   projection     the step's own: the same fp32 operations as the photometric term, so the taps, the strict in-view
+ *                  flag inb (transform.py:128-131) and the bilinear weights w1..w4 are bitwise those of the warp.
+ *   validity       a pair is valid iff inb.  An invalid pair contributes nothing to the geometry term and has M = 1 (its
+ *                  photometric term is already masked by the x2 rule).
+ *   computed depth z' = q2, the third row of P_s . [X, Y, Z, 1] before the + 1e-10 (the source-camera depth: row 2 of K is
+ *                  (0, 0, 1)).  sfm_intrinsics_grad afterwards therefore stays exact.
+ *   projected depth D' = ((w1 * 1/d'00 + w2 * 1/d'01) + w3 * 1/d'10) + w4 * 1/d'11, d' = src_disps[s] of (b, i), the
+ *                  reciprocals as the march forms 1/disp (correctly rounded), products and sums individually rounded.
+ *   depth diff     D_diff = clip(|z' - D'| / (z' + D'), 0, 1) in fp32.  Derivative with torch's conventions: sign(0) = 0,
+ *                  and the clip passes the gradient on the closed interval [0, 1] and blocks it outside.  A point behind
+ *                  the source camera that still projects into view (z' + D' <= 0, or z' < 0) clips and has gradient 0.
+ *   geometry term  L_geo = sum_s sum_i sum_{b, p valid} D_diff / (B_global * h_s * w_s): no 2^-s and no 1/S, as the
+ *                  released code sums over the sources.  The step adds geometry_reg * L_geo to the total; snippet weights
+ *                  and gy apply to it as to every other term.
+ *   self-mask      (self_mask != 0) the photometric terms are those of sfm_loss_weighted with M_i(p) = 1 - D_diff_i(p),
+ *                  L1 and SSIM parts, with its denominators; the gradient includes the product-rule term through M.
+ *   reporting      losses_out[0] (total) includes geometry_reg * L_geo; losses_out[3] REPORTS geometry_reg * L_geo: that
+ *                  slot is the explainability regulariser's, which this entry point excludes, so it carries the geometry
+ *                  term here (also in the rows of SfmSnippetTerms and in the peer sum).  losses_out[1] and [4] are the
+ *                  (masked) L1 and SSIM parts, [2] the smoothness term.
+ *   gradients      gdisps, gposes, the dL/dP cells (hence sfm_intrinsics_grad afterwards) and gsrc_disps are those of
+ *                  this total.  gdisps are bitwise reproducible from run to run; gsrc_disps are accumulated with fp32
+ *                  atomics after the step zeroes them, and their last bits vary with the order, as gsrc's do.
+ * Computed as prologue -> (smoothness kernels) -> geometry forward (D_diff, M, the loss) -> the march (per-pixel instances
+ * with the M planes under the self-mask, the plain ones without it) -> geometry backward -> epilogue; graph-capturable. */
+typedef struct SfmGeometry {
+  const float* src_disps[SFM_MAX_SCALES];  /* (B,S,h_s,w_s) device, activated disparity of every source frame */
+  float* gsrc_disps[SFM_MAX_SCALES];       /* (B,S,h_s,w_s) device: d total / d src_disps (overwritten), or NULL */
+  float* diff_maps[SFM_MAX_SCALES];        /* (B,S,h_s,w_s) device: D_diff (0 for invalid pairs), or NULL */
+  float geometry_reg;                      /* SC-SfMLearner's w3 (0.5 in its released setting) */
+  int32_t self_mask;                       /* != 0: the photometric terms are weighted by M = 1 - D_diff */
+} SfmGeometry;
+
+/* sfm_loss_snippets with the geometry consistency term and, optionally, the self-discovered mask.  desc->flags must
+ * contain SFM_FLAG_GEOMETRY_CONSISTENCY (else SFM_E_INVALID_DESC; the workspace is sized with it), geo must not be NULL
+ * and geo->src_disps[s] must be set for every s < n_scales (else SFM_E_NULL_POINTER).  grads == NULL: forward only (the
+ * losses and diff_maps; gsrc_disps is then not written).  Composes with snippet terms, the peer sum (diff_maps stay per
+ * rank), raw target disparity (raw_disp_scales) and raw pose, the axis-angle pose with its invert bits, either smoothness
+ * with SFM_FLAG_MEAN_NORM_SMOOTH / SFM_FLAG_EDGE_MEAN_ABS, SFM_FLAG_TABLES_PROVIDED, SFM_FLAG_REUSE_PYRAMID,
+ * sfm_intrinsics_grad afterwards and CUDA-graph capture.  src_disps are activated disparities (raw source maps are not
+ * supported).  SFM_E_UNSUPPORTED: exp_reg != 0 (the self-mask replaces the explainability branch and its slot carries the
+ * geometry term), SFM_FLAG_FULL_RES_MULTISCALE, SFM_FLAG_BORDER_PADDING or SFM_FLAG_MIN_REPROJECTION in the same call;
+ * sfm_host_ctx_create with the flag.  Image gradients and debug dumps have no argument here.
+ * SC-SfMLearner applies the pair loss in both directions; the reverse direction is a second call on a batch of B*S
+ * snippets with S = 1 (target = source frame i, source = the target frame, disparities swapped, the inverse pose: with
+ * SFM_FLAG_AXISANGLE_POSE the same rows with the invert bit flipped), which also supplies the smoothness of the sources
+ * (INTEGRATION.md §6). */
+int sfm_loss_geometry(const SfmDesc* desc, const SfmInputs* in, const SfmSnippetTerms* terms, const SfmGeometry* geo,
+                      float* losses_out, const SfmGrads* grads, void* workspace, SfmPeer* peer, void* stream);
 
 #ifdef __cplusplus
 }

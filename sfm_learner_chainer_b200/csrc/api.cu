@@ -180,7 +180,7 @@ int num_sms() {
 int run_loss(const SfmDesc* d, const SfmInputs* in, float* losses_out, const SfmGrads* grads, const float* gy,
              const SfmDebug* dbg, void* workspace, cudaStream_t st, const SfmPeerDev* peer = nullptr,
              const SfmImageGrads* ig = nullptr, const SfmSnippetTerms* snip = nullptr, const SfmPixelTerms* pix = nullptr,
-             const SfmMinReprojection* mr = nullptr) {
+             const SfmMinReprojection* mr = nullptr, const SfmGeometry* geo = nullptr) {
   int rc = sfm_validate_desc(d);
   if (rc) return rc;
   // SFM_FLAG_BORDER_PADDING runs the per-pixel instances (weights and maps NULL unless the caller passed them)
@@ -222,6 +222,8 @@ int run_loss(const SfmDesc* d, const SfmInputs* in, float* losses_out, const Sfm
   if (pix) mode |= SFM_MODE_PIX;
   if (mr) mode |= SFM_MODE_PIX | SFM_MODE_MINREP;
   if (border) mode |= SFM_MODE_PIX | SFM_MODE_BORDER;
+  const bool self_mask = geo && geo->self_mask != 0;
+  if (self_mask) mode |= SFM_MODE_PIX;             // the per-pixel instances with the mask planes as weights
   const SfmStepPlan plan = sfm_plan_step(d, mode, num_sms());
   SfmWsLayout L;
   sfm_ws_layout(d, &L);
@@ -260,6 +262,11 @@ int run_loss(const SfmDesc* d, const SfmInputs* in, float* losses_out, const Sfm
       p.pix_map[s] = pix->losses[s];
     }
     if (mr) p.pix_w[s] = (const float*)(ws + L.off_mrw[s]);   // the one-hot weights, made by the select kernel
+    if (self_mask) {
+      // M = 1 - D_diff, made by the geometry forward kernel; the maps d total / d M feed its backward kernel
+      p.pix_w[s] = (const float*)(ws + L.off_geow[s]);
+      p.pix_map[s] = grads ? (float*)(ws + L.off_geomap[s]) : nullptr;
+    }
   }
   auto photometric_consts = [&](int s) {              // from the size of the photometric terms of scale s
     const int h = p.h[s], w = p.w[s];
@@ -388,6 +395,29 @@ int run_loss(const SfmDesc* d, const SfmInputs* in, float* losses_out, const Sfm
     SFM_CUDA_CHECK(cudaMemsetAsync(ig->gsrc, 0, (size_t)d->B * d->S * 3 * d->H * d->W * sizeof(float), st));
     if (L.gsrc_bytes) SFM_CUDA_CHECK(cudaMemsetAsync(ws + L.off_gsrc[1], 0, L.gsrc_bytes, st));
   }
+  SfmGeoArgs ga{};
+  if (geo) {
+    ga.geometry_reg = geo->geometry_reg;
+    int nf = 0, nb = 0;
+    for (int s = 0; s < SFM_MAX_SCALES; ++s) {
+      ga.fwd_begin[s] = nf;
+      ga.bwd_begin[s] = nb;
+      if (s >= d->n_scales) continue;
+      const long long plane = (long long)p.h[s] * p.w[s];
+      const int per = (int)((plane + 255) / 256);
+      nf += d->B * d->S * per;
+      nb += d->B * per;
+      ga.src_disps[s] = geo->src_disps[s];
+      ga.diff_maps[s] = geo->diff_maps[s];
+      ga.gsrc_disps[s] = grads ? geo->gsrc_disps[s] : nullptr;
+      ga.mask[s] = self_mask ? (float*)(ws + L.off_geow[s]) : nullptr;
+      ga.map[s] = self_mask ? p.pix_map[s] : nullptr;
+      // gsrc_disps is accumulated with fp32 reductions
+      if (ga.gsrc_disps[s]) SFM_CUDA_CHECK(cudaMemsetAsync(ga.gsrc_disps[s], 0, (size_t)d->B * d->S * plane * sizeof(float), st));
+    }
+    ga.fwd_begin[SFM_MAX_SCALES] = nf;
+    ga.bwd_begin[SFM_MAX_SCALES] = nb;
+  }
   if (fr && (rc = sfm_launch_full_res_upsample(f, st))) return rc;
   rc = sfm_launch_prep(pp, &sm, (grads ? 2 : 1) + ((snip || mean_norm) ? 2 : 0), st, p.pose_flags);
   if (rc) return rc;
@@ -397,7 +427,7 @@ int run_loss(const SfmDesc* d, const SfmInputs* in, float* losses_out, const Sfm
     for (int s = 0; s < d->n_scales; ++s) a.selection[s] = mr->selection[s];
   }
   rc = sfm_launch_fused(p, plan, st, mr ? &a : nullptr, fr ? &native : nullptr, mean_norm ? &mn : nullptr,
-                        (d->flags & SFM_FLAG_EDGE_MEAN_ABS) != 0);
+                        (d->flags & SFM_FLAG_EDGE_MEAN_ABS) != 0, geo ? &ga : nullptr);
   if (rc || !fr || !grads) return rc;
   return sfm_launch_full_res_adjoint(f, st);
 }
@@ -537,6 +567,44 @@ extern "C" int sfm_loss_min_reprojection(const SfmDesc* desc, const SfmInputs* i
   }
   return run_loss(desc, in, losses_out, grads, nullptr, nullptr, workspace, (cudaStream_t)stream, dev, nullptr,
                   snip ? terms : nullptr, nullptr, mr);
+}
+
+extern "C" int sfm_loss_geometry(const SfmDesc* desc, const SfmInputs* in, const SfmSnippetTerms* terms,
+                                 const SfmGeometry* geo, float* losses_out, const SfmGrads* grads, void* workspace, SfmPeer* peer,
+                                 void* stream) {
+  int rc = sfm_validate_desc(desc);
+  if (rc) return rc;
+  if (!(desc->flags & SFM_FLAG_GEOMETRY_CONSISTENCY)) {
+    sfm_set_error("sfm_loss_geometry: desc->flags lacks SFM_FLAG_GEOMETRY_CONSISTENCY (the workspace must be sized with it)");
+    return SFM_E_INVALID_DESC;
+  }
+  if (desc->exp_reg != 0.f) {
+    sfm_set_error("unsupported: geometry consistency together with the explainability branch (exp_reg != 0)");
+    return SFM_E_UNSUPPORTED;
+  }
+  const unsigned excl = desc->flags & (SFM_FLAG_FULL_RES_MULTISCALE | SFM_FLAG_BORDER_PADDING | SFM_FLAG_MIN_REPROJECTION);
+  if (excl) {
+    sfm_set_error("unsupported: geometry consistency together with %s",
+                  (excl & SFM_FLAG_FULL_RES_MULTISCALE) ? "SFM_FLAG_FULL_RES_MULTISCALE"
+                  : (excl & SFM_FLAG_BORDER_PADDING) ? "SFM_FLAG_BORDER_PADDING" : "SFM_FLAG_MIN_REPROJECTION");
+    return SFM_E_UNSUPPORTED;
+  }
+  if (!geo) { sfm_set_error("SfmGeometry is NULL"); return SFM_E_NULL_POINTER; }
+  for (int s = 0; s < desc->n_scales; ++s)
+    if (!geo->src_disps[s]) { sfm_set_error("SfmGeometry.src_disps[%d] is NULL", s); return SFM_E_NULL_POINTER; }
+  const bool snip = terms && (terms->weights || terms->losses);
+  if (snip && !(desc->flags & SFM_FLAG_SNIPPET_TERMS)) {
+    sfm_set_error("sfm_loss_geometry: desc->flags lacks SFM_FLAG_SNIPPET_TERMS (the workspace must be sized with it)");
+    return SFM_E_INVALID_DESC;
+  }
+  if (!losses_out) { sfm_set_error("losses_out is NULL"); return SFM_E_NULL_POINTER; }
+  const SfmPeerDev* dev = nullptr;
+  if (peer && !(dev = sfm_peer_dev(peer))) {
+    sfm_set_error("sfm_loss_geometry: the peer object is not connected (sfm_peer_connect)");
+    return SFM_E_UNSUPPORTED;
+  }
+  return run_loss(desc, in, losses_out, grads, nullptr, nullptr, workspace, (cudaStream_t)stream, dev, nullptr,
+                  snip ? terms : nullptr, nullptr, nullptr, geo);
 }
 
 extern "C" int sfm_scale_image_grads(const SfmDesc* desc, const float* gy, const SfmImageGrads* igrads, void* stream) {
@@ -744,6 +812,10 @@ extern "C" int sfm_host_ctx_create(const SfmDesc* desc, SfmHostCtx** ctx_out) {
   }
   if (desc->flags & SFM_FLAG_AXISANGLE_POSE) {
     sfm_set_error("unsupported: the host-buffer path with SFM_FLAG_AXISANGLE_POSE");
+    return SFM_E_UNSUPPORTED;
+  }
+  if (desc->flags & SFM_FLAG_GEOMETRY_CONSISTENCY) {
+    sfm_set_error("unsupported: the host-buffer path with SFM_FLAG_GEOMETRY_CONSISTENCY");
     return SFM_E_UNSUPPORTED;
   }
   int ndev = 0;

@@ -62,6 +62,11 @@ struct SfmWsLayout {
   size_t off_mnmean;                // float [B][ns][SFM_MN_SLOTS]
   size_t off_mnedge;                // float [B][ns][SFM_MN_SLOTS]
   size_t off_mnloss;                // float [B]
+  // SFM_FLAG_GEOMETRY_CONSISTENCY: the self-discovered mask M = 1 - D_diff of every (pixel, source), written by the
+  // geometry forward kernel, and the per-pixel maps d total / d M of the march, read by the geometry backward kernel.
+  // 0 without the flag.  (The loss partials ride in the fp64 cells.)
+  size_t off_geow[SFM_MAX_SCALES];  // float [B][S][h][w]
+  size_t off_geomap[SFM_MAX_SCALES];  // float [B][S][h][w]
   size_t acc_doubles;
   size_t total;
 };
@@ -187,6 +192,17 @@ static inline void sfm_ws_layout(const SfmDesc* d, SfmWsLayout* L) {
     off = sfm_align_up(off + slots, 256);
     L->off_mnloss = off;
     off = sfm_align_up(off + (size_t)d->B * sizeof(float), 256);
+  }
+  for (int s = 0; s < SFM_MAX_SCALES; ++s) L->off_geow[s] = L->off_geomap[s] = 0;
+  if (d->flags & SFM_FLAG_GEOMETRY_CONSISTENCY) {
+    for (int s = 0; s < d->n_scales; ++s) {
+      L->off_geow[s] = off;
+      off = sfm_align_up(off + (size_t)d->B * d->S * (d->H >> s) * (d->W >> s) * sizeof(float), 256);
+    }
+    for (int s = 0; s < d->n_scales; ++s) {
+      L->off_geomap[s] = off;
+      off = sfm_align_up(off + (size_t)d->B * d->S * (d->H >> s) * (d->W >> s) * sizeof(float), 256);
+    }
   }
   L->total = off;
 }

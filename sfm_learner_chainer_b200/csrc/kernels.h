@@ -238,8 +238,25 @@ int sfm_launch_mean_norm_fix(const SfmMeanNorm& m, bool grad, cudaStream_t strea
 // native: with SFM_FLAG_FULL_RES_MULTISCALE, the parameters of the native-resolution scales (dims, disparity, gradient,
 // pyramid, raw bits), read by the edge-aware smoothness kernel and by the epilogue's layout of the smoothness tasks.
 // mn: SFM_FLAG_MEAN_NORM_SMOOTH with a smoothness term (nullptr otherwise); edge_mean_abs: SFM_FLAG_EDGE_MEAN_ABS
+// Geometry consistency (sfm_loss_geometry, geometry.cuh): the forward kernel runs ahead of the march and writes D_diff,
+// the mask planes (p.pix_w under the self-mask) and the loss partials; the backward kernel runs behind it (gradient steps)
+// and chains the upstream of D_diff into gdisp, the dL/dP cells and gsrc_disps.  Block grids: scale s holds blocks
+// [fwd_begin[s], fwd_begin[s+1]) of the forward kernel, (b, i) x ceil(h w / 256) each, and [bwd_begin[s], bwd_begin[s+1])
+// of the backward kernel, b x ceil(h w / 256) each.
+struct SfmGeoArgs {
+  const float* src_disps[SFM_MAX_SCALES];
+  float* gsrc_disps[SFM_MAX_SCALES];   // zeroed by the step (nullptr: not wanted)
+  float* diff_maps[SFM_MAX_SCALES];    // nullptr: not wanted
+  float* mask[SFM_MAX_SCALES];         // self-mask: M planes (the march's pix_w); nullptr without the self-mask
+  const float* map[SFM_MAX_SCALES];    // self-mask, gradient steps: the march's maps d total / d M (nullptr otherwise)
+  float geometry_reg;
+  int fwd_begin[SFM_MAX_SCALES + 1];
+  int bwd_begin[SFM_MAX_SCALES + 1];
+};
+// mr: minimum reprojection; geo: geometry consistency (at most one of them)
 int sfm_launch_fused(SfmFusedParams& p, const SfmStepPlan& plan, cudaStream_t stream, const SfmMinRepArgs* mr = nullptr,
-                     const SfmFusedParams* native = nullptr, const SfmMeanNorm* mn = nullptr, bool edge_mean_abs = false);
+                     const SfmFusedParams* native = nullptr, const SfmMeanNorm* mn = nullptr, bool edge_mean_abs = false,
+                     const SfmGeoArgs* geo = nullptr);
 // smooth.cu; slots (SFM_FLAG_MEAN_NORM_SMOOTH): the per-CTA loss partials [B][ns][SFM_MN_SLOTS] instead of the cells
 int sfm_launch_edge_smooth(const SfmFusedParams& p, bool grad, bool mean_abs, float* slots, cudaStream_t stream);
 extern thread_local cudaEvent_t sfm_ev_start, sfm_ev_stop;   // profiling hook (sfm_set_kernel_events)

@@ -69,13 +69,36 @@ class ViewSynthesisLoss(object):
     inverted, [R^T | -R^T t] (Monodepth2 inverts the pose of every source that precedes the target: frame ids
     [0, -1, 1] give invert_sources=(0,)); needs axisangle_pose and is checked against S at call time.  See
     SFM_FLAG_AXISANGLE_POSE in include/sfmloss.h.
+    geometry_consistency: SC-SfMLearner's geometry consistency term (Bian et al., NeurIPS 2019): every target pixel is
+    projected into each source frame and its computed depth z' is compared with the source frame's own predicted depth
+    D' sampled there, D_diff = clip(|z' - D'| / (z' + D'), 0, 1) on the in-view pairs; geometry_reg times its mean over
+    the target pixels (summed over the sources and scales) is added to the total and reported in the exp_loss slot.
+    forward and forward_backward then take `src_disps`, a list of n_scales (B,S,h_s,w_s) arrays with the activated
+    disparity of every source frame, and return `geometry_diff` (the D_diff maps, like src_disps) appended to the
+    forward's tuple / in the grads dict, where forward_backward also puts `gsrc_disps`, the gradient w.r.t. src_disps.
+    self_mask: the photometric terms of every (pixel, source) are weighted by M = 1 - D_diff, with the gradient through
+    M (SC-SfMLearner's self-discovered mask).  See sfm_loss_geometry in include/sfmloss.h.  Not with exp_reg,
+    image_grads, pixel_terms, min_reprojection, full_res_multiscale, border_padding or debug dumps.
     """
 
     def __init__(self, smooth_reg=0.0, exp_reg=0.0, ssim_rate=0.0, n_scales=N_SCALES, B_global=None,
                  raw_disp_scales=0, raw_pose=False, edge_aware_smooth=False, image_grads=False,
                  intrinsics_grad=False, snippet_terms=False, pixel_terms=False, min_reprojection=False, automask=True,
                  full_res_multiscale=False, mean_norm_smooth=False, edge_mean_abs=False, border_padding=False,
-                 axisangle_pose=False, invert_sources=()):
+                 axisangle_pose=False, invert_sources=(), geometry_consistency=False, geometry_reg=0.5, self_mask=False):
+        if self_mask and not geometry_consistency:
+            raise ValueError('self_mask needs geometry_consistency')
+        if geometry_consistency:
+            for name, on in (('image_grads', image_grads), ('pixel_terms', pixel_terms),
+                             ('min_reprojection', min_reprojection), ('full_res_multiscale', full_res_multiscale),
+                             ('border_padding', border_padding)):
+                if on:
+                    raise ValueError('geometry_consistency is not supported together with %s' % name)
+            if float(exp_reg or 0.0) != 0.0:
+                raise ValueError('geometry_consistency is not supported together with the explainability branch (exp_reg)')
+        self.geometry_consistency = bool(geometry_consistency)
+        self.geometry_reg = float(geometry_reg)
+        self.self_mask = bool(self_mask)
         invert_sources = tuple(int(i) for i in (invert_sources or ()))
         if invert_sources and not axisangle_pose:
             raise ValueError('invert_sources needs axisangle_pose')
@@ -152,6 +175,8 @@ class ViewSynthesisLoss(object):
             flags |= L.SFM_FLAG_EDGE_MEAN_ABS
         if self.border_padding:
             flags |= L.SFM_FLAG_BORDER_PADDING
+        if self.geometry_consistency:
+            flags |= L.SFM_FLAG_GEOMETRY_CONSISTENCY
         if self.axisangle_pose:
             flags |= L.SFM_FLAG_AXISANGLE_POSE
             for i in self.invert_sources:
@@ -165,7 +190,7 @@ class ViewSynthesisLoss(object):
         # the image-gradient, snippet-terms, min-reprojection, full-resolution and mean-normalisation flags size the
         # workspace; the per-call flags (tables, reused pyramid) do not
         sizing = (L.SFM_FLAG_IMAGE_GRADS | L.SFM_FLAG_SNIPPET_TERMS | L.SFM_FLAG_MIN_REPROJECTION
-                  | L.SFM_FLAG_FULL_RES_MULTISCALE | L.SFM_FLAG_MEAN_NORM_SMOOTH)
+                  | L.SFM_FLAG_FULL_RES_MULTISCALE | L.SFM_FLAG_MEAN_NORM_SMOOTH | L.SFM_FLAG_GEOMETRY_CONSISTENCY)
         key = (desc.B, desc.S, desc.H, desc.W, desc.n_scales, desc.flags & sizing,
                str(getattr(like, 'device', '')))
         ws = self._ws.get(key)
@@ -301,19 +326,53 @@ class ViewSynthesisLoss(object):
             mr.selection[s] = D.ptr(sel[s])
         return mr, sel
 
+    def _geometry(self, desc, tgt, src_disps, want_grads):
+        """-> (SfmGeometry, D_diff maps, gsrc_disps or None), each a list of n_scales (B,S,h_s,w_s) arrays."""
+        if src_disps is None or len(src_disps) != self.n_scales:
+            raise ValueError('geometry_consistency needs src_disps, a list of %d (B,S,h,w) source disparity maps'
+                             % self.n_scales)
+        ge = L.SfmGeometry()
+        ge.geometry_reg = self.geometry_reg
+        ge.self_mask = 1 if self.self_mask else 0
+        diff, gsd = [], [] if want_grads else None
+        for s in range(self.n_scales):
+            shape = (desc.B, desc.S, desc.H >> s, desc.W >> s)
+            D.check_array(src_disps[s], 'src_disps[%d]' % s, shape)
+            ge.src_disps[s] = D.ptr(src_disps[s])
+            diff.append(D.empty(tgt, shape))
+            ge.diff_maps[s] = D.ptr(diff[s])
+            if want_grads:
+                gsd.append(D.empty(tgt, shape))
+                ge.gsrc_disps[s] = D.ptr(gsd[s])
+        return ge, diff, gsd
+
     # ---- operators
     def forward(self, tgt, src, intrinsics, disps, poses, logits=None, proj=None, kinv=None, debug=False,
-                snippet_weights=None, pixel_weights=None):
+                snippet_weights=None, pixel_weights=None, src_disps=None):
         """-> losses (5,) device array in the order of lib.LOSS_KEYS [, debug dict].
         With the operator's snippet_terms: -> (losses, snippet losses (B,5)), losses = sum_b w_b * l_b.
         With the operator's pixel_terms the per-pixel loss maps (list of n_scales (B,S,h,w)) are appended as the last
         element: (losses, maps) or (losses, snippet losses, maps).
-        With the operator's min_reprojection the selection maps (list of n_scales (B,h,w) int8) are appended likewise."""
-        if debug and (self.snippet_terms or self.pixel_terms or self.min_reprojection or self.border_padding):
-            raise ValueError('debug dumps are not available on an operator with snippet_terms, pixel_terms, min_reprojection '
-                             'or border_padding')
+        With the operator's min_reprojection the selection maps (list of n_scales (B,h,w) int8) are appended likewise.
+        With the operator's geometry_consistency: src_disps (list of n_scales (B,S,h,w)) is required and the D_diff maps
+        (list of n_scales (B,S,h,w)) are appended likewise."""
+        if debug and (self.snippet_terms or self.pixel_terms or self.min_reprojection or self.border_padding
+                      or self.geometry_consistency):
+            raise ValueError('debug dumps are not available on an operator with snippet_terms, pixel_terms, min_reprojection, '
+                             'border_padding or geometry_consistency')
+        if src_disps is not None and not self.geometry_consistency:
+            raise ValueError('src_disps needs ViewSynthesisLoss(geometry_consistency=True)')
         desc, inp = self._pack(tgt, src, intrinsics, disps, poses, logits, proj, kinv)
         losses = D.empty(tgt, (5,))
+        if self.geometry_consistency:
+            terms, rows = self._snippet_terms(desc, tgt, snippet_weights)
+            if pixel_weights is not None:
+                raise ValueError('pixel_weights needs ViewSynthesisLoss(pixel_terms=True)')
+            ge, diff, _ = self._geometry(desc, tgt, src_disps, False)
+            L.check(self._lib.sfm_loss_geometry(C.byref(desc), C.byref(inp), C.byref(terms) if terms else None,
+                                                C.byref(ge), _vp(losses), None, self._workspace(desc, tgt), None,
+                                                C.c_void_p(D.current_stream(tgt))))
+            return (losses,) + ((rows,) if self.snippet_terms else ()) + (diff,)
         if self.min_reprojection:
             terms, rows = self._snippet_terms(desc, tgt, snippet_weights)
             if pixel_weights is not None:
@@ -384,7 +443,7 @@ class ViewSynthesisLoss(object):
 
     def forward_backward(self, tgt, src, intrinsics, disps, poses, logits=None, proj=None, kinv=None, reuse_pyramid=False,
                          peer=None, image_grads=('tgt', 'src'), intrinsics_grad=True, snippet_weights=None,
-                         pixel_weights=None):
+                         pixel_weights=None, src_disps=None):
         """Single fused pass: -> (losses (5,), dict(gdisps, gposes, glogits)) for upstream gradient 1.
         reuse_pyramid: the workspace already holds this batch's pyramid (build_pyramid).
         peer: a distributed.PeerLossSum -- the batch is sharded by snippet over several GPUs (B_global set) and the
@@ -399,7 +458,12 @@ class ViewSynthesisLoss(object):
         photometric terms per (pixel, source), and the dict also holds pixel_losses, the maps d total / d weights
         (this shard's, under peer).
         With the operator's min_reprojection the dict also holds selection (list of n_scales (B,h,w) int8; this
-        shard's, under peer)."""
+        shard's, under peer).
+        With the operator's geometry_consistency: src_disps (list of n_scales (B,S,h,w) activated source disparities) is
+        required, and the dict also holds geometry_diff (the D_diff maps, this shard's under peer) and gsrc_disps (the
+        gradient w.r.t. src_disps)."""
+        if src_disps is not None and not self.geometry_consistency:
+            raise ValueError('src_disps needs ViewSynthesisLoss(geometry_consistency=True)')
         want_k = self._want_intrinsics_grad(intrinsics_grad, proj, kinv)
         desc, inp = self._pack(tgt, src, intrinsics, disps, poses, logits, proj, kinv)
         if reuse_pyramid:
@@ -413,6 +477,16 @@ class ViewSynthesisLoss(object):
         pt, maps = self._pixel_terms(desc, tgt, pixel_weights)
         if maps is not None:
             out['pixel_losses'] = maps
+        if self.geometry_consistency:
+            ge, out['geometry_diff'], out['gsrc_disps'] = self._geometry(desc, tgt, src_disps, True)
+            L.check(self._lib.sfm_loss_geometry(C.byref(desc), C.byref(inp), C.byref(terms) if terms else None,
+                                                C.byref(ge), _vp(losses), C.byref(g), self._workspace(desc, tgt),
+                                                peer.handle if peer is not None else None,
+                                                C.c_void_p(D.current_stream(tgt))))
+            self._intrinsics_grad(desc, inp, tgt, out, want_k)
+            if self._ev_pyramid is not None:
+                self._ev_loss = D.record_event(tgt)
+            return losses, out
         if self.min_reprojection:
             mr, out['selection'] = self._min_reprojection(desc, tgt)
             L.check(self._lib.sfm_loss_min_reprojection(C.byref(desc), C.byref(inp), C.byref(terms) if terms else None,
@@ -442,7 +516,8 @@ class ViewSynthesisLoss(object):
         return losses, out
 
     def scale_grads(self, grads, gy, B, S, H, W):
-        """grads *= gy (device scalar); a no-op on the device when gy == 1."""
+        """grads *= gy (device scalar); a no-op on the device when gy == 1.  gsrc_disps (geometry_consistency) is not
+        touched: it has the shape of a per-pixel map and is scaled by the caller as the maps are."""
         gp_shape = tuple(grads['gposes'].shape)
         desc = self._desc(B, S, H, W, 0, int(gp_shape[2] * (gp_shape[3] if len(gp_shape) > 3 else 1)) if self.raw_pose else 0)
         g = L.SfmGrads()

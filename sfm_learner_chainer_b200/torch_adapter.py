@@ -11,7 +11,11 @@ from .functions import ViewSynthesisLoss
 class _ViewSynthesisLossFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, op, tgt, src, intrinsics, weights, n_scales, use_exp, n_pred, *rest):
-        preds, pix_w = rest[:n_pred], rest[n_pred:]      # pix_w: n_scales per-pixel weights (or None) with op.pixel_terms
+        preds, extra = rest[:n_pred], rest[n_pred:]
+        # extra: n_scales per-pixel weights (or None) with op.pixel_terms, n_scales source disparities with
+        # op.geometry_consistency
+        pix_w = extra if op.pixel_terms else ()
+        src_d = extra if op.geometry_consistency else ()
         disps = [p.contiguous() for p in preds[:n_scales]]
         poses = preds[n_scales].contiguous()
         logits = [p.contiguous() for p in preds[n_scales + 1:]] if use_exp else None
@@ -27,7 +31,9 @@ class _ViewSynthesisLossFn(torch.autograd.Function):
                                             intrinsics_grad=ctx.want_k,
                                             snippet_weights=weights.detach().contiguous() if weights is not None else None,
                                             **(dict(pixel_weights=[w.detach().contiguous() if w is not None else None
-                                                                   for w in pix_w]) if op.pixel_terms else {}))
+                                                                   for w in pix_w]) if op.pixel_terms else {}),
+                                            **(dict(src_disps=[d.detach().contiguous() for d in src_d])
+                                               if op.geometry_consistency else {}))
         ctx.op, ctx.grads, ctx.shape = op, grads, tuple(src.shape)
         ctx.n_scales, ctx.use_exp = n_scales, use_exp
         ctx.consumed = False
@@ -43,6 +49,9 @@ class _ViewSynthesisLossFn(torch.autograd.Function):
         ctx.want_pw = [w is not None and ctx.needs_input_grad[8 + n_pred + s] for s, w in enumerate(pix_w)]
         outs += ctx.maps
         outs += grads.get('selection') or []      # min_reprojection: the selection maps, non-differentiable
+        outs += grads.get('geometry_diff') or []  # geometry_consistency: the D_diff maps
+        ctx.gsrc_d = grads.get('gsrc_disps') or []
+        ctx.want_sd = [ctx.needs_input_grad[8 + n_pred + s] for s in range(len(src_d))]
         ctx.mark_non_differentiable(*outs)
         return (losses[0].clone(),) + tuple(outs)
 
@@ -67,11 +76,12 @@ class _ViewSynthesisLossFn(torch.autograd.Function):
         gsrc = g.get('gsrc') if ctx.want_src else None
         gk = g.get('gintrinsics') if ctx.want_k else None
         gpw = tuple(gy * m if want else None for m, want in zip(ctx.maps, ctx.want_pw))
-        return (None, gtgt, gsrc, gk, gw, None, None, None) + tuple(out) + gpw
+        gsd = tuple(gy * m if want else None for m, want in zip(ctx.gsrc_d, ctx.want_sd))
+        return (None, gtgt, gsrc, gk, gw, None, None, None) + tuple(out) + gpw + gsd
 
 
 def view_synthesis_loss(op, tgt, src, intrinsics, pred_disps, pred_poses, pred_maskes=None, snippet_weights=None,
-                        pixel_weights=None):
+                        pixel_weights=None, src_disps=None):
     """-> (total_loss scalar tensor with grad_fn, losses (5,) tensor [total, pixel, smooth, exp, ssim]).
 
     pred_poses: (B,S,6) tensor or a tuple of S (B,6) tensors as PoseNet returns them (pose_net.py:52-54).
@@ -83,6 +93,9 @@ def view_synthesis_loss(op, tgt, src, intrinsics, pred_disps, pred_poses, pred_m
     the returned tuple; weights that require grad receive gy * pixel_losses[s].
     With op.min_reprojection: the selection maps (list of n_scales (B,h,w) int8 tensors: the chosen source, -1
     auto-masked, -2 no candidate) are appended to the returned tuple; they are not differentiable.
+    With op.geometry_consistency: src_disps (list of n_scales (B,S,h,w) tensors, the activated disparity of every source
+    frame, e.g. DispNet run on the source frames) is required and receives its gradient through autograd; the D_diff maps
+    (list of n_scales (B,S,h,w) tensors, not differentiable) are appended to the returned tuple.
     """
     assert isinstance(op, ViewSynthesisLoss)
     if snippet_weights is not None and not op.snippet_terms:
@@ -96,10 +109,18 @@ def view_synthesis_loss(op, tgt, src, intrinsics, pred_disps, pred_poses, pred_m
             raise ValueError('pixel_weights must hold %d entries (one per scale, None = 1)' % op.n_scales)
     if isinstance(pred_poses, (tuple, list)):
         pred_poses = torch.stack(list(pred_poses), dim=1)
+    src_d = []
+    if op.geometry_consistency:
+        if src_disps is None or len(src_disps) != op.n_scales:
+            raise ValueError('geometry_consistency needs src_disps, a list of %d (B,S,h,w) tensors' % op.n_scales)
+        src_d = list(src_disps)
+    elif src_disps is not None:
+        raise ValueError('src_disps needs ViewSynthesisLoss(geometry_consistency=True)')
     use_exp = op.use_exp
     preds = list(pred_disps) + [pred_poses] + (list(pred_maskes) if use_exp else [])
-    res = _ViewSynthesisLossFn.apply(op, tgt, src, intrinsics, snippet_weights, op.n_scales, use_exp, len(preds), *preds, *pix_w)
-    if not (op.pixel_terms or op.min_reprojection):
+    res = _ViewSynthesisLossFn.apply(op, tgt, src, intrinsics, snippet_weights, op.n_scales, use_exp, len(preds), *preds,
+                                     *pix_w, *src_d)
+    if not (op.pixel_terms or op.min_reprojection or op.geometry_consistency):
         return res
     k = len(res) - op.n_scales
     return tuple(res[:k]) + (list(res[k:]),)

@@ -13,7 +13,10 @@ without mean_norm_smooth + edge_mean_abs: Monodepth2's whole loss against the sa
 the last four have default configs cfg2 and cfg5.  border_padding (ViewSynthesisLoss(border_padding=True), Monodepth2's
 image borders) and monodepth2_border (Monodepth2's whole loss, as the second variant of monodepth2, with and without
 border_padding) have default configs cfg2 and cfg5 too, as has axisangle_pose (ViewSynthesisLoss(axisangle_pose=True,
-invert_sources=(0,)), Monodepth2's pose with the first source inverted, against the Euler pose).
+invert_sources=(0,)), Monodepth2's pose with the first source inverted, against the Euler pose).  geometry
+(ViewSynthesisLoss(geometry_consistency=True, self_mask=True), SC-SfMLearner's geometry consistency term and
+self-discovered mask, with the source disparities as an extra input) and geometry_nomask (the same without the
+self-mask) have default configs cfg2 and cfg5 and compare against the plain step.
 
 For each config the step (forward_backward on device tensors) is captured four times into one CUDA graph and the graph
 is replayed; the two variants alternate, and the median over the repeats is reported per step.  Prints one JSON line
@@ -24,7 +27,7 @@ min_reprojection, full_res_multiscale and full_res_min_reprojection, the added m
 relative overhead for border_padding and monodepth2_border, and the added microseconds for axisangle_pose.
 usage: python tools/time_opt_in_grads.py OUT.json {image_grads,intrinsics_grad,snippet_terms,pixel_terms,min_reprojection,
        full_res_multiscale,full_res_min_reprojection,mean_norm_smooth,mean_norm_smooth_edge,edge_mean_abs,monodepth2,
-       border_padding,monodepth2_border,axisangle_pose}
+       border_padding,monodepth2_border,axisangle_pose,geometry,geometry_nomask}
        [cfg ...]"""
 import json
 import os
@@ -55,6 +58,8 @@ LAST_COLUMN = {
     'border_padding': ('overhead', lambda p, q: round(q / p - 1.0, 4)),
     'monodepth2_border': ('overhead', lambda p, q: round(q / p - 1.0, 4)),
     'axisangle_pose': ('extra_us', lambda p, q: round(q - p, 2)),
+    'geometry': ('overhead', lambda p, q: round(q / p - 1.0, 4)),
+    'geometry_nomask': ('overhead', lambda p, q: round(q / p - 1.0, 4)),
 }
 EDGE = dict(edge_aware_smooth=True)
 MONODEPTH2 = dict(full_res_multiscale=True, min_reprojection=True, edge_aware_smooth=True)
@@ -65,11 +70,14 @@ VARIANTS = {'full_res_min_reprojection': (dict(min_reprojection=True), dict(min_
             'edge_mean_abs': (EDGE, dict(EDGE, edge_mean_abs=True)),
             'monodepth2': (MONODEPTH2, MONODEPTH2_SMOOTH),
             'monodepth2_border': (MONODEPTH2_SMOOTH, dict(MONODEPTH2_SMOOTH, border_padding=True)),
-            'axisangle_pose': ({}, dict(axisangle_pose=True, invert_sources=(0,)))}
+            'axisangle_pose': ({}, dict(axisangle_pose=True, invert_sources=(0,))),
+            'geometry': ({}, dict(geometry_consistency=True, self_mask=True)),
+            'geometry_nomask': ({}, dict(geometry_consistency=True))}
 DEFAULT_CONFIGS = {'min_reprojection': ['cfg1', 'cfg2', 'cfg5'], 'full_res_multiscale': ['cfg1', 'cfg2', 'cfg5'],
                    'full_res_min_reprojection': ['cfg2', 'cfg5'], 'mean_norm_smooth': ['cfg2', 'cfg5'],
                    'mean_norm_smooth_edge': ['cfg2', 'cfg5'], 'edge_mean_abs': ['cfg2', 'cfg5'], 'monodepth2': ['cfg2', 'cfg5'],
-                   'border_padding': ['cfg2', 'cfg5'], 'monodepth2_border': ['cfg2', 'cfg5'], 'axisangle_pose': ['cfg2', 'cfg5']}
+                   'border_padding': ['cfg2', 'cfg5'], 'monodepth2_border': ['cfg2', 'cfg5'], 'axisangle_pose': ['cfg2', 'cfg5'],
+                   'geometry': ['cfg2', 'cfg5'], 'geometry_nomask': ['cfg2', 'cfg5']}
 
 
 def card():
@@ -130,6 +138,10 @@ def main():
             gen = torch.Generator(device='cuda').manual_seed(0)
             pw = [torch.rand((c['B'], c['S'], c['H'] >> s, c['W'] >> s), device='cuda', generator=gen) for s in range(4)]
             kw = {option: dict(pixel_weights=pw)}
+        if option.startswith('geometry'):
+            # the source frames' disparities: the target's maps of the snippets in a rolled order
+            sd = [dev(np.repeat(x[np.roll(np.arange(c['B']), 1)], c['S'], axis=1)) for x in d['disps']]
+            kw = {option: dict(src_disps=sd)}
         graphs = {k: make_graph(op, args, **kw.get(k, {})) for k, op in ops.items()}
         replays = 10 if name == 'cfg5' else 200
         t = {k: [] for k in graphs}
