@@ -77,6 +77,10 @@ extern "C" {
                                          map planes of sfm_loss_geometry (B*S*sum_s h_s*w_s floats each); see "Geometry
                                          consistency" below.  Every other entry point accepts the flag and behaves exactly
                                          as without it */
+#define SFM_FLAG_VALID_MEAN 0x2000u    /* the workspace also holds the valid-pixel masks (B*S*sum_s h_s*w_s bytes) and the
+                                         pixel counts (n_scales*S*B int32) of sfm_loss_geometry_valid_mean; see "Valid-pixel
+                                         means" below.  Every other entry point accepts the flag and behaves exactly as
+                                         without it */
 #define SFM_FLAG_POSE_INVERT_SHIFT 16   /* flags bits 16..23: with SFM_FLAG_AXISANGLE_POSE, bit 16 + i inverts the
                                          transform of source i (Monodepth2's frame ids < 0) */
 #define SFM_FLAG_POSE_INVERT(i) (1u << (SFM_FLAG_POSE_INVERT_SHIFT + (i)))
@@ -632,6 +636,49 @@ typedef struct SfmGeometry {
  * (INTEGRATION.md §6). */
 int sfm_loss_geometry(const SfmDesc* desc, const SfmInputs* in, const SfmSnippetTerms* terms, const SfmGeometry* geo,
                       float* losses_out, const SfmGrads* grads, void* workspace, SfmPeer* peer, void* stream);
+
+/* Valid-pixel means (SC-SfMLearner's released compute_pairwise_loss with --with-auto-mask), sfm_loss_geometry_valid_mean.
+ * sfm_loss_geometry divides every term by B_global * h_s * w_s; the released code takes each (source, scale) term as a
+ * mean over the pixels that count (mean_on_mask), clamps the L1 difference and can drop the pixels that a static camera
+ * would explain better.  Per scale s, source i, snippet b and target pixel p, with T the target, W the warped source and
+ * S_i the unwarped source at level s:
+ *   valid          inb, the step's strict in-view flag (the geometry term's validity), and w_b != 0 when snippet weights
+ *                  are given: a padding snippet of weight 0 counts nowhere.
+ *   L1             E_c = min(|T_c - W_c|, 1); the gradient passes where |T_c - W_c| <= 1 (torch's closed interval),
+ *                  sign(0) = 0.  The SSIM part stays clip((1 - SSIM) / 2, 0, 1) on zero-padded 3x3 windows.
+ *   auto-mask      automask != 0: a = valid * [((E_0 + E_1) + E_2) / 3 < ((|T_0 - S_0| + |T_1 - S_1|) + |T_2 - S_2|) / 3]
+ *                  in fp32 (strict <; the identity difference is not clamped; W bitwise the march's warped value).
+ *                  automask == 0: a = valid.
+ *   count          n_{s,i,g} = sum over the snippets b = g mod G (w_b != 0) and pixels p of a (exact integer counts).
+ *   photometric    the terms of sfm_loss_weighted with the weight a * M * (B h_s w_s) / n in place of M (M = 1 - D_diff
+ *                  under the self-mask, else 1): L1 and SSIM are means over 3 n entries.  A (s, i, g) with 3 n <= min_count
+ *                  contributes 0.
+ *   geometry       geometry_reg * sum_{a = 1} D_diff / n per (s, i, g); 0 where n <= min_count.
+ *   reporting      as sfm_loss_geometry: [1] L1, [4] SSIM, [3] geometry, [2] smoothness, [0] total; the snippet rows
+ *                  use the group's shared count, so they still sum to the total.
+ *   gradients      of this total; a, valid and n are piecewise constant (derivative 0); through M the upstream of D_diff
+ *                  carries the factor B h w / n.  gdisps stay bitwise reproducible.
+ * Computed as prologue -> geometry forward (D_diff, a, the counts) -> normalise (the weight planes, the geometry loss)
+ * -> the march (per-pixel instances with the clamped L1) -> geometry backward -> epilogue; the counts are reset inside
+ * the step, which stays graph-capturable. */
+typedef struct SfmValidMean {
+  int32_t automask;                    /* != 0: SC-SfMLearner's auto-mask (--with-auto-mask) */
+  int32_t groups;                      /* G, 1 <= G <= B: snippet b counts in group b mod G (1: one batch-wide count) */
+  float min_count;                     /* released value 10000; >= 0 and finite */
+  int32_t reserved_;
+  uint8_t* masks[SFM_MAX_SCALES];      /* (B,S,h_s,w_s) device out: a (1 where the pair counts), or NULL */
+  int32_t* counts;                     /* (n_scales,S,G) device out: n, or NULL */
+} SfmValidMean;
+
+/* sfm_loss_geometry with valid-pixel means.  vm == NULL: exactly sfm_loss_geometry.  Otherwise desc->flags must also
+ * contain SFM_FLAG_VALID_MEAN (else SFM_E_INVALID_DESC; the workspace is sized with it).  SFM_E_INVALID_DESC: groups
+ * outside [1, B], min_count negative or not finite.  SFM_E_UNSUPPORTED: a peer (the counts are batch-global; exchanging
+ * them across ranks is not implemented), B_global != B, and everything sfm_loss_geometry refuses.
+ * SC-SfMLearner's reverse direction (INTEGRATION.md §6) is a second call on B*S one-source snippets ordered (b, i) with
+ * groups = S, so that each source frame keeps its own count as in the released per-reference call. */
+int sfm_loss_geometry_valid_mean(const SfmDesc* desc, const SfmInputs* in, const SfmSnippetTerms* terms,
+                                 const SfmGeometry* geo, const SfmValidMean* vm, float* losses_out, const SfmGrads* grads,
+                                 void* workspace, SfmPeer* peer, void* stream);
 
 #ifdef __cplusplus
 }

@@ -9,7 +9,7 @@ ROOT = os.path.dirname(HERE)
 CSRC = os.path.join(HERE, 'csrc')
 LIB = os.path.join(HERE, 'libsfmloss.so')
 SOURCES = ['api.cu', 'plan.cu', 'prep.cu', 'smooth.cu', 'fused_loss.cu', 'full_res.cu', 'mean_norm.cu', 'stage.cu', 'ingest.cu', 'eval.cu', 'comm.cu']
-HEADERS = ['common.cuh', 'kernels.h', 'ssim_march.cuh', 'min_reprojection.cuh', 'smooth_task.cuh', os.path.join(ROOT, 'include', 'sfmloss.h')]
+HEADERS = ['common.cuh', 'kernels.h', 'ssim_march.cuh', 'min_reprojection.cuh', 'geometry.cuh', 'smooth_task.cuh', os.path.join(ROOT, 'include', 'sfmloss.h')]
 
 
 def _nvcc():

@@ -180,7 +180,7 @@ int num_sms() {
 int run_loss(const SfmDesc* d, const SfmInputs* in, float* losses_out, const SfmGrads* grads, const float* gy,
              const SfmDebug* dbg, void* workspace, cudaStream_t st, const SfmPeerDev* peer = nullptr,
              const SfmImageGrads* ig = nullptr, const SfmSnippetTerms* snip = nullptr, const SfmPixelTerms* pix = nullptr,
-             const SfmMinReprojection* mr = nullptr, const SfmGeometry* geo = nullptr) {
+             const SfmMinReprojection* mr = nullptr, const SfmGeometry* geo = nullptr, const SfmValidMean* vm = nullptr) {
   int rc = sfm_validate_desc(d);
   if (rc) return rc;
   // SFM_FLAG_BORDER_PADDING runs the per-pixel instances (weights and maps NULL unless the caller passed them)
@@ -224,6 +224,7 @@ int run_loss(const SfmDesc* d, const SfmInputs* in, float* losses_out, const Sfm
   if (border) mode |= SFM_MODE_PIX | SFM_MODE_BORDER;
   const bool self_mask = geo && geo->self_mask != 0;
   if (self_mask) mode |= SFM_MODE_PIX;             // the per-pixel instances with the mask planes as weights
+  if (vm) mode |= SFM_MODE_PIX | SFM_MODE_CLAMP;   // the weight planes a M (B h w) / n, the clamped L1
   const SfmStepPlan plan = sfm_plan_step(d, mode, num_sms());
   SfmWsLayout L;
   sfm_ws_layout(d, &L);
@@ -262,10 +263,11 @@ int run_loss(const SfmDesc* d, const SfmInputs* in, float* losses_out, const Sfm
       p.pix_map[s] = pix->losses[s];
     }
     if (mr) p.pix_w[s] = (const float*)(ws + L.off_mrw[s]);   // the one-hot weights, made by the select kernel
-    if (self_mask) {
-      // M = 1 - D_diff, made by the geometry forward kernel; the maps d total / d M feed its backward kernel
+    if (self_mask || vm) {
+      // M = 1 - D_diff, made by the geometry forward kernel (valid-pixel means: a M (B h w) / n, by the normalise
+      // kernel); the maps d total / d M feed its backward kernel
       p.pix_w[s] = (const float*)(ws + L.off_geow[s]);
-      p.pix_map[s] = grads ? (float*)(ws + L.off_geomap[s]) : nullptr;
+      p.pix_map[s] = (grads && self_mask) ? (float*)(ws + L.off_geomap[s]) : nullptr;
     }
   }
   auto photometric_consts = [&](int s) {              // from the size of the photometric terms of scale s
@@ -410,13 +412,28 @@ int run_loss(const SfmDesc* d, const SfmInputs* in, float* losses_out, const Sfm
       ga.src_disps[s] = geo->src_disps[s];
       ga.diff_maps[s] = geo->diff_maps[s];
       ga.gsrc_disps[s] = grads ? geo->gsrc_disps[s] : nullptr;
-      ga.mask[s] = self_mask ? (float*)(ws + L.off_geow[s]) : nullptr;
+      ga.mask[s] = (self_mask || vm) ? (float*)(ws + L.off_geow[s]) : nullptr;
+      if (vm) {
+        ga.vm_mask[s] = (uint8_t*)(ws + L.off_vmmask[s]);
+        ga.vm_out[s] = vm->masks[s];
+      }
       ga.map[s] = self_mask ? p.pix_map[s] : nullptr;
       // gsrc_disps is accumulated with fp32 reductions
       if (ga.gsrc_disps[s]) SFM_CUDA_CHECK(cudaMemsetAsync(ga.gsrc_disps[s], 0, (size_t)d->B * d->S * plane * sizeof(float), st));
     }
     ga.fwd_begin[SFM_MAX_SCALES] = nf;
     ga.bwd_begin[SFM_MAX_SCALES] = nb;
+    if (vm) {
+      ga.vm = 1;
+      ga.automask = vm->automask != 0 ? 1 : 0;
+      ga.self_mask = self_mask ? 1 : 0;
+      ga.groups = vm->groups;
+      ga.min_count = vm->min_count;
+      ga.counts = (int*)(ws + L.off_vmcount);
+      ga.counts_out = vm->counts;
+      // the counts are reset inside the step (a memset node under graph capture)
+      SFM_CUDA_CHECK(cudaMemsetAsync(ga.counts, 0, (size_t)d->n_scales * d->S * vm->groups * sizeof(int32_t), st));
+    }
   }
   if (fr && (rc = sfm_launch_full_res_upsample(f, st))) return rc;
   rc = sfm_launch_prep(pp, &sm, (grads ? 2 : 1) + ((snip || mean_norm) ? 2 : 0), st, p.pose_flags);
@@ -605,6 +622,60 @@ extern "C" int sfm_loss_geometry(const SfmDesc* desc, const SfmInputs* in, const
   }
   return run_loss(desc, in, losses_out, grads, nullptr, nullptr, workspace, (cudaStream_t)stream, dev, nullptr,
                   snip ? terms : nullptr, nullptr, nullptr, geo);
+}
+
+extern "C" int sfm_loss_geometry_valid_mean(const SfmDesc* desc, const SfmInputs* in, const SfmSnippetTerms* terms,
+                                            const SfmGeometry* geo, const SfmValidMean* vm, float* losses_out,
+                                            const SfmGrads* grads, void* workspace, SfmPeer* peer, void* stream) {
+  if (!vm) return sfm_loss_geometry(desc, in, terms, geo, losses_out, grads, workspace, peer, stream);
+  int rc = sfm_validate_desc(desc);
+  if (rc) return rc;
+  if (!(desc->flags & SFM_FLAG_VALID_MEAN)) {
+    sfm_set_error("sfm_loss_geometry_valid_mean: desc->flags lacks SFM_FLAG_VALID_MEAN (the workspace must be sized with it)");
+    return SFM_E_INVALID_DESC;
+  }
+  if (vm->groups < 1 || vm->groups > desc->B) {
+    sfm_set_error("SfmValidMean.groups = %d outside [1, B = %d]", vm->groups, desc->B);
+    return SFM_E_INVALID_DESC;
+  }
+  if (!(vm->min_count >= 0.f) || !isfinite(vm->min_count)) {
+    sfm_set_error("SfmValidMean.min_count must be finite and >= 0");
+    return SFM_E_INVALID_DESC;
+  }
+  if (peer) {
+    sfm_set_error("unsupported: valid-pixel means with a peer (the counts are batch-global)");
+    return SFM_E_UNSUPPORTED;
+  }
+  if (desc->B_global > 0 && desc->B_global != desc->B) {
+    sfm_set_error("unsupported: valid-pixel means with B_global != B (the counts are batch-global)");
+    return SFM_E_UNSUPPORTED;
+  }
+  if (!(desc->flags & SFM_FLAG_GEOMETRY_CONSISTENCY)) {
+    sfm_set_error("sfm_loss_geometry_valid_mean: desc->flags lacks SFM_FLAG_GEOMETRY_CONSISTENCY (the workspace must be sized with it)");
+    return SFM_E_INVALID_DESC;
+  }
+  if (desc->exp_reg != 0.f) {
+    sfm_set_error("unsupported: geometry consistency together with the explainability branch (exp_reg != 0)");
+    return SFM_E_UNSUPPORTED;
+  }
+  const unsigned excl = desc->flags & (SFM_FLAG_FULL_RES_MULTISCALE | SFM_FLAG_BORDER_PADDING | SFM_FLAG_MIN_REPROJECTION);
+  if (excl) {
+    sfm_set_error("unsupported: geometry consistency together with %s",
+                  (excl & SFM_FLAG_FULL_RES_MULTISCALE) ? "SFM_FLAG_FULL_RES_MULTISCALE"
+                  : (excl & SFM_FLAG_BORDER_PADDING) ? "SFM_FLAG_BORDER_PADDING" : "SFM_FLAG_MIN_REPROJECTION");
+    return SFM_E_UNSUPPORTED;
+  }
+  if (!geo) { sfm_set_error("SfmGeometry is NULL"); return SFM_E_NULL_POINTER; }
+  for (int s = 0; s < desc->n_scales; ++s)
+    if (!geo->src_disps[s]) { sfm_set_error("SfmGeometry.src_disps[%d] is NULL", s); return SFM_E_NULL_POINTER; }
+  const bool snip = terms && (terms->weights || terms->losses);
+  if (snip && !(desc->flags & SFM_FLAG_SNIPPET_TERMS)) {
+    sfm_set_error("sfm_loss_geometry_valid_mean: desc->flags lacks SFM_FLAG_SNIPPET_TERMS (the workspace must be sized with it)");
+    return SFM_E_INVALID_DESC;
+  }
+  if (!losses_out) { sfm_set_error("losses_out is NULL"); return SFM_E_NULL_POINTER; }
+  return run_loss(desc, in, losses_out, grads, nullptr, nullptr, workspace, (cudaStream_t)stream, nullptr, nullptr,
+                  snip ? terms : nullptr, nullptr, nullptr, geo, vm);
 }
 
 extern "C" int sfm_scale_image_grads(const SfmDesc* desc, const float* gy, const SfmImageGrads* igrads, void* stream) {
@@ -816,6 +887,10 @@ extern "C" int sfm_host_ctx_create(const SfmDesc* desc, SfmHostCtx** ctx_out) {
   }
   if (desc->flags & SFM_FLAG_GEOMETRY_CONSISTENCY) {
     sfm_set_error("unsupported: the host-buffer path with SFM_FLAG_GEOMETRY_CONSISTENCY");
+    return SFM_E_UNSUPPORTED;
+  }
+  if (desc->flags & SFM_FLAG_VALID_MEAN) {
+    sfm_set_error("unsupported: the host-buffer path with SFM_FLAG_VALID_MEAN");
     return SFM_E_UNSUPPORTED;
   }
   int ndev = 0;

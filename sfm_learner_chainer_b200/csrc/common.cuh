@@ -67,6 +67,10 @@ struct SfmWsLayout {
   // 0 without the flag.  (The loss partials ride in the fp64 cells.)
   size_t off_geow[SFM_MAX_SCALES];  // float [B][S][h][w]
   size_t off_geomap[SFM_MAX_SCALES];  // float [B][S][h][w]
+  // SFM_FLAG_VALID_MEAN: the byte a of every (pixel, source) and the counts n of every (scale, source, group <= B); 0
+  // without the flag
+  size_t off_vmmask[SFM_MAX_SCALES];  // uint8 [B][S][h][w]
+  size_t off_vmcount;                 // int32 [ns][S][B]
   size_t acc_doubles;
   size_t total;
 };
@@ -203,6 +207,16 @@ static inline void sfm_ws_layout(const SfmDesc* d, SfmWsLayout* L) {
       L->off_geomap[s] = off;
       off = sfm_align_up(off + (size_t)d->B * d->S * (d->H >> s) * (d->W >> s) * sizeof(float), 256);
     }
+  }
+  for (int s = 0; s < SFM_MAX_SCALES; ++s) L->off_vmmask[s] = 0;
+  L->off_vmcount = 0;
+  if (d->flags & SFM_FLAG_VALID_MEAN) {
+    for (int s = 0; s < d->n_scales; ++s) {
+      L->off_vmmask[s] = off;
+      off = sfm_align_up(off + (size_t)d->B * d->S * (d->H >> s) * (d->W >> s), 256);
+    }
+    L->off_vmcount = off;
+    off = sfm_align_up(off + (size_t)d->n_scales * d->S * d->B * sizeof(int32_t), 256);
   }
   L->total = off;
 }

@@ -15,6 +15,14 @@
 //             chained through z' = q2 and D' into the target's gdisp (read-modify-write, one store per pixel: bitwise
 //             reproducible), the 12 dL/dP cells of (snippet, source, scale) (the march's layout, so the epilogue's pose
 //             chain and sfm_intrinsics_grad see the whole gradient) and gsrc_disps (fp32 atomics).
+// Valid-pixel means (sfm_loss_geometry_valid_mean, VM instances of their own so that the plain ones keep their code):
+//   forward   also forms the pair's validity a (in view, snippet weight != 0 and, with the auto-mask, the clamped L1 of
+//             the warped value -- the march's taps and blend -- below the unclamped L1 of the unwarped source), stores it
+//             as a byte, stores D_diff (not M) into the mask plane and adds the block's count of a into its (s, i, g)
+//             counter with one integer atomic: exact, whatever the order.  No loss partial: it needs the count.
+//   normalise behind a kernel boundary, so the counts are complete: turns the mask plane into the march's weight
+//             a M (B h w) / n (0 where 3 n <= min_count) and adds geometry_reg sum_{a} D_diff / n (0 where n <= min_count).
+//   backward  the upstream of D_diff is a (gy w_b geometry_reg / n - map (B h w) / n), with the same thresholds.
 // PDL: the epilogue reads the smoothness partials ahead of its own cudaGridDependencySynchronize(), relying on "launched
 // => the kernel before it passed its dependency wait" holding transitively back to the prologue.  Both kernels therefore
 // call cudaGridDependencySynchronize() before cudaTriggerProgrammaticLaunchCompletion().
@@ -76,6 +84,14 @@ __device__ __forceinline__ void geo_eval(const float* __restrict__ sd, const Geo
   r.rc = __fdiv_rn(1.f, c);
 }
 
+// Valid-pixel means: the factor (B h w) / n of the photometric weights of a (s, i, g) with count n, 0 where 3 n <= min_count
+__device__ __forceinline__ float vm_photometric_factor(int n, float min_count, int bhw) {
+  return (n > 0 && 3.0 * (double)n > (double)min_count) ? (float)((double)bhw / (double)n) : 0.f;
+}
+__device__ __forceinline__ int vm_count(const SfmGeoArgs& a, int s, int i, int b, int S) {
+  return __ldcg(a.counts + ((size_t)s * S + i) * a.groups + b % a.groups);
+}
+
 // Loads the 3x4 projection of (b, i, s)
 __device__ __forceinline__ void geo_proj(const SfmFusedParams& p, int b, int i, int s, float* P) {
   const float* q = p.proj + (((size_t)b * p.S + i) * p.ns + s) * 12;
@@ -83,6 +99,7 @@ __device__ __forceinline__ void geo_proj(const SfmFusedParams& p, int b, int i, 
   for (int k = 0; k < 12; ++k) P[k] = __ldg(q + k);
 }
 
+template <bool VM>
 __global__ void __launch_bounds__(kGeoThreads) sfm_geometry_forward_kernel(const __grid_constant__ SfmFusedParams p,
                                                                            const __grid_constant__ SfmGeoArgs a) {
   __shared__ float s_part[kGeoWarps];
@@ -97,6 +114,7 @@ __global__ void __launch_bounds__(kGeoThreads) sfm_geometry_forward_kernel(const
   cudaGridDependencySynchronize();
   cudaTriggerProgrammaticLaunchCompletion();
   float diff = 0.f;
+  bool on = false;                                 // VM: the pair counts
   if (act) {
     float X, Y, Z, dsc;
     geo_camera(p, s, b, pix, w, X, Y, Z, dsc);
@@ -112,7 +130,37 @@ __global__ void __launch_bounds__(kGeoThreads) sfm_geometry_forward_kernel(const
     }
     const size_t o = (size_t)bi * plane + pix;
     if (a.diff_maps[s]) a.diff_maps[s][o] = diff;
-    if (a.mask[s]) a.mask[s][o] = __fsub_rn(1.f, diff);
+    if constexpr (VM) {
+      on = f.inb && !(p.snip_w && __ldg(p.snip_w + b) == 0.f);
+      if (on && a.automask) {
+        // the warped value exactly as the march forms it, against the unwarped source
+        const float* img = p.src_pl[s] + (size_t)bi * 3 * plane;
+        const float* tg = p.tgt_pl[s] + (size_t)b * 3 * plane + pix;
+        Taps t;
+        gather_taps(img, g, f, t);
+        const float w1 = __fmul_rn(f.wa, f.wc), w2 = __fmul_rn(f.wb, f.wc);
+        const float w3 = __fmul_rn(f.wa, f.wd), w4 = __fmul_rn(f.wb, f.wd);
+        float e = 0.f, e_id = 0.f;
+#pragma unroll
+        for (int c = 0; c < 3; ++c) {
+          const float W = sfm_blend(w1, w2, w3, w4, t.a[c], t.b[c], t.c[c], t.d[c]);
+          const float T = __ldg(tg + (size_t)c * plane), Sc = __ldg(img + (size_t)c * plane + pix);
+          e = __fadd_rn(e, l1_abs<true>(__fsub_rn(W, T)));
+          e_id = __fadd_rn(e_id, fabsf(__fsub_rn(T, Sc)));
+        }
+        on = __fdiv_rn(e, 3.f) < __fdiv_rn(e_id, 3.f);
+      }
+      a.mask[s][o] = diff;                         // D_diff: the normalise kernel makes the weight of it
+      a.vm_mask[s][o] = on ? 1 : 0;
+      if (a.vm_out[s]) a.vm_out[s][o] = on ? 1 : 0;
+    } else if (a.mask[s]) {
+      a.mask[s][o] = __fsub_rn(1.f, diff);
+    }
+  }
+  if constexpr (VM) {
+    const int n = __syncthreads_count(on);
+    if (threadIdx.x == 0 && n) atomicAdd(a.counts + ((size_t)s * S + i) * a.groups + b % a.groups, n);
+    return;
   }
   // loss partial: warp sums, then the block's warps in order, one fp64 atomic per block
   const float ws = sfm_warp_sum(diff);
@@ -129,6 +177,45 @@ __global__ void __launch_bounds__(kGeoThreads) sfm_geometry_forward_kernel(const
   }
 }
 
+// Valid-pixel means, behind the forward kernel (same grid): the weight planes of the march and the geometry loss partials
+__global__ void __launch_bounds__(kGeoThreads) sfm_valid_mean_normalise_kernel(const __grid_constant__ SfmFusedParams p,
+                                                                               const __grid_constant__ SfmGeoArgs a) {
+  __shared__ float s_part[kGeoWarps];
+  const int s = geo_scale(a.fwd_begin, p.ns);
+  const int plane = p.h[s] * p.w[s], S = p.S;
+  const int per = (plane + kGeoThreads - 1) / kGeoThreads;
+  const int rel = (int)blockIdx.x - a.fwd_begin[s];
+  const int bi = rel / per, b = bi / S, i = bi - b * S;
+  const int pix = (rel - bi * per) * kGeoThreads + (int)threadIdx.x;
+  // the forward kernel's counts are complete
+  cudaGridDependencySynchronize();
+  cudaTriggerProgrammaticLaunchCompletion();
+  const int n = vm_count(a, s, i, b, S);
+  const float fph = vm_photometric_factor(n, a.min_count, p.B * plane);
+  float dsum = 0.f;
+  if (pix < plane) {
+    const size_t o = (size_t)bi * plane + pix;
+    const float dd = a.mask[s][o];
+    const bool on = a.vm_mask[s][o] != 0;
+    const float M = a.self_mask ? __fsub_rn(1.f, dd) : 1.f;
+    a.mask[s][o] = on ? __fmul_rn(M, fph) : 0.f;
+    dsum = on ? dd : 0.f;
+  }
+  const float ws = sfm_warp_sum(dsum);
+  if ((threadIdx.x & 31) == 0) s_part[threadIdx.x >> 5] = ws;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    float t = 0.f;
+#pragma unroll
+    for (int k = 0; k < kGeoWarps; ++k) t += s_part[k];
+    if (t != 0.f && (double)n > (double)a.min_count)
+      atomicAdd(p.acc + (p.snip_cell0 ? p.snip_cell0 + 4 * (size_t)b : 0) + 2, (double)t * (double)a.geometry_reg / (double)n);
+  }
+  if (blockIdx.x == 0 && a.counts_out)
+    for (int k = threadIdx.x; k < p.ns * S * a.groups; k += kGeoThreads) a.counts_out[k] = __ldcg(a.counts + k);
+}
+
+template <bool VM>
 __global__ void __launch_bounds__(kGeoThreads) sfm_geometry_backward_kernel(const __grid_constant__ SfmFusedParams p,
                                                                             const __grid_constant__ SfmGeoArgs a) {
   __shared__ float s_red[kGeoWarps][12];
@@ -145,7 +232,7 @@ __global__ void __launch_bounds__(kGeoThreads) sfm_geometry_backward_kernel(cons
   cudaTriggerProgrammaticLaunchCompletion();
   float gyv = p.gy ? __ldg(p.gy) : 1.f;
   if (p.snip_w) gyv *= __ldg(p.snip_w + b);
-  const float wgeo = gyv * a.geometry_reg * p.inv_n1[s];
+  const float wgeo = VM ? gyv * a.geometry_reg : gyv * a.geometry_reg * p.inv_n1[s];   // VM: / n per source below
   float X = 0.f, Y = 0.f, Z = 0.f, dsc = 0.f;
   if (act) geo_camera(p, s, b, pix, w, X, Y, Z, dsc);
   const Geo g = make_geo(p, s);
@@ -157,14 +244,20 @@ __global__ void __launch_bounds__(kGeoThreads) sfm_geometry_backward_kernel(cons
     float acc[12];
 #pragma unroll
     for (int k = 0; k < 12; ++k) acc[k] = 0.f;
+    float wg = wgeo, fph = 1.f;
+    if constexpr (VM) {
+      const int n = vm_count(a, s, i, b, S);
+      wg = (double)n > (double)a.min_count ? __fdiv_rn(wgeo, (float)n) : 0.f;
+      fph = vm_photometric_factor(n, a.min_count, p.B * plane);
+    }
     if (act) {
       PairFwd f;
       pair_project(P, X, Y, Z, g, f);
-      if (f.inb) {
+      if (f.inb && (!VM || a.vm_mask[s][bi * plane + pix])) {
         GeoRec r;
         geo_eval(a.src_disps[s] + bi * plane, g, f, r);
-        float up = wgeo;
-        if (a.map[s]) up -= __ldcg(a.map[s] + bi * plane + pix);
+        float up = wg;
+        if (a.map[s]) up -= VM ? __ldcg(a.map[s] + bi * plane + pix) * fph : __ldcg(a.map[s] + bi * plane + pix);
         // clip: the gradient passes on the closed interval [0, 1]; sign(0) = 0
         const bool pass = (r.ratio >= 0.f) && (r.ratio <= 1.f);
         const float sa = (r.a > 0.f) ? 1.f : (r.a < 0.f) ? -1.f : 0.f;

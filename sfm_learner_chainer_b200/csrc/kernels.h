@@ -184,14 +184,15 @@ constexpr int SFM_SSIM_REG_MIN_WARPS = 8;
 constexpr int SFM_SSIM_IMG_MIN_WARPS = 10;
 
 // Launch plan of one fused step (plan.cu, the whole launch policy).  The marching kernel instance is
-// sfm_l1_march_kernel<exp, grad, accum, debug, raw, img, snip, pix, border> or
-// sfm_ssim_march_kernel<grad, accum, debug, raw, nw, srec, img, snip, pix, border>.
+// sfm_l1_march_kernel<exp, grad, accum, debug, raw, img, snip, pix, border, clamp> or
+// sfm_ssim_march_kernel<grad, accum, debug, raw, nw, srec, img, snip, pix, border, clamp>.
 struct SfmStepPlan {
   bool ssim;                           // kernel family
   bool exp, grad, accum, debug, raw;   // accum: a smoothness kernel has initialised gdisp
   bool img;                            // image gradients (grad, !debug; SSIM: nw = 1 with shared-memory records)
   bool pix;                            // per-pixel terms (!debug, !img; SSIM: nw = 1 with shared-memory records)
   bool border;                         // SFM_FLAG_BORDER_PADDING (pix, !exp): border-clamped sampler, reflection-padded SSIM
+  bool clamp;                          // valid-pixel means (pix, !border, !exp): the L1 difference clamped to [0, 1]
   bool minrep;                         // minimum reprojection (pix): a forward per-pixel march with the task table pre_tasks
                                        // and the select kernel run ahead of the march of this plan
   SfmTaskTable pre_tasks;
@@ -204,7 +205,7 @@ struct SfmStepPlan {
 };
 // mode bits of the planner
 enum { SFM_MODE_EXP = 1, SFM_MODE_SSIM = 2, SFM_MODE_GRAD = 4, SFM_MODE_DEBUG = 8, SFM_MODE_SMOOTH = 16, SFM_MODE_IMG = 32,
-       SFM_MODE_PIX = 64, SFM_MODE_MINREP = 128, SFM_MODE_BORDER = 256 };
+       SFM_MODE_PIX = 64, SFM_MODE_MINREP = 128, SFM_MODE_BORDER = 256, SFM_MODE_CLAMP = 512 };
 SfmStepPlan sfm_plan_step(const SfmDesc* d, int mode, int num_sms);
 int sfm_plan_band(const SfmDesc* d);
 // Minimum reprojection (sfm_loss_min_reprojection): the planes p.pix_w[s] are written by the forward march and turned
@@ -252,6 +253,15 @@ struct SfmGeoArgs {
   float geometry_reg;
   int fwd_begin[SFM_MAX_SCALES + 1];
   int bwd_begin[SFM_MAX_SCALES + 1];
+  // valid-pixel means (sfm_loss_geometry_valid_mean; vm == 0 otherwise): the forward kernel writes D_diff into `mask`, the
+  // byte a into vm_mask (and vm_out) and counts it into counts[(s S + i) G + b mod G]; the normalise kernel, behind it,
+  // turns `mask` into the march's weights a M (B h w) / n and adds the geometry loss; the backward kernel reads a and n
+  int vm, automask, self_mask, groups;
+  float min_count;
+  uint8_t* vm_mask[SFM_MAX_SCALES];     // workspace (B,S,h,w)
+  uint8_t* vm_out[SFM_MAX_SCALES];      // the caller's masks, nullptr: not wanted
+  int* counts;                          // workspace (ns,S,G), reset by the step
+  int* counts_out;                      // the caller's copy, nullptr: not wanted
 };
 // mr: minimum reprojection; geo: geometry consistency (at most one of them)
 int sfm_launch_fused(SfmFusedParams& p, const SfmStepPlan& plan, cudaStream_t stream, const SfmMinRepArgs* mr = nullptr,

@@ -186,6 +186,7 @@ SfmStepPlan sfm_plan_step(const SfmDesc* d, int mode, int num_sms) {
   q.pix = !q.debug && !q.img && (mode & SFM_MODE_PIX) != 0;
   q.minrep = q.pix && (mode & SFM_MODE_MINREP) != 0;
   q.border = q.pix && !q.exp && (mode & SFM_MODE_BORDER) != 0;
+  q.clamp = q.pix && !q.exp && !q.border && (mode & SFM_MODE_CLAMP) != 0;
   // under SFM_FLAG_FULL_RES_MULTISCALE the upsample kernel activates the raw scales >= 1 and the march sees bit 0 only
   q.raw = (sfm_full_res(d) ? d->raw_disp_scales & 1u : d->raw_disp_scales) != 0;
   const bool smooth = (mode & SFM_MODE_SMOOTH) != 0;

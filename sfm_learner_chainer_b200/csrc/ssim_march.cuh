@@ -113,13 +113,15 @@ enum RowStages {
 // feed only windows outside the image.  The adjoint of the padding folds the window terms of column 0 / w-1 twice into
 // column 1 / w-2 (stage D: 2 up + self + down, up + self + 2 down) and those of row 0 / h-1 into row 1 / h-2 (stage E),
 // whose product is the 2-D adjoint; both test the image column / row, so a halo or a task boundary anywhere is fine.
+// CLAMP (PIX, no BORDER): valid-pixel means, the L1 part's difference clamped to [0, 1] (l1_abs); SSIM is unchanged.
 template <bool GRAD, bool ACCUM, bool DEBUG, bool RAW, int NW, bool SREC = true, bool IMG = false, bool SNIP = false,
-          bool PIX = false, bool BORDER = false>
+          bool PIX = false, bool BORDER = false, bool CLAMP = false>
 __global__ void __launch_bounds__(32 * NW, (IMG ? SFM_SSIM_IMG_MIN_WARPS : SREC ? SFM_SSIM_MIN_WARPS : SFM_SSIM_REG_MIN_WARPS) / NW)
 sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
   static_assert(!IMG || (GRAD && NW == 1 && SREC), "image gradients: GRAD, one warp per CTA, shared-memory records");
   static_assert(!PIX || (NW == 1 && SREC && !IMG && !DEBUG), "per-pixel terms: one warp per CTA, shared-memory records");
   static_assert(!BORDER || PIX, "border padding: per-pixel instances");
+  static_assert(!CLAMP || (PIX && !BORDER), "clamped L1: per-pixel instances without border padding");
   constexpr int NREC = IMG ? 21 : PIX ? 19 : 18;        // fields of a forward record
   constexpr int NG = IMG ? 4 : 3;                       // gradient fields: g_a, g_s, g_c (, h_a)
   __shared__ float4 sP_all[NW][3];
@@ -324,7 +326,7 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
                               : (P0 == 0.f) && (P1 == 0.f) && (P2 == 0.f);         // true outside the image / view
         const bool own = col_own && (r >= t.y0) && (r < t.y1);
         if (PIX) {
-          e_cur = m ? 0.f : (fabsf(P0 - T[0]) + fabsf(P1 - T[1]) + fabsf(P2 - T[2]));
+          e_cur = m ? 0.f : (l1_abs<CLAMP>(P0 - T[0]) + l1_abs<CLAMP>(P1 - T[1]) + l1_abs<CLAMP>(P2 - T[2]));
           pix_part += own ? e_cur * m_cur : 0.f;
         } else {
           pix_part += (own && !m) ? (fabsf(P0 - T[0]) + fabsf(P1 - T[1]) + fabsf(P2 - T[2])) : 0.f;
@@ -492,7 +494,7 @@ sfm_ssim_march_kernel(const __grid_constant__ SfmFusedParams p) {
           }
 #pragma unroll
           for (int c = 0; c < 3; ++c) {
-            const float gl1 = mf ? 0.f : sfm_sign_times(rb.P[c] - rb.T[c], wpf);
+            const float gl1 = mf ? 0.f : l1_sign_times<CLAMP>(rb.P[c] - rb.T[c], wpf);
             gP[c] = do_f ? gs3[c] + gl1 : 0.f;
             if (IMG) gT[c] = do_f ? gt3[c] - gl1 : 0.f;
           }

@@ -1,6 +1,7 @@
 """Host-side operators of the view-synthesis loss path (thin: argument checks, output allocation and
 one C-ABI call each).  Names and argument meaning follow the reference."""
 import ctypes as C
+import math
 
 from . import device as D
 from . import lib as L
@@ -79,15 +80,39 @@ class ViewSynthesisLoss(object):
     self_mask: the photometric terms of every (pixel, source) are weighted by M = 1 - D_diff, with the gradient through
     M (SC-SfMLearner's self-discovered mask).  See sfm_loss_geometry in include/sfmloss.h.  Not with exp_reg,
     image_grads, pixel_terms, min_reprojection, full_res_multiscale, border_padding or debug dumps.
+    valid_mean: SC-SfMLearner's means over the valid pixels (its released compute_pairwise_loss / mean_on_mask; needs
+    geometry_consistency): each (scale, source) term is a mean over the pairs that count instead of over B_global h w,
+    and the L1 difference is clamped to 1.  valid_automask: a pair counts only where the clamped L1 of the warped source
+    is below the L1 of the unwarped source (--with-auto-mask); else every in-view pair counts.  valid_min_count: a term
+    whose count (3 n for the photometric terms, n for the geometry term) is <= it contributes 0 (released value 10000).
+    count_groups: G, snippet b counts in group b mod G (1: one batch-wide count per source and scale; S for the reverse
+    direction of INTEGRATION.md §6).  forward and forward_backward then also return `valid_masks` (list of n_scales
+    (B,S,h,w) uint8, 1 where the pair counts) and `valid_counts` ((n_scales,S,G) int32), appended to the forward's tuple
+    after the D_diff maps / in the grads dict.  Not with a peer or B_global != B.  See sfm_loss_geometry_valid_mean in
+    include/sfmloss.h.
     """
 
     def __init__(self, smooth_reg=0.0, exp_reg=0.0, ssim_rate=0.0, n_scales=N_SCALES, B_global=None,
                  raw_disp_scales=0, raw_pose=False, edge_aware_smooth=False, image_grads=False,
                  intrinsics_grad=False, snippet_terms=False, pixel_terms=False, min_reprojection=False, automask=True,
                  full_res_multiscale=False, mean_norm_smooth=False, edge_mean_abs=False, border_padding=False,
-                 axisangle_pose=False, invert_sources=(), geometry_consistency=False, geometry_reg=0.5, self_mask=False):
+                 axisangle_pose=False, invert_sources=(), geometry_consistency=False, geometry_reg=0.5, self_mask=False,
+                 valid_mean=False, valid_automask=True, valid_min_count=10000.0, count_groups=1):
         if self_mask and not geometry_consistency:
             raise ValueError('self_mask needs geometry_consistency')
+        if valid_mean:
+            if not geometry_consistency:
+                raise ValueError('valid_mean needs geometry_consistency')
+            if B_global is not None:
+                raise ValueError('valid_mean is not supported with B_global (the counts are batch-global)')
+            if not math.isfinite(float(valid_min_count)) or float(valid_min_count) < 0.0:
+                raise ValueError('valid_min_count must be finite and >= 0, got %r' % (valid_min_count,))
+            if int(count_groups) < 1:
+                raise ValueError('count_groups must be >= 1, got %r' % (count_groups,))
+        self.valid_mean = bool(valid_mean)
+        self.valid_automask = bool(valid_automask)
+        self.valid_min_count = float(valid_min_count)
+        self.count_groups = int(count_groups)
         if geometry_consistency:
             for name, on in (('image_grads', image_grads), ('pixel_terms', pixel_terms),
                              ('min_reprojection', min_reprojection), ('full_res_multiscale', full_res_multiscale),
@@ -177,6 +202,8 @@ class ViewSynthesisLoss(object):
             flags |= L.SFM_FLAG_BORDER_PADDING
         if self.geometry_consistency:
             flags |= L.SFM_FLAG_GEOMETRY_CONSISTENCY
+        if self.valid_mean:
+            flags |= L.SFM_FLAG_VALID_MEAN
         if self.axisangle_pose:
             flags |= L.SFM_FLAG_AXISANGLE_POSE
             for i in self.invert_sources:
@@ -190,7 +217,8 @@ class ViewSynthesisLoss(object):
         # the image-gradient, snippet-terms, min-reprojection, full-resolution and mean-normalisation flags size the
         # workspace; the per-call flags (tables, reused pyramid) do not
         sizing = (L.SFM_FLAG_IMAGE_GRADS | L.SFM_FLAG_SNIPPET_TERMS | L.SFM_FLAG_MIN_REPROJECTION
-                  | L.SFM_FLAG_FULL_RES_MULTISCALE | L.SFM_FLAG_MEAN_NORM_SMOOTH | L.SFM_FLAG_GEOMETRY_CONSISTENCY)
+                  | L.SFM_FLAG_FULL_RES_MULTISCALE | L.SFM_FLAG_MEAN_NORM_SMOOTH | L.SFM_FLAG_GEOMETRY_CONSISTENCY
+                  | L.SFM_FLAG_VALID_MEAN)
         key = (desc.B, desc.S, desc.H, desc.W, desc.n_scales, desc.flags & sizing,
                str(getattr(like, 'device', '')))
         ws = self._ws.get(key)
@@ -346,6 +374,33 @@ class ViewSynthesisLoss(object):
                 ge.gsrc_disps[s] = D.ptr(gsd[s])
         return ge, diff, gsd
 
+    def _valid_mean(self, desc, tgt):
+        """-> (SfmValidMean or None, masks (list of n_scales (B,S,h_s,w_s) uint8), counts (n_scales,S,G) int32)."""
+        if not self.valid_mean:
+            return None, None, None
+        if not 1 <= self.count_groups <= desc.B:
+            raise ValueError('count_groups = %d must lie in [1, B = %d]' % (self.count_groups, desc.B))
+        vm = L.SfmValidMean()
+        vm.automask = 1 if self.valid_automask else 0
+        vm.groups = self.count_groups
+        vm.min_count = self.valid_min_count
+        masks = []
+        for s in range(self.n_scales):
+            masks.append(D.empty(tgt, (desc.B, desc.S, desc.H >> s, desc.W >> s), 'uint8'))
+            vm.masks[s] = D.ptr(masks[s])
+        counts = D.empty(tgt, (self.n_scales, desc.S, self.count_groups), 'int32')
+        vm.counts = D.ptr(counts)
+        return vm, masks, counts
+
+    def _run_geometry(self, desc, inp, terms, ge, vm, losses, grads, tgt, peer):
+        args = (C.byref(desc), C.byref(inp), C.byref(terms) if terms else None, C.byref(ge))
+        tail = (_vp(losses), C.byref(grads) if grads is not None else None, self._workspace(desc, tgt), peer,
+                C.c_void_p(D.current_stream(tgt)))
+        if vm is None:
+            L.check(self._lib.sfm_loss_geometry(*args, *tail))
+        else:
+            L.check(self._lib.sfm_loss_geometry_valid_mean(*args, C.byref(vm), *tail))
+
     # ---- operators
     def forward(self, tgt, src, intrinsics, disps, poses, logits=None, proj=None, kinv=None, debug=False,
                 snippet_weights=None, pixel_weights=None, src_disps=None):
@@ -355,7 +410,7 @@ class ViewSynthesisLoss(object):
         element: (losses, maps) or (losses, snippet losses, maps).
         With the operator's min_reprojection the selection maps (list of n_scales (B,h,w) int8) are appended likewise.
         With the operator's geometry_consistency: src_disps (list of n_scales (B,S,h,w)) is required and the D_diff maps
-        (list of n_scales (B,S,h,w)) are appended likewise."""
+        (list of n_scales (B,S,h,w)) are appended likewise; with valid_mean then also the masks and the counts."""
         if debug and (self.snippet_terms or self.pixel_terms or self.min_reprojection or self.border_padding
                       or self.geometry_consistency):
             raise ValueError('debug dumps are not available on an operator with snippet_terms, pixel_terms, min_reprojection, '
@@ -369,10 +424,9 @@ class ViewSynthesisLoss(object):
             if pixel_weights is not None:
                 raise ValueError('pixel_weights needs ViewSynthesisLoss(pixel_terms=True)')
             ge, diff, _ = self._geometry(desc, tgt, src_disps, False)
-            L.check(self._lib.sfm_loss_geometry(C.byref(desc), C.byref(inp), C.byref(terms) if terms else None,
-                                                C.byref(ge), _vp(losses), None, self._workspace(desc, tgt), None,
-                                                C.c_void_p(D.current_stream(tgt))))
-            return (losses,) + ((rows,) if self.snippet_terms else ()) + (diff,)
+            vm, masks, counts = self._valid_mean(desc, tgt)
+            self._run_geometry(desc, inp, terms, ge, vm, losses, None, tgt, None)
+            return (losses,) + ((rows,) if self.snippet_terms else ()) + (diff,) + ((masks, counts) if vm else ())
         if self.min_reprojection:
             terms, rows = self._snippet_terms(desc, tgt, snippet_weights)
             if pixel_weights is not None:
@@ -461,7 +515,7 @@ class ViewSynthesisLoss(object):
         shard's, under peer).
         With the operator's geometry_consistency: src_disps (list of n_scales (B,S,h,w) activated source disparities) is
         required, and the dict also holds geometry_diff (the D_diff maps, this shard's under peer) and gsrc_disps (the
-        gradient w.r.t. src_disps)."""
+        gradient w.r.t. src_disps); with valid_mean also valid_masks and valid_counts."""
         if src_disps is not None and not self.geometry_consistency:
             raise ValueError('src_disps needs ViewSynthesisLoss(geometry_consistency=True)')
         want_k = self._want_intrinsics_grad(intrinsics_grad, proj, kinv)
@@ -479,10 +533,12 @@ class ViewSynthesisLoss(object):
             out['pixel_losses'] = maps
         if self.geometry_consistency:
             ge, out['geometry_diff'], out['gsrc_disps'] = self._geometry(desc, tgt, src_disps, True)
-            L.check(self._lib.sfm_loss_geometry(C.byref(desc), C.byref(inp), C.byref(terms) if terms else None,
-                                                C.byref(ge), _vp(losses), C.byref(g), self._workspace(desc, tgt),
-                                                peer.handle if peer is not None else None,
-                                                C.c_void_p(D.current_stream(tgt))))
+            vm, masks, counts = self._valid_mean(desc, tgt)
+            if vm is not None:
+                if peer is not None:
+                    raise ValueError('valid_mean is not supported with a peer (the counts are batch-global)')
+                out['valid_masks'], out['valid_counts'] = masks, counts
+            self._run_geometry(desc, inp, terms, ge, vm, losses, g, tgt, peer.handle if peer is not None else None)
             self._intrinsics_grad(desc, inp, tgt, out, want_k)
             if self._ev_pyramid is not None:
                 self._ev_loss = D.record_event(tgt)

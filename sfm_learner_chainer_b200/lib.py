@@ -21,6 +21,7 @@ SFM_FLAG_EDGE_MEAN_ABS = 0x200
 SFM_FLAG_BORDER_PADDING = 0x400
 SFM_FLAG_AXISANGLE_POSE = 0x800
 SFM_FLAG_GEOMETRY_CONSISTENCY = 0x1000
+SFM_FLAG_VALID_MEAN = 0x2000
 SFM_FLAG_POSE_INVERT_SHIFT = 16          # flags bit 16 + i: invert the transform of source i
 
 SFM_E_INVALID_DESC = -1
@@ -74,6 +75,11 @@ class SfmGeometry(C.Structure):
                 ('diff_maps', _vp * SFM_MAX_SCALES), ('geometry_reg', C.c_float), ('self_mask', C.c_int32)]
 
 
+class SfmValidMean(C.Structure):
+    _fields_ = [('automask', C.c_int32), ('groups', C.c_int32), ('min_count', C.c_float), ('reserved_', C.c_int32),
+                ('masks', _vp * SFM_MAX_SCALES), ('counts', _vp)]
+
+
 class SfmAugment(C.Structure):
     _fields_ = [('out_h', C.c_int32), ('out_w', C.c_int32), ('off_y', C.c_int32), ('off_x', C.c_int32),
                 ('flip', C.c_int32), ('reserved_', C.c_int32), ('x_scaling', C.c_double), ('y_scaling', C.c_double)]
@@ -92,6 +98,7 @@ _ST = C.POINTER(SfmSnippetTerms)
 _PT = C.POINTER(SfmPixelTerms)
 _MR = C.POINTER(SfmMinReprojection)
 _GE = C.POINTER(SfmGeometry)
+_VM = C.POINTER(SfmValidMean)
 SYMBOLS = {
     'sfm_version': (_i, []),
     'sfm_last_error': (C.c_char_p, []),
@@ -139,6 +146,7 @@ SYMBOLS = {
     'sfm_loss_weighted': (_i, [_D, _I, _ST, _PT, _vp, _G, _IG, _vp, _vp, _vp]),
     'sfm_loss_min_reprojection': (_i, [_D, _I, _ST, _MR, _vp, _G, _vp, _vp, _vp]),
     'sfm_loss_geometry': (_i, [_D, _I, _ST, _GE, _vp, _G, _vp, _vp, _vp]),
+    'sfm_loss_geometry_valid_mean': (_i, [_D, _I, _ST, _GE, _VM, _vp, _G, _vp, _vp, _vp]),
 }
 
 _lib = None

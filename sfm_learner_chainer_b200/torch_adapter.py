@@ -50,6 +50,9 @@ class _ViewSynthesisLossFn(torch.autograd.Function):
         outs += ctx.maps
         outs += grads.get('selection') or []      # min_reprojection: the selection maps, non-differentiable
         outs += grads.get('geometry_diff') or []  # geometry_consistency: the D_diff maps
+        if 'valid_counts' in grads:               # valid_mean: the masks and the counts, non-differentiable
+            outs += grads['valid_masks']
+            outs.append(grads['valid_counts'])
         ctx.gsrc_d = grads.get('gsrc_disps') or []
         ctx.want_sd = [ctx.needs_input_grad[8 + n_pred + s] for s in range(len(src_d))]
         ctx.mark_non_differentiable(*outs)
@@ -96,6 +99,8 @@ def view_synthesis_loss(op, tgt, src, intrinsics, pred_disps, pred_poses, pred_m
     With op.geometry_consistency: src_disps (list of n_scales (B,S,h,w) tensors, the activated disparity of every source
     frame, e.g. DispNet run on the source frames) is required and receives its gradient through autograd; the D_diff maps
     (list of n_scales (B,S,h,w) tensors, not differentiable) are appended to the returned tuple.
+    With op.valid_mean the valid-pixel masks (list of n_scales (B,S,h,w) uint8 tensors) and the counts ((n_scales,S,G)
+    int32 tensor) follow the D_diff maps; neither is differentiable.
     """
     assert isinstance(op, ViewSynthesisLoss)
     if snippet_weights is not None and not op.snippet_terms:
@@ -122,5 +127,8 @@ def view_synthesis_loss(op, tgt, src, intrinsics, pred_disps, pred_poses, pred_m
                                      *pix_w, *src_d)
     if not (op.pixel_terms or op.min_reprojection or op.geometry_consistency):
         return res
+    if op.valid_mean:
+        k = len(res) - 2 * op.n_scales - 1
+        return tuple(res[:k]) + (list(res[k:k + op.n_scales]), list(res[k + op.n_scales:-1]), res[-1])
     k = len(res) - op.n_scales
     return tuple(res[:k]) + (list(res[k:]),)

@@ -16,7 +16,10 @@ border_padding) have default configs cfg2 and cfg5 too, as has axisangle_pose (V
 invert_sources=(0,)), Monodepth2's pose with the first source inverted, against the Euler pose).  geometry
 (ViewSynthesisLoss(geometry_consistency=True, self_mask=True), SC-SfMLearner's geometry consistency term and
 self-discovered mask, with the source disparities as an extra input) and geometry_nomask (the same without the
-self-mask) have default configs cfg2 and cfg5 and compare against the plain step.
+self-mask) have default configs cfg2 and cfg5 and compare against the plain step.  valid_mean
+(ViewSynthesisLoss(geometry_consistency=True, self_mask=True, valid_mean=True), SC-SfMLearner's valid-pixel means with
+its auto-mask) and valid_mean_noauto (the same without the auto-mask) have default configs cfg2 and cfg5 and compare
+against the geometry step with the self-mask; the plain step is timed alongside as a third column.
 
 For each config the step (forward_backward on device tensors) is captured four times into one CUDA graph and the graph
 is replayed; the two variants alternate, and the median over the repeats is reported per step.  Prints one JSON line
@@ -27,7 +30,7 @@ min_reprojection, full_res_multiscale and full_res_min_reprojection, the added m
 relative overhead for border_padding and monodepth2_border, and the added microseconds for axisangle_pose.
 usage: python tools/time_opt_in_grads.py OUT.json {image_grads,intrinsics_grad,snippet_terms,pixel_terms,min_reprojection,
        full_res_multiscale,full_res_min_reprojection,mean_norm_smooth,mean_norm_smooth_edge,edge_mean_abs,monodepth2,
-       border_padding,monodepth2_border,axisangle_pose,geometry,geometry_nomask}
+       border_padding,monodepth2_border,axisangle_pose,geometry,geometry_nomask,valid_mean,valid_mean_noauto}
        [cfg ...]"""
 import json
 import os
@@ -60,7 +63,10 @@ LAST_COLUMN = {
     'axisangle_pose': ('extra_us', lambda p, q: round(q - p, 2)),
     'geometry': ('overhead', lambda p, q: round(q / p - 1.0, 4)),
     'geometry_nomask': ('overhead', lambda p, q: round(q / p - 1.0, 4)),
+    'valid_mean': ('extra_us', lambda p, q: round(q - p, 2)),
+    'valid_mean_noauto': ('extra_us', lambda p, q: round(q - p, 2)),
 }
+GEOMETRY = dict(geometry_consistency=True, self_mask=True)
 EDGE = dict(edge_aware_smooth=True)
 MONODEPTH2 = dict(full_res_multiscale=True, min_reprojection=True, edge_aware_smooth=True)
 MONODEPTH2_SMOOTH = dict(MONODEPTH2, mean_norm_smooth=True, edge_mean_abs=True)
@@ -72,12 +78,17 @@ VARIANTS = {'full_res_min_reprojection': (dict(min_reprojection=True), dict(min_
             'monodepth2_border': (MONODEPTH2_SMOOTH, dict(MONODEPTH2_SMOOTH, border_padding=True)),
             'axisangle_pose': ({}, dict(axisangle_pose=True, invert_sources=(0,))),
             'geometry': ({}, dict(geometry_consistency=True, self_mask=True)),
-            'geometry_nomask': ({}, dict(geometry_consistency=True))}
+            'geometry_nomask': ({}, dict(geometry_consistency=True)),
+            'valid_mean': (GEOMETRY, dict(GEOMETRY, valid_mean=True)),
+            'valid_mean_noauto': (GEOMETRY, dict(GEOMETRY, valid_mean=True, valid_automask=False))}
+# options whose baseline is itself an option: the plain step is timed as a third column
+THIRD = {'valid_mean', 'valid_mean_noauto'}
 DEFAULT_CONFIGS = {'min_reprojection': ['cfg1', 'cfg2', 'cfg5'], 'full_res_multiscale': ['cfg1', 'cfg2', 'cfg5'],
                    'full_res_min_reprojection': ['cfg2', 'cfg5'], 'mean_norm_smooth': ['cfg2', 'cfg5'],
                    'mean_norm_smooth_edge': ['cfg2', 'cfg5'], 'edge_mean_abs': ['cfg2', 'cfg5'], 'monodepth2': ['cfg2', 'cfg5'],
                    'border_padding': ['cfg2', 'cfg5'], 'monodepth2_border': ['cfg2', 'cfg5'], 'axisangle_pose': ['cfg2', 'cfg5'],
-                   'geometry': ['cfg2', 'cfg5'], 'geometry_nomask': ['cfg2', 'cfg5']}
+                   'geometry': ['cfg2', 'cfg5'], 'geometry_nomask': ['cfg2', 'cfg5'], 'valid_mean': ['cfg2', 'cfg5'],
+                   'valid_mean_noauto': ['cfg2', 'cfg5']}
 
 
 def card():
@@ -129,6 +140,8 @@ def main():
         # the operators own the workspaces the graphs write: they live as long as the graphs
         base_kw, option_kw = VARIANTS.get(option, ({}, {option: True}))
         ops = {'plain': ViewSynthesisLoss(**base_kw, **flags), option: ViewSynthesisLoss(**option_kw, **flags)}
+        if option in THIRD:
+            ops['step'] = ViewSynthesisLoss(**flags)
         # snippet_terms: weights of a padded batch (the last snippet weighs 0)
         w = torch.full((c['B'],), 1.0, device='cuda')
         w[-1] = 0.0
@@ -138,10 +151,12 @@ def main():
             gen = torch.Generator(device='cuda').manual_seed(0)
             pw = [torch.rand((c['B'], c['S'], c['H'] >> s, c['W'] >> s), device='cuda', generator=gen) for s in range(4)]
             kw = {option: dict(pixel_weights=pw)}
-        if option.startswith('geometry'):
+        if option.startswith('geometry') or option in THIRD:
             # the source frames' disparities: the target's maps of the snippets in a rolled order
             sd = [dev(np.repeat(x[np.roll(np.arange(c['B']), 1)], c['S'], axis=1)) for x in d['disps']]
             kw = {option: dict(src_disps=sd)}
+            if option in THIRD:
+                kw['plain'] = dict(src_disps=sd)
         graphs = {k: make_graph(op, args, **kw.get(k, {})) for k, op in ops.items()}
         replays = 10 if name == 'cfg5' else 200
         t = {k: [] for k in graphs}
