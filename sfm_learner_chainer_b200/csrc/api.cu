@@ -177,23 +177,96 @@ int num_sms() {
   return n;
 }
 
-int run_loss(const SfmDesc* d, const SfmInputs* in, float* losses_out, const SfmGrads* grads, const float* gy,
-             const SfmDebug* dbg, void* workspace, cudaStream_t st, const SfmPeerDev* peer = nullptr,
-             const SfmImageGrads* ig = nullptr, const SfmSnippetTerms* snip = nullptr, const SfmPixelTerms* pix = nullptr,
-             const SfmMinReprojection* mr = nullptr, const SfmGeometry* geo = nullptr, const SfmValidMean* vm = nullptr) {
+// Everything a loss entry point can pass.  `need` names the members its own signature makes mandatory; a mandatory
+// igrads, mr or geo also puts that option in play when the pointer is NULL (the call is then refused for it).
+enum : unsigned { NEED_LOSSES = 1, NEED_GRADS = 2, NEED_PEER = 4, NEED_IGRADS = 8, NEED_MR = 16, NEED_GEO = 32 };
+struct LossCall {
+  float* losses_out = nullptr;
+  const SfmGrads* grads = nullptr;
+  const float* gy = nullptr;
+  const SfmDebug* dbg = nullptr;
+  SfmPeer* peer = nullptr;
+  const SfmImageGrads* igrads = nullptr;
+  const SfmSnippetTerms* terms = nullptr;
+  const SfmPixelTerms* pix = nullptr;
+  const SfmMinReprojection* mr = nullptr;
+  const SfmGeometry* geo = nullptr;
+  const SfmValidMean* vm = nullptr;
+  unsigned need = 0;
+  const SfmPeerDev* peer_dev = nullptr;   // set by check_call: the connected peer's device view
+};
+
+// the name of the lowest flag of `bits`, for messages
+const char* flag_name(unsigned bits) {
+#define SFM_NAMED(f) {f, #f}
+  static const struct { unsigned bit; const char* name; } names[] = {
+      SFM_NAMED(SFM_FLAG_EDGE_AWARE_SMOOTH), SFM_NAMED(SFM_FLAG_MIN_REPROJECTION), SFM_NAMED(SFM_FLAG_FULL_RES_MULTISCALE),
+      SFM_NAMED(SFM_FLAG_MEAN_NORM_SMOOTH), SFM_NAMED(SFM_FLAG_EDGE_MEAN_ABS), SFM_NAMED(SFM_FLAG_BORDER_PADDING),
+      SFM_NAMED(SFM_FLAG_AXISANGLE_POSE), SFM_NAMED(SFM_FLAG_GEOMETRY_CONSISTENCY), SFM_NAMED(SFM_FLAG_VALID_MEAN)};
+#undef SFM_NAMED
+  for (const auto& n : names)
+    if (bits & n.bit) return n.name;
+  return "an unknown flag";
+}
+
+// Every rule of the loss entry points, in the order that decides which code a call breaking several of them gets.
+// Normalises the record: empty snippet or per-pixel terms become NULL (off).  The device probe comes last, and
+// run_loss refuses nothing after it.
+int check_call(const SfmDesc* d, const SfmInputs* in, LossCall& c, const void* workspace) {
   int rc = sfm_validate_desc(d);
   if (rc) return rc;
-  // SFM_FLAG_BORDER_PADDING runs the per-pixel instances (weights and maps NULL unless the caller passed them)
-  const bool border = (d->flags & SFM_FLAG_BORDER_PADDING) != 0;
-  if (border && (modes_of(d).use_exp || ig || dbg)) {
-    sfm_set_error("unsupported: SFM_FLAG_BORDER_PADDING together with %s", modes_of(d).use_exp ? "the explainability branch (exp_reg != 0)"
-                  : ig ? "image gradients" : "debug dumps");
-    return SFM_E_UNSUPPORTED;
-  }
-  const bool reuse = (d->flags & SFM_FLAG_REUSE_PYRAMID) != 0;
-  rc = check_inputs(d, in, true);      // the images are always needed: scale 0 is read from the caller's tensors
-  if (rc) return rc;
-  if (grads && (rc = check_grads(d, grads))) return rc;
+  if (c.terms && !c.terms->weights && !c.terms->losses) c.terms = nullptr;
+  bool pixel = false;                  // per-pixel terms: some member of a scale < n_scales is set
+  for (int s = 0; c.pix && s < d->n_scales; ++s) pixel = pixel || c.pix->weights[s] || c.pix->losses[s];
+  if (!pixel) c.pix = nullptr;
+  const unsigned fl = d->flags;
+  const bool exp = d->exp_reg != 0.f;
+  const bool ig = c.igrads || (c.need & NEED_IGRADS), mr = c.mr || (c.need & NEED_MR), geo = c.geo || (c.need & NEED_GEO);
+  const unsigned geo_excl = fl & (SFM_FLAG_FULL_RES_MULTISCALE | SFM_FLAG_BORDER_PADDING | SFM_FLAG_MIN_REPROJECTION);
+  const unsigned ig_excl = fl & (SFM_FLAG_EDGE_AWARE_SMOOTH | SFM_FLAG_FULL_RES_MULTISCALE);
+#define SFM_REFUSE(cond, code, ...) \
+  do { if (cond) { sfm_set_error(__VA_ARGS__); return code; } } while (0)
+#define SIZED " in desc->flags (the workspace is sized with it)"
+  SFM_REFUSE(c.vm && !(fl & SFM_FLAG_VALID_MEAN), SFM_E_INVALID_DESC, "valid-pixel means (vm) need SFM_FLAG_VALID_MEAN" SIZED);
+  SFM_REFUSE(c.vm && (c.vm->groups < 1 || c.vm->groups > d->B), SFM_E_INVALID_DESC,
+             "SfmValidMean.groups = %d outside [1, B = %d]", c.vm->groups, d->B);
+  SFM_REFUSE(c.vm && !(c.vm->min_count >= 0.f && isfinite(c.vm->min_count)), SFM_E_INVALID_DESC,
+             "SfmValidMean.min_count must be finite and >= 0");
+  SFM_REFUSE(c.vm && c.peer, SFM_E_UNSUPPORTED, "unsupported: valid-pixel means (vm) with a peer (the counts are batch-global)");
+  SFM_REFUSE(c.vm && d->B_global > 0 && d->B_global != d->B, SFM_E_UNSUPPORTED,
+             "unsupported: valid-pixel means (vm) with B_global != B (the counts are batch-global)");
+  SFM_REFUSE(geo && !(fl & SFM_FLAG_GEOMETRY_CONSISTENCY), SFM_E_INVALID_DESC,
+             "geometry consistency (geo) needs SFM_FLAG_GEOMETRY_CONSISTENCY" SIZED);
+  SFM_REFUSE(mr && !(fl & SFM_FLAG_MIN_REPROJECTION), SFM_E_INVALID_DESC, "minimum reprojection (mr) needs SFM_FLAG_MIN_REPROJECTION" SIZED);
+  SFM_REFUSE(mr && !(d->ssim_rate >= 0.f && d->ssim_rate <= 1.f), SFM_E_INVALID_DESC,
+             "minimum reprojection (mr): ssim_rate=%g outside [0, 1] (the selection needs a non-negative error)", (double)d->ssim_rate);
+  SFM_REFUSE((geo || mr) && exp, SFM_E_UNSUPPORTED, "unsupported: %s together with the explainability branch (exp_reg != 0)",
+             geo ? "geometry consistency (geo)" : "minimum reprojection (mr)");
+  SFM_REFUSE(geo && geo_excl, SFM_E_UNSUPPORTED, "unsupported: geometry consistency (geo) together with %s", flag_name(geo_excl));
+  SFM_REFUSE(c.mr && c.mr->reserved_ != 0, SFM_E_INVALID_DESC, "SfmMinReprojection.reserved_ must be 0");
+  SFM_REFUSE(c.terms && !(fl & SFM_FLAG_SNIPPET_TERMS), SFM_E_INVALID_DESC, "snippet terms (terms) need SFM_FLAG_SNIPPET_TERMS" SIZED);
+  SFM_REFUSE(ig && !(fl & SFM_FLAG_IMAGE_GRADS), SFM_E_INVALID_DESC, "image gradients (igrads) need SFM_FLAG_IMAGE_GRADS" SIZED);
+  SFM_REFUSE(ig && ig_excl, SFM_E_UNSUPPORTED, "unsupported: image gradients (igrads) together with %s", flag_name(ig_excl));
+  SFM_REFUSE(ig && (!c.igrads || (!c.igrads->gtgt && !c.igrads->gsrc)), SFM_E_NULL_POINTER, "igrads is NULL or has neither gtgt nor gsrc");
+  SFM_REFUSE(ig && !c.grads, SFM_E_NULL_POINTER, "image gradients (igrads) need grads, which is NULL");
+  SFM_REFUSE((c.need & NEED_LOSSES) && !c.losses_out, SFM_E_NULL_POINTER, "losses_out is NULL");
+  SFM_REFUSE((c.need & NEED_GRADS) && !c.grads, SFM_E_NULL_POINTER, "grads is NULL");
+  SFM_REFUSE((c.need & NEED_PEER) && !c.peer, SFM_E_NULL_POINTER, "peer is NULL");
+  SFM_REFUSE(mr && !c.mr, SFM_E_NULL_POINTER, "SfmMinReprojection is NULL");
+  SFM_REFUSE(geo && !c.geo, SFM_E_NULL_POINTER, "SfmGeometry is NULL");
+  for (int s = 0; c.geo && s < d->n_scales; ++s)
+    SFM_REFUSE(!c.geo->src_disps[s], SFM_E_NULL_POINTER, "SfmGeometry.src_disps[%d] is NULL", s);
+  SFM_REFUSE(c.pix && ig, SFM_E_UNSUPPORTED, "unsupported: per-pixel terms (pix) together with image gradients (igrads)");
+  SFM_REFUSE(c.peer && !(c.peer_dev = sfm_peer_dev(c.peer)), SFM_E_UNSUPPORTED,
+             "unsupported: the peer object is not connected (sfm_peer_connect)");
+  SFM_REFUSE((fl & SFM_FLAG_BORDER_PADDING) && (exp || ig || c.dbg), SFM_E_UNSUPPORTED, "unsupported: SFM_FLAG_BORDER_PADDING together with %s",
+             exp ? "the explainability branch (exp_reg != 0)" : ig ? "image gradients (igrads)" : "debug dumps");
+  SFM_REFUSE(sfm_full_res(d) && exp, SFM_E_UNSUPPORTED, "unsupported: SFM_FLAG_FULL_RES_MULTISCALE together with the explainability "
+             "branch (exp_reg != 0): the logits live at scale resolution");
+#undef SIZED
+#undef SFM_REFUSE
+  if ((rc = check_inputs(d, in, true))) return rc;      // the images are always needed: scale 0 is read from the caller's tensors
+  if (c.grads && (rc = check_grads(d, c.grads))) return rc;
   if (!workspace) { sfm_set_error("workspace is NULL"); return SFM_E_NULL_POINTER; }
   if (((uintptr_t)workspace & 255) != 0) { sfm_set_error("workspace must be 256-byte aligned"); return SFM_E_INVALID_DESC; }
   int ndev = 0;
@@ -201,17 +274,25 @@ int run_loss(const SfmDesc* d, const SfmInputs* in, float* losses_out, const Sfm
     sfm_set_error("no CUDA device: libsfmloss has no CPU fallback");
     return SFM_E_NO_DEVICE;
   }
+  return 0;
+}
+
+int run_loss(const SfmDesc* d, const SfmInputs* in, LossCall c, void* workspace, cudaStream_t st) {
+  int rc = check_call(d, in, c, workspace);
+  if (rc) return rc;
+  const SfmGrads* grads = c.grads;
+  const float* gy = c.gy;
+  const SfmDebug* dbg = c.dbg;
+  const SfmImageGrads* ig = c.igrads;
+  const SfmSnippetTerms* snip = c.terms;
+  const SfmPixelTerms* pix = c.pix;
+  const SfmMinReprojection* mr = c.mr;
+  const SfmGeometry* geo = c.geo;
+  const SfmValidMean* vm = c.vm;
+  const bool border = (d->flags & SFM_FLAG_BORDER_PADDING) != 0;
+  const bool reuse = (d->flags & SFM_FLAG_REUSE_PYRAMID) != 0;
   const Modes m = modes_of(d);
   const bool fr = sfm_full_res(d);
-  if (fr && m.use_exp) {
-    sfm_set_error("unsupported: SFM_FLAG_FULL_RES_MULTISCALE together with the explainability branch (exp_reg != 0): the logits "
-                  "live at scale resolution");
-    return SFM_E_UNSUPPORTED;
-  }
-  if (fr && ig) {
-    sfm_set_error("unsupported: image gradients together with SFM_FLAG_FULL_RES_MULTISCALE");
-    return SFM_E_UNSUPPORTED;
-  }
   int mode = 0;
   if (m.use_exp) mode |= SFM_MODE_EXP;
   if (m.use_ssim) mode |= SFM_MODE_SSIM;
@@ -288,9 +369,9 @@ int run_loss(const SfmDesc* d, const SfmInputs* in, float* losses_out, const Sfm
   p.raw_disp_mask = d->raw_disp_scales;
   p.gy = gy;
   p.acc = (double*)(ws + L.off_acc);
-  p.losses_out = losses_out;
+  p.losses_out = c.losses_out;
   p.peer = SfmPeerDev{};
-  if (peer) p.peer = *peer;
+  if (c.peer_dev) p.peer = *c.peer_dev;
   p.gposes = grads ? grads->gposes : nullptr;
   p.smooth_reg = d->smooth_reg;
   p.exp_reg = m.use_exp ? d->exp_reg : 0.f;
@@ -451,56 +532,46 @@ int run_loss(const SfmDesc* d, const SfmInputs* in, float* losses_out, const Sfm
 
 }  // namespace
 
+// The loss entry points fill the call record from their arguments; check_call holds every rule.
 extern "C" int sfm_loss_forward(const SfmDesc* desc, const SfmInputs* in, float* losses_out, const SfmDebug* debug,
                                 void* workspace, void* stream) {
-  if (!losses_out) { sfm_set_error("losses_out is NULL"); return SFM_E_NULL_POINTER; }
-  return run_loss(desc, in, losses_out, nullptr, nullptr, debug, workspace, (cudaStream_t)stream);
+  LossCall c;
+  c.need = NEED_LOSSES;
+  c.losses_out = losses_out; c.dbg = debug;
+  return run_loss(desc, in, c, workspace, (cudaStream_t)stream);
 }
 
 extern "C" int sfm_loss_backward(const SfmDesc* desc, const SfmInputs* in, const float* gy, const SfmGrads* grads,
                                  void* workspace, void* stream) {
-  if (!grads) { sfm_set_error("grads is NULL"); return SFM_E_NULL_POINTER; }
-  return run_loss(desc, in, nullptr, grads, gy, nullptr, workspace, (cudaStream_t)stream);
+  LossCall c;
+  c.need = NEED_GRADS;
+  c.gy = gy; c.grads = grads;
+  return run_loss(desc, in, c, workspace, (cudaStream_t)stream);
 }
 
 extern "C" int sfm_loss_forward_backward(const SfmDesc* desc, const SfmInputs* in, float* losses_out,
                                          const SfmGrads* grads, void* workspace, void* stream) {
-  if (!losses_out) { sfm_set_error("losses_out is NULL"); return SFM_E_NULL_POINTER; }
-  if (!grads) { sfm_set_error("grads is NULL"); return SFM_E_NULL_POINTER; }
-  return run_loss(desc, in, losses_out, grads, nullptr, nullptr, workspace, (cudaStream_t)stream);
+  LossCall c;
+  c.need = NEED_LOSSES | NEED_GRADS;
+  c.losses_out = losses_out; c.grads = grads;
+  return run_loss(desc, in, c, workspace, (cudaStream_t)stream);
 }
 
 extern "C" int sfm_loss_forward_backward_peer(const SfmDesc* desc, const SfmInputs* in, float* losses_out,
                                               const SfmGrads* grads, void* workspace, SfmPeer* peer, void* stream) {
-  if (!losses_out) { sfm_set_error("losses_out is NULL"); return SFM_E_NULL_POINTER; }
-  if (!grads) { sfm_set_error("grads is NULL"); return SFM_E_NULL_POINTER; }
-  if (!peer) { sfm_set_error("peer is NULL"); return SFM_E_NULL_POINTER; }
-  const SfmPeerDev* dev = sfm_peer_dev(peer);
-  if (!dev) { sfm_set_error("sfm_loss_forward_backward_peer: the peer object is not connected (sfm_peer_connect)"); return SFM_E_UNSUPPORTED; }
-  return run_loss(desc, in, losses_out, grads, nullptr, nullptr, workspace, (cudaStream_t)stream, dev);
+  LossCall c;
+  c.need = NEED_LOSSES | NEED_GRADS | NEED_PEER;
+  c.losses_out = losses_out; c.grads = grads; c.peer = peer;
+  return run_loss(desc, in, c, workspace, (cudaStream_t)stream);
 }
 
 extern "C" int sfm_loss_forward_backward_images(const SfmDesc* desc, const SfmInputs* in, float* losses_out,
                                                 const SfmGrads* grads, const SfmImageGrads* igrads, void* workspace,
                                                 void* stream) {
-  int rc = sfm_validate_desc(desc);
-  if (rc) return rc;
-  if (!(desc->flags & SFM_FLAG_IMAGE_GRADS)) {
-    sfm_set_error("sfm_loss_forward_backward_images: desc->flags lacks SFM_FLAG_IMAGE_GRADS (the workspace must be sized with it)");
-    return SFM_E_INVALID_DESC;
-  }
-  if (desc->flags & SFM_FLAG_EDGE_AWARE_SMOOTH) {
-    sfm_set_error("unsupported: image gradients through the edge-aware smoothness term (SFM_FLAG_EDGE_AWARE_SMOOTH)");
-    return SFM_E_UNSUPPORTED;
-  }
-  if (desc->flags & SFM_FLAG_FULL_RES_MULTISCALE) {
-    sfm_set_error("unsupported: image gradients together with SFM_FLAG_FULL_RES_MULTISCALE");
-    return SFM_E_UNSUPPORTED;
-  }
-  if (!igrads || (!igrads->gtgt && !igrads->gsrc)) { sfm_set_error("igrads is NULL or has neither gtgt nor gsrc"); return SFM_E_NULL_POINTER; }
-  if (!losses_out) { sfm_set_error("losses_out is NULL"); return SFM_E_NULL_POINTER; }
-  if (!grads) { sfm_set_error("grads is NULL"); return SFM_E_NULL_POINTER; }
-  return run_loss(desc, in, losses_out, grads, nullptr, nullptr, workspace, (cudaStream_t)stream, nullptr, igrads);
+  LossCall c;
+  c.need = NEED_LOSSES | NEED_GRADS | NEED_IGRADS;
+  c.losses_out = losses_out; c.grads = grads; c.igrads = igrads;
+  return run_loss(desc, in, c, workspace, (cudaStream_t)stream);
 }
 
 extern "C" int sfm_loss_snippets(const SfmDesc* desc, const SfmInputs* in, const SfmSnippetTerms* terms, float* losses_out,
@@ -512,170 +583,34 @@ extern "C" int sfm_loss_snippets(const SfmDesc* desc, const SfmInputs* in, const
 extern "C" int sfm_loss_weighted(const SfmDesc* desc, const SfmInputs* in, const SfmSnippetTerms* terms, const SfmPixelTerms* pix,
                                  float* losses_out, const SfmGrads* grads, const SfmImageGrads* igrads, void* workspace,
                                  SfmPeer* peer, void* stream) {
-  int rc = sfm_validate_desc(desc);
-  if (rc) return rc;
-  const bool snip = terms && (terms->weights || terms->losses);
-  if (snip && !(desc->flags & SFM_FLAG_SNIPPET_TERMS)) {
-    sfm_set_error("sfm_loss_snippets: desc->flags lacks SFM_FLAG_SNIPPET_TERMS (the workspace must be sized with it)");
-    return SFM_E_INVALID_DESC;
-  }
-  if (igrads) {
-    if (!(desc->flags & SFM_FLAG_IMAGE_GRADS)) {
-      sfm_set_error("sfm_loss_snippets: igrads given but desc->flags lacks SFM_FLAG_IMAGE_GRADS (the workspace must be sized with it)");
-      return SFM_E_INVALID_DESC;
-    }
-    if (desc->flags & SFM_FLAG_EDGE_AWARE_SMOOTH) {
-      sfm_set_error("unsupported: image gradients through the edge-aware smoothness term (SFM_FLAG_EDGE_AWARE_SMOOTH)");
-      return SFM_E_UNSUPPORTED;
-    }
-    if (desc->flags & SFM_FLAG_FULL_RES_MULTISCALE) {
-      sfm_set_error("unsupported: image gradients together with SFM_FLAG_FULL_RES_MULTISCALE");
-      return SFM_E_UNSUPPORTED;
-    }
-    if (!igrads->gtgt && !igrads->gsrc) { sfm_set_error("igrads has neither gtgt nor gsrc"); return SFM_E_NULL_POINTER; }
-    if (!grads) { sfm_set_error("sfm_loss_snippets: igrads needs grads"); return SFM_E_NULL_POINTER; }
-  }
-  bool pixel = false;                  // per-pixel terms: some member of a scale < n_scales is set
-  for (int s = 0; pix && s < desc->n_scales; ++s) pixel = pixel || pix->weights[s] || pix->losses[s];
-  if (pixel && igrads) {
-    sfm_set_error("unsupported: per-pixel terms (SfmPixelTerms) together with image gradients (igrads)");
-    return SFM_E_UNSUPPORTED;
-  }
-  if (!losses_out) { sfm_set_error("losses_out is NULL"); return SFM_E_NULL_POINTER; }
-  const SfmPeerDev* dev = nullptr;
-  if (peer && !(dev = sfm_peer_dev(peer))) {
-    sfm_set_error("sfm_loss_snippets: the peer object is not connected (sfm_peer_connect)");
-    return SFM_E_UNSUPPORTED;
-  }
-  return run_loss(desc, in, losses_out, grads, nullptr, nullptr, workspace, (cudaStream_t)stream, dev, igrads,
-                  snip ? terms : nullptr, pixel ? pix : nullptr);
+  LossCall c;
+  c.need = NEED_LOSSES;
+  c.terms = terms; c.pix = pix; c.losses_out = losses_out; c.grads = grads; c.igrads = igrads; c.peer = peer;
+  return run_loss(desc, in, c, workspace, (cudaStream_t)stream);
 }
 
 extern "C" int sfm_loss_min_reprojection(const SfmDesc* desc, const SfmInputs* in, const SfmSnippetTerms* terms,
                                          const SfmMinReprojection* mr, float* losses_out, const SfmGrads* grads, void* workspace,
                                          SfmPeer* peer, void* stream) {
-  int rc = sfm_validate_desc(desc);
-  if (rc) return rc;
-  if (!(desc->flags & SFM_FLAG_MIN_REPROJECTION)) {
-    sfm_set_error("sfm_loss_min_reprojection: desc->flags lacks SFM_FLAG_MIN_REPROJECTION (the workspace must be sized with it)");
-    return SFM_E_INVALID_DESC;
-  }
-  if (!(desc->ssim_rate >= 0.f && desc->ssim_rate <= 1.f)) {
-    sfm_set_error("sfm_loss_min_reprojection: ssim_rate=%g outside [0, 1] (the selection needs a non-negative error)",
-                  (double)desc->ssim_rate);
-    return SFM_E_INVALID_DESC;
-  }
-  if (desc->exp_reg != 0.f) {
-    sfm_set_error("unsupported: minimum reprojection together with the explainability branch (exp_reg != 0)");
-    return SFM_E_UNSUPPORTED;
-  }
-  if (!mr) { sfm_set_error("SfmMinReprojection is NULL"); return SFM_E_NULL_POINTER; }
-  if (mr->reserved_ != 0) { sfm_set_error("SfmMinReprojection.reserved_ must be 0"); return SFM_E_INVALID_DESC; }
-  const bool snip = terms && (terms->weights || terms->losses);
-  if (snip && !(desc->flags & SFM_FLAG_SNIPPET_TERMS)) {
-    sfm_set_error("sfm_loss_min_reprojection: desc->flags lacks SFM_FLAG_SNIPPET_TERMS (the workspace must be sized with it)");
-    return SFM_E_INVALID_DESC;
-  }
-  if (!losses_out) { sfm_set_error("losses_out is NULL"); return SFM_E_NULL_POINTER; }
-  const SfmPeerDev* dev = nullptr;
-  if (peer && !(dev = sfm_peer_dev(peer))) {
-    sfm_set_error("sfm_loss_min_reprojection: the peer object is not connected (sfm_peer_connect)");
-    return SFM_E_UNSUPPORTED;
-  }
-  return run_loss(desc, in, losses_out, grads, nullptr, nullptr, workspace, (cudaStream_t)stream, dev, nullptr,
-                  snip ? terms : nullptr, nullptr, mr);
+  LossCall c;
+  c.need = NEED_LOSSES | NEED_MR;
+  c.terms = terms; c.mr = mr; c.losses_out = losses_out; c.grads = grads; c.peer = peer;
+  return run_loss(desc, in, c, workspace, (cudaStream_t)stream);
 }
 
 extern "C" int sfm_loss_geometry(const SfmDesc* desc, const SfmInputs* in, const SfmSnippetTerms* terms,
                                  const SfmGeometry* geo, float* losses_out, const SfmGrads* grads, void* workspace, SfmPeer* peer,
                                  void* stream) {
-  int rc = sfm_validate_desc(desc);
-  if (rc) return rc;
-  if (!(desc->flags & SFM_FLAG_GEOMETRY_CONSISTENCY)) {
-    sfm_set_error("sfm_loss_geometry: desc->flags lacks SFM_FLAG_GEOMETRY_CONSISTENCY (the workspace must be sized with it)");
-    return SFM_E_INVALID_DESC;
-  }
-  if (desc->exp_reg != 0.f) {
-    sfm_set_error("unsupported: geometry consistency together with the explainability branch (exp_reg != 0)");
-    return SFM_E_UNSUPPORTED;
-  }
-  const unsigned excl = desc->flags & (SFM_FLAG_FULL_RES_MULTISCALE | SFM_FLAG_BORDER_PADDING | SFM_FLAG_MIN_REPROJECTION);
-  if (excl) {
-    sfm_set_error("unsupported: geometry consistency together with %s",
-                  (excl & SFM_FLAG_FULL_RES_MULTISCALE) ? "SFM_FLAG_FULL_RES_MULTISCALE"
-                  : (excl & SFM_FLAG_BORDER_PADDING) ? "SFM_FLAG_BORDER_PADDING" : "SFM_FLAG_MIN_REPROJECTION");
-    return SFM_E_UNSUPPORTED;
-  }
-  if (!geo) { sfm_set_error("SfmGeometry is NULL"); return SFM_E_NULL_POINTER; }
-  for (int s = 0; s < desc->n_scales; ++s)
-    if (!geo->src_disps[s]) { sfm_set_error("SfmGeometry.src_disps[%d] is NULL", s); return SFM_E_NULL_POINTER; }
-  const bool snip = terms && (terms->weights || terms->losses);
-  if (snip && !(desc->flags & SFM_FLAG_SNIPPET_TERMS)) {
-    sfm_set_error("sfm_loss_geometry: desc->flags lacks SFM_FLAG_SNIPPET_TERMS (the workspace must be sized with it)");
-    return SFM_E_INVALID_DESC;
-  }
-  if (!losses_out) { sfm_set_error("losses_out is NULL"); return SFM_E_NULL_POINTER; }
-  const SfmPeerDev* dev = nullptr;
-  if (peer && !(dev = sfm_peer_dev(peer))) {
-    sfm_set_error("sfm_loss_geometry: the peer object is not connected (sfm_peer_connect)");
-    return SFM_E_UNSUPPORTED;
-  }
-  return run_loss(desc, in, losses_out, grads, nullptr, nullptr, workspace, (cudaStream_t)stream, dev, nullptr,
-                  snip ? terms : nullptr, nullptr, nullptr, geo);
+  return sfm_loss_geometry_valid_mean(desc, in, terms, geo, nullptr, losses_out, grads, workspace, peer, stream);
 }
 
 extern "C" int sfm_loss_geometry_valid_mean(const SfmDesc* desc, const SfmInputs* in, const SfmSnippetTerms* terms,
                                             const SfmGeometry* geo, const SfmValidMean* vm, float* losses_out,
                                             const SfmGrads* grads, void* workspace, SfmPeer* peer, void* stream) {
-  if (!vm) return sfm_loss_geometry(desc, in, terms, geo, losses_out, grads, workspace, peer, stream);
-  int rc = sfm_validate_desc(desc);
-  if (rc) return rc;
-  if (!(desc->flags & SFM_FLAG_VALID_MEAN)) {
-    sfm_set_error("sfm_loss_geometry_valid_mean: desc->flags lacks SFM_FLAG_VALID_MEAN (the workspace must be sized with it)");
-    return SFM_E_INVALID_DESC;
-  }
-  if (vm->groups < 1 || vm->groups > desc->B) {
-    sfm_set_error("SfmValidMean.groups = %d outside [1, B = %d]", vm->groups, desc->B);
-    return SFM_E_INVALID_DESC;
-  }
-  if (!(vm->min_count >= 0.f) || !isfinite(vm->min_count)) {
-    sfm_set_error("SfmValidMean.min_count must be finite and >= 0");
-    return SFM_E_INVALID_DESC;
-  }
-  if (peer) {
-    sfm_set_error("unsupported: valid-pixel means with a peer (the counts are batch-global)");
-    return SFM_E_UNSUPPORTED;
-  }
-  if (desc->B_global > 0 && desc->B_global != desc->B) {
-    sfm_set_error("unsupported: valid-pixel means with B_global != B (the counts are batch-global)");
-    return SFM_E_UNSUPPORTED;
-  }
-  if (!(desc->flags & SFM_FLAG_GEOMETRY_CONSISTENCY)) {
-    sfm_set_error("sfm_loss_geometry_valid_mean: desc->flags lacks SFM_FLAG_GEOMETRY_CONSISTENCY (the workspace must be sized with it)");
-    return SFM_E_INVALID_DESC;
-  }
-  if (desc->exp_reg != 0.f) {
-    sfm_set_error("unsupported: geometry consistency together with the explainability branch (exp_reg != 0)");
-    return SFM_E_UNSUPPORTED;
-  }
-  const unsigned excl = desc->flags & (SFM_FLAG_FULL_RES_MULTISCALE | SFM_FLAG_BORDER_PADDING | SFM_FLAG_MIN_REPROJECTION);
-  if (excl) {
-    sfm_set_error("unsupported: geometry consistency together with %s",
-                  (excl & SFM_FLAG_FULL_RES_MULTISCALE) ? "SFM_FLAG_FULL_RES_MULTISCALE"
-                  : (excl & SFM_FLAG_BORDER_PADDING) ? "SFM_FLAG_BORDER_PADDING" : "SFM_FLAG_MIN_REPROJECTION");
-    return SFM_E_UNSUPPORTED;
-  }
-  if (!geo) { sfm_set_error("SfmGeometry is NULL"); return SFM_E_NULL_POINTER; }
-  for (int s = 0; s < desc->n_scales; ++s)
-    if (!geo->src_disps[s]) { sfm_set_error("SfmGeometry.src_disps[%d] is NULL", s); return SFM_E_NULL_POINTER; }
-  const bool snip = terms && (terms->weights || terms->losses);
-  if (snip && !(desc->flags & SFM_FLAG_SNIPPET_TERMS)) {
-    sfm_set_error("sfm_loss_geometry_valid_mean: desc->flags lacks SFM_FLAG_SNIPPET_TERMS (the workspace must be sized with it)");
-    return SFM_E_INVALID_DESC;
-  }
-  if (!losses_out) { sfm_set_error("losses_out is NULL"); return SFM_E_NULL_POINTER; }
-  return run_loss(desc, in, losses_out, grads, nullptr, nullptr, workspace, (cudaStream_t)stream, nullptr, nullptr,
-                  snip ? terms : nullptr, nullptr, nullptr, geo, vm);
+  LossCall c;
+  c.need = NEED_LOSSES | NEED_GEO;
+  c.terms = terms; c.geo = geo; c.vm = vm; c.losses_out = losses_out; c.grads = grads; c.peer = peer;
+  return run_loss(desc, in, c, workspace, (cudaStream_t)stream);
 }
 
 extern "C" int sfm_scale_image_grads(const SfmDesc* desc, const float* gy, const SfmImageGrads* igrads, void* stream) {
@@ -869,28 +804,11 @@ extern "C" int sfm_host_ctx_create(const SfmDesc* desc, SfmHostCtx** ctx_out) {
   int rc = sfm_validate_desc(desc);
   if (rc) return rc;
   if (!ctx_out) { sfm_set_error("ctx_out is NULL"); return SFM_E_NULL_POINTER; }
-  if (desc->flags & SFM_FLAG_FULL_RES_MULTISCALE) {
-    sfm_set_error("unsupported: the host-buffer path with SFM_FLAG_FULL_RES_MULTISCALE");
-    return SFM_E_UNSUPPORTED;
-  }
-  if (desc->flags & (SFM_FLAG_MEAN_NORM_SMOOTH | SFM_FLAG_EDGE_MEAN_ABS)) {
-    sfm_set_error("unsupported: the host-buffer path with SFM_FLAG_MEAN_NORM_SMOOTH or SFM_FLAG_EDGE_MEAN_ABS");
-    return SFM_E_UNSUPPORTED;
-  }
-  if (desc->flags & SFM_FLAG_BORDER_PADDING) {
-    sfm_set_error("unsupported: the host-buffer path with SFM_FLAG_BORDER_PADDING");
-    return SFM_E_UNSUPPORTED;
-  }
-  if (desc->flags & SFM_FLAG_AXISANGLE_POSE) {
-    sfm_set_error("unsupported: the host-buffer path with SFM_FLAG_AXISANGLE_POSE");
-    return SFM_E_UNSUPPORTED;
-  }
-  if (desc->flags & SFM_FLAG_GEOMETRY_CONSISTENCY) {
-    sfm_set_error("unsupported: the host-buffer path with SFM_FLAG_GEOMETRY_CONSISTENCY");
-    return SFM_E_UNSUPPORTED;
-  }
-  if (desc->flags & SFM_FLAG_VALID_MEAN) {
-    sfm_set_error("unsupported: the host-buffer path with SFM_FLAG_VALID_MEAN");
+  const unsigned unsupported = desc->flags & (SFM_FLAG_FULL_RES_MULTISCALE | SFM_FLAG_MEAN_NORM_SMOOTH | SFM_FLAG_EDGE_MEAN_ABS |
+                                               SFM_FLAG_BORDER_PADDING | SFM_FLAG_AXISANGLE_POSE | SFM_FLAG_GEOMETRY_CONSISTENCY |
+                                               SFM_FLAG_VALID_MEAN);
+  if (unsupported) {
+    sfm_set_error("unsupported: the host-buffer path with %s", flag_name(unsupported));
     return SFM_E_UNSUPPORTED;
   }
   int ndev = 0;

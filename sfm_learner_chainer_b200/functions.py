@@ -92,72 +92,59 @@ class ViewSynthesisLoss(object):
     include/sfmloss.h.
     """
 
+    # constructor options that need another one, and pairs that exclude each other (exp_reg and B_global count as on
+    # when set); the C entry points enforce the same rules on the descriptor (include/sfmloss.h)
+    NEEDS = (('self_mask', 'geometry_consistency'), ('valid_mean', 'geometry_consistency'),
+             ('invert_sources', 'axisangle_pose'), ('edge_mean_abs', 'edge_aware_smooth'))
+    EXCLUDES = tuple((a, b) for a, bs in (
+        ('geometry_consistency', ('image_grads', 'pixel_terms', 'min_reprojection', 'full_res_multiscale', 'border_padding',
+                                  'exp_reg')),
+        ('valid_mean', ('B_global',)),
+        ('border_padding', ('image_grads', 'exp_reg')),
+        ('full_res_multiscale', ('image_grads', 'exp_reg')),
+        ('image_grads', ('edge_aware_smooth', 'pixel_terms')),
+        ('min_reprojection', ('image_grads', 'pixel_terms', 'exp_reg'))) for b in bs)
+
     def __init__(self, smooth_reg=0.0, exp_reg=0.0, ssim_rate=0.0, n_scales=N_SCALES, B_global=None,
                  raw_disp_scales=0, raw_pose=False, edge_aware_smooth=False, image_grads=False,
                  intrinsics_grad=False, snippet_terms=False, pixel_terms=False, min_reprojection=False, automask=True,
                  full_res_multiscale=False, mean_norm_smooth=False, edge_mean_abs=False, border_padding=False,
                  axisangle_pose=False, invert_sources=(), geometry_consistency=False, geometry_reg=0.5, self_mask=False,
                  valid_mean=False, valid_automask=True, valid_min_count=10000.0, count_groups=1):
-        if self_mask and not geometry_consistency:
-            raise ValueError('self_mask needs geometry_consistency')
+        invert_sources = tuple(int(i) for i in (invert_sources or ()))
+        on = dict(self_mask=self_mask, valid_mean=valid_mean, invert_sources=invert_sources, edge_mean_abs=edge_mean_abs,
+                  geometry_consistency=geometry_consistency, axisangle_pose=axisangle_pose,
+                  edge_aware_smooth=edge_aware_smooth, image_grads=image_grads, pixel_terms=pixel_terms,
+                  min_reprojection=min_reprojection, full_res_multiscale=full_res_multiscale, border_padding=border_padding,
+                  exp_reg=float(exp_reg or 0.0) != 0.0, B_global=B_global is not None)
+        for a, b in self.NEEDS:
+            if on[a] and not on[b]:
+                raise ValueError('%s needs %s' % (a, b))
+        for a, b in self.EXCLUDES:
+            if on[a] and on[b]:
+                raise ValueError('%s is not supported together with %s' % (a, b))
         if valid_mean:
-            if not geometry_consistency:
-                raise ValueError('valid_mean needs geometry_consistency')
-            if B_global is not None:
-                raise ValueError('valid_mean is not supported with B_global (the counts are batch-global)')
             if not math.isfinite(float(valid_min_count)) or float(valid_min_count) < 0.0:
                 raise ValueError('valid_min_count must be finite and >= 0, got %r' % (valid_min_count,))
             if int(count_groups) < 1:
                 raise ValueError('count_groups must be >= 1, got %r' % (count_groups,))
+        if any(i < 0 for i in invert_sources):
+            raise ValueError('invert_sources must hold source indices >= 0, got %r' % (invert_sources,))
+        if min_reprojection and not 0.0 <= float(ssim_rate or 0.0) <= 1.0:
+            raise ValueError('min_reprojection needs ssim_rate in [0, 1]')
         self.valid_mean = bool(valid_mean)
         self.valid_automask = bool(valid_automask)
         self.valid_min_count = float(valid_min_count)
         self.count_groups = int(count_groups)
-        if geometry_consistency:
-            for name, on in (('image_grads', image_grads), ('pixel_terms', pixel_terms),
-                             ('min_reprojection', min_reprojection), ('full_res_multiscale', full_res_multiscale),
-                             ('border_padding', border_padding)):
-                if on:
-                    raise ValueError('geometry_consistency is not supported together with %s' % name)
-            if float(exp_reg or 0.0) != 0.0:
-                raise ValueError('geometry_consistency is not supported together with the explainability branch (exp_reg)')
         self.geometry_consistency = bool(geometry_consistency)
         self.geometry_reg = float(geometry_reg)
         self.self_mask = bool(self_mask)
-        invert_sources = tuple(int(i) for i in (invert_sources or ()))
-        if invert_sources and not axisangle_pose:
-            raise ValueError('invert_sources needs axisangle_pose')
-        if any(i < 0 for i in invert_sources):
-            raise ValueError('invert_sources must hold source indices >= 0, got %r' % (invert_sources,))
         self.axisangle_pose = bool(axisangle_pose)
         self.invert_sources = invert_sources
-        if edge_mean_abs and not edge_aware_smooth:
-            raise ValueError('edge_mean_abs needs edge_aware_smooth')
-        if border_padding:
-            if image_grads:
-                raise ValueError('border_padding is not supported together with image_grads')
-            if float(exp_reg or 0.0) != 0.0:
-                raise ValueError('border_padding is not supported together with the explainability branch (exp_reg)')
         self.border_padding = bool(border_padding)
         self.mean_norm_smooth = bool(mean_norm_smooth)
         self.edge_mean_abs = bool(edge_mean_abs)
-        if full_res_multiscale:
-            if image_grads:
-                raise ValueError('full_res_multiscale is not supported together with image_grads')
-            if float(exp_reg or 0.0) != 0.0:
-                raise ValueError('full_res_multiscale is not supported together with the explainability branch (exp_reg)')
         self.full_res_multiscale = bool(full_res_multiscale)
-        if image_grads and edge_aware_smooth:
-            raise ValueError('image_grads is not supported together with edge_aware_smooth')
-        if image_grads and pixel_terms:
-            raise ValueError('image_grads is not supported together with pixel_terms')
-        if min_reprojection:
-            if image_grads or pixel_terms:
-                raise ValueError('min_reprojection is not supported together with image_grads or pixel_terms')
-            if float(exp_reg or 0.0) != 0.0:
-                raise ValueError('min_reprojection is not supported together with the explainability branch (exp_reg)')
-            if not 0.0 <= float(ssim_rate or 0.0) <= 1.0:
-                raise ValueError('min_reprojection needs ssim_rate in [0, 1]')
         self.min_reprojection = bool(min_reprojection)
         self.automask = bool(automask)
         self.pixel_terms = bool(pixel_terms)
@@ -392,14 +379,51 @@ class ViewSynthesisLoss(object):
         vm.counts = D.ptr(counts)
         return vm, masks, counts
 
-    def _run_geometry(self, desc, inp, terms, ge, vm, losses, grads, tgt, peer):
-        args = (C.byref(desc), C.byref(inp), C.byref(terms) if terms else None, C.byref(ge))
-        tail = (_vp(losses), C.byref(grads) if grads is not None else None, self._workspace(desc, tgt), peer,
-                C.c_void_p(D.current_stream(tgt)))
-        if vm is None:
-            L.check(self._lib.sfm_loss_geometry(*args, *tail))
+    def _loss(self, desc, inp, tgt, losses, g, out, snippet_weights, pixel_weights, src_disps, peer=None, image_grads=(),
+              dbg=None):
+        """The one loss call of forward (g None) and forward_backward: builds the blocks of the operator's options, adds
+        their outputs to `out` (snippet_losses, pixel_losses, selection, geometry_diff, gsrc_disps, valid_masks,
+        valid_counts, gtgt, gsrc) and calls the entry point that takes them: sfm_loss_forward for debug dumps,
+        sfm_loss_geometry_valid_mean, sfm_loss_min_reprojection or sfm_loss_weighted."""
+        terms, rows = self._snippet_terms(desc, tgt, snippet_weights)
+        if rows is not None:
+            out['snippet_losses'] = rows
+        pt, maps = self._pixel_terms(desc, tgt, pixel_weights)
+        if maps is not None:
+            out['pixel_losses'] = maps
+        mr, sel = self._min_reprojection(desc, tgt)
+        if sel is not None:
+            out['selection'] = sel
+        ge = vm = None
+        if self.geometry_consistency:
+            ge, out['geometry_diff'], gsd = self._geometry(desc, tgt, src_disps, g is not None)
+            if gsd is not None:
+                out['gsrc_disps'] = gsd
+            vm, masks, counts = self._valid_mean(desc, tgt)
+            if vm is not None:
+                if peer is not None:
+                    raise ValueError('valid_mean is not supported with a peer (the counts are batch-global)')
+                out['valid_masks'], out['valid_counts'] = masks, counts
+        ig = None
+        want = set(image_grads) if self.image_grads else set()
+        if want:
+            if not want <= {'tgt', 'src'}:
+                raise ValueError("image_grads must be a subset of ('tgt', 'src')")
+            out['gtgt'] = D.empty(tgt, (desc.B, 3, desc.H, desc.W)) if 'tgt' in want else None
+            out['gsrc'] = D.empty(tgt, (desc.B, desc.S, 3, desc.H, desc.W)) if 'src' in want else None
+            ig = L.SfmImageGrads(_vp(out['gtgt']), _vp(out['gsrc']))
+        ref = lambda s: C.byref(s) if s is not None else None
+        head = (C.byref(desc), C.byref(inp))
+        ws, ph, st = self._workspace(desc, tgt), peer.handle if peer is not None else None, C.c_void_p(D.current_stream(tgt))
+        if dbg is not None:
+            rc = self._lib.sfm_loss_forward(*head, _vp(losses), C.byref(dbg), ws, st)
+        elif self.geometry_consistency:
+            rc = self._lib.sfm_loss_geometry_valid_mean(*head, ref(terms), C.byref(ge), ref(vm), _vp(losses), ref(g), ws, ph, st)
+        elif self.min_reprojection:
+            rc = self._lib.sfm_loss_min_reprojection(*head, ref(terms), C.byref(mr), _vp(losses), ref(g), ws, ph, st)
         else:
-            L.check(self._lib.sfm_loss_geometry_valid_mean(*args, C.byref(vm), *tail))
+            rc = self._lib.sfm_loss_weighted(*head, ref(terms), ref(pt), _vp(losses), ref(g), ref(ig), ws, ph, st)
+        L.check(rc)
 
     # ---- operators
     def forward(self, tgt, src, intrinsics, disps, poses, logits=None, proj=None, kinv=None, debug=False,
@@ -419,35 +443,6 @@ class ViewSynthesisLoss(object):
             raise ValueError('src_disps needs ViewSynthesisLoss(geometry_consistency=True)')
         desc, inp = self._pack(tgt, src, intrinsics, disps, poses, logits, proj, kinv)
         losses = D.empty(tgt, (5,))
-        if self.geometry_consistency:
-            terms, rows = self._snippet_terms(desc, tgt, snippet_weights)
-            if pixel_weights is not None:
-                raise ValueError('pixel_weights needs ViewSynthesisLoss(pixel_terms=True)')
-            ge, diff, _ = self._geometry(desc, tgt, src_disps, False)
-            vm, masks, counts = self._valid_mean(desc, tgt)
-            self._run_geometry(desc, inp, terms, ge, vm, losses, None, tgt, None)
-            return (losses,) + ((rows,) if self.snippet_terms else ()) + (diff,) + ((masks, counts) if vm else ())
-        if self.min_reprojection:
-            terms, rows = self._snippet_terms(desc, tgt, snippet_weights)
-            if pixel_weights is not None:
-                raise ValueError('pixel_weights needs ViewSynthesisLoss(pixel_terms=True)')
-            mr, sel = self._min_reprojection(desc, tgt)
-            L.check(self._lib.sfm_loss_min_reprojection(C.byref(desc), C.byref(inp), C.byref(terms) if terms else None,
-                                                        C.byref(mr), _vp(losses), None, self._workspace(desc, tgt), None,
-                                                        C.c_void_p(D.current_stream(tgt))))
-            return (losses,) + ((rows,) if self.snippet_terms else ()) + (sel,)
-        if self.snippet_terms or self.pixel_terms:
-            terms, rows = self._snippet_terms(desc, tgt, snippet_weights)
-            pt, maps = self._pixel_terms(desc, tgt, pixel_weights)
-            L.check(self._lib.sfm_loss_weighted(C.byref(desc), C.byref(inp), C.byref(terms) if terms else None,
-                                                C.byref(pt) if pt else None, _vp(losses), None, None,
-                                                self._workspace(desc, tgt), None, C.c_void_p(D.current_stream(tgt))))
-            out = (losses,) + ((rows,) if self.snippet_terms else ()) + ((maps,) if self.pixel_terms else ())
-            return out
-        if snippet_weights is not None:
-            raise ValueError('snippet_weights needs ViewSynthesisLoss(snippet_terms=True)')
-        if pixel_weights is not None:
-            raise ValueError('pixel_weights needs ViewSynthesisLoss(pixel_terms=True)')
         dbg_struct, dbg = None, None
         if debug:
             B, S, H, W = desc.B, desc.S, desc.H, desc.W
@@ -461,10 +456,13 @@ class ViewSynthesisLoss(object):
                 dbg['inb'].append(D.empty(tgt, (B, S, h, w), 'uint8'))
                 dbg_struct.P[s], dbg_struct.u0[s] = D.ptr(dbg['P'][s]), D.ptr(dbg['u0'][s])
                 dbg_struct.v0[s], dbg_struct.inb[s] = D.ptr(dbg['v0'][s]), D.ptr(dbg['inb'][s])
-        L.check(self._lib.sfm_loss_forward(C.byref(desc), C.byref(inp), _vp(losses),
-                                           C.byref(dbg_struct) if debug else None,
-                                           self._workspace(desc, tgt), C.c_void_p(D.current_stream(tgt))))
-        return (losses, dbg) if debug else losses
+        out = {}
+        self._loss(desc, inp, tgt, losses, None, out, snippet_weights, pixel_weights, src_disps, dbg=dbg_struct)
+        if debug:
+            return losses, dbg
+        res = (losses,) + tuple(out[k] for k in ('snippet_losses', 'pixel_losses', 'selection', 'geometry_diff', 'valid_masks',
+                                                 'valid_counts') if k in out)
+        return res if len(res) > 1 else losses
 
     def backward(self, tgt, src, intrinsics, disps, poses, logits=None, gy=None, proj=None, kinv=None,
                  intrinsics_grad=True):
@@ -525,47 +523,7 @@ class ViewSynthesisLoss(object):
             D.wait_event(tgt, self._ev_pyramid)     # build_pyramid may have run on another stream
         g, out = self._alloc_grads(desc, tgt)
         losses = D.empty(tgt, (5,))
-        terms, rows = self._snippet_terms(desc, tgt, snippet_weights)
-        if rows is not None:
-            out['snippet_losses'] = rows
-        pt, maps = self._pixel_terms(desc, tgt, pixel_weights)
-        if maps is not None:
-            out['pixel_losses'] = maps
-        if self.geometry_consistency:
-            ge, out['geometry_diff'], out['gsrc_disps'] = self._geometry(desc, tgt, src_disps, True)
-            vm, masks, counts = self._valid_mean(desc, tgt)
-            if vm is not None:
-                if peer is not None:
-                    raise ValueError('valid_mean is not supported with a peer (the counts are batch-global)')
-                out['valid_masks'], out['valid_counts'] = masks, counts
-            self._run_geometry(desc, inp, terms, ge, vm, losses, g, tgt, peer.handle if peer is not None else None)
-            self._intrinsics_grad(desc, inp, tgt, out, want_k)
-            if self._ev_pyramid is not None:
-                self._ev_loss = D.record_event(tgt)
-            return losses, out
-        if self.min_reprojection:
-            mr, out['selection'] = self._min_reprojection(desc, tgt)
-            L.check(self._lib.sfm_loss_min_reprojection(C.byref(desc), C.byref(inp), C.byref(terms) if terms else None,
-                                                        C.byref(mr), _vp(losses), C.byref(g), self._workspace(desc, tgt),
-                                                        peer.handle if peer is not None else None,
-                                                        C.c_void_p(D.current_stream(tgt))))
-            self._intrinsics_grad(desc, inp, tgt, out, want_k)
-            if self._ev_pyramid is not None:
-                self._ev_loss = D.record_event(tgt)
-            return losses, out
-        ig = None
-        want = set(image_grads) if self.image_grads else set()
-        if want:
-            if not want <= {'tgt', 'src'}:
-                raise ValueError("image_grads must be a subset of ('tgt', 'src')")
-            out['gtgt'] = D.empty(tgt, (desc.B, 3, desc.H, desc.W)) if 'tgt' in want else None
-            out['gsrc'] = D.empty(tgt, (desc.B, desc.S, 3, desc.H, desc.W)) if 'src' in want else None
-            ig = L.SfmImageGrads(_vp(out['gtgt']), _vp(out['gsrc']))
-        # one entry point for every combination of image gradients, peer sum, snippet and per-pixel terms
-        L.check(self._lib.sfm_loss_weighted(C.byref(desc), C.byref(inp), C.byref(terms) if terms else None,
-                                            C.byref(pt) if pt else None, _vp(losses), C.byref(g), C.byref(ig) if ig else None,
-                                            self._workspace(desc, tgt), peer.handle if peer is not None else None,
-                                            C.c_void_p(D.current_stream(tgt))))
+        self._loss(desc, inp, tgt, losses, g, out, snippet_weights, pixel_weights, src_disps, peer, image_grads)
         self._intrinsics_grad(desc, inp, tgt, out, want_k)
         if self._ev_pyramid is not None:
             self._ev_loss = D.record_event(tgt)

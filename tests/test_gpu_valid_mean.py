@@ -113,8 +113,11 @@ def test_clamped_pixels():
     _check(l, gg, L, G, 4, 'clamped')
 
 
-def test_without_struct_is_sfm_loss_geometry():
-    """vm == NULL: bitwise sfm_loss_geometry (the entry point with a descriptor carrying SFM_FLAG_VALID_MEAN)."""
+def test_vm_null_is_sfm_loss_geometry():
+    """vm == NULL: bitwise sfm_loss_geometry (the entry point with a descriptor carrying SFM_FLAG_VALID_MEAN), and both
+    bitwise the geometry operator without valid_mean."""
+    import ctypes as C
+    from sfm_learner_chainer_b200 import device as Dv, lib as Lb
     flags = FLAGSETS['cfg2']
     d, sd = _case(2, 2, 128, 416, 6301, True)
     g = dev_inputs(d)
@@ -122,26 +125,24 @@ def test_without_struct_is_sfm_loss_geometry():
     ref = make_op(flags, geometry_consistency=True, geometry_reg=REG, self_mask=True)
     lp, gp = _run(ref, g, flags, sdd)
     op = _op(flags, self_mask=True)
-    orig = op._valid_mean
-    op._valid_mean = lambda desc, tgt: (None, None, None)   # the operator then calls sfm_loss_geometry ...
-    calls = []
-    lib = op._lib
-    real = lib.sfm_loss_geometry_valid_mean
-
-    class Proxy:                                             # ... route it through the new entry point with vm = NULL
-        def __getattr__(self, k):
-            if k == 'sfm_loss_geometry':
-                return lambda desc, inp, terms, ge, *rest: calls.append(1) or real(desc, inp, terms, ge, None, *rest)
-            return getattr(lib, k)
-    op._lib = Proxy()
-    l, gg = _run(op, g, flags, sdd)
-    op._lib, op._valid_mean = lib, orig
-    assert calls
-    np.testing.assert_array_equal(host(l), host(lp))
-    for s in range(4):
-        np.testing.assert_array_equal(host(gg['gdisps'][s]), host(gp['gdisps'][s]))
-        np.testing.assert_array_equal(host(gg['geometry_diff'][s]), host(gp['geometry_diff'][s]))
-    np.testing.assert_allclose(host(gg['gposes']), host(gp['gposes']), rtol=1e-5, atol=1e-6 * np.abs(host(gp['gposes'])).max())
+    args = op_args(g, flags)
+    tgt = args[0]
+    desc, inp = op._pack(*args)
+    assert desc.flags & Lb.SFM_FLAG_VALID_MEAN
+    so, ws, st = op._lib, op._workspace(desc, tgt), C.c_void_p(Dv.current_stream(tgt))
+    for name in ('sfm_loss_geometry', 'sfm_loss_geometry_valid_mean'):
+        l = Dv.empty(tgt, (5,))
+        grads, gg = op._alloc_grads(desc, tgt)
+        ge, gg['geometry_diff'], _ = op._geometry(desc, tgt, sdd, True)
+        vm = () if name == 'sfm_loss_geometry' else (None,)
+        Lb.check(getattr(so, name)(C.byref(desc), C.byref(inp), None, C.byref(ge), *vm, C.c_void_p(Dv.ptr(l)),
+                                   C.byref(grads), ws, None, st))
+        np.testing.assert_array_equal(host(l), host(lp))
+        for s in range(4):
+            np.testing.assert_array_equal(host(gg['gdisps'][s]), host(gp['gdisps'][s]))
+            np.testing.assert_array_equal(host(gg['geometry_diff'][s]), host(gp['geometry_diff'][s]))
+        np.testing.assert_allclose(host(gg['gposes']), host(gp['gposes']), rtol=1e-5,
+                                   atol=1e-6 * np.abs(host(gp['gposes'])).max())
 
 
 def test_groups_equal_separate_calls():
